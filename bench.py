@@ -2,7 +2,7 @@
 PSD -> PSF -> Moffat fit).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 1|2|3|4|5]
-                    [--scaling strong|weak] [--draws D]
+                    [--scaling strong|weak] [--draws D] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[3] - the sweep of 4096 random (seeing, GL, L0,
 Cn2 profile) draws x 35 wavelengths (`--draws` changes the count).  One step = the whole path for
@@ -13,7 +13,9 @@ the fit records are gathered to rank 0 over NCCL inside the timed region; `--sca
 rank its own sweep instead (rank r: seed 12345 + r).  `--config` times another BASELINE config on one
 GPU (1, 2, 3: latency of one call; 5: dim 2560 x 100 wavelengths).
 
-One JSON line on rank 0; DESIGN.md section 6 says how each field is obtained.
+One JSON line on rank 0; DESIGN.md section 6 says how each field is obtained.  `--dump-outputs DIR`
+writes what the timed config-4 path returned in its last timed step as .npy files (see dump_outputs), so
+that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -25,6 +27,8 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # no __pycache__: the benchmark writes nothing into the tree it runs from,
+os.environ['PYTHONDONTWRITEBYTECODE'] = '1'     # nor do the joblib workers of the CPU arm
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 NLAM = int(os.environ.get('PSFR_BENCH_NLAM', '35'))   # 35 = BASELINE config; env override for tuning only
@@ -340,6 +344,30 @@ def own_bytes(ctx_info, nplanes, ndraw, nlam, dim):
     return hot, hot + stage_a + tail
 
 
+DUMP_FIT_BYTES = 24 << 20       # the two budgets keep a dump under 64 MB whatever --draws is
+DUMP_CUBE_BYTES = 36 << 20
+
+
+def dump_outputs(out_dir, cube, fit, first_draw):
+    """Write what one compute_batch call returned, as float64 .npy files in out_dir:
+        fit.npy              [n, wavelengths, FIT_NPAR] fit records (psfr.h PSFR_FIT_*)
+        fit_draws.npy        [n] sweep index of each draw in fit.npy
+        psf_cube.npy         [m, wavelengths, 40, 40] PSF cubes
+        psf_cube_draws.npy   [m] sweep index of each draw in psf_cube.npy
+    Every draw goes in where its records fit the budget; beyond that a fixed, seeded sample of draws
+    (in sweep order).  `first_draw` is the sweep index of the buffers' first draw (the rank's block)."""
+    import torch
+    nd = cube.shape[0]
+    order = np.random.default_rng(0).permutation(nd)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, buf, budget in (('fit', fit, DUMP_FIT_BYTES), ('psf_cube', cube, DUMP_CUBE_BYTES)):
+        per_draw = (buf[0].numel() + 1) * 8
+        pick = np.sort(order[:min(nd, budget // per_draw)])
+        rows = buf.index_select(0, torch.as_tensor(pick, device=buf.device))
+        np.save(os.path.join(out_dir, name + '.npy'), rows.cpu().numpy())
+        np.save(os.path.join(out_dir, name + '_draws.npy'), (first_draw + pick).astype(np.float64))
+
+
 def run_gpu(args):
     from muse_psfr_b200 import _lib, psfrec, sharding
     g = Gpu()
@@ -404,6 +432,8 @@ def run_gpu(args):
     ms_total = g.timed(step_device, args.steps, 0, after_step=collect_hot)
     launches = ctx.kernel_launches() - launches0
     gather_ms = float(np.mean([a.elapsed_time(b) for a, b in gather_ev[-args.steps:]])) if gather_ev else None
+    if args.dump_outputs and g.rank == 0:      # before the legs below reuse d_cube / d_fit
+        dump_outputs(args.dump_outputs, d_cube, d_fit, loc.start)
 
     # ---- the same leg with both precision grades off (everything FP64): 3 steps, same draws
     ms_fp64 = None
@@ -667,7 +697,14 @@ def main():
     ap.add_argument('--f32-rows', type=float, default=None, dest='f32_rows', help='PSFR_OPT_F32_ROWS override (tuning)')
     ap.add_argument('--row-kernel', type=int, default=None, dest='row_kernel', help='PSFR_OPT_ROW_KERNEL override (tuning)')
     ap.add_argument('--exp-cut', type=float, default=None, dest='exp_cut', help='PSFR_OPT_EXP_CUT override (tuning)')
+    ap.add_argument('--dump-outputs', default=None, dest='dump_outputs', metavar='DIR',
+                    help='write the fit records and PSF cubes of the last timed step to DIR/*.npy (config 4; on N GPUs '
+                         'rank 0\'s draws)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and (args.impl != 'b200' or args.config != 4):
+        ap.error('--dump-outputs dumps the config-4 sweep of the b200 implementation')
     own_stdout()
     if args.impl == 'reference':
         run_reference(args)

@@ -1,9 +1,8 @@
 """Load the reference's numeric core (``/root/reference/muse_psfr/psfrec.py``) in a
 container that lacks astropy / mpdaf / matplotlib (SURVEY F3).
 
-TEST INFRASTRUCTURE ONLY: used by ``oracle/make_goldens.py`` and by the CPU tests
-that pin the oracle to the real reference when ``/root/reference`` is present
-(it is absent on the GPU box; those tests skip there).
+TEST INFRASTRUCTURE ONLY: used by ``oracle/make_goldens.py`` to write the reference's
+outputs into ``tests/golden/ref_*.npz``, which the tests compare against.
 
 The third-party symbols the numeric core never touches are replaced by stubs that
 fail loudly if used, so only the reference's own numpy/scipy code runs:
@@ -11,15 +10,10 @@ fail loudly if used, so only the reference's own numpy/scipy code runs:
 ``psf_muse``, ``muse_intrinsic_psf``, ``fit_psf_with_polynom``.
 """
 import importlib.util
-import os
 import sys
 import types
 
 REFERENCE_FILE = '/root/reference/muse_psfr/psfrec.py'
-
-
-def reference_available():
-    return os.path.isfile(REFERENCE_FILE)
 
 
 class _Missing:
