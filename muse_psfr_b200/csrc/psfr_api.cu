@@ -111,10 +111,14 @@ static int set_lambda_tables(Ctx* c, int nlam, const double* lam_host, cudaStrea
         const double conv = 2 * 3.141592653589793 / lb;        // convnm, psfrec.py:717 (lbda*1e9 = nm)
         cl[l] = 0.5 * (conv * conv);
         const long npix = (long)(std::nearbyint(((kPSF * 0.2 * 2 * 8 * 4.85 * 1000) / lb) / 2) * 2);
-        if (npix > kN || npix < 2 * kPSF)
+        if (npix > kN)
             return set_error(c, PSFR_E_UNSUPPORTED,
                              "wavelength %g nm needs a %ld-pixel crop but dim is %d (reference: psf_muse fails)",
                              lb, npix, kN);
+        if (npix < kNS)   // two distinct samples per output pixel and axis: crops of at least 80 pixels
+            return set_error(c, PSFR_E_UNSUPPORTED,
+                             "wavelength %g nm needs a %ld-pixel crop, fewer than the %d samples per axis this "
+                             "library resamples from", lb, npix, kNS);
         const long origin = kN / 2 - npix / 2;
         for (int y = 0; y < kPSF; ++y) {
             const double pos = (double)(y * npix) / kPSF;
