@@ -166,6 +166,18 @@ PSFR_API int psfr_compute_groups(psfr_ctx* ctx, int ndraw, const double* draws, 
                         int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                         double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream);
 
+/* psfr_compute_groups without the field average: the PSF of every draw at every one of the ndir
+ * positions of dirs [2][ndir] (arcsec, ndir <= 256 and <= max_planes).  The PSF at position k of draw d
+ * is the reference's psf_muse of that direction's PSD alone, convolved with draw d's kernels and fitted:
+ * bit for bit what psfr_compute_batch / psfr_compute_groups give for draw d with dirs = position k only.
+ * Arguments and checks as psfr_compute_groups; the outputs gain a position axis:
+ * out_cube [ndraw][ndir][nlam][40][40], out_fit [ndraw][ndir][nlam][PSFR_FIT_NPAR],
+ * out_mean [ngroup][ndir][nlam][40][40] and out_mean_fit [ngroup][ndir][nlam][PSFR_FIT_NPAR], where
+ * out_mean[g][k] and its fit are psfr_mean_refit of exposure g's cubes at position k, bit for bit. */
+PSFR_API int psfr_compute_field(psfr_ctx* ctx, int ndraw, const double* draws, int npos, const double* poslgs,
+                       int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                       double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream);
+
 /* Time-mean of ncube cubes + refit (psfrec.py:1104-1105). cubes [ncube][nlam][40][40]. */
 PSFR_API int psfr_mean_refit(psfr_ctx* ctx, int ncube, int nlam, const double* cubes,
                     double* out_mean, double* out_fit, void* stream);

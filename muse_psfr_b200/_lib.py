@@ -67,6 +67,7 @@ _SIGNATURES = {
     'psfr_moffat_fit': (_I, [_P, _I, _I, _I, _P, _P, _P]),
     'psfr_compute_batch': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P]),
     'psfr_compute_groups': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
+    'psfr_compute_field': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     'psfr_mean_refit': (_I, [_P, _I, _I, _P, _P, _P, _P]),
     'psfr_polyfit': (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     'psfr_set_option': (_I, [_P, _I, _D]),
@@ -293,6 +294,19 @@ class Context:
         DRAW_NGS (first stars of ``poslgs`` [2, npos]), exposures closed at the draw indices of
         ``group_end`` (int32); per-draw outputs as ``compute_batch``, per-exposure ``out_mean``
         [ngroup, nl, 40, 40] and ``out_mean_fit`` [ngroup, nl, FIT_NPAR]."""
+        self._groups(self._lib.psfr_compute_groups, False, draws, dirs, poslgs, lambda_nm, group_end, out_cube,
+                     out_fit, out_mean, out_mean_fit, stream)
+
+    def compute_field(self, draws, dirs, poslgs, lambda_nm, group_end=None, out_cube=None, out_fit=None,
+                      out_mean=None, out_mean_fit=None, stream=None):
+        """psfr_compute_field: ``compute_groups`` with one PSF per field position of ``dirs`` [2, npos]
+        instead of their average.  Outputs ``out_cube`` [ndraw, npos, nl, 40, 40], ``out_fit`` [ndraw, npos,
+        nl, FIT_NPAR], ``out_mean`` [ngroup, npos, nl, 40, 40], ``out_mean_fit`` [ngroup, npos, nl, FIT_NPAR]."""
+        self._groups(self._lib.psfr_compute_field, True, draws, dirs, poslgs, lambda_nm, group_end, out_cube,
+                     out_fit, out_mean, out_mean_fit, stream)
+
+    def _groups(self, fn, field, draws, dirs, poslgs, lambda_nm, group_end, out_cube, out_fit, out_mean,
+                out_mean_fit, stream):
         if not hasattr(draws, 'data_ptr'):
             draws = f64(draws)
         if len(draws.shape) != 2 or draws.shape[1] != DRAW_NPAR:
@@ -300,14 +314,15 @@ class Context:
         dirs, poslgs, lam = f64(dirs), f64(poslgs), f64(lambda_nm)
         nd = int(draws.shape[0])
         ng, gp = group_end_ptr(group_end)
-        img = lam.size * PSF_DIM * PSF_DIM
-        self._check(self._lib.psfr_compute_groups(
+        nimg = lam.size * (dirs.shape[1] if field else 1)      # images per draw and per exposure
+        img = nimg * PSF_DIM * PSF_DIM
+        self._check(fn(
             self._handle(), nd, self._buf(draws, nd * DRAW_NPAR, 'draws'), poslgs.shape[1], ptr(poslgs),
             dirs.shape[1], ptr(dirs), lam.size, ptr(lam), ng, gp,
             self._buf(out_cube, nd * img, 'out_cube', True),
-            self._buf(out_fit, nd * lam.size * FIT_NPAR, 'out_fit', True),
+            self._buf(out_fit, nd * nimg * FIT_NPAR, 'out_fit', True),
             self._buf(out_mean, ng * img, 'out_mean', True),
-            self._buf(out_mean_fit, ng * lam.size * FIT_NPAR, 'out_mean_fit', True), stream))
+            self._buf(out_mean_fit, ng * nimg * FIT_NPAR, 'out_mean_fit', True), stream))
 
     def mean_refit(self, ncube, nlam, cubes, out_mean=None, out_fit=None, stream=None):
         ncube, nlam = int(ncube), int(nlam)

@@ -279,14 +279,17 @@ static int hot_begin(Ctx* c) {
     return 0;
 }
 
-// The fused pipeline of psfr_compute_batch and psfr_compute_groups, chunk by chunk of max_planes / ndir
-// draws: PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit, and with ngroup > 0
-// the time mean of every exposure (draws [group_end[g-1], group_end[g])) and its fit in the chunk where the
-// exposure's last draw lies.  Host outputs leave through a second stream: the results of chunk i are
-// copied out while chunk i + 1 computes, from staging buffers that alternate between two sets.
+// The fused pipeline of psfr_compute_batch, psfr_compute_groups and psfr_compute_field, chunk by chunk of
+// max_planes / ndir draws: PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit, and
+// with ngroup > 0 the time mean of every exposure (draws [group_end[g-1], group_end[g])) and its fit in the
+// chunk where the exposure's last draw lies.  field: every (draw, direction) plane keeps its own PSF instead
+// of the draw's field mean, so a draw owns ndir x nlam images in every output.  Host outputs leave through
+// a second stream: the results of chunk i are copied out while chunk i + 1 computes, from staging buffers
+// that alternate between two sets.
 static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs, int npos,
                      const double* poslgs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
-                     double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, cudaStream_t s) {
+                     bool field, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
+                     cudaStream_t s) {
     PSFR_CUDA(c, cudaSetDevice(c->device));
     std::vector<double> lam;
     int rc = small_to_host(c, lam, lambda_nm, nlam > 0 ? nlam : 0, s);
@@ -300,7 +303,11 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     hot_begin(c);
     c->hot_timed = true;
     const int per_chunk = c->max_planes / ndir;
-    const size_t img = (size_t)kPSF * kPSF, elems = (size_t)nlam * img;
+    // output planes per draw; a chunk's nd * ppd * nlam images fit every [max_planes * max_lambda]-image
+    // buffer (d_samp, d_cube*, d_fit*, d_mean[b], d_mfit[b], d_carry) because nd * ndir <= max_planes
+    const int ppd = field ? ndir : 1;
+    const size_t img = (size_t)kPSF * kPSF, imgs = (size_t)ppd * nlam, elems = imgs * img;
+    const size_t fits = imgs * PSFR_FIT_NPAR;   // fit records per draw
     const bool cube_dev = out_cube && is_device_ptr(out_cube);
     const bool fit_dev = out_fit && is_device_ptr(out_fit);
     const bool mean_dev = out_mean && is_device_ptr(out_mean);
@@ -319,21 +326,22 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
         if (rc) break;
         if ((rc = run_psd(c, nd, ndir, ngs, npos, s, false))) break;
         if ((rc = run_structure_function(c, nd * ndir, s, true, ndir))) break;
-        if ((rc = run_pruned_psf(c, nd, ndir, nlam, s))) break;
-        if ((rc = run_resample(c, nd * nlam, nlam, c->d_cube, s))) break;
+        // field mode: one column pass per plane (scale 1, no sum over directions), as ndir = 1 calls would run it
+        if ((rc = field ? run_pruned_psf(c, nd * ndir, 1, nlam, s) : run_pruned_psf(c, nd, ndir, nlam, s))) break;
+        if ((rc = run_resample(c, nd * ppd * nlam, nlam, c->d_cube, s))) break;
         if ((rc = run_build_kernels(c, nd, nlam, lam.data(), true, false, s))) break;
         if (host_out && chunk >= 2 && cudaStreamWaitEvent(s, c->ev_copied[b], 0) != cudaSuccess) {
             rc = set_error(c, PSFR_E_CUDA, "stream wait failed: %s", cudaGetErrorString(cudaGetLastError()));
             break;
         }
         double* conv = cube_dev ? out_cube + (size_t)d0 * elems : (b ? c->d_cube3 : c->d_cube2);
-        if ((rc = run_convolve(c, nd, nlam, c->d_cube, conv, s))) break;
-        double* fit = fit_dev ? out_fit + (size_t)d0 * nlam * PSFR_FIT_NPAR : (b ? c->d_fit2 : c->d_fit);
-        if (out_fit && (rc = run_fit(c, nd * nlam, kPSF, kPSF, conv, fit, s))) break;
+        if ((rc = run_convolve(c, nd, ppd, nlam, c->d_cube, conv, s))) break;
+        double* fit = fit_dev ? out_fit + (size_t)d0 * fits : (b ? c->d_fit2 : c->d_fit);
+        if (out_fit && (rc = run_fit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, s))) break;
         // exposures g0, g0 + 1, ... that have draws in [d0, d0 + nd): all but possibly the last end here
         int ndone = 0;
         double* mean = mean_dev ? out_mean + (size_t)g0 * elems : c->d_mean[b];
-        double* mfit = mfit_dev ? out_mean_fit + (size_t)g0 * nlam * PSFR_FIT_NPAR : c->d_mfit[b];
+        double* mfit = mfit_dev ? out_mean_fit + (size_t)g0 * fits : c->d_mfit[b];
         if (means) {
             seg.clear();
             for (int g = g0; g < ngroup && (g == g0 || group_end[g - 1] < d0 + nd); ++g) {
@@ -348,7 +356,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                 break;
             }
             if ((rc = run_group_mean(c, (int)elems, conv, seg_dev, (int)seg.size() / 2, carry_in, mean, s))) break;
-            if (out_mean_fit && ndone && (rc = run_fit(c, ndone * nlam, kPSF, kPSF, mean, mfit, s))) break;
+            if (out_mean_fit && ndone && (rc = run_fit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, s))) break;
         }
         if (host_out) {
             cudaError_t e = cudaEventRecord(c->ev_done[b], s);
@@ -357,15 +365,14 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                 e = cudaMemcpyAsync(out_cube + (size_t)d0 * elems, conv, (size_t)nd * elems * sizeof(double),
                                     cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess && out_fit && !fit_dev)
-                e = cudaMemcpyAsync(out_fit + (size_t)d0 * nlam * PSFR_FIT_NPAR, fit,
-                                    (size_t)nd * nlam * PSFR_FIT_NPAR * sizeof(double), cudaMemcpyDefault, c->copy_stream);
+                e = cudaMemcpyAsync(out_fit + (size_t)d0 * fits, fit, (size_t)nd * fits * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess && ndone && out_mean && !mean_dev)
                 e = cudaMemcpyAsync(out_mean + (size_t)g0 * elems, mean, (size_t)ndone * elems * sizeof(double),
                                     cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess && ndone && out_mean_fit && !mfit_dev)
-                e = cudaMemcpyAsync(out_mean_fit + (size_t)g0 * nlam * PSFR_FIT_NPAR, mfit,
-                                    (size_t)ndone * nlam * PSFR_FIT_NPAR * sizeof(double), cudaMemcpyDefault,
-                                    c->copy_stream);
+                e = cudaMemcpyAsync(out_mean_fit + (size_t)g0 * fits, mfit, (size_t)ndone * fits * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess) e = cudaEventRecord(c->ev_copied[b], c->copy_stream);
             if (e != cudaSuccess) {
                 rc = set_error(c, PSFR_E_CUDA, "result copy failed: %s", cudaGetErrorString(e));
@@ -386,7 +393,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 101; }
+int psfr_version(void) { return 102; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -516,7 +523,7 @@ int psfr_create(int device, int dim, int max_planes, int max_lambda, psfr_ctx** 
     CK(dev_alloc(c, &c->d_fit, P * LM * PSFR_FIT_NPAR));
     CK(dev_alloc(c, &c->d_cube3, P * LM * kPSF * kPSF));
     CK(dev_alloc(c, &c->d_fit2, P * LM * PSFR_FIT_NPAR));
-    CK(dev_alloc(c, &c->d_carry, LM * kPSF * kPSF));
+    CK(dev_alloc(c, &c->d_carry, P * LM * kPSF * kPSF));
     for (int i = 0; i < 2; ++i) {
         CK(dev_alloc(c, &c->d_mean[i], P * LM * kPSF * kPSF));
         CK(dev_alloc(c, &c->d_mfit[i], P * LM * PSFR_FIT_NPAR));
@@ -682,7 +689,7 @@ int psfr_convolve(psfr_ctx* c, int ndraw, int nlam, const double* lambda_nm, con
         src = c->d_cube;
     }
     double* dst = is_device_ptr(out_cube) ? out_cube : c->d_cube2;
-    rc = run_convolve(c, ndraw, nlam, src, dst, s);
+    rc = run_convolve(c, ndraw, 1, nlam, src, dst, s);
     if (rc) return rc;
     if (dst != out_cube) return from_device(c, out_cube, dst, bytes, s);
     return PSFR_OK;
@@ -725,13 +732,14 @@ int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, co
     if (ndraw < 1 || ndir < 1 || ndir > c->max_planes)
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d ndir=%d max_planes=%d", ndraw, ndir, c->max_planes);
     if (ngs < 1) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
-    return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, out_cube, out_fit,
-                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
+    return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, false, out_cube,
+                     out_fit, nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
-int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
-                        const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
-                        double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
+// the arguments of psfr_compute_groups and psfr_compute_field that run_batch does not check itself
+static int check_groups(Ctx* c, int ndraw, const double* draws, const double* poslgs, int ndir, const double* dirs,
+                        const double* lambda_nm, int ngroup, const int* group_end, const double* out_mean,
+                        const double* out_mean_fit) {
     if (!c || !draws || !dirs || !poslgs || !lambda_nm || (ngroup > 0 && !group_end))
         return set_error(c, PSFR_E_ARG, "NULL argument");
     if (ndraw < 1 || ndir < 1 || ndir > c->max_planes)
@@ -744,8 +752,25 @@ int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, c
             return set_error(c, PSFR_E_ARG, "group_end[%d]=%d does not close a non-empty exposure", g, group_end[g]);
     if (ngroup > 0 && group_end[ngroup - 1] != ndraw)
         return set_error(c, PSFR_E_ARG, "group_end ends at %d, not at ndraw=%d", group_end[ngroup - 1], ndraw);
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, out_cube,
-                     out_fit, out_mean, out_mean_fit, static_cast<cudaStream_t>(stream));
+    return PSFR_OK;
+}
+
+int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
+                        const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                        double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean, out_mean_fit))
+        return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, false,
+                     out_cube, out_fit, out_mean, out_mean_fit, static_cast<cudaStream_t>(stream));
+}
+
+int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
+                       const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                       double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean, out_mean_fit))
+        return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
+                     out_cube, out_fit, out_mean, out_mean_fit, static_cast<cudaStream_t>(stream));
 }
 
 int psfr_mean_refit(psfr_ctx* c, int ncube, int nlam, const double* cubes, double* out_mean, double* out_fit,

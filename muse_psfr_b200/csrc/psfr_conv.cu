@@ -309,10 +309,11 @@ kernel_spectrum_kernel(const double* __restrict__ kern, double2* __restrict__ kh
 
 __global__ void __launch_bounds__(kConvThreads, 3)
 fft_convolve_kernel(const double* __restrict__ in, const double2* __restrict__ khat_tt,
-                    const double2* __restrict__ khat_mu, int nlam, double* __restrict__ out) {
+                    const double2* __restrict__ khat_mu, int nlam, int per_draw, double* __restrict__ out) {
     extern __shared__ __align__(16) unsigned char conv_smem_raw[];
     ConvSmem& S = *reinterpret_cast<ConvSmem*>(conv_smem_raw);
-    const int img = blockIdx.x, draw = img / nlam, lam = img % nlam;
+    // a draw owns per_draw consecutive images (its field positions x wavelengths) and one tip-tilt spectrum
+    const int img = blockIdx.x, draw = img / per_draw, lam = img % nlam;
     constexpr int kImg = kPSF * kPSF;
     load_twiddles(S);
     for (int i = threadIdx.x; i < kImg; i += kConvThreads) S.img[(i / kPSF) * kIST + i % kPSF] = in[(size_t)img * kImg + i];
@@ -338,10 +339,10 @@ int run_kernel_spectra(Ctx* c, int nk, const double* kern_dev, double2* khat_dev
     return PSFR_OK;
 }
 
-int run_fft_convolve(Ctx* c, int ndraw, int nlam, const double* in_dev, double* out_dev, cudaStream_t s) {
+int run_fft_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev, double* out_dev, cudaStream_t s) {
     if (int rc = ensure_dynamic_smem(c, fft_convolve_kernel, sizeof(ConvSmem))) return rc;
-    fft_convolve_kernel<<<ndraw * nlam, kConvThreads, sizeof(ConvSmem), s>>>(in_dev, c->d_khat_tt, c->d_khat_mu, nlam,
-                                                                              out_dev);
+    fft_convolve_kernel<<<ndraw * ndir * nlam, kConvThreads, sizeof(ConvSmem), s>>>(in_dev, c->d_khat_tt, c->d_khat_mu,
+                                                                                     nlam, ndir * nlam, out_dev);
     PSFR_LAUNCH_CHECK(c);
     return PSFR_OK;
 }

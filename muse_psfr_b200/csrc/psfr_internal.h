@@ -139,7 +139,8 @@ struct Ctx {
     double* d_cube3 = nullptr;   // third staging buffer (double-buffered device -> host copies)
     double* d_fit = nullptr;     // [max_planes*max_lambda][PSFR_FIT_NPAR]
     double* d_fit2 = nullptr;    // second fit buffer (double-buffered device -> host copies)
-    double* d_carry = nullptr;   // [max_lambda][40][40] unnormalised sum of the exposure open at a chunk edge
+    double* d_carry = nullptr;   // [max_planes*max_lambda][40][40] unnormalised sum of the exposure open at a chunk
+                                 // edge: [ndir][nlam][40][40] in psfr_compute_field, and ndir <= max_planes
     double* d_mean[2] = {nullptr, nullptr};  // [max_planes*max_lambda][40][40] exposure means finished in a chunk
     double* d_mfit[2] = {nullptr, nullptr};  // [max_planes*max_lambda][PSFR_FIT_NPAR] their fits
     cudaStream_t copy_stream = nullptr;      // device -> host copies of finished chunks
@@ -242,9 +243,10 @@ int run_build_kernels(Ctx* c, int ndraw, int nlam, const double* lambda_nm_host,
 int run_resample(Ctx* c, int nimg, int nlam, double* cube_dev, cudaStream_t s);
 // psfr_conv.cu: spectra of nk 41x41 kernels, and the two FFT convolutions of every image
 int run_kernel_spectra(Ctx* c, int nk, const double* kern_dev, double2* khat_dev, cudaStream_t s);
-int run_fft_convolve(Ctx* c, int ndraw, int nlam, const double* in_dev, double* out_dev, cudaStream_t s);
-// two Moffat convolutions; img index = draw*nlam + lam
-int run_convolve(Ctx* c, int ndraw, int nlam, const double* in_dev, double* out_dev, cudaStream_t s);
+int run_fft_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev, double* out_dev, cudaStream_t s);
+// two Moffat convolutions; img index = (draw*ndir + k)*nlam + lam, one tip-tilt kernel per draw (ndir = 1
+// unless every field position of a draw keeps its own image, psfr_compute_field)
+int run_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev, double* out_dev, cudaStream_t s);
 int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit_dev, cudaStream_t s);
 // out = (running sum of the cubes) ; first: start from zero, last: divide by ntotal
 int run_mean(Ctx* c, int ncube, int plane_elems, const double* cubes_dev, double* out_dev,

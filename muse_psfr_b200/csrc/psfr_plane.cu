@@ -585,8 +585,8 @@ int run_resample(Ctx* c, int nimg, int nlam, double* cube_dev, cudaStream_t s) {
     return PSFR_OK;
 }
 
-int run_convolve(Ctx* c, int ndraw, int nlam, const double* in_dev, double* out_dev, cudaStream_t s) {
-    return run_fft_convolve(c, ndraw, nlam, in_dev, out_dev, s);
+int run_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev, double* out_dev, cudaStream_t s) {
+    return run_fft_convolve(c, ndraw, ndir, nlam, in_dev, out_dev, s);
 }
 
 int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit_dev, cudaStream_t s) {

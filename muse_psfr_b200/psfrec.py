@@ -17,7 +17,7 @@ from ._lib import PsfrError
 
 __all__ = ['compute_psf_from_sparta', 'compute_psf_from_sparta_batch', 'compute_psf', 'compute_psf_batch',
            'reconstruct_psf', 'create_sparta_table', 'fit_psf_with_polynom', 'simul_psd_wfm', 'psd_to_psf', 'psf_muse',
-           'convolve_final_psf', 'fit_psf_cube',
+           'convolve_final_psf', 'fit_psf_cube', 'compute_psf_field',
            'muse_intrinsic_psf', 'direction_perf', 'seeing2r01', 'pupil_mask', 'select_sparta_rows', 'FitTable',
            'PsfrError', 'MIN_L0', 'MAX_L0']
 
@@ -30,6 +30,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _WIND_DIR = np.array([0.628163, -0.326497])      # psfrec.py:66
 _DIM = 1280                                      # psfrec.py:955 (compute_psf's fixed grid)
 _DIMS = (1280, 2560)                             # grids the CUDA library is built for
+_MAX_POSITIONS = 256                             # directions per draw the library takes (kMaxDir)
 _CONTEXTS = {}
 _DEFAULT_DEVICE = [None]
 
@@ -453,6 +454,29 @@ def _mode_records(three, seeing, GL, L0, h=(100, 10000), zenith=0., Cn2=None, wi
     return recs
 
 
+def _mode_flags(three_lgs_mode, nd):
+    """One three-lasers flag per draw from one flag or a sequence of nd flags."""
+    three = np.asarray(three_lgs_mode, dtype=bool)
+    if three.ndim == 0:
+        return np.full(nd, bool(three))
+    if three.shape != (nd,):
+        raise ValueError('three_lgs_mode must be one flag or one flag per draw (got shape %s for %d draws)'
+                         % (three.shape, nd))
+    return three
+
+
+def _field_positions(positions):
+    """Field positions [2, npos] in arcsec (x row, then y row) as a C-contiguous float64 array, checked."""
+    pos = np.array(positions, dtype=float, ndmin=2)
+    if pos.ndim != 2 or pos.shape[0] != 2:
+        raise ValueError('positions must be [2, npos] (x row, then y row, arcsec); got shape %s' % (pos.shape,))
+    if not 1 <= pos.shape[1] <= _MAX_POSITIONS:
+        raise ValueError('positions must hold 1 to %d field positions (got %d)' % (_MAX_POSITIONS, pos.shape[1]))
+    if not np.all(np.isfinite(pos)):
+        raise ValueError('positions must be finite')
+    return np.ascontiguousarray(pos)
+
+
 def _planes_context(nd, ndir, nlam, max_planes, device, dim):
     if max_planes is None:
         max_planes = 128 if dim == _DIM else 16      # planes per chunk of the fused pipeline (~8 GB of workspace)
@@ -476,10 +500,7 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         raise ValueError('seeing, GL and L0 must have one entry per draw (got %d, %d, %d)' % (nd, GL.size, L0.size))
     per_draw = np.ndim(three_lgs_mode) > 0
     if per_draw:
-        three = np.asarray(three_lgs_mode, dtype=bool)
-        if three.shape != (nd,):
-            raise ValueError('three_lgs_mode must be one flag or one flag per draw (got shape %s for %d draws)'
-                             % (three.shape, nd))
+        three = _mode_flags(three_lgs_mode, nd)
     if nd == 0 or lam.size == 0:
         # nothing to compute: empty results of the right shape, written through nothing
         return (np.empty((nd, lam.size, _lib.FIT_NPAR)),
@@ -502,6 +523,49 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         else:
             ctx.compute_batch(recs, dirs, _lgs_positions(three_lgs_mode), lam, out_cube=out_cube,
                               out_fit=out_fit, stream=stream)
+    except PsfrError as exc:
+        if exc.code == _lib.E_UNSUPPORTED:
+            raise ValueError(str(exc))
+        raise
+    return out_fit, out_cube
+
+
+def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_size=60, h=(100, 10000),
+                      three_lgs_mode=False, out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None,
+                      stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None):
+    """Field-resolved ``compute_psf_batch``: the PSF of every draw at every field position instead of
+    their average.
+
+    ``positions`` is [2, npos] in arcsec (x row, then y row, the convention of ``direction_perf``), at most
+    256 positions; the default is ``direction_perf(npsflin, field_size)``.  The PSF at position k of a draw
+    is the reference's ``psf_muse`` of that direction's PSD alone, then ``convolve_final_psf`` and the
+    Moffat fit: bit for bit what ``compute_psf_batch`` gives for that draw with the single direction k
+    (so ``positions=[[0], [0]]`` reproduces ``compute_psf_batch(npsflin=1)``).  It is not the field mean
+    ``compute_psf_batch(npsflin=n)`` returns, and the field mean is not the average of these PSFs (each
+    is normalised on its own).  Other arguments as ``compute_psf_batch``.  Returns (fit [ndraw, npos, nl,
+    FIT_NPAR], cube [ndraw, npos, nl, 40, 40])."""
+    pos = _field_positions(direction_perf(npsflin, field_size) if positions is None else positions)
+    npos = pos.shape[1]
+    lam = np.atleast_1d(np.asarray(lbda, dtype=float))
+    seeing, GL, L0 = (np.atleast_1d(np.asarray(v, dtype=float)) for v in (seeing, GL, L0))
+    nd = seeing.size
+    if GL.size != nd or L0.size != nd:
+        raise ValueError('seeing, GL and L0 must have one entry per draw (got %d, %d, %d)' % (nd, GL.size, L0.size))
+    three = _mode_flags(three_lgs_mode, nd)
+    if nd == 0 or lam.size == 0:
+        return (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
+                np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
+    # the records compute_psf_batch builds in either laser mode; the three-laser asterism is the first three
+    # stars of the four-laser one
+    recs = _mode_records(three, seeing, GL, L0, h, zenith, Cn2, wind_dir)
+    dim = _check_dim(dim)
+    ctx = _planes_context(nd, npos, lam.size, max_planes, device, dim)
+    if out_fit is None:
+        out_fit = np.empty((nd, npos, lam.size, _lib.FIT_NPAR))
+    if out_cube is None and want_cube:
+        out_cube = np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
+    try:
+        ctx.compute_field(recs, pos, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit, stream=stream)
     except PsfrError as exc:
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
@@ -576,7 +640,7 @@ def _fit_columns(lam, fit):
 
 def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                             lbda=None, h=(100, 10000), n_jobs=-1, plot=False, mean_of_lgs=True,
-                            verbose=True, device=None):
+                            verbose=True, device=None, field_positions=None):
     """Reconstruct a PSF from SPARTA data (psfrec.py:981-1120).
 
     ``filename``: path of a FITS file, a binary file object, or an HDUList (this package's or
@@ -584,17 +648,19 @@ def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin
     batched GPU call (the reference fans them out over joblib processes, psfrec.py:1082-1083;
     ``n_jobs`` is accepted and only reported).  Returns an HDUList [PRIMARY, <extname>, FIT_ROWS,
     FIT_MEAN, PSF_MEAN] - an ``astropy.io.fits.HDUList`` when astropy is installed, otherwise
-    the equivalent object of ``muse_psfr_b200._fits`` - or None when no row is valid."""
+    the equivalent object of ``muse_psfr_b200._fits`` - or None when no row is valid.  With
+    ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow: see
+    ``compute_psf_from_sparta_batch``."""
     if plot:
         raise NotImplementedError('plotting is outside the B200 hot path')
     return compute_psf_from_sparta_batch([filename], extname=extname, npsflin=npsflin, lmin=lmin, lmax=lmax, nl=nl,
                                          lbda=lbda, h=h, n_jobs=n_jobs, mean_of_lgs=mean_of_lgs, verbose=verbose,
-                                         device=device)[0]
+                                         device=device, field_positions=field_positions)[0]
 
 
 def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                                   lbda=None, h=(100, 10000), n_jobs=-1, mean_of_lgs=True, verbose=True,
-                                  device=None, max_planes=None):
+                                  device=None, max_planes=None, field_positions=None):
     """``compute_psf_from_sparta`` for many exposures in one device pass: returns one entry per source,
     the HDUList ``compute_psf_from_sparta(source, ...)`` returns, bit for bit, or None for a table
     without a valid row.
@@ -603,10 +669,17 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     exposure's time-mean PSF and its refit are formed on the device while its draws are resident, and
     only the fit records and the means come back to the host.  Each table logs the messages of a
     single-table call, in the same order.  ``max_planes`` caps the (draw x direction) planes per
-    chunk of the pipeline, as in ``compute_psf_batch``."""
+    chunk of the pipeline, as in ``compute_psf_batch``.
+
+    ``field_positions`` [2, npos] (arcsec, x row then y row, as ``direction_perf``) adds the exposure's
+    time-mean PSF at each of those positions, from one more device pass over the same draws
+    (``compute_psf_field``): FIT_FIELD, the columns of FIT_MEAN plus ``x`` and ``y`` [arcsec], one row per
+    (position, wavelength), position-major, with the cards of FIT_MEAN; and PSF_FIELD, an image [npos,
+    nl, 40, 40].  The first five HDUs are those of a call without ``field_positions``, bit for bit."""
     if lbda is None:
         lbda = np.linspace(lmin, lmax, nl)
     lbda = np.atleast_1d(np.asarray(lbda, dtype=float))
+    pos = None if field_positions is None else _field_positions(field_positions)
     files, recs = [], []
     for source in sources:
         hdul = _fits.from_any(source, only={extname.upper()})
@@ -644,6 +717,13 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     try:
         ctx.compute_groups(draws, dirs, _lgs_positions(False), lbda, group_end, out_fit=fit, out_mean=psftot,
                            out_mean_fit=fit_mean)
+        if pos is not None:
+            npos = pos.shape[1]
+            psf_field = np.empty((ng, npos, nlam, _lib.PSF_DIM, _lib.PSF_DIM))
+            fit_field = np.empty((ng, npos, nlam, _lib.FIT_NPAR))
+            ctx = _planes_context(nd, npos, nlam, max_planes, device, _DIM)
+            ctx.compute_field(draws, pos, _lgs_positions(False), lbda, group_end, out_mean=psf_field,
+                              out_mean_fit=fit_field)
     except PsfrError as exc:
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
@@ -671,6 +751,12 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
         meta = {'SEEING': float(med[0]), 'GL': float(med[1]), 'L0': float(med[2])}
         out.append(_fits.table_to_hdu(_fit_columns(lbda, fit_mean[g][None]), meta=meta, name='FIT_MEAN'))
         out.append(_fits.ImageHDU(data=psftot[g], name='PSF_MEAN'))
+        if pos is not None:
+            cols = _fit_columns(lbda, fit_field[g])
+            cols['x'] = np.repeat(pos[0], nlam)
+            cols['y'] = np.repeat(pos[1], nlam)
+            out.append(_fits.table_to_hdu(cols, meta=meta, name='FIT_FIELD'))
+            out.append(_fits.ImageHDU(data=psf_field[g], name='PSF_FIELD'))
         try:
             results.append(_fits.to_astropy(out))
         except ImportError:
