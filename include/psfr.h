@@ -89,6 +89,32 @@ enum {
     PSFR_FIT_NPAR = 16
 };
 
+/* Per-image record of the elliptical Moffat fit, f = I (1 + A dp^2 + B dq^2 + C dp dq)^(-n) with dp = p - y0
+ * (row) and dq = q - x0 (column), fitted over theta = (I, y0, x0, A, B, C, n) from the image's circular record.
+ * The reference has no elliptical fit (it calls mpdaf's moffat_fit with circular=True): these columns are
+ * this library's own and their parity with mpdaf's elliptical fit is unpinned.  Widths and FWHM in pixels.
+ * Every err_* entry is sqrt(grad g^T Sigma grad g) of its quantity g, Sigma = (J^T J)^-1 chi^2/dof over theta,
+ * dof = npx - 7 (the delta method; not mpdaf's err_fwhm = err_a * n). */
+enum {
+    PSFR_EFIT_PEAK = 0, PSFR_EFIT_Y0 = 1, PSFR_EFIT_X0 = 2,   /* as the circular record */
+    PSFR_EFIT_A_MAJOR = 3,   /* 1/sqrt(lambda_min) of [[A, C/2], [C/2, B]] */
+    PSFR_EFIT_A_MINOR = 4,   /* 1/sqrt(lambda_max) */
+    PSFR_EFIT_PA = 5,        /* major axis [deg] in [0, 180), from +x (column) toward +y (row); 0 at a circle */
+    PSFR_EFIT_N = 6,         /* beta */
+    PSFR_EFIT_FWHM_MAJOR = 7, PSFR_EFIT_FWHM_MINOR = 8,   /* a 2 sqrt(2^(1/n) - 1) */
+    PSFR_EFIT_AXIS_RATIO = 9,   /* minor / major, in (0, 1] */
+    PSFR_EFIT_CHISQ = 10,
+    PSFR_EFIT_ITER = 11,     /* LM iterations of the elliptical stage; negative = not converged */
+    PSFR_EFIT_ERR_PEAK = 12, PSFR_EFIT_ERR_Y0 = 13, PSFR_EFIT_ERR_X0 = 14,
+    PSFR_EFIT_ERR_A_MAJOR = 15, PSFR_EFIT_ERR_A_MINOR = 16,
+    PSFR_EFIT_ERR_PA = 17,   /* [deg]; +inf at an exact circle */
+    PSFR_EFIT_ERR_N = 18, PSFR_EFIT_ERR_FWHM_MAJOR = 19, PSFR_EFIT_ERR_FWHM_MINOR = 20,
+    PSFR_EFIT_ERR_AXIS_RATIO = 21,
+    PSFR_EFIT_FLUX = 22,     /* pi I a_major a_minor / (n - 1) */
+    PSFR_EFIT_ERR_FLUX = 23,
+    PSFR_EFIT_NPAR = 24
+};
+
 /* Context ------------------------------------------------------------------------- */
 
 /* dim: PSD grid size (1280; the reference hard-codes it in compute_psf, psfrec.py:955).
@@ -144,6 +170,12 @@ PSFR_API int psfr_convolve(psfr_ctx* ctx, int ndraw, int nlam, const double* lam
 PSFR_API int psfr_moffat_fit(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs,
                     double* params, void* stream);
 
+/* Elliptical Moffat fit of every image (PSFR_EFIT_* record): the circular fit of psfr_moffat_fit, then a
+ * 7-parameter Levenberg-Marquardt from its converged record, one warp per image.  Images, sizes, host / device
+ * handling and refusals as psfr_moffat_fit, and ny*nx must exceed 7.  params [nimg][PSFR_EFIT_NPAR]. */
+PSFR_API int psfr_moffat_fit_elliptical(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs,
+                                        double* params, void* stream);
+
 /* compute_psf (psfrec.py:933-978) for a batch of draws, fused on the device:
  * PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit.
  * out_cube [ndraw][nlam][40][40] and out_fit [ndraw][nlam][PSFR_FIT_NPAR]; either may be NULL.
@@ -177,6 +209,16 @@ PSFR_API int psfr_compute_groups(psfr_ctx* ctx, int ndraw, const double* draws, 
 PSFR_API int psfr_compute_field(psfr_ctx* ctx, int ndraw, const double* draws, int npos, const double* poslgs,
                        int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                        double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream);
+
+/* psfr_compute_field plus the elliptical fit of every image it fits: out_efit [ndraw][ndir][nlam][PSFR_EFIT_NPAR]
+ * of the per-draw cubes and out_mean_efit [ngroup][ndir][nlam][PSFR_EFIT_NPAR] of the exposure means, each
+ * bit for bit psfr_moffat_fit_elliptical of the images in out_cube / out_mean.  The elliptical fit runs in the
+ * chunk of its images, right after their circular fit.  Every output may be NULL; the other outputs are those
+ * of psfr_compute_field, bit for bit. */
+PSFR_API int psfr_compute_field_shapes(psfr_ctx* ctx, int ndraw, const double* draws, int npos, const double* poslgs,
+                       int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                       double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
+                       double* out_efit, double* out_mean_efit, void* stream);
 
 /* Time-mean of ncube cubes + refit (psfrec.py:1104-1105). cubes [ncube][nlam][40][40]. */
 PSFR_API int psfr_mean_refit(psfr_ctx* ctx, int ncube, int nlam, const double* cubes,

@@ -27,6 +27,12 @@ def layer_slot(layer, field):
 FIT_PEAK, FIT_Y0, FIT_X0, FIT_ALPHA, FIT_N, FIT_FWHM, FIT_CHISQ, FIT_ITER = range(8)
 FIT_ERR_PEAK, FIT_ERR_Y0, FIT_ERR_X0, FIT_ERR_ALPHA, FIT_ERR_N, FIT_ERR_FWHM, FIT_FLUX, FIT_ERR_FLUX = range(8, 16)
 FIT_NPAR = 16
+# elliptical record (PSFR_EFIT_*): widths and FWHM in pixels, PA in degrees
+(EFIT_PEAK, EFIT_Y0, EFIT_X0, EFIT_A_MAJOR, EFIT_A_MINOR, EFIT_PA, EFIT_N, EFIT_FWHM_MAJOR, EFIT_FWHM_MINOR,
+ EFIT_AXIS_RATIO, EFIT_CHISQ, EFIT_ITER) = range(12)
+(EFIT_ERR_PEAK, EFIT_ERR_Y0, EFIT_ERR_X0, EFIT_ERR_A_MAJOR, EFIT_ERR_A_MINOR, EFIT_ERR_PA, EFIT_ERR_N,
+ EFIT_ERR_FWHM_MAJOR, EFIT_ERR_FWHM_MINOR, EFIT_ERR_AXIS_RATIO, EFIT_FLUX, EFIT_ERR_FLUX) = range(12, 24)
+EFIT_NPAR = 24
 AO_DIM = 80
 PSF_DIM = 40
 
@@ -65,9 +71,11 @@ _SIGNATURES = {
     'psfr_psf_cube': (_I, [_P, _I, _I, _I, _P, _P, _P]),
     'psfr_convolve': (_I, [_P, _I, _I, _P, _P, _P, _P, _P]),
     'psfr_moffat_fit': (_I, [_P, _I, _I, _I, _P, _P, _P]),
+    'psfr_moffat_fit_elliptical': (_I, [_P, _I, _I, _I, _P, _P, _P]),
     'psfr_compute_batch': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P]),
     'psfr_compute_groups': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     'psfr_compute_field': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
+    'psfr_compute_field_shapes': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     'psfr_mean_refit': (_I, [_P, _I, _I, _P, _P, _P, _P]),
     'psfr_polyfit': (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     'psfr_set_option': (_I, [_P, _I, _D]),
@@ -275,6 +283,13 @@ class Context:
         self._check(self._lib.psfr_moffat_fit(self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
                                               self._buf(params, nimg * FIT_NPAR, 'params', True), stream))
 
+    def moffat_fit_elliptical(self, nimg, ny, nx, imgs, params, stream=None):
+        """psfr_moffat_fit_elliptical: ``params`` [nimg, EFIT_NPAR]."""
+        nimg, ny, nx = int(nimg), int(ny), int(nx)
+        self._check(self._lib.psfr_moffat_fit_elliptical(
+            self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
+            self._buf(params, nimg * EFIT_NPAR, 'params', True), stream))
+
     def compute_batch(self, draws, dirs, poslgs, lambda_nm, out_cube=None, out_fit=None, stream=None):
         if not hasattr(draws, 'data_ptr'):      # numpy / sequence; torch tensors pass through as buffers
             draws = f64(draws)
@@ -298,15 +313,21 @@ class Context:
                      out_fit, out_mean, out_mean_fit, stream)
 
     def compute_field(self, draws, dirs, poslgs, lambda_nm, group_end=None, out_cube=None, out_fit=None,
-                      out_mean=None, out_mean_fit=None, stream=None):
+                      out_mean=None, out_mean_fit=None, stream=None, out_efit=None, out_mean_efit=None):
         """psfr_compute_field: ``compute_groups`` with one PSF per field position of ``dirs`` [2, npos]
         instead of their average.  Outputs ``out_cube`` [ndraw, npos, nl, 40, 40], ``out_fit`` [ndraw, npos,
-        nl, FIT_NPAR], ``out_mean`` [ngroup, npos, nl, 40, 40], ``out_mean_fit`` [ngroup, npos, nl, FIT_NPAR]."""
-        self._groups(self._lib.psfr_compute_field, True, draws, dirs, poslgs, lambda_nm, group_end, out_cube,
-                     out_fit, out_mean, out_mean_fit, stream)
+        nl, FIT_NPAR], ``out_mean`` [ngroup, npos, nl, 40, 40], ``out_mean_fit`` [ngroup, npos, nl, FIT_NPAR].
+        ``out_efit`` [ndraw, npos, nl, EFIT_NPAR] and ``out_mean_efit`` [ngroup, npos, nl, EFIT_NPAR], the
+        elliptical fits of the same images, bind psfr_compute_field_shapes instead."""
+        if out_efit is None and out_mean_efit is None:
+            self._groups(self._lib.psfr_compute_field, True, draws, dirs, poslgs, lambda_nm, group_end, out_cube,
+                         out_fit, out_mean, out_mean_fit, stream)
+        else:
+            self._groups(self._lib.psfr_compute_field_shapes, True, draws, dirs, poslgs, lambda_nm, group_end,
+                         out_cube, out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit))
 
     def _groups(self, fn, field, draws, dirs, poslgs, lambda_nm, group_end, out_cube, out_fit, out_mean,
-                out_mean_fit, stream):
+                out_mean_fit, stream, shapes=None):
         if not hasattr(draws, 'data_ptr'):
             draws = f64(draws)
         if len(draws.shape) != 2 or draws.shape[1] != DRAW_NPAR:
@@ -316,13 +337,16 @@ class Context:
         ng, gp = group_end_ptr(group_end)
         nimg = lam.size * (dirs.shape[1] if field else 1)      # images per draw and per exposure
         img = nimg * PSF_DIM * PSF_DIM
-        self._check(fn(
-            self._handle(), nd, self._buf(draws, nd * DRAW_NPAR, 'draws'), poslgs.shape[1], ptr(poslgs),
-            dirs.shape[1], ptr(dirs), lam.size, ptr(lam), ng, gp,
-            self._buf(out_cube, nd * img, 'out_cube', True),
-            self._buf(out_fit, nd * nimg * FIT_NPAR, 'out_fit', True),
-            self._buf(out_mean, ng * img, 'out_mean', True),
-            self._buf(out_mean_fit, ng * nimg * FIT_NPAR, 'out_mean_fit', True), stream))
+        args = [self._handle(), nd, self._buf(draws, nd * DRAW_NPAR, 'draws'), poslgs.shape[1], ptr(poslgs),
+                dirs.shape[1], ptr(dirs), lam.size, ptr(lam), ng, gp,
+                self._buf(out_cube, nd * img, 'out_cube', True),
+                self._buf(out_fit, nd * nimg * FIT_NPAR, 'out_fit', True),
+                self._buf(out_mean, ng * img, 'out_mean', True),
+                self._buf(out_mean_fit, ng * nimg * FIT_NPAR, 'out_mean_fit', True)]
+        if shapes is not None:
+            args += [self._buf(shapes[0], nd * nimg * EFIT_NPAR, 'out_efit', True),
+                     self._buf(shapes[1], ng * nimg * EFIT_NPAR, 'out_mean_efit', True)]
+        self._check(fn(*args, stream))
 
     def mean_refit(self, ncube, nlam, cubes, out_mean=None, out_fit=None, stream=None):
         ncube, nlam = int(ncube), int(nlam)

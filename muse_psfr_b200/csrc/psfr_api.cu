@@ -289,7 +289,7 @@ static int hot_begin(Ctx* c) {
 static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs, int npos,
                      const double* poslgs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                      bool field, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
-                     cudaStream_t s) {
+                     double* out_efit, double* out_mean_efit, cudaStream_t s) {
     PSFR_CUDA(c, cudaSetDevice(c->device));
     std::vector<double> lam;
     int rc = small_to_host(c, lam, lambda_nm, nlam > 0 ? nlam : 0, s);
@@ -308,13 +308,16 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     const int ppd = field ? ndir : 1;
     const size_t img = (size_t)kPSF * kPSF, imgs = (size_t)ppd * nlam, elems = imgs * img;
     const size_t fits = imgs * PSFR_FIT_NPAR;   // fit records per draw
+    const size_t efits = imgs * PSFR_EFIT_NPAR;  // elliptical records per draw
     const bool cube_dev = out_cube && is_device_ptr(out_cube);
     const bool fit_dev = out_fit && is_device_ptr(out_fit);
     const bool mean_dev = out_mean && is_device_ptr(out_mean);
     const bool mfit_dev = out_mean_fit && is_device_ptr(out_mean_fit);
-    const bool means = out_mean || out_mean_fit;
+    const bool efit_dev = out_efit && is_device_ptr(out_efit);
+    const bool mefit_dev = out_mean_efit && is_device_ptr(out_mean_efit);
+    const bool means = out_mean || out_mean_fit || out_mean_efit;
     const bool host_out = (out_cube && !cube_dev) || (out_fit && !fit_dev) || (out_mean && !mean_dev) ||
-                          (out_mean_fit && !mfit_dev);
+                          (out_mean_fit && !mfit_dev) || (out_efit && !efit_dev) || (out_mean_efit && !mefit_dev);
     int* seg_dev = reinterpret_cast<int*>(c->d_misc + misc_groups(c->max_planes));
     std::vector<int> seg;
     int g0 = 0;   // first exposure not finished in an earlier chunk
@@ -337,11 +340,15 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
         double* conv = cube_dev ? out_cube + (size_t)d0 * elems : (b ? c->d_cube3 : c->d_cube2);
         if ((rc = run_convolve(c, nd, ppd, nlam, c->d_cube, conv, s))) break;
         double* fit = fit_dev ? out_fit + (size_t)d0 * fits : (b ? c->d_fit2 : c->d_fit);
-        if (out_fit && (rc = run_fit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, s))) break;
+        // the elliptical fit starts from the circular records of the same images
+        if ((out_fit || out_efit) && (rc = run_fit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, s))) break;
+        double* efit = efit_dev ? out_efit + (size_t)d0 * efits : (b ? c->d_efit2 : c->d_efit);
+        if (out_efit && (rc = run_efit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, efit, s))) break;
         // exposures g0, g0 + 1, ... that have draws in [d0, d0 + nd): all but possibly the last end here
         int ndone = 0;
         double* mean = mean_dev ? out_mean + (size_t)g0 * elems : c->d_mean[b];
         double* mfit = mfit_dev ? out_mean_fit + (size_t)g0 * fits : c->d_mfit[b];
+        double* mefit = mefit_dev ? out_mean_efit + (size_t)g0 * efits : c->d_mefit[b];
         if (means) {
             seg.clear();
             for (int g = g0; g < ngroup && (g == g0 || group_end[g - 1] < d0 + nd); ++g) {
@@ -356,7 +363,9 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                 break;
             }
             if ((rc = run_group_mean(c, (int)elems, conv, seg_dev, (int)seg.size() / 2, carry_in, mean, s))) break;
-            if (out_mean_fit && ndone && (rc = run_fit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, s))) break;
+            if ((out_mean_fit || out_mean_efit) && ndone && (rc = run_fit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, s)))
+                break;
+            if (out_mean_efit && ndone && (rc = run_efit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, mefit, s))) break;
         }
         if (host_out) {
             cudaError_t e = cudaEventRecord(c->ev_done[b], s);
@@ -372,6 +381,12 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                                     cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess && ndone && out_mean_fit && !mfit_dev)
                 e = cudaMemcpyAsync(out_mean_fit + (size_t)g0 * fits, mfit, (size_t)ndone * fits * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
+            if (e == cudaSuccess && out_efit && !efit_dev)
+                e = cudaMemcpyAsync(out_efit + (size_t)d0 * efits, efit, (size_t)nd * efits * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
+            if (e == cudaSuccess && ndone && out_mean_efit && !mefit_dev)
+                e = cudaMemcpyAsync(out_mean_efit + (size_t)g0 * efits, mefit, (size_t)ndone * efits * sizeof(double),
                                     cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess) e = cudaEventRecord(c->ev_copied[b], c->copy_stream);
             if (e != cudaSuccess) {
@@ -393,7 +408,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 102; }
+int psfr_version(void) { return 103; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -406,8 +421,8 @@ void psfr_destroy(psfr_ctx* c) {
     cudaFree(c->d_kern_tt); cudaFree(c->d_kern_mu); cudaFree(c->d_cube); cudaFree(c->d_cube2);
     cudaFree(c->d_fit); cudaFree(c->d_poly); cudaFree(c->d_dmin); cudaFree(c->d_counter);
     cudaFree(c->d_twc); cudaFree(c->d_wsamp); cudaFree(c->d_wcol); cudaFree(c->d_kcol); cudaFree(c->d_xmap); cudaFree(c->d_khat_tt); cudaFree(c->d_khat_mu);
-    cudaFree(c->d_cube3); cudaFree(c->d_fit2); cudaFree(c->d_carry);
-    for (int i = 0; i < 2; ++i) { cudaFree(c->d_mean[i]); cudaFree(c->d_mfit[i]); }
+    cudaFree(c->d_cube3); cudaFree(c->d_fit2); cudaFree(c->d_carry); cudaFree(c->d_efit); cudaFree(c->d_efit2);
+    for (int i = 0; i < 2; ++i) { cudaFree(c->d_mean[i]); cudaFree(c->d_mfit[i]); cudaFree(c->d_mefit[i]); }
     cudaFree(c->d_dphi32); cudaFree(c->d_otf32); cudaFree(c->d_tw32); cudaFree(c->d_twg); cudaFree(c->d_twg32); cudaFree(c->d_p3); cudaFree(c->d_p2mask); cudaFree(c->d_csort); cudaFree(c->d_lorder); cudaFree(c->d_kaddr);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     for (int i = 0; i < 2; ++i) {
@@ -524,9 +539,12 @@ int psfr_create(int device, int dim, int max_planes, int max_lambda, psfr_ctx** 
     CK(dev_alloc(c, &c->d_cube3, P * LM * kPSF * kPSF));
     CK(dev_alloc(c, &c->d_fit2, P * LM * PSFR_FIT_NPAR));
     CK(dev_alloc(c, &c->d_carry, P * LM * kPSF * kPSF));
+    CK(dev_alloc(c, &c->d_efit, P * LM * PSFR_EFIT_NPAR));
+    CK(dev_alloc(c, &c->d_efit2, P * LM * PSFR_EFIT_NPAR));
     for (int i = 0; i < 2; ++i) {
         CK(dev_alloc(c, &c->d_mean[i], P * LM * kPSF * kPSF));
         CK(dev_alloc(c, &c->d_mfit[i], P * LM * PSFR_FIT_NPAR));
+        CK(dev_alloc(c, &c->d_mefit[i], P * LM * PSFR_EFIT_NPAR));
     }
     CKC(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; ++i) {
@@ -725,6 +743,41 @@ int psfr_moffat_fit(psfr_ctx* c, int nimg, int ny, int nx, const double* imgs, d
     return PSFR_OK;
 }
 
+int psfr_moffat_fit_elliptical(psfr_ctx* c, int nimg, int ny, int nx, const double* imgs, double* params,
+                               void* stream) {
+    if (!c || !imgs || !params) return set_error(c, PSFR_E_ARG, "NULL argument");
+    if (nimg < 1 || ny < 3 || nx < 3) return set_error(c, PSFR_E_ARG, "nimg=%d ny=%d nx=%d", nimg, ny, nx);
+    if ((long long)ny * nx <= 7)
+        return set_error(c, PSFR_E_ARG, "image %dx%d: the elliptical fit needs more than 7 pixels", ny, nx);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    const size_t cap = (size_t)c->max_planes * c->max_lambda;
+    const size_t per = (size_t)ny * nx;
+    const bool in_dev = is_device_ptr(imgs), out_dev = is_device_ptr(params);
+    // the circular records go to d_fit and, for host outputs, the elliptical ones to d_efit: both hold cap records
+    const size_t chunk_imgs = std::min(cap, (cap * kPSF * kPSF) / per);
+    if (chunk_imgs < 1) return set_error(c, PSFR_E_CAPACITY, "image %dx%d does not fit the staging buffer", ny, nx);
+    for (size_t i0 = 0; i0 < (size_t)nimg; i0 += chunk_imgs) {
+        const int n = (int)std::min(chunk_imgs, (size_t)nimg - i0);
+        const double* src = imgs + i0 * per;
+        if (!in_dev) {
+            int rc = to_device(c, c->d_cube, src, (size_t)n * per * sizeof(double), s);
+            if (rc) return rc;
+            src = c->d_cube;
+        }
+        double* dst = out_dev ? params + i0 * PSFR_EFIT_NPAR : c->d_efit;
+        int rc = run_fit(c, n, ny, nx, src, c->d_fit, s);
+        if (rc) return rc;
+        rc = run_efit(c, n, ny, nx, src, c->d_fit, dst, s);
+        if (rc) return rc;
+        if (!out_dev) {
+            rc = from_device(c, params + i0 * PSFR_EFIT_NPAR, dst, (size_t)n * PSFR_EFIT_NPAR * sizeof(double), s);
+            if (rc) return rc;
+        }
+    }
+    return PSFR_OK;
+}
+
 int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs,
                        const double* poslgs, int nlam, const double* lambda_nm, double* out_cube,
                        double* out_fit, void* stream) {
@@ -733,19 +786,18 @@ int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, co
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d ndir=%d max_planes=%d", ndraw, ndir, c->max_planes);
     if (ngs < 1) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
     return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, false, out_cube,
-                     out_fit, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+                     out_fit, nullptr, nullptr, nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 // the arguments of psfr_compute_groups and psfr_compute_field that run_batch does not check itself
 static int check_groups(Ctx* c, int ndraw, const double* draws, const double* poslgs, int ndir, const double* dirs,
-                        const double* lambda_nm, int ngroup, const int* group_end, const double* out_mean,
-                        const double* out_mean_fit) {
+                        const double* lambda_nm, int ngroup, const int* group_end, bool means) {
     if (!c || !draws || !dirs || !poslgs || !lambda_nm || (ngroup > 0 && !group_end))
         return set_error(c, PSFR_E_ARG, "NULL argument");
     if (ndraw < 1 || ndir < 1 || ndir > c->max_planes)
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d ndir=%d max_planes=%d", ndraw, ndir, c->max_planes);
     if (ngroup < 0) return set_error(c, PSFR_E_ARG, "ngroup=%d", ngroup);
-    if (ngroup == 0 && (out_mean || out_mean_fit))
+    if (ngroup == 0 && means)
         return set_error(c, PSFR_E_ARG, "exposure means need at least one exposure (ngroup=0)");
     for (int g = 0; g < ngroup; ++g)
         if (group_end[g] <= (g ? group_end[g - 1] : 0))
@@ -758,19 +810,31 @@ static int check_groups(Ctx* c, int ndraw, const double* draws, const double* po
 int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
                         const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                         double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean, out_mean_fit))
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean || out_mean_fit))
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, false,
-                     out_cube, out_fit, out_mean, out_mean_fit, static_cast<cudaStream_t>(stream));
+                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
                        const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                        double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean, out_mean_fit))
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean || out_mean_fit))
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
-                     out_cube, out_fit, out_mean, out_mean_fit, static_cast<cudaStream_t>(stream));
+                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+int psfr_compute_field_shapes(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
+                              const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                              double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
+                              double* out_efit, double* out_mean_efit, void* stream) {
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
+                              out_mean || out_mean_fit || out_mean_efit))
+        return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
+                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int psfr_mean_refit(psfr_ctx* c, int ncube, int nlam, const double* cubes, double* out_mean, double* out_fit,

@@ -143,6 +143,9 @@ struct Ctx {
                                  // edge: [ndir][nlam][40][40] in psfr_compute_field, and ndir <= max_planes
     double* d_mean[2] = {nullptr, nullptr};  // [max_planes*max_lambda][40][40] exposure means finished in a chunk
     double* d_mfit[2] = {nullptr, nullptr};  // [max_planes*max_lambda][PSFR_FIT_NPAR] their fits
+    double* d_efit = nullptr;    // [max_planes*max_lambda][PSFR_EFIT_NPAR] elliptical records (double-buffered
+    double* d_efit2 = nullptr;   // with d_efit2 as d_fit / d_fit2)
+    double* d_mefit[2] = {nullptr, nullptr};  // [max_planes*max_lambda][PSFR_EFIT_NPAR] elliptical fits of the means
     cudaStream_t copy_stream = nullptr;      // device -> host copies of finished chunks
     cudaEvent_t ev_done[2] = {nullptr, nullptr};    // chunk results ready (compute stream)
     cudaEvent_t ev_copied[2] = {nullptr, nullptr};  // chunk results copied out (copy stream)
@@ -248,6 +251,9 @@ int run_fft_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev
 // unless every field position of a draw keeps its own image, psfr_compute_field)
 int run_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev, double* out_dev, cudaStream_t s);
 int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit_dev, cudaStream_t s);
+// elliptical fit of every image from its circular record circ_dev [nimg][PSFR_FIT_NPAR]
+int run_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* circ_dev, double* efit_dev,
+             cudaStream_t s);
 // out = (running sum of the cubes) ; first: start from zero, last: divide by ntotal
 int run_mean(Ctx* c, int ncube, int plane_elems, const double* cubes_dev, double* out_dev,
              cudaStream_t s, bool first, bool last, int ntotal);

@@ -105,15 +105,23 @@ constexpr int kFitWarps = 4;
 #ifndef PSFR_FIT_TOL2
 #define PSFR_FIT_TOL2 2.2e-16
 #endif
-constexpr int kNP = 5;
-constexpr int kNSUM = 21;  // 15 (J^T J upper) + 5 (J^T r) + 1 (cost)
+// Sizes of the normal equations of an NP-parameter least-squares fit: the packed upper triangle of J^T J,
+// then J^T r, then the cost r.r.
+template <int NP>
+struct Normal {
+    static constexpr int NJJ = NP * (NP + 1) / 2;
+    static constexpr int NSUM = NJJ + NP + 1;
+    static constexpr int COST = NSUM - 1;
+};
 
 // packed-upper index of (i, j), i <= j
-__device__ __forceinline__ constexpr int pk(int i, int j) { return i * kNP - i * (i - 1) / 2 + (j - i); }
+template <int NP>
+__device__ __forceinline__ constexpr int pk(int i, int j) { return i * NP - i * (i - 1) / 2 + (j - i); }
 
+template <int NSUM>
 __device__ __forceinline__ void warp_sum_vec(double* v) {
 #pragma unroll
-    for (int k = 0; k < kNSUM; ++k) {
+    for (int k = 0; k < NSUM; ++k) {
         double t = v[k];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
@@ -157,42 +165,101 @@ __device__ __forceinline__ double log_ge1(double u) {
     return fma(kf, kLn2[0], r);
 }
 
-// one pixel's contribution to the normal equations
-__device__ __forceinline__ void accumulate_pixel(double dp, double dq, double pix, double I, double n, double ia2,
-                                                 double ia, double* sums) {
-    const double rho2 = (dp * dp + dq * dq) * ia2;
-    const double uu = 1.0 + rho2;
-    const double lu = log_ge1(uu);
-    const double m = fast_exp(-n * lu);        // u^-n
-    const double f = I * m;
-    const double g = 2.0 * n * f * rcp_pos(uu);  // 2 I n u^(-n-1)
-    double J[kNP];
-    J[0] = m;
-    J[1] = g * dp * ia2;
-    J[2] = g * dq * ia2;
-    J[3] = g * rho2 * ia;
-    J[4] = -f * lu;
-    const double r = f - pix;
+// packed indices of the diagonal of J^T J
+template <int NP>
+struct DiagIndex {
+    int v[NP];
+    __device__ constexpr DiagIndex() : v() {
+        for (int i = 0; i < NP; ++i) v[i] = pk<NP>(i, i);
+    }
+};
+
+// one pixel's contribution J (NP entries) and residual r to the normal equations
+template <int NP>
+__device__ __forceinline__ void add_normal(const double* J, double r, double* sums) {
+    constexpr int NJJ = Normal<NP>::NJJ;
 #pragma unroll
-    for (int i = 0; i < kNP; ++i)
+    for (int i = 0; i < NP; ++i)
 #pragma unroll
-        for (int j = i; j < kNP; ++j) sums[pk(i, j)] = fma(J[i], J[j], sums[pk(i, j)]);
+        for (int j = i; j < NP; ++j) sums[pk<NP>(i, j)] = fma(J[i], J[j], sums[pk<NP>(i, j)]);
 #pragma unroll
-    for (int i = 0; i < kNP; ++i) sums[15 + i] = fma(J[i], r, sums[15 + i]);
-    sums[20] = fma(r, r, sums[20]);
+    for (int i = 0; i < NP; ++i) sums[NJJ + i] = fma(J[i], r, sums[NJJ + i]);
+    sums[NJJ + NP] = fma(r, r, sums[NJJ + NP]);
 }
+
+// The models the Levenberg-Marquardt driver below fits.  Each is built from the parameter vector x once
+// per pass over the image (per-pass constants), gives one pixel's contribution to the normal equations at
+// offset (dp, dq) = (row - y0, column - x0), and says which trial points it refuses.
+//
+// Circular Moffat f = I (1 + ((p-y0)^2 + (q-x0)^2)/a^2)^(-n), x = [I, y0, x0, a, n].
+struct CircularMoffat {
+    static constexpr int NP = 5;
+    double I, n, ia2, ia;
+    __device__ __forceinline__ explicit CircularMoffat(const double* x)
+        : I(x[0]), n(x[4]), ia2(1.0 / (x[3] * x[3])), ia(1.0 / x[3]) {}
+    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double* sums) const {
+        const double rho2 = (dp * dp + dq * dq) * ia2;
+        const double uu = 1.0 + rho2;
+        const double lu = log_ge1(uu);
+        const double m = fast_exp(-n * lu);        // u^-n
+        const double f = I * m;
+        const double g = 2.0 * n * f * rcp_pos(uu);  // 2 I n u^(-n-1)
+        double J[NP];
+        J[0] = m;
+        J[1] = g * dp * ia2;
+        J[2] = g * dq * ia2;
+        J[3] = g * rho2 * ia;
+        J[4] = -f * lu;
+        add_normal<NP>(J, f - pix, sums);
+    }
+    static __device__ __forceinline__ bool refuses(const double* xt) {
+        return !(xt[3] > 0.0) || !(xt[4] > 0.0) || !isfinite(xt[0]);
+    }
+};
+
+// Elliptical Moffat f = I (1 + A dp^2 + B dq^2 + C dp dq)^(-n), x = [I, y0, x0, A, B, C, n].  The quadratic
+// form keeps every Jacobian column alive at a circle (A = B, C = 0), where the rotation column of the
+// (a, e, rot) parameterisation vanishes.
+struct EllipticalMoffat {
+    static constexpr int NP = 7;
+    double I, A, B, C, n;
+    __device__ __forceinline__ explicit EllipticalMoffat(const double* x)
+        : I(x[0]), A(x[3]), B(x[4]), C(x[5]), n(x[6]) {}
+    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double* sums) const {
+        const double pp = dp * dp, qq = dq * dq, pq = dp * dq;
+        const double uu = 1.0 + fma(A, pp, fma(B, qq, C * pq));
+        const double lu = log_ge1(uu);
+        const double m = fast_exp(-n * lu);        // u^-n
+        const double f = I * m;
+        const double g = n * f * rcp_pos(uu);        // I n u^(-n-1)
+        double J[NP];
+        J[0] = m;
+        J[1] = g * fma(2.0 * A, dp, C * dq);
+        J[2] = g * fma(2.0 * B, dq, C * dp);
+        J[3] = -g * pp;
+        J[4] = -g * qq;
+        J[5] = -g * pq;
+        J[6] = -f * lu;
+        add_normal<NP>(J, f - pix, sums);
+    }
+    // the form must stay positive definite (u >= 1 everywhere)
+    static __device__ __forceinline__ bool refuses(const double* xt) {
+        return !(xt[3] > 0.0) || !(xt[4] > 0.0) || !(4.0 * xt[3] * xt[4] - xt[5] * xt[5] > 0.0) || !(xt[6] > 0.0) ||
+               !isfinite(xt[0]);
+    }
+};
 
 // accumulate normal equations at x over this lane's pixels (two independent pixel chains per
 // trip so that the log / exp latencies overlap), then reduce over the warp.  STEP = 1 visits every
 // pixel; STEP = 4 every fourth pixel of each lane (a quasi-uniform quarter of the image), used
 // by the coarse first stage of the fit.
-template <int STEP>
+template <class M, int STEP>
 __device__ __forceinline__ void accumulate(const double* __restrict__ img, int npx, int nx, const double* x,
                                            double* sums) {
 #pragma unroll
-    for (int k = 0; k < kNSUM; ++k) sums[k] = 0.0;
-    const double I = x[0], y0 = x[1], x0 = x[2], a = x[3], n = x[4];
-    const double ia2 = 1.0 / (a * a), ia = 1.0 / a;
+    for (int k = 0; k < Normal<M::NP>::NSUM; ++k) sums[k] = 0.0;
+    const double y0 = x[1], x0 = x[2];
+    const M model(x);
     const int lane = threadIdx.x & 31;
     int pr = lane / nx, qc = lane % nx;          // once per call; then stepped incrementally
     const int dpr = (32 * STEP) / nx, dqc = (32 * STEP) % nx;
@@ -210,22 +277,23 @@ __device__ __forceinline__ void accumulate(const double* __restrict__ img, int n
         step();
         const double dp1 = (double)pr - y0, dq1 = (double)qc - x0;
         step();
-        accumulate_pixel(dp0, dq0, img[idx], I, n, ia2, ia, sums);
-        accumulate_pixel(dp1, dq1, img[idx + 32 * STEP], I, n, ia2, ia, sums);
+        model.pixel(dp0, dq0, img[idx], sums);
+        model.pixel(dp1, dq1, img[idx + 32 * STEP], sums);
     }
-    if (idx < npx) accumulate_pixel((double)pr - y0, (double)qc - x0, img[idx], I, n, ia2, ia, sums);
-    warp_sum_vec(sums);
+    if (idx < npx) model.pixel((double)pr - y0, (double)qc - x0, img[idx], sums);
+    warp_sum_vec<Normal<M::NP>::NSUM>(sums);
 }
 
 // Cholesky of A + mu diag(A) (A from the packed sums), fully unrolled in registers.
 // L holds the factor with the RECIPROCAL of the diagonal on the diagonal.
-__device__ __forceinline__ bool cholesky(const double* s, double mu, double (&L)[kNP][kNP]) {
+template <int NP>
+__device__ __forceinline__ bool cholesky(const double* s, double mu, double (&L)[NP][NP]) {
     bool ok = true;
 #pragma unroll
-    for (int i = 0; i < kNP; ++i) {
+    for (int i = 0; i < NP; ++i) {
 #pragma unroll
         for (int j = 0; j <= i; ++j) {
-            double t = s[pk(j, i)];
+            double t = s[pk<NP>(j, i)];
             if (i == j) t *= (1.0 + mu);
 #pragma unroll
             for (int q = 0; q < j; ++q) t = fma(-L[i][q], L[j][q], t);
@@ -241,34 +309,36 @@ __device__ __forceinline__ bool cholesky(const double* s, double mu, double (&L)
 }
 
 // solve L L^T z = b in place
-__device__ __forceinline__ void chol_solve(const double (&L)[kNP][kNP], double* z) {
+template <int NP>
+__device__ __forceinline__ void chol_solve(const double (&L)[NP][NP], double* z) {
 #pragma unroll
-    for (int i = 0; i < kNP; ++i) {
+    for (int i = 0; i < NP; ++i) {
         double t = z[i];
 #pragma unroll
         for (int q = 0; q < i; ++q) t = fma(-L[i][q], z[q], t);
         z[i] = t * L[i][i];
     }
 #pragma unroll
-    for (int i = kNP - 1; i >= 0; --i) {
+    for (int i = NP - 1; i >= 0; --i) {
         double t = z[i];
 #pragma unroll
-        for (int q = i + 1; q < kNP; ++q) t = fma(-L[q][i], z[q], t);
+        for (int q = i + 1; q < NP; ++q) t = fma(-L[q][i], z[q], t);
         z[i] = t * L[i][i];
     }
 }
 
-// Levenberg-Marquardt on the pixel subset STEP from the start point x (updated in place);
+// Levenberg-Marquardt of model M on the pixel subset STEP from the start point x (updated in place);
 // sums holds the normal equations at the final x.  tol2 = square of the relative step at which
 // to stop (MINPACK, the reference's solver, stops at 1.49e-8; so does the final stage).
-template <int STEP>
+template <class M, int STEP>
 __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx, int nx, double* x, double* sums,
                                          double tol2, int max_iter, int& iter, int& status) {
+    constexpr int kNP = M::NP, NJJ = Normal<kNP>::NJJ, kNSUM = Normal<kNP>::NSUM, COST = Normal<kNP>::COST;
     double trial[kNSUM], xt[kNP], d[kNP];
-    accumulate<STEP>(img, npx, nx, x, sums);
+    accumulate<M, STEP>(img, npx, nx, x, sums);
     double mu = 1e-3, nu = 2.0;
     status = -1;
-    constexpr int dia[kNP] = {pk(0, 0), pk(1, 1), pk(2, 2), pk(3, 3), pk(4, 4)};
+    constexpr DiagIndex<kNP> dia;
     double L[kNP][kNP];
     for (iter = 1; iter <= max_iter; ++iter) {
         // every lane runs the identical solve on bit-identical sums
@@ -279,31 +349,31 @@ __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx
             continue;
         }
 #pragma unroll
-        for (int i = 0; i < kNP; ++i) d[i] = -sums[15 + i];
+        for (int i = 0; i < kNP; ++i) d[i] = -sums[NJJ + i];
         chol_solve(L, d);
         double dn = 0.0, xn = 0.0, pred = 0.0;
 #pragma unroll
         for (int i = 0; i < kNP; ++i) {
             xt[i] = x[i] + d[i];
-            const double sc2 = sums[dia[i]];                  // |J column|^2
+            const double sc2 = sums[dia.v[i]];           // |J column|^2
             dn = fma(d[i] * d[i], sc2, dn);
             xn = fma(x[i] * x[i], sc2, xn);
             // predicted decrease of r.r : d.(mu D d - g)
-            pred += d[i] * (mu * sc2 * d[i] - sums[15 + i]);
+            pred += d[i] * (mu * sc2 * d[i] - sums[NJJ + i]);
         }
-        if (!(xt[3] > 0.0) || !(xt[4] > 0.0) || !isfinite(xt[0])) {
+        if (M::refuses(xt)) {
             mu *= nu;
             nu *= 2.0;
             if (mu > 1e15) break;
             continue;
         }
-        accumulate<STEP>(img, npx, nx, xt, trial);
-        const double actual = sums[20] - trial[20];
+        accumulate<M, STEP>(img, npx, nx, xt, trial);
+        const double actual = sums[COST] - trial[COST];
         // near the minimum the cost is flat to rounding: tolerate a noise-level increase so that
         // Gauss-Newton steps keep contracting, and stop on the (column-scaled) step size
         // MINPACK (the reference, through mpdaf -> scipy leastsq) stops at a relative step of 1.49e-8
         const bool small = dn <= tol2 * (xn + 1e-300);            // relative step <= sqrt(tol2)
-        if (isfinite(trial[20]) && actual >= -1e-13 * sums[20]) {
+        if (isfinite(trial[COST]) && actual >= -1e-13 * sums[COST]) {
             const double rho = pred > 0.0 ? actual / pred : 1.0;
 #pragma unroll
             for (int i = 0; i < kNP; ++i) x[i] = xt[i];
@@ -332,6 +402,7 @@ __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx
 __global__ void __launch_bounds__(kFitWarps * 32, PSFR_FIT_MINBLOCKS)
 fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __restrict__ out,
            int* __restrict__ next_image) {
+    constexpr int kNP = CircularMoffat::NP, kNSUM = Normal<kNP>::NSUM, COST = Normal<kNP>::COST;
     extern __shared__ double sm[];
     const int npx = ny * nx, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double* img = sm + (size_t)warp * (npx + nx);    // npx pixels + nx column weights
@@ -396,9 +467,9 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     // only moves the start point (the converged minimum does not depend on it); stage 2: all
     // pixels down to MINPACK's own tolerance, 1.49e-8.
     int iter = 0, status = -1;
-    lm_solve<PSFR_FIT_COARSE_STEP>(img, npx, nx, x, sums, PSFR_FIT_COARSE_TOL2, 12, iter, status);
+    lm_solve<CircularMoffat, PSFR_FIT_COARSE_STEP>(img, npx, nx, x, sums, PSFR_FIT_COARSE_TOL2, 12, iter, status);
     const int coarse_iter = iter;
-    lm_solve<1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, 200, iter, status);
+    lm_solve<CircularMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, 200, iter, status);
     iter += coarse_iter;
     if (status > 0) status += coarse_iter;
     const int max_iter = 212;
@@ -412,7 +483,7 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
         o[PSFR_FIT_ALPHA] = a;
         o[PSFR_FIT_N] = n;
         o[PSFR_FIT_FWHM] = a * kf;
-        o[PSFR_FIT_CHISQ] = sums[20];
+        o[PSFR_FIT_CHISQ] = sums[COST];
         o[PSFR_FIT_ITER] = (status > 0) ? (double)status : -(double)(iter > max_iter ? max_iter : iter);
         const double dof = (double)(npx - kNP);
         double L[kNP][kNP];
@@ -424,7 +495,7 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
 #pragma unroll
                 for (int i = 0; i < kNP; ++i) z[i] = (i == c) ? 1.0 : 0.0;
                 chol_solve(L, z);
-                e[c] = sqrt(fabs(z[c]) * fabs(sums[20] / dof));
+                e[c] = sqrt(fabs(z[c]) * fabs(sums[COST] / dof));
             }
             o[PSFR_FIT_ERR_PEAK] = e[0];
             o[PSFR_FIT_ERR_Y0] = e[1];
@@ -443,6 +514,144 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     }
     __syncwarp();
     }   // next image
+}
+
+// ---------------------------------------------------------------- elliptical Moffat fit
+// resident CTAs per SM the elliptical fitter is compiled for: 36 sums, 36 trial sums and the 7 x 7 factor
+// live in registers, so it runs at half the circular fitter's occupancy
+#ifndef PSFR_EFIT_MINBLOCKS
+#define PSFR_EFIT_MINBLOCKS 2
+#endif
+constexpr int kEfitMaxIter = 200;
+
+// g^T (J^T J)^-1 g from the Cholesky factor of J^T J
+template <int NP>
+__device__ __forceinline__ double inv_quad(const double (&L)[NP][NP], const double* g) {
+    double z[NP];
+#pragma unroll
+    for (int i = 0; i < NP; ++i) z[i] = g[i];
+    chol_solve<NP>(L, z);
+    double t = 0.0;
+#pragma unroll
+    for (int i = 0; i < NP; ++i) t = fma(g[i], z[i], t);
+    return t;
+}
+
+// The elliptical record of x = [I, y0, x0, A, B, C, n] (include/psfr.h, PSFR_EFIT_*).  Each derived quantity
+// q gets the error sqrt(grad q^T Sigma grad q), Sigma = (J^T J)^-1 chi^2/dof, with the gradient written out.
+__device__ void write_efit_record(const double* x, const double* sums, int npx, int iter, int status, double* o) {
+    constexpr int NP = EllipticalMoffat::NP, COST = Normal<NP>::COST;
+    constexpr double kPi = 3.141592653589793, kDeg = 180.0 / kPi;
+    const double I = x[0], A = x[3], B = x[4], C = x[5], n = x[6];
+    // eigenvalues of [[A, C/2], [C/2, B]]: the major axis belongs to the smaller one
+    const double hd = 0.5 * (A - B), hc = 0.5 * C, S = 0.5 * (A + B);
+    const double R2 = hd * hd + hc * hc, R = sqrt(R2);
+    const double lmin = S - R, lmax = S + R;
+    const double amaj = 1.0 / sqrt(lmin), amin = 1.0 / sqrt(lmax);
+    // major axis from +x (column) toward +y (row): B x^2 + C x y + A y^2 is smallest along
+    // angle 0.5 atan2(-C, A - B)
+    double pa = 0.0;
+    if (R2 != 0.0) {
+        pa = 0.5 * atan2(-C, A - B);
+        if (pa < 0.0) pa += kPi;
+        pa *= kDeg;
+        if (pa >= 180.0) pa -= 180.0;
+        pa = fabs(pa);       // 0, not -0, for a major axis along +x
+    }
+    const double kf = 2.0 * sqrt(pow(2.0, 1.0 / n) - 1.0);
+    const double dkf = -2.0 * pow(2.0, 1.0 / n) * 0.6931471805599453 / (n * n * kf);   // d kf / d n
+    const double q = sqrt(lmin / lmax);
+    const double flux = kPi * I * amaj * amin / (n - 1.0);
+    o[PSFR_EFIT_PEAK] = I;
+    o[PSFR_EFIT_Y0] = x[1];
+    o[PSFR_EFIT_X0] = x[2];
+    o[PSFR_EFIT_A_MAJOR] = amaj;
+    o[PSFR_EFIT_A_MINOR] = amin;
+    o[PSFR_EFIT_PA] = pa;
+    o[PSFR_EFIT_N] = n;
+    o[PSFR_EFIT_FWHM_MAJOR] = amaj * kf;
+    o[PSFR_EFIT_FWHM_MINOR] = amin * kf;
+    o[PSFR_EFIT_AXIS_RATIO] = q;
+    o[PSFR_EFIT_CHISQ] = sums[COST];
+    o[PSFR_EFIT_ITER] = (status > 0) ? (double)status : -(double)(iter > kEfitMaxIter ? kEfitMaxIter : iter);
+    o[PSFR_EFIT_FLUX] = flux;
+    double L[NP][NP];
+    if (!cholesky<NP>(sums, 0.0, L)) {
+        for (int i = PSFR_EFIT_ERR_PEAK; i <= PSFR_EFIT_ERR_AXIS_RATIO; ++i) o[i] = nan("");
+        o[PSFR_EFIT_ERR_FLUX] = nan("");
+        if (R2 == 0.0) o[PSFR_EFIT_ERR_PA] = INFINITY;
+        return;
+    }
+    const double s2 = fabs(sums[COST] / (double)(npx - NP));
+    auto err = [&](const double* g) { return sqrt(fabs(inv_quad<NP>(L, g)) * s2); };
+    // the eigenvalues are not differentiable at a circle (R = 0): there their mean (A + B)/2 stands in
+    const double ca = R > 0.0 ? hd / (2.0 * R) : 0.0, cc = R > 0.0 ? hc / (2.0 * R) : 0.0;
+    const double gmaj = -0.5 * amaj * amaj * amaj, gmin = -0.5 * amin * amin * amin;   // d a / d lambda
+    const double g_amaj[NP] = {0, 0, 0, gmaj * (0.5 - ca), gmaj * (0.5 + ca), -gmaj * cc, 0};
+    const double g_amin[NP] = {0, 0, 0, gmin * (0.5 + ca), gmin * (0.5 - ca), gmin * cc, 0};
+    double g[NP];
+#pragma unroll
+    for (int c = 0; c < NP; ++c) {
+        if (c == 3 || c == 4 || c == 5) continue;
+#pragma unroll
+        for (int i = 0; i < NP; ++i) g[i] = (i == c) ? 1.0 : 0.0;
+        o[c == 6 ? PSFR_EFIT_ERR_N : PSFR_EFIT_ERR_PEAK + c] = err(g);
+    }
+    o[PSFR_EFIT_ERR_A_MAJOR] = err(g_amaj);
+    o[PSFR_EFIT_ERR_A_MINOR] = err(g_amin);
+    if (R2 == 0.0) {
+        o[PSFR_EFIT_ERR_PA] = INFINITY;
+    } else {
+        const double k = kDeg * 0.5 / (4.0 * R2);      // d atan2(-C, A - B) / 2, in degrees
+        const double g_pa[NP] = {0, 0, 0, k * C, -k * C, -k * (A - B), 0};
+        o[PSFR_EFIT_ERR_PA] = err(g_pa);
+    }
+#pragma unroll
+    for (int i = 0; i < NP; ++i) g[i] = kf * g_amaj[i];
+    g[6] = amaj * dkf;
+    o[PSFR_EFIT_ERR_FWHM_MAJOR] = err(g);
+#pragma unroll
+    for (int i = 0; i < NP; ++i) g[i] = kf * g_amin[i];
+    g[6] = amin * dkf;
+    o[PSFR_EFIT_ERR_FWHM_MINOR] = err(g);
+#pragma unroll
+    for (int i = 0; i < NP; ++i) g[i] = q * (g_amin[i] / amin - g_amaj[i] / amaj);
+    o[PSFR_EFIT_ERR_AXIS_RATIO] = err(g);
+    // flux = pi I / ((n - 1) sqrt(det)), det = A B - C^2 / 4
+    const double det = A * B - hc * hc, fd = -flux / (2.0 * det);
+    const double g_flux[NP] = {kPi * amaj * amin / (n - 1.0), 0, 0, fd * B, fd * A, -fd * hc, -flux / (n - 1.0)};
+    o[PSFR_EFIT_ERR_FLUX] = err(g_flux);
+}
+
+// Elliptical Moffat fit of every image, one warp per image as fit_kernel, from the image's converged
+// circular record circ [nimg][PSFR_FIT_NPAR]: (I, y0, x0, 1/a^2, 1/a^2, 0, n), all pixels, down to the
+// final stage's tolerance.  out [nimg][PSFR_EFIT_NPAR].
+__global__ void __launch_bounds__(kFitWarps * 32, PSFR_EFIT_MINBLOCKS)
+efit_kernel(const double* __restrict__ imgs, const double* __restrict__ circ, int nimg, int ny, int nx,
+            double* __restrict__ out, int* __restrict__ next_image) {
+    constexpr int kNP = EllipticalMoffat::NP, kNSUM = Normal<kNP>::NSUM;
+    extern __shared__ double sm[];
+    const int npx = ny * nx, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double* img = sm + (size_t)warp * npx;
+#pragma unroll 1
+    for (;;) {
+        int image = 0;
+        if (lane == 0) image = atomicAdd(next_image, 1);
+        image = __shfl_sync(0xffffffffu, image, 0);
+        if (image >= nimg) return;
+        __syncwarp();
+        const double* src = imgs + (size_t)image * npx;
+        for (int i = lane; i < npx; i += 32) img[i] = src[i];
+        __syncwarp();
+        const double* c = circ + (size_t)image * PSFR_FIT_NPAR;
+        const double ia2 = 1.0 / (c[PSFR_FIT_ALPHA] * c[PSFR_FIT_ALPHA]);
+        double x[kNP] = {c[PSFR_FIT_PEAK], c[PSFR_FIT_Y0], c[PSFR_FIT_X0], ia2, ia2, 0.0, c[PSFR_FIT_N]};
+        double sums[kNSUM];
+        int iter = 0, status = -1;
+        lm_solve<EllipticalMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
+        if (lane == 0) write_efit_record(x, sums, npx, iter, status, out + (size_t)image * PSFR_EFIT_NPAR);
+        __syncwarp();
+    }
 }
 
 // ---------------------------------------------------------------- mean of cubes
@@ -604,6 +813,26 @@ int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit
     if (grid > resident) grid = resident;
     PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 1, 0, sizeof(int), s));
     fit_kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, nimg, ny, nx, fit_dev, c->d_counter + 1);
+    PSFR_LAUNCH_CHECK(c);
+    return PSFR_OK;
+}
+
+int run_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* circ_dev, double* efit_dev,
+             cudaStream_t s) {
+    const size_t smem = (size_t)kFitWarps * ny * nx * sizeof(double);
+    if (smem > 200 * 1024) return set_error(c, PSFR_E_UNSUPPORTED, "image %dx%d too large for the fitter", ny, nx);
+    if (int rc = ensure_dynamic_smem(c, efit_kernel, smem)) return rc;
+    int grid = (nimg + kFitWarps - 1) / kFitWarps;
+    int per_sm = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, efit_kernel, kFitWarps * 32, smem) != cudaSuccess ||
+        per_sm < 1) {
+        cudaGetLastError();
+        per_sm = 1;
+    }
+    const int resident = c->sm_count * per_sm;
+    if (grid > resident) grid = resident;
+    PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 2, 0, sizeof(int), s));
+    efit_kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, circ_dev, nimg, ny, nx, efit_dev, c->d_counter + 2);
     PSFR_LAUNCH_CHECK(c);
     return PSFR_OK;
 }

@@ -291,6 +291,36 @@ def _table_from_fit(lbda, fit, pixscale=0.2):
     })
 
 
+def _shape_table_from_fit(lbda, efit, pixscale=0.2):
+    """Columns of the elliptical fit (``fit_psf_cube(circular=False)``) for records [n, EFIT_NPAR]: ``fwhm`` and
+    ``err_fwhm`` hold (major, minor) in arcsec in the reference's two-element columns, ``pa`` and ``err_pa``
+    are in degrees (major axis from +x toward +y), ``center`` in pixels.  The reference has no elliptical
+    fit: these columns are this package's own (DESIGN.md section 5.3).  ``converged`` as ``_table_from_fit``."""
+    converged = efit[:, _lib.EFIT_ITER] > 0
+    if not converged.all():
+        bad = np.flatnonzero(~converged)
+        logger.warning('elliptical Moffat fit did not converge for %d of %d images (first at index %d)',
+                       bad.size, len(efit), bad[0])
+    return FitTable({
+        'lbda': np.asarray(lbda, dtype=float),
+        'center': efit[:, [_lib.EFIT_Y0, _lib.EFIT_X0]].copy(),
+        'fwhm': efit[:, [_lib.EFIT_FWHM_MAJOR, _lib.EFIT_FWHM_MINOR]] * pixscale,
+        'axis_ratio': efit[:, _lib.EFIT_AXIS_RATIO].copy(),
+        'pa': efit[:, _lib.EFIT_PA].copy(),
+        'n': efit[:, _lib.EFIT_N].copy(),
+        'peak': efit[:, _lib.EFIT_PEAK].copy(),
+        'flux': efit[:, _lib.EFIT_FLUX].copy(),
+        'err_center': efit[:, [_lib.EFIT_ERR_Y0, _lib.EFIT_ERR_X0]].copy(),
+        'err_fwhm': efit[:, [_lib.EFIT_ERR_FWHM_MAJOR, _lib.EFIT_ERR_FWHM_MINOR]] * pixscale,
+        'err_axis_ratio': efit[:, _lib.EFIT_ERR_AXIS_RATIO].copy(),
+        'err_pa': efit[:, _lib.EFIT_ERR_PA].copy(),
+        'err_n': efit[:, _lib.EFIT_ERR_N].copy(),
+        'err_peak': efit[:, _lib.EFIT_ERR_PEAK].copy(),
+        'err_flux': efit[:, _lib.EFIT_ERR_FLUX].copy(),
+        'converged': converged.astype(np.int64),
+    })
+
+
 # --------------------------------------------------------------------------- reference API
 def simul_psd_wfm(Cn2, h, seeing, L0, zenith=0., plot=False, npsflin=1, dim=1280,
                   three_lgs_mode=False, verbose=True, wind_dir=None):
@@ -386,13 +416,22 @@ def convolve_final_psf(lbda, seeing, GL, L0, psf):
     return out
 
 
-def fit_psf_cube(lbda, psfcube):
+def fit_psf_cube(lbda, psfcube, circular=True):
     """Fit a Moffat PSF on each wavelength plane (psfrec.py:861-871).  ``psfcube`` is an
-    array [nl, ny, nx] (or anything with a ``.data`` array, like an mpdaf Cube)."""
+    array [nl, ny, nx] (or anything with a ``.data`` array, like an mpdaf Cube).
+
+    ``circular=False`` (mpdaf's keyword; the reference passes True) fits an elliptical Moffat instead and
+    returns the columns of ``_shape_table_from_fit``: ``fwhm`` = (major, minor), ``axis_ratio``, ``pa`` [deg]
+    and their errors."""
     data = getattr(psfcube, 'data', psfcube)
     data = np.ascontiguousarray(np.ma.getdata(data), dtype=np.float64)
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
     nimg, ny, nx = data.shape
+    if not circular:
+        efit = np.empty((nimg, _lib.EFIT_NPAR))
+        if nimg:
+            get_context().moffat_fit_elliptical(nimg, ny, nx, data, efit)
+        return _shape_table_from_fit(lam, efit)
     ctx = get_context()
     fit = np.empty((nimg, _lib.FIT_NPAR))
     ctx.moffat_fit(nimg, ny, nx, data, fit)
@@ -532,7 +571,7 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
 
 def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_size=60, h=(100, 10000),
                       three_lgs_mode=False, out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None,
-                      stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None):
+                      stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None, elliptical=False):
     """Field-resolved ``compute_psf_batch``: the PSF of every draw at every field position instead of
     their average.
 
@@ -543,7 +582,11 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     (so ``positions=[[0], [0]]`` reproduces ``compute_psf_batch(npsflin=1)``).  It is not the field mean
     ``compute_psf_batch(npsflin=n)`` returns, and the field mean is not the average of these PSFs (each
     is normalised on its own).  Other arguments as ``compute_psf_batch``.  Returns (fit [ndraw, npos, nl,
-    FIT_NPAR], cube [ndraw, npos, nl, 40, 40])."""
+    FIT_NPAR], cube [ndraw, npos, nl, 40, 40]).
+
+    ``elliptical=True`` also fits an elliptical Moffat to every PSF on the device, right after its circular fit
+    and from it, and returns (fit, cube, efit) with efit [ndraw, npos, nl, EFIT_NPAR] (``_lib.EFIT_*``); fit and
+    cube are those of a call without it, bit for bit."""
     pos = _field_positions(direction_perf(npsflin, field_size) if positions is None else positions)
     npos = pos.shape[1]
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
@@ -552,9 +595,11 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     if GL.size != nd or L0.size != nd:
         raise ValueError('seeing, GL and L0 must have one entry per draw (got %d, %d, %d)' % (nd, GL.size, L0.size))
     three = _mode_flags(three_lgs_mode, nd)
+    efit = np.empty((nd, npos, lam.size, _lib.EFIT_NPAR)) if elliptical else None
     if nd == 0 or lam.size == 0:
-        return (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
-                np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
+        empty = (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
+                 np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
+        return empty + (efit,) if elliptical else empty
     # the records compute_psf_batch builds in either laser mode; the three-laser asterism is the first three
     # stars of the four-laser one
     recs = _mode_records(three, seeing, GL, L0, h, zenith, Cn2, wind_dir)
@@ -565,12 +610,13 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        ctx.compute_field(recs, pos, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit, stream=stream)
+        ctx.compute_field(recs, pos, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit, stream=stream,
+                          out_efit=efit)
     except PsfrError as exc:
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
         raise
-    return out_fit, out_cube
+    return (out_fit, out_cube, efit) if elliptical else (out_fit, out_cube)
 
 
 def _norm_lbda(lbda, lb1, lb2):
@@ -638,9 +684,17 @@ def _fit_columns(lam, fit):
     return {k: tab[k] for k in tab.colnames}
 
 
+def _shape_columns(lam, efit):
+    """Columns of the elliptical fit table for records [n, nl, EFIT_NPAR] (flattened)."""
+    nl = lam.size
+    efit = np.asarray(efit).reshape(-1, _lib.EFIT_NPAR)
+    tab = _shape_table_from_fit(np.tile(lam, len(efit) // nl), efit)
+    return {k: tab[k] for k in tab.colnames}
+
+
 def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                             lbda=None, h=(100, 10000), n_jobs=-1, plot=False, mean_of_lgs=True,
-                            verbose=True, device=None, field_positions=None):
+                            verbose=True, device=None, field_positions=None, elliptical=False):
     """Reconstruct a PSF from SPARTA data (psfrec.py:981-1120).
 
     ``filename``: path of a FITS file, a binary file object, or an HDUList (this package's or
@@ -649,18 +703,18 @@ def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin
     ``n_jobs`` is accepted and only reported).  Returns an HDUList [PRIMARY, <extname>, FIT_ROWS,
     FIT_MEAN, PSF_MEAN] - an ``astropy.io.fits.HDUList`` when astropy is installed, otherwise
     the equivalent object of ``muse_psfr_b200._fits`` - or None when no row is valid.  With
-    ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow: see
-    ``compute_psf_from_sparta_batch``."""
+    ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow, and with ``elliptical=True``
+    SHAPE_MEAN (and SHAPE_FIELD): see ``compute_psf_from_sparta_batch``."""
     if plot:
         raise NotImplementedError('plotting is outside the B200 hot path')
     return compute_psf_from_sparta_batch([filename], extname=extname, npsflin=npsflin, lmin=lmin, lmax=lmax, nl=nl,
                                          lbda=lbda, h=h, n_jobs=n_jobs, mean_of_lgs=mean_of_lgs, verbose=verbose,
-                                         device=device, field_positions=field_positions)[0]
+                                         device=device, field_positions=field_positions, elliptical=elliptical)[0]
 
 
 def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                                   lbda=None, h=(100, 10000), n_jobs=-1, mean_of_lgs=True, verbose=True,
-                                  device=None, max_planes=None, field_positions=None):
+                                  device=None, max_planes=None, field_positions=None, elliptical=False):
     """``compute_psf_from_sparta`` for many exposures in one device pass: returns one entry per source,
     the HDUList ``compute_psf_from_sparta(source, ...)`` returns, bit for bit, or None for a table
     without a valid row.
@@ -675,7 +729,12 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     time-mean PSF at each of those positions, from one more device pass over the same draws
     (``compute_psf_field``): FIT_FIELD, the columns of FIT_MEAN plus ``x`` and ``y`` [arcsec], one row per
     (position, wavelength), position-major, with the cards of FIT_MEAN; and PSF_FIELD, an image [npos,
-    nl, 40, 40].  The first five HDUs are those of a call without ``field_positions``, bit for bit."""
+    nl, 40, 40].  The first five HDUs are those of a call without ``field_positions``, bit for bit.
+
+    ``elliptical=True`` appends SHAPE_MEAN, the elliptical fit table (``fit_psf_cube(circular=False)``
+    columns) of PSF_MEAN with the cards of FIT_MEAN, and with ``field_positions`` SHAPE_FIELD, the same
+    columns plus ``x`` and ``y`` for the PSFs of PSF_FIELD, position-major.  Every HDU before them is that of
+    a call without ``elliptical``, bit for bit."""
     if lbda is None:
         lbda = np.linspace(lmin, lmax, nl)
     lbda = np.atleast_1d(np.asarray(lbda, dtype=float))
@@ -722,8 +781,12 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
             psf_field = np.empty((ng, npos, nlam, _lib.PSF_DIM, _lib.PSF_DIM))
             fit_field = np.empty((ng, npos, nlam, _lib.FIT_NPAR))
             ctx = _planes_context(nd, npos, nlam, max_planes, device, _DIM)
+            shape_field = np.empty((ng, npos, nlam, _lib.EFIT_NPAR)) if elliptical else None
             ctx.compute_field(draws, pos, _lgs_positions(False), lbda, group_end, out_mean=psf_field,
-                              out_mean_fit=fit_field)
+                              out_mean_fit=fit_field, out_mean_efit=shape_field)
+        if elliptical:      # the time means are on the host already: one standalone fit of all of them
+            shape_mean = np.empty((ng, nlam, _lib.EFIT_NPAR))
+            ctx.moffat_fit_elliptical(ng * nlam, _lib.PSF_DIM, _lib.PSF_DIM, psftot, shape_mean)
     except PsfrError as exc:
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
@@ -757,6 +820,13 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
             cols['y'] = np.repeat(pos[1], nlam)
             out.append(_fits.table_to_hdu(cols, meta=meta, name='FIT_FIELD'))
             out.append(_fits.ImageHDU(data=psf_field[g], name='PSF_FIELD'))
+        if elliptical:
+            out.append(_fits.table_to_hdu(_shape_columns(lbda, shape_mean[g]), meta=meta, name='SHAPE_MEAN'))
+            if pos is not None:
+                cols = _shape_columns(lbda, shape_field[g])
+                cols['x'] = np.repeat(pos[0], nlam)
+                cols['y'] = np.repeat(pos[1], nlam)
+                out.append(_fits.table_to_hdu(cols, meta=meta, name='SHAPE_FIELD'))
         try:
             results.append(_fits.to_astropy(out))
         except ImportError:
