@@ -115,6 +115,19 @@ enum {
     PSFR_EFIT_NPAR = 24
 };
 
+/* Encircled energy (DESIGN.md section 5.4).  Pixel (p, q) is the unit square [p - 1/2, p + 1/2] x [q - 1/2, q + 1/2]
+ * with its value spread uniformly over it; EE(r) = sum img[p][q] * area(pixel AND disc(centre, r)), the exact
+ * overlap area in FP64, over the pixels of the image only (a circle that leaves the image is clipped by its edge),
+ * in the image's own units (no renormalisation).  A record of nrad + 1 + nfrac doubles per image: */
+#define PSFR_EE_MAX_RADII 64
+#define PSFR_EE_MAX_FRACTIONS 16
+/*  [0, nrad)              EE(radii[k])
+ *  [nrad]                 TOTAL = sum img, summed in the order of the EE sums (EE == TOTAL bit for bit once the
+ *                         circle contains every pixel)
+ *  [nrad + 1 + j]         the smallest r >= 0 with EE(r) >= fracs[j] * TOTAL [px], to a bracket of 1e-10 px;
+ *                         NaN when TOTAL <= 0 (or NaN)
+ * Radii must be finite and >= 0, fractions in (0, 1), centres finite; otherwise PSFR_E_ARG, nothing written. */
+
 /* Context ------------------------------------------------------------------------- */
 
 /* dim: PSD grid size (1280; the reference hard-codes it in compute_psf, psfrec.py:955).
@@ -219,6 +232,27 @@ PSFR_API int psfr_compute_field_shapes(psfr_ctx* ctx, int ndraw, const double* d
                        int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                        double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
                        double* out_efit, double* out_mean_efit, void* stream);
+
+/* Encircled-energy record of every image.  centres [nimg][2] = (y0, x0) in pixels (row, column; pixel centres at
+ * integers), or NULL for (ny / 2, nx / 2) - pixel (20, 20) of a 40 x 40 PSF, its point of symmetry.  radii_px
+ * [nrad] (0 <= nrad <= PSFR_EE_MAX_RADII), fracs [nfrac] (0 <= nfrac <= PSFR_EE_MAX_FRACTIONS); out
+ * [nimg][nrad + 1 + nfrac].  Image sizes, host / device handling and refusals as psfr_moffat_fit. */
+PSFR_API int psfr_encircled_energy(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs, const double* centres,
+                                   int nrad, const double* radii_px, int nfrac, const double* fracs, double* out,
+                                   void* stream);
+
+/* The fused pipeline with the encircled energy of every image it returns.  field = 0: psfr_compute_groups (the
+ * field mean of the ndir directions of every draw), field != 0: psfr_compute_field (one PSF per direction);
+ * arguments and checks as those entry points.  out_efit / out_mean_efit as psfr_compute_field_shapes, in either
+ * mode.  out_ee [ndraw][P][nlam][nrad + 1 + nfrac] and out_mean_ee [ngroup][P][nlam][nrad + 1 + nfrac] (P = ndir
+ * with field, 1 without) are psfr_encircled_energy of the images in out_cube / out_mean about their default
+ * centre, bit for bit; each runs in the chunk of its images, right after their fits.  Every output may be NULL;
+ * the other outputs are those of psfr_compute_groups / psfr_compute_field_shapes, bit for bit. */
+PSFR_API int psfr_compute_energy(psfr_ctx* ctx, int field, int ndraw, const double* draws, int npos,
+                       const double* poslgs, int ndir, const double* dirs, int nlam, const double* lambda_nm,
+                       int ngroup, const int* group_end, int nrad, const double* radii_px, int nfrac,
+                       const double* fracs, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
+                       double* out_efit, double* out_mean_efit, double* out_ee, double* out_mean_ee, void* stream);
 
 /* Time-mean of ncube cubes + refit (psfrec.py:1104-1105). cubes [ncube][nlam][40][40]. */
 PSFR_API int psfr_mean_refit(psfr_ctx* ctx, int ncube, int nlam, const double* cubes,

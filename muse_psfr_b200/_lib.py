@@ -33,6 +33,16 @@ FIT_NPAR = 16
 (EFIT_ERR_PEAK, EFIT_ERR_Y0, EFIT_ERR_X0, EFIT_ERR_A_MAJOR, EFIT_ERR_A_MINOR, EFIT_ERR_PA, EFIT_ERR_N,
  EFIT_ERR_FWHM_MAJOR, EFIT_ERR_FWHM_MINOR, EFIT_ERR_AXIS_RATIO, EFIT_FLUX, EFIT_ERR_FLUX) = range(12, 24)
 EFIT_NPAR = 24
+# encircled-energy record (include/psfr.h): EE at nrad radii, TOTAL, then the radius at each of nfrac fractions
+EE_MAX_RADII = 64
+EE_MAX_FRACTIONS = 16
+
+
+def ee_slots(nrad, nfrac):
+    """(EE slice, TOTAL index, radius-at-fraction slice, record length) of an encircled-energy record."""
+    nrad, nfrac = int(nrad), int(nfrac)
+    return slice(0, nrad), nrad, slice(nrad + 1, nrad + 1 + nfrac), nrad + 1 + nfrac
+
 AO_DIM = 80
 PSF_DIM = 40
 
@@ -76,6 +86,9 @@ _SIGNATURES = {
     'psfr_compute_groups': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     'psfr_compute_field': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     'psfr_compute_field_shapes': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'psfr_encircled_energy': (_I, [_P, _I, _I, _I, _P, _P, _I, _P, _I, _P, _P, _P]),
+    'psfr_compute_energy': (_I, [_P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P,
+                                 _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     'psfr_mean_refit': (_I, [_P, _I, _I, _P, _P, _P, _P]),
     'psfr_polyfit': (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     'psfr_set_option': (_I, [_P, _I, _D]),
@@ -290,6 +303,29 @@ class Context:
             self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
             self._buf(params, nimg * EFIT_NPAR, 'params', True), stream))
 
+    def encircled_energy(self, nimg, ny, nx, imgs, radii_px, fracs, out, centres=None, stream=None):
+        """psfr_encircled_energy: ``out`` [nimg, len(radii_px) + 1 + len(fracs)]; ``centres`` [nimg, 2] (y0, x0)
+        in pixels or None for (ny // 2, nx // 2)."""
+        nimg, ny, nx = int(nimg), int(ny), int(nx)
+        rad, fr = f64(radii_px).ravel(), f64(fracs).ravel()
+        rec = ee_slots(rad.size, fr.size)[3]
+        self._check(self._lib.psfr_encircled_energy(
+            self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
+            self._buf(centres, 2 * nimg, 'centres'), rad.size, ptr(rad) if rad.size else None, fr.size,
+            ptr(fr) if fr.size else None, self._buf(out, nimg * rec, 'out', True), stream))
+
+    def compute_energy(self, field, draws, dirs, poslgs, lambda_nm, radii_px, fracs, group_end=None, out_cube=None,
+                       out_fit=None, out_mean=None, out_mean_fit=None, out_efit=None, out_mean_efit=None, out_ee=None,
+                       out_mean_ee=None, stream=None):
+        """psfr_compute_energy: ``compute_groups`` (``field`` false) or ``compute_field`` (``field`` true) with the
+        encircled-energy records of every returned image, ``out_ee`` [ndraw, P, nl, rec] and ``out_mean_ee``
+        [ngroup, P, nl, rec] (P = npos with ``field``, 1 without; rec = len(radii_px) + 1 + len(fracs)), and the
+        elliptical fits ``out_efit`` / ``out_mean_efit`` of ``compute_field``."""
+        rad, fr = f64(radii_px).ravel(), f64(fracs).ravel()
+        self._groups(self._lib.psfr_compute_energy, bool(field), draws, dirs, poslgs, lambda_nm, group_end, out_cube,
+                     out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit),
+                     energy=(rad, fr, out_ee, out_mean_ee))
+
     def compute_batch(self, draws, dirs, poslgs, lambda_nm, out_cube=None, out_fit=None, stream=None):
         if not hasattr(draws, 'data_ptr'):      # numpy / sequence; torch tensors pass through as buffers
             draws = f64(draws)
@@ -327,7 +363,7 @@ class Context:
                          out_cube, out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit))
 
     def _groups(self, fn, field, draws, dirs, poslgs, lambda_nm, group_end, out_cube, out_fit, out_mean,
-                out_mean_fit, stream, shapes=None):
+                out_mean_fit, stream, shapes=None, energy=None):
         if not hasattr(draws, 'data_ptr'):
             draws = f64(draws)
         if len(draws.shape) != 2 or draws.shape[1] != DRAW_NPAR:
@@ -338,14 +374,22 @@ class Context:
         nimg = lam.size * (dirs.shape[1] if field else 1)      # images per draw and per exposure
         img = nimg * PSF_DIM * PSF_DIM
         args = [self._handle(), nd, self._buf(draws, nd * DRAW_NPAR, 'draws'), poslgs.shape[1], ptr(poslgs),
-                dirs.shape[1], ptr(dirs), lam.size, ptr(lam), ng, gp,
-                self._buf(out_cube, nd * img, 'out_cube', True),
-                self._buf(out_fit, nd * nimg * FIT_NPAR, 'out_fit', True),
-                self._buf(out_mean, ng * img, 'out_mean', True),
-                self._buf(out_mean_fit, ng * nimg * FIT_NPAR, 'out_mean_fit', True)]
+                dirs.shape[1], ptr(dirs), lam.size, ptr(lam), ng, gp]
+        if energy is not None:
+            rad, fr = energy[0], energy[1]
+            args = args[:1] + [int(field)] + args[1:] + [rad.size, ptr(rad) if rad.size else None, fr.size,
+                                                         ptr(fr) if fr.size else None]
+        args += [self._buf(out_cube, nd * img, 'out_cube', True),
+                 self._buf(out_fit, nd * nimg * FIT_NPAR, 'out_fit', True),
+                 self._buf(out_mean, ng * img, 'out_mean', True),
+                 self._buf(out_mean_fit, ng * nimg * FIT_NPAR, 'out_mean_fit', True)]
         if shapes is not None:
             args += [self._buf(shapes[0], nd * nimg * EFIT_NPAR, 'out_efit', True),
                      self._buf(shapes[1], ng * nimg * EFIT_NPAR, 'out_mean_efit', True)]
+        if energy is not None:
+            rec = ee_slots(energy[0].size, energy[1].size)[3]
+            args += [self._buf(energy[2], nd * nimg * rec, 'out_ee', True),
+                     self._buf(energy[3], ng * nimg * rec, 'out_mean_ee', True)]
         self._check(fn(*args, stream))
 
     def mean_refit(self, ncube, nlam, cubes, out_mean=None, out_fit=None, stream=None):

@@ -259,6 +259,32 @@ static int upload_draws(Ctx* c, int ndraw, const double* draws, int ndir, cudaSt
     return PSFR_OK;
 }
 
+// Radii and fractions of an encircled-energy call: checked on the host (either side's arrays), then radii followed
+// by fractions to d_eepar, stream-ordered before the kernels that read them.
+static int upload_ee_params(Ctx* c, int nrad, const double* radii, int nfrac, const double* fracs, cudaStream_t s) {
+    if (nrad < 0 || nrad > PSFR_EE_MAX_RADII)
+        return set_error(c, PSFR_E_ARG, "nrad=%d outside [0, %d]", nrad, PSFR_EE_MAX_RADII);
+    if (nfrac < 0 || nfrac > PSFR_EE_MAX_FRACTIONS)
+        return set_error(c, PSFR_E_ARG, "nfrac=%d outside [0, %d]", nfrac, PSFR_EE_MAX_FRACTIONS);
+    if ((nrad && !radii) || (nfrac && !fracs)) return set_error(c, PSFR_E_ARG, "NULL radii or fractions");
+    std::vector<double> r, f;
+    int rc = small_to_host(c, r, radii, (size_t)nrad, s);
+    if (!rc) rc = small_to_host(c, f, fracs, (size_t)nfrac, s);
+    if (rc) return rc;
+    for (int k = 0; k < nrad; ++k)
+        if (!(std::isfinite(r[k]) && r[k] >= 0.0))
+            return set_error(c, PSFR_E_ARG, "radius %d is %g: radii must be finite and >= 0", k, r[k]);
+    for (int j = 0; j < nfrac; ++j)
+        if (!(f[j] > 0.0 && f[j] < 1.0))
+            return set_error(c, PSFR_E_ARG, "fraction %d is %g: fractions must lie in (0, 1)", j, f[j]);
+    c->ee_par = r;
+    c->ee_par.insert(c->ee_par.end(), f.begin(), f.end());
+    if (!c->ee_par.empty())
+        PSFR_CUDA(c, cudaMemcpyAsync(c->d_eepar, c->ee_par.data(), c->ee_par.size() * sizeof(double),
+                                     cudaMemcpyHostToDevice, s));
+    return PSFR_OK;
+}
+
 constexpr int kMaxHotEvents = 512;
 struct HotTimer {
     cudaEvent_t ev[2 * kMaxHotEvents];
@@ -289,7 +315,8 @@ static int hot_begin(Ctx* c) {
 static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs, int npos,
                      const double* poslgs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                      bool field, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
-                     double* out_efit, double* out_mean_efit, cudaStream_t s) {
+                     double* out_efit, double* out_mean_efit, int nrad, int nfrac, double* out_ee,
+                     double* out_mean_ee, cudaStream_t s) {
     PSFR_CUDA(c, cudaSetDevice(c->device));
     std::vector<double> lam;
     int rc = small_to_host(c, lam, lambda_nm, nlam > 0 ? nlam : 0, s);
@@ -309,15 +336,19 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     const size_t img = (size_t)kPSF * kPSF, imgs = (size_t)ppd * nlam, elems = imgs * img;
     const size_t fits = imgs * PSFR_FIT_NPAR;   // fit records per draw
     const size_t efits = imgs * PSFR_EFIT_NPAR;  // elliptical records per draw
+    const size_t ees = imgs * (size_t)(nrad + 1 + nfrac);   // encircled-energy values per draw
     const bool cube_dev = out_cube && is_device_ptr(out_cube);
     const bool fit_dev = out_fit && is_device_ptr(out_fit);
     const bool mean_dev = out_mean && is_device_ptr(out_mean);
     const bool mfit_dev = out_mean_fit && is_device_ptr(out_mean_fit);
     const bool efit_dev = out_efit && is_device_ptr(out_efit);
     const bool mefit_dev = out_mean_efit && is_device_ptr(out_mean_efit);
-    const bool means = out_mean || out_mean_fit || out_mean_efit;
+    const bool ee_dev = out_ee && is_device_ptr(out_ee);
+    const bool mee_dev = out_mean_ee && is_device_ptr(out_mean_ee);
+    const bool means = out_mean || out_mean_fit || out_mean_efit || out_mean_ee;
     const bool host_out = (out_cube && !cube_dev) || (out_fit && !fit_dev) || (out_mean && !mean_dev) ||
-                          (out_mean_fit && !mfit_dev) || (out_efit && !efit_dev) || (out_mean_efit && !mefit_dev);
+                          (out_mean_fit && !mfit_dev) || (out_efit && !efit_dev) || (out_mean_efit && !mefit_dev) ||
+                          (out_ee && !ee_dev) || (out_mean_ee && !mee_dev);
     int* seg_dev = reinterpret_cast<int*>(c->d_misc + misc_groups(c->max_planes));
     std::vector<int> seg;
     int g0 = 0;   // first exposure not finished in an earlier chunk
@@ -344,11 +375,14 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
         if ((out_fit || out_efit) && (rc = run_fit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, s))) break;
         double* efit = efit_dev ? out_efit + (size_t)d0 * efits : (b ? c->d_efit2 : c->d_efit);
         if (out_efit && (rc = run_efit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, efit, s))) break;
+        double* ee = ee_dev ? out_ee + (size_t)d0 * ees : c->d_ee[b];
+        if (out_ee && (rc = run_ee(c, nd * (int)imgs, kPSF, kPSF, conv, nullptr, nrad, nfrac, ee, s))) break;
         // exposures g0, g0 + 1, ... that have draws in [d0, d0 + nd): all but possibly the last end here
         int ndone = 0;
         double* mean = mean_dev ? out_mean + (size_t)g0 * elems : c->d_mean[b];
         double* mfit = mfit_dev ? out_mean_fit + (size_t)g0 * fits : c->d_mfit[b];
         double* mefit = mefit_dev ? out_mean_efit + (size_t)g0 * efits : c->d_mefit[b];
+        double* mee = mee_dev ? out_mean_ee + (size_t)g0 * ees : c->d_mee[b];
         if (means) {
             seg.clear();
             for (int g = g0; g < ngroup && (g == g0 || group_end[g - 1] < d0 + nd); ++g) {
@@ -366,6 +400,8 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
             if ((out_mean_fit || out_mean_efit) && ndone && (rc = run_fit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, s)))
                 break;
             if (out_mean_efit && ndone && (rc = run_efit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, mefit, s))) break;
+            if (out_mean_ee && ndone && (rc = run_ee(c, ndone * (int)imgs, kPSF, kPSF, mean, nullptr, nrad, nfrac, mee, s)))
+                break;
         }
         if (host_out) {
             cudaError_t e = cudaEventRecord(c->ev_done[b], s);
@@ -388,6 +424,12 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
             if (e == cudaSuccess && ndone && out_mean_efit && !mefit_dev)
                 e = cudaMemcpyAsync(out_mean_efit + (size_t)g0 * efits, mefit, (size_t)ndone * efits * sizeof(double),
                                     cudaMemcpyDefault, c->copy_stream);
+            if (e == cudaSuccess && out_ee && !ee_dev)
+                e = cudaMemcpyAsync(out_ee + (size_t)d0 * ees, ee, (size_t)nd * ees * sizeof(double), cudaMemcpyDefault,
+                                    c->copy_stream);
+            if (e == cudaSuccess && ndone && out_mean_ee && !mee_dev)
+                e = cudaMemcpyAsync(out_mean_ee + (size_t)g0 * ees, mee, (size_t)ndone * ees * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess) e = cudaEventRecord(c->ev_copied[b], c->copy_stream);
             if (e != cudaSuccess) {
                 rc = set_error(c, PSFR_E_CUDA, "result copy failed: %s", cudaGetErrorString(e));
@@ -408,7 +450,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 103; }
+int psfr_version(void) { return 104; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -423,6 +465,8 @@ void psfr_destroy(psfr_ctx* c) {
     cudaFree(c->d_twc); cudaFree(c->d_wsamp); cudaFree(c->d_wcol); cudaFree(c->d_kcol); cudaFree(c->d_xmap); cudaFree(c->d_khat_tt); cudaFree(c->d_khat_mu);
     cudaFree(c->d_cube3); cudaFree(c->d_fit2); cudaFree(c->d_carry); cudaFree(c->d_efit); cudaFree(c->d_efit2);
     for (int i = 0; i < 2; ++i) { cudaFree(c->d_mean[i]); cudaFree(c->d_mfit[i]); cudaFree(c->d_mefit[i]); }
+    for (int i = 0; i < 2; ++i) { cudaFree(c->d_ee[i]); cudaFree(c->d_mee[i]); }
+    cudaFree(c->d_eepar); cudaFree(c->d_eecen);
     cudaFree(c->d_dphi32); cudaFree(c->d_otf32); cudaFree(c->d_tw32); cudaFree(c->d_twg); cudaFree(c->d_twg32); cudaFree(c->d_p3); cudaFree(c->d_p2mask); cudaFree(c->d_csort); cudaFree(c->d_lorder); cudaFree(c->d_kaddr);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     for (int i = 0; i < 2; ++i) {
@@ -545,7 +589,11 @@ int psfr_create(int device, int dim, int max_planes, int max_lambda, psfr_ctx** 
         CK(dev_alloc(c, &c->d_mean[i], P * LM * kPSF * kPSF));
         CK(dev_alloc(c, &c->d_mfit[i], P * LM * PSFR_FIT_NPAR));
         CK(dev_alloc(c, &c->d_mefit[i], P * LM * PSFR_EFIT_NPAR));
+        CK(dev_alloc(c, &c->d_ee[i], P * LM * kEeMaxRecord));
+        CK(dev_alloc(c, &c->d_mee[i], P * LM * kEeMaxRecord));
     }
+    CK(dev_alloc(c, &c->d_eepar, (size_t)PSFR_EE_MAX_RADII + PSFR_EE_MAX_FRACTIONS));
+    CK(dev_alloc(c, &c->d_eecen, P * LM * 2));
     CKC(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; ++i) {
         CKC(cudaEventCreateWithFlags(&c->ev_done[i], cudaEventDisableTiming));
@@ -778,6 +826,47 @@ int psfr_moffat_fit_elliptical(psfr_ctx* c, int nimg, int ny, int nx, const doub
     return PSFR_OK;
 }
 
+int psfr_encircled_energy(psfr_ctx* c, int nimg, int ny, int nx, const double* imgs, const double* centres, int nrad,
+                          const double* radii_px, int nfrac, const double* fracs, double* out, void* stream) {
+    if (!c || !imgs || !out) return set_error(c, PSFR_E_ARG, "NULL argument");
+    if (nimg < 1 || ny < 3 || nx < 3) return set_error(c, PSFR_E_ARG, "nimg=%d ny=%d nx=%d", nimg, ny, nx);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s);
+    if (rc) return rc;
+    if (centres) {
+        std::vector<double> h;
+        if ((rc = small_to_host(c, h, centres, (size_t)nimg * 2, s))) return rc;
+        for (size_t i = 0; i < h.size(); ++i)
+            if (!std::isfinite(h[i]))
+                return set_error(c, PSFR_E_ARG, "centre of image %zu is not finite", i / 2);
+    }
+    const size_t cap = (size_t)c->max_planes * c->max_lambda;
+    const size_t per = (size_t)ny * nx, rec = (size_t)nrad + 1 + nfrac;
+    const bool in_dev = is_device_ptr(imgs), out_dev = is_device_ptr(out);
+    const bool cen_dev = centres && is_device_ptr(centres);
+    // host images, centres and records go through d_cube, d_eecen and d_ee[0]: each holds cap images' worth
+    const size_t chunk_imgs = std::min(cap, (cap * kPSF * kPSF) / per);
+    if (chunk_imgs < 1) return set_error(c, PSFR_E_CAPACITY, "image %dx%d does not fit the staging buffer", ny, nx);
+    for (size_t i0 = 0; i0 < (size_t)nimg; i0 += chunk_imgs) {
+        const int n = (int)std::min(chunk_imgs, (size_t)nimg - i0);
+        const double* src = imgs + i0 * per;
+        if (!in_dev) {
+            if ((rc = to_device(c, c->d_cube, src, (size_t)n * per * sizeof(double), s))) return rc;
+            src = c->d_cube;
+        }
+        const double* cen = centres ? centres + 2 * i0 : nullptr;
+        if (centres && !cen_dev) {
+            if ((rc = to_device(c, c->d_eecen, cen, (size_t)n * 2 * sizeof(double), s))) return rc;
+            cen = c->d_eecen;
+        }
+        double* dst = out_dev ? out + i0 * rec : c->d_ee[0];
+        if ((rc = run_ee(c, n, ny, nx, src, cen, nrad, nfrac, dst, s))) return rc;
+        if (!out_dev && (rc = from_device(c, out + i0 * rec, dst, (size_t)n * rec * sizeof(double), s))) return rc;
+    }
+    return PSFR_OK;
+}
+
 int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs,
                        const double* poslgs, int nlam, const double* lambda_nm, double* out_cube,
                        double* out_fit, void* stream) {
@@ -786,7 +875,8 @@ int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, co
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d ndir=%d max_planes=%d", ndraw, ndir, c->max_planes);
     if (ngs < 1) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
     return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, false, out_cube,
-                     out_fit, nullptr, nullptr, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+                     out_fit, nullptr, nullptr, nullptr, nullptr, 0, 0, nullptr, nullptr,
+                     static_cast<cudaStream_t>(stream));
 }
 
 // the arguments of psfr_compute_groups and psfr_compute_field that run_batch does not check itself
@@ -813,7 +903,8 @@ int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, c
     if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean || out_mean_fit))
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, false,
-                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, 0, 0, nullptr, nullptr,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
@@ -822,7 +913,8 @@ int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, co
     if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean || out_mean_fit))
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
-                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, 0, 0, nullptr, nullptr,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field_shapes(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
@@ -833,8 +925,24 @@ int psfr_compute_field_shapes(psfr_ctx* c, int ndraw, const double* draws, int n
                               out_mean || out_mean_fit || out_mean_efit))
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
-                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit,
+                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, 0, 0, nullptr, nullptr,
                      static_cast<cudaStream_t>(stream));
+}
+
+int psfr_compute_energy(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs,
+                        int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                        int nrad, const double* radii_px, int nfrac, const double* fracs, double* out_cube,
+                        double* out_fit, double* out_mean, double* out_mean_fit, double* out_efit,
+                        double* out_mean_efit, double* out_ee, double* out_mean_ee, void* stream) {
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
+                              out_mean || out_mean_fit || out_mean_efit || out_mean_ee))
+        return rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
+                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
+                     out_mean_ee, s);
 }
 
 int psfr_mean_refit(psfr_ctx* c, int ncube, int nlam, const double* cubes, double* out_mean, double* out_fit,

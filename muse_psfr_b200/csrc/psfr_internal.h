@@ -65,6 +65,7 @@ constexpr int kKW = 41;                 // Moffat kernel width
 constexpr int kMaxGS = 4;
 constexpr int kMaxDir = 256;            // field directions per draw
 constexpr int kMaxLambdaCap = 4096;
+constexpr int kEeMaxRecord = PSFR_EE_MAX_RADII + 1 + PSFR_EE_MAX_FRACTIONS;   // doubles per EE record, at most
 
 // layout of the small scratch array d_misc (doubles)
 constexpr int kMiscDirs = 0;            // [2][ndir]
@@ -146,6 +147,11 @@ struct Ctx {
     double* d_efit = nullptr;    // [max_planes*max_lambda][PSFR_EFIT_NPAR] elliptical records (double-buffered
     double* d_efit2 = nullptr;   // with d_efit2 as d_fit / d_fit2)
     double* d_mefit[2] = {nullptr, nullptr};  // [max_planes*max_lambda][PSFR_EFIT_NPAR] elliptical fits of the means
+    double* d_ee[2] = {nullptr, nullptr};     // [max_planes*max_lambda][kEeMaxRecord] encircled-energy records
+    double* d_mee[2] = {nullptr, nullptr};    // the same for the exposure means (double-buffered as d_mean)
+    double* d_eepar = nullptr;   // [PSFR_EE_MAX_RADII + PSFR_EE_MAX_FRACTIONS] radii then fractions of the call
+    double* d_eecen = nullptr;   // [max_planes*max_lambda][2] staging for host centres (psfr_encircled_energy)
+    std::vector<double> ee_par;  // host copy of d_eepar's contents (outlives the asynchronous upload)
     cudaStream_t copy_stream = nullptr;      // device -> host copies of finished chunks
     cudaEvent_t ev_done[2] = {nullptr, nullptr};    // chunk results ready (compute stream)
     cudaEvent_t ev_copied[2] = {nullptr, nullptr};  // chunk results copied out (copy stream)
@@ -254,6 +260,10 @@ int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit
 // elliptical fit of every image from its circular record circ_dev [nimg][PSFR_FIT_NPAR]
 int run_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* circ_dev, double* efit_dev,
              cudaStream_t s);
+// psfr_energy.cu: encircled-energy record [nimg][nrad + 1 + nfrac] of every image, radii and fractions from
+// d_eepar, centres_dev [nimg][2] (row, column) or nullptr for (ny / 2, nx / 2)
+int run_ee(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* centres_dev, int nrad, int nfrac,
+           double* out_dev, cudaStream_t s);
 // out = (running sum of the cubes) ; first: start from zero, last: divide by ntotal
 int run_mean(Ctx* c, int ncube, int plane_elems, const double* cubes_dev, double* out_dev,
              cudaStream_t s, bool first, bool last, int ntotal);

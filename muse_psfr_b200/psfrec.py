@@ -17,7 +17,7 @@ from ._lib import PsfrError
 
 __all__ = ['compute_psf_from_sparta', 'compute_psf_from_sparta_batch', 'compute_psf', 'compute_psf_batch',
            'reconstruct_psf', 'create_sparta_table', 'fit_psf_with_polynom', 'simul_psd_wfm', 'psd_to_psf', 'psf_muse',
-           'convolve_final_psf', 'fit_psf_cube', 'compute_psf_field',
+           'convolve_final_psf', 'fit_psf_cube', 'compute_psf_field', 'encircled_energy',
            'muse_intrinsic_psf', 'direction_perf', 'seeing2r01', 'pupil_mask', 'select_sparta_rows', 'FitTable',
            'PsfrError', 'MIN_L0', 'MAX_L0']
 
@@ -31,6 +31,7 @@ _WIND_DIR = np.array([0.628163, -0.326497])      # psfrec.py:66
 _DIM = 1280                                      # psfrec.py:955 (compute_psf's fixed grid)
 _DIMS = (1280, 2560)                             # grids the CUDA library is built for
 _MAX_POSITIONS = 256                             # directions per draw the library takes (kMaxDir)
+_PIXSCALE = 0.2                                  # arcsec per pixel of the 40 x 40 PSFs (psfrec.py:901)
 _CONTEXTS = {}
 _DEFAULT_DEVICE = [None]
 
@@ -321,6 +322,40 @@ def _shape_table_from_fit(lbda, efit, pixscale=0.2):
     })
 
 
+def _ee_params(radii, fractions, pixscale=_PIXSCALE):
+    """Radii [arcsec] and fractions of an encircled-energy request, checked, as (radii [px], fractions)."""
+    rad = np.array(radii, dtype=float, ndmin=1)
+    frac = np.array(fractions, dtype=float, ndmin=1)
+    if rad.ndim != 1 or frac.ndim != 1:
+        raise ValueError('radii and fractions must be 1-D sequences')
+    if rad.size > _lib.EE_MAX_RADII or frac.size > _lib.EE_MAX_FRACTIONS:
+        raise ValueError('at most %d radii and %d fractions (got %d and %d)'
+                         % (_lib.EE_MAX_RADII, _lib.EE_MAX_FRACTIONS, rad.size, frac.size))
+    if not np.all(np.isfinite(rad)) or np.any(rad < 0):
+        raise ValueError('radii must be finite and >= 0 (got %s)' % rad.tolist())
+    if not np.all((frac > 0) & (frac < 1)):
+        raise ValueError('fractions must lie in (0, 1) (got %s)' % frac.tolist())
+    if not (np.isfinite(pixscale) and pixscale > 0):
+        raise ValueError('pixscale must be positive')
+    return np.ascontiguousarray(rad / pixscale), np.ascontiguousarray(frac)
+
+
+def _ee_table(lbda, ee, radii, fractions, pixscale=_PIXSCALE):
+    """Columns of the encircled-energy table for records [n, nrad + 1 + nfrac] (``_lib.ee_slots``): ``ee``
+    [n, nrad] (flux inside each radius, in the images' units), ``ee_total`` (the sum of each image), ``r_ee``
+    [n, nfrac] in arcsec.  ``radii`` [arcsec] and ``fractions`` go to the meta."""
+    radii = np.array(radii, dtype=float, ndmin=1)
+    fractions = np.array(fractions, dtype=float, ndmin=1)
+    sl_ee, i_tot, sl_r, rec = _lib.ee_slots(radii.size, fractions.size)
+    ee = np.asarray(ee).reshape(-1, rec)
+    return FitTable({
+        'lbda': np.asarray(lbda, dtype=float),
+        'ee': ee[:, sl_ee].copy(),
+        'ee_total': ee[:, i_tot].copy(),
+        'r_ee': ee[:, sl_r] * pixscale,
+    }, meta={'radii': radii, 'fractions': fractions})
+
+
 # --------------------------------------------------------------------------- reference API
 def simul_psd_wfm(Cn2, h, seeing, L0, zenith=0., plot=False, npsflin=1, dim=1280,
                   three_lgs_mode=False, verbose=True, wind_dir=None):
@@ -438,6 +473,43 @@ def fit_psf_cube(lbda, psfcube, circular=True):
     return _table_from_fit(lam, fit)
 
 
+def encircled_energy(lbda, psfcube, radii, fractions=(0.5, 0.8), center=None, pixscale=_PIXSCALE):
+    """Encircled energy of each plane of ``psfcube`` [nl, ny, nx] on the device (DESIGN.md section 5.4).
+
+    Pixel (p, q) is the unit square about (p, q) with its value spread uniformly over it, and EE(r) is the sum
+    of every pixel times the exact area of its overlap with the disc of radius r: no supersampling, no
+    renormalisation (the flux inside the aperture in the cube's own units).  ``radii`` and the returned radii are
+    in arcsec at ``pixscale`` arcsec per pixel.  ``center`` is (y0, x0) in pixels (row, column; pixel centres at
+    integers) for every plane or [nl, 2] per plane; the default (ny // 2, nx // 2) is pixel (20, 20) of a 40 x 40
+    PSF of this package, its point of symmetry.  The image stops 19.5 px beyond that centre on its high side, so a
+    larger circle is clipped by the edge.
+
+    Returns a ``FitTable`` with ``lbda``, ``ee`` [nl, nrad], ``ee_total`` (the sum of the plane) and ``r_ee`` [nl,
+    nfrac], the smallest radius holding each fraction of ``ee_total`` (NaN where ``ee_total`` <= 0); its meta
+    holds the radii and fractions.  Invalid radii, fractions or centres raise ValueError before any device call."""
+    data = getattr(psfcube, 'data', psfcube)
+    data = np.ascontiguousarray(np.ma.getdata(data), dtype=np.float64)
+    if data.ndim != 3:
+        raise ValueError('psfcube must be [nl, ny, nx]')
+    lam = np.atleast_1d(np.asarray(lbda, dtype=float))
+    nimg, ny, nx = data.shape
+    rad_px, frac = _ee_params(radii, fractions, pixscale)
+    cen = None
+    if center is not None:
+        cen = np.array(center, dtype=float)
+        if cen.shape == (2,):
+            cen = np.tile(cen, (nimg, 1))
+        if cen.shape != (nimg, 2):
+            raise ValueError('center must be (y0, x0) or [nl, 2] (got shape %s)' % (cen.shape,))
+        if not np.all(np.isfinite(cen)):
+            raise ValueError('center must be finite')
+        cen = np.ascontiguousarray(cen)
+    ee = np.empty((nimg, _lib.ee_slots(rad_px.size, frac.size)[3]))
+    if nimg:
+        get_context().encircled_energy(nimg, ny, nx, data, rad_px, frac, ee, centres=cen)
+    return _ee_table(lam, ee, rad_px * pixscale, frac, pixscale)
+
+
 def compute_psf(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs_mode=False, verbose=True,
                 dim=_DIM, zenith=0., Cn2=None, wind_dir=None):
     """Reconstruct a PSF from seeing, GL and L0 (psfrec.py:933-978): returns (table, psf).
@@ -525,13 +597,19 @@ def _planes_context(nd, ndir, nlam, max_planes, device, dim):
 
 def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs_mode=False,
                       out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None, stream=None,
-                      dim=_DIM, zenith=0., Cn2=None, wind_dir=None):
+                      dim=_DIM, zenith=0., Cn2=None, wind_dir=None, ee_radii=None, ee_fractions=(0.5, 0.8)):
     """Batched ``compute_psf``: one fused device pipeline for many (seeing, GL, L0[, h]) draws.
 
     ``h`` is one (h0, h1) pair or an array [ndraw, 2].  ``three_lgs_mode`` is one flag for all draws or
     one per draw; each draw gives the same bits as in a call of its own mode.  Returns (fit [ndraw, nl,
     FIT_NPAR], cube [ndraw, nl, 40, 40]); ``out_cube`` / ``out_fit`` may be preallocated numpy arrays or
-    torch tensors (host-pinned or device) used as plain buffers."""
+    torch tensors (host-pinned or device) used as plain buffers.
+
+    ``ee_radii`` [arcsec] adds the encircled energy of every returned PSF about its centre pixel (20, 20),
+    computed on the device right after its fit (``encircled_energy``): the result gains a third entry, the raw
+    records [ndraw, nl, nrad + 1 + nfrac] in pixels (``_lib.ee_slots``; ``_ee_table`` turns them into the
+    columns of ``encircled_energy``), for the fractions ``ee_fractions``.  With ``want_cube=False`` no cube leaves
+    the device.  fit and cube are those of a call without ``ee_radii``, bit for bit."""
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
     seeing, GL, L0 = (np.atleast_1d(np.asarray(v, dtype=float)) for v in (seeing, GL, L0))
     nd = seeing.size
@@ -540,14 +618,21 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     per_draw = np.ndim(three_lgs_mode) > 0
     if per_draw:
         three = _mode_flags(three_lgs_mode, nd)
+    energy = ee_radii is not None
+    if energy:
+        rad_px, frac = _ee_params(ee_radii, ee_fractions)
+        ee = np.empty((nd, lam.size, _lib.ee_slots(rad_px.size, frac.size)[3]))
     if nd == 0 or lam.size == 0:
         # nothing to compute: empty results of the right shape, written through nothing
-        return (np.empty((nd, lam.size, _lib.FIT_NPAR)),
-                np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
+        empty = (np.empty((nd, lam.size, _lib.FIT_NPAR)),
+                 np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
+        return empty + (ee,) if energy else empty
     if per_draw:
         recs = _mode_records(three, seeing, GL, L0, h, zenith, Cn2, wind_dir)
     else:
         recs = _batch_records(seeing, GL, L0, h, zenith, Cn2, wind_dir)
+        if energy:      # the groups path takes each draw's guide-star count from its record
+            recs[:, _lib.DRAW_NGS] = 3 if three_lgs_mode else 4
     dirs = direction_perf(npsflin)
     dim = _check_dim(dim)
     ctx = _planes_context(nd, dirs.shape[1], lam.size, max_planes, device, dim)
@@ -556,7 +641,10 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        if per_draw:    # the three-laser asterism is the first three stars of the four-laser one
+        if energy:
+            ctx.compute_energy(False, recs, dirs, _lgs_positions(False), lam, rad_px, frac, out_cube=out_cube,
+                               out_fit=out_fit, out_ee=ee, stream=stream)
+        elif per_draw:    # the three-laser asterism is the first three stars of the four-laser one
             ctx.compute_groups(recs, dirs, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit,
                                stream=stream)
         else:
@@ -566,12 +654,13 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
         raise
-    return out_fit, out_cube
+    return (out_fit, out_cube, ee) if energy else (out_fit, out_cube)
 
 
 def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_size=60, h=(100, 10000),
                       three_lgs_mode=False, out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None,
-                      stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None, elliptical=False):
+                      stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None, elliptical=False, ee_radii=None,
+                      ee_fractions=(0.5, 0.8)):
     """Field-resolved ``compute_psf_batch``: the PSF of every draw at every field position instead of
     their average.
 
@@ -586,7 +675,10 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
 
     ``elliptical=True`` also fits an elliptical Moffat to every PSF on the device, right after its circular fit
     and from it, and returns (fit, cube, efit) with efit [ndraw, npos, nl, EFIT_NPAR] (``_lib.EFIT_*``); fit and
-    cube are those of a call without it, bit for bit."""
+    cube are those of a call without it, bit for bit.
+
+    ``ee_radii`` [arcsec] appends the encircled-energy records [ndraw, npos, nl, nrad + 1 + nfrac] of every PSF, in
+    pixels, as ``compute_psf_batch(ee_radii=...)`` does, after ``efit`` where present."""
     pos = _field_positions(direction_perf(npsflin, field_size) if positions is None else positions)
     npos = pos.shape[1]
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
@@ -596,10 +688,14 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
         raise ValueError('seeing, GL and L0 must have one entry per draw (got %d, %d, %d)' % (nd, GL.size, L0.size))
     three = _mode_flags(three_lgs_mode, nd)
     efit = np.empty((nd, npos, lam.size, _lib.EFIT_NPAR)) if elliptical else None
+    energy = ee_radii is not None
+    if energy:
+        rad_px, frac = _ee_params(ee_radii, ee_fractions)
+        ee = np.empty((nd, npos, lam.size, _lib.ee_slots(rad_px.size, frac.size)[3]))
+    extra = ((efit,) if elliptical else ()) + ((ee,) if energy else ())
     if nd == 0 or lam.size == 0:
-        empty = (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
-                 np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
-        return empty + (efit,) if elliptical else empty
+        return (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
+                np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None) + extra
     # the records compute_psf_batch builds in either laser mode; the three-laser asterism is the first three
     # stars of the four-laser one
     recs = _mode_records(three, seeing, GL, L0, h, zenith, Cn2, wind_dir)
@@ -610,13 +706,17 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        ctx.compute_field(recs, pos, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit, stream=stream,
-                          out_efit=efit)
+        if energy:
+            ctx.compute_energy(True, recs, pos, _lgs_positions(False), lam, rad_px, frac, out_cube=out_cube,
+                               out_fit=out_fit, out_efit=efit, out_ee=ee, stream=stream)
+        else:
+            ctx.compute_field(recs, pos, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit,
+                              stream=stream, out_efit=efit)
     except PsfrError as exc:
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
         raise
-    return (out_fit, out_cube, efit) if elliptical else (out_fit, out_cube)
+    return (out_fit, out_cube) + extra
 
 
 def _norm_lbda(lbda, lb1, lb2):
@@ -692,9 +792,25 @@ def _shape_columns(lam, efit):
     return {k: tab[k] for k in tab.colnames}
 
 
+def _ee_columns(lam, ee, radii, fractions):
+    """Columns of the encircled-energy table for records [n, nl, nrad + 1 + nfrac] (flattened)."""
+    ee = np.asarray(ee).reshape(-1, _lib.ee_slots(len(radii), len(fractions))[3])
+    tab = _ee_table(np.tile(lam, len(ee) // lam.size), ee, radii, fractions)
+    return {k: tab[k] for k in tab.colnames}
+
+
+def _ee_cards(meta, radii, fractions):
+    """``meta`` plus one card per radius [arcsec] (EERADk) and per fraction (EEFRACk), k from 1."""
+    cards = dict(meta)
+    cards.update({'EERAD%d' % (k + 1): float(r) for k, r in enumerate(radii)})
+    cards.update({'EEFRAC%d' % (j + 1): float(f) for j, f in enumerate(fractions)})
+    return cards
+
+
 def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                             lbda=None, h=(100, 10000), n_jobs=-1, plot=False, mean_of_lgs=True,
-                            verbose=True, device=None, field_positions=None, elliptical=False):
+                            verbose=True, device=None, field_positions=None, elliptical=False, ee_radii=None,
+                            ee_fractions=(0.5, 0.8)):
     """Reconstruct a PSF from SPARTA data (psfrec.py:981-1120).
 
     ``filename``: path of a FITS file, a binary file object, or an HDUList (this package's or
@@ -703,18 +819,21 @@ def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin
     ``n_jobs`` is accepted and only reported).  Returns an HDUList [PRIMARY, <extname>, FIT_ROWS,
     FIT_MEAN, PSF_MEAN] - an ``astropy.io.fits.HDUList`` when astropy is installed, otherwise
     the equivalent object of ``muse_psfr_b200._fits`` - or None when no row is valid.  With
-    ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow, and with ``elliptical=True``
-    SHAPE_MEAN (and SHAPE_FIELD): see ``compute_psf_from_sparta_batch``."""
+    ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow, with ``elliptical=True``
+    SHAPE_MEAN (and SHAPE_FIELD), and with ``ee_radii`` EE_MEAN (and EE_FIELD): see
+    ``compute_psf_from_sparta_batch``."""
     if plot:
         raise NotImplementedError('plotting is outside the B200 hot path')
     return compute_psf_from_sparta_batch([filename], extname=extname, npsflin=npsflin, lmin=lmin, lmax=lmax, nl=nl,
                                          lbda=lbda, h=h, n_jobs=n_jobs, mean_of_lgs=mean_of_lgs, verbose=verbose,
-                                         device=device, field_positions=field_positions, elliptical=elliptical)[0]
+                                         device=device, field_positions=field_positions, elliptical=elliptical,
+                                         ee_radii=ee_radii, ee_fractions=ee_fractions)[0]
 
 
 def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                                   lbda=None, h=(100, 10000), n_jobs=-1, mean_of_lgs=True, verbose=True,
-                                  device=None, max_planes=None, field_positions=None, elliptical=False):
+                                  device=None, max_planes=None, field_positions=None, elliptical=False,
+                                  ee_radii=None, ee_fractions=(0.5, 0.8)):
     """``compute_psf_from_sparta`` for many exposures in one device pass: returns one entry per source,
     the HDUList ``compute_psf_from_sparta(source, ...)`` returns, bit for bit, or None for a table
     without a valid row.
@@ -734,11 +853,22 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     ``elliptical=True`` appends SHAPE_MEAN, the elliptical fit table (``fit_psf_cube(circular=False)``
     columns) of PSF_MEAN with the cards of FIT_MEAN, and with ``field_positions`` SHAPE_FIELD, the same
     columns plus ``x`` and ``y`` for the PSFs of PSF_FIELD, position-major.  Every HDU before them is that of
-    a call without ``elliptical``, bit for bit."""
+    a call without ``elliptical``, bit for bit.
+
+    ``ee_radii`` [arcsec] appends EE_MEAN, the ``encircled_energy`` table of PSF_MEAN (radii ``ee_radii``, fractions
+    ``ee_fractions``) with the cards of FIT_MEAN plus EERADk / EEFRACk, and with ``field_positions`` EE_FIELD, the
+    same columns plus ``x`` and ``y`` for the PSFs of PSF_FIELD, position-major.  Both are computed on the device
+    in the passes that form the means, and follow the SHAPE_* HDUs; every HDU before them is that of a call
+    without ``ee_radii``, bit for bit."""
     if lbda is None:
         lbda = np.linspace(lmin, lmax, nl)
     lbda = np.atleast_1d(np.asarray(lbda, dtype=float))
     pos = None if field_positions is None else _field_positions(field_positions)
+    energy = ee_radii is not None
+    if energy:
+        rad_px, frac = _ee_params(ee_radii, ee_fractions)
+        ee_rec = _lib.ee_slots(rad_px.size, frac.size)[3]
+        ee_rad = rad_px * _PIXSCALE
     files, recs = [], []
     for source in sources:
         hdul = _fits.from_any(source, only={extname.upper()})
@@ -774,16 +904,27 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     dirs = direction_perf(npsflin)
     ctx = _planes_context(nd, dirs.shape[1], nlam, max_planes, device, _DIM)
     try:
-        ctx.compute_groups(draws, dirs, _lgs_positions(False), lbda, group_end, out_fit=fit, out_mean=psftot,
-                           out_mean_fit=fit_mean)
+        if energy:
+            ee_mean = np.empty((ng, nlam, ee_rec))
+            ctx.compute_energy(False, draws, dirs, _lgs_positions(False), lbda, rad_px, frac, group_end, out_fit=fit,
+                               out_mean=psftot, out_mean_fit=fit_mean, out_mean_ee=ee_mean)
+        else:
+            ctx.compute_groups(draws, dirs, _lgs_positions(False), lbda, group_end, out_fit=fit, out_mean=psftot,
+                               out_mean_fit=fit_mean)
         if pos is not None:
             npos = pos.shape[1]
             psf_field = np.empty((ng, npos, nlam, _lib.PSF_DIM, _lib.PSF_DIM))
             fit_field = np.empty((ng, npos, nlam, _lib.FIT_NPAR))
             ctx = _planes_context(nd, npos, nlam, max_planes, device, _DIM)
             shape_field = np.empty((ng, npos, nlam, _lib.EFIT_NPAR)) if elliptical else None
-            ctx.compute_field(draws, pos, _lgs_positions(False), lbda, group_end, out_mean=psf_field,
-                              out_mean_fit=fit_field, out_mean_efit=shape_field)
+            if energy:
+                ee_field = np.empty((ng, npos, nlam, ee_rec))
+                ctx.compute_energy(True, draws, pos, _lgs_positions(False), lbda, rad_px, frac, group_end,
+                                   out_mean=psf_field, out_mean_fit=fit_field, out_mean_efit=shape_field,
+                                   out_mean_ee=ee_field)
+            else:
+                ctx.compute_field(draws, pos, _lgs_positions(False), lbda, group_end, out_mean=psf_field,
+                                  out_mean_fit=fit_field, out_mean_efit=shape_field)
         if elliptical:      # the time means are on the host already: one standalone fit of all of them
             shape_mean = np.empty((ng, nlam, _lib.EFIT_NPAR))
             ctx.moffat_fit_elliptical(ng * nlam, _lib.PSF_DIM, _lib.PSF_DIM, psftot, shape_mean)
@@ -827,6 +968,14 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
                 cols['x'] = np.repeat(pos[0], nlam)
                 cols['y'] = np.repeat(pos[1], nlam)
                 out.append(_fits.table_to_hdu(cols, meta=meta, name='SHAPE_FIELD'))
+        if energy:
+            cards = _ee_cards(meta, ee_rad, frac)
+            out.append(_fits.table_to_hdu(_ee_columns(lbda, ee_mean[g], ee_rad, frac), meta=cards, name='EE_MEAN'))
+            if pos is not None:
+                cols = _ee_columns(lbda, ee_field[g], ee_rad, frac)
+                cols['x'] = np.repeat(pos[0], nlam)
+                cols['y'] = np.repeat(pos[1], nlam)
+                out.append(_fits.table_to_hdu(cols, meta=cards, name='EE_FIELD'))
         try:
             results.append(_fits.to_astropy(out))
         except ImportError:
