@@ -124,8 +124,10 @@ enum {
 /*  [0, nrad)              EE(radii[k])
  *  [nrad]                 TOTAL = sum img, summed in the order of the EE sums (EE == TOTAL bit for bit once the
  *                         circle contains every pixel)
- *  [nrad + 1 + j]         the smallest r >= 0 with EE(r) >= fracs[j] * TOTAL [px], to a bracket of 1e-10 px;
- *                         NaN when TOTAL <= 0 (or NaN)
+ *  [nrad + 1 + j]         r_q [px] for q = fracs[j], to a bracket of 1e-10 px; NaN when TOTAL <= 0 (or NaN).
+ *                         Without negative pixels, the smallest r >= 0 with EE(r) >= q TOTAL; with them, an r
+ *                         where EE crosses q TOTAL from below: EE(r) >= q TOTAL > EE(r') for an r' less than
+ *                         1e-10 px below r
  * Radii must be finite and >= 0, fractions in (0, 1), centres finite; otherwise PSFR_E_ARG, nothing written. */
 
 /* Context ------------------------------------------------------------------------- */

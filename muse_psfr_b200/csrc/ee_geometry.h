@@ -109,4 +109,30 @@ EE_HD void pixel_dist2(double dy, double dx, double* near2, double* far2) {
     *far2 = (ay + 0.5) * (ay + 0.5) + (ax + 0.5) * (ax + 0.5);
 }
 
+// Rows [*p0, *p1) of an image of ny rows that the disc of radius r about row y0 can reach: row p spans
+// [p - 1/2, p + 1/2], so it is reached when y0 - r - 1/2 <= p <= y0 + r + 1/2; the window keeps a row of margin
+// on each side against rounding.  Both ends are clamped to [0, ny] in double before the conversion to int, so a
+// centre far outside the image gives an empty window (*p0 >= *p1) and nothing overflows; r may be +inf.
+EE_HD void row_window(double y0, double r, int ny, int* p0, int* p1) {
+    *p0 = (int)fmin(fmax(0.0, floor(y0 - r - 0.5)), (double)ny);
+    *p1 = (int)fmax(0.0, fmin((double)ny, ceil(y0 + r + 0.5) + 1.0));
+}
+
+// Starting bracket of the radius at which EE reaches target > 0, from n tabulated radii r[k] with e[k] = EE(r[k])
+// and the farthest pixel corner rmax, where EE = total >= target: *hi is the smallest tabulated radius with
+// EE >= target (rmax if there is none), *lo the largest tabulated radius below *hi with EE < target (0 if there is
+// none, where EE = 0).  So lo < hi and EE(lo) < target <= EE(hi) also where EE falls (negative pixels), and the
+// bracket does not depend on the order of the radii.
+EE_HD void fraction_bracket(const double* r, const double* e, int n, double target, double rmax, double total,
+                            double* lo, double* elo, double* hi, double* ehi) {
+    *hi = rmax;
+    *ehi = total;
+    for (int k = 0; k < n; ++k)
+        if (e[k] >= target && r[k] < *hi) { *hi = r[k]; *ehi = e[k]; }
+    *lo = 0.0;
+    *elo = 0.0;
+    for (int k = 0; k < n; ++k)
+        if (e[k] < target && r[k] < *hi && r[k] > *lo) { *lo = r[k]; *elo = e[k]; }
+}
+
 }  // namespace ee

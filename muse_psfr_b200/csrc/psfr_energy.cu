@@ -30,7 +30,8 @@ __device__ __forceinline__ double ee_eval(const double* img, unsigned short* lst
     const int lane = threadIdx.x & 31;
     const unsigned lt = (1u << lane) - 1u;
     const double r2 = r * r;
-    const int p0 = (int)fmax(0.0, floor(y0 - r - 0.5)), p1 = (int)fmin((double)ny, ceil(y0 + r + 0.5) + 1.0);
+    int p0, p1;
+    ee::row_window(y0, r, ny, &p0, &p1);
     const int i0 = p0 * nx, i1 = p1 * nx;
     double t = 0.0;
     int nst = 0;
@@ -107,20 +108,17 @@ ee_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, const doubl
         // farthest pixel corner: EE there is TOTAL, bit for bit
         const double fy = fmax(y0 + 0.5, ny - 0.5 - y0), fx = fmax(x0 + 0.5, nx - 0.5 - x0);
         const double rmax = sqrt(fy * fy + fx * fx);
-        // smallest r with EE(r) >= frac * TOTAL.  The bracket [lo, hi] keeps EE(lo) < target <= EE(hi); it starts
-        // from the tabulated radii, and the first trial point interpolates inside it.  Newton steps inside the
-        // bracket, bisection when Newton leaves it or does not halve the step of two iterations back, and a step
-        // of tol / 2 across the root once Newton's steps are that small, which closes the bracket.
+        // r where EE crosses frac * TOTAL from below (the smallest such r when no pixel is negative).  The bracket
+        // [lo, hi] keeps EE(lo) < target <= EE(hi); it starts from the tabulated radii, and the first trial point
+        // interpolates inside it.  Newton steps inside the bracket, bisection when Newton leaves it or does not
+        // halve the step of two iterations back, and a step of tol / 2 across the root once Newton's steps are
+        // that small, which closes the bracket.
         for (int j = 0; j < nfrac; ++j) {
             double res = CUDART_NAN;
             if (total > 0.0) {
                 const double target = par[nrad + j] * total;
-                double lo = 0.0, hi = rmax, elo = 0.0, ehi = total;
-                for (int k = 0; k < nrad; ++k) {
-                    const double rk = par[k], ek = o[k];
-                    if (ek < target) { if (rk > lo) { lo = rk; elo = ek; } }
-                    else if (rk < hi) { hi = rk; ehi = ek; }
-                }
+                double lo, hi, elo, ehi;
+                ee::fraction_bracket(par, o, nrad, target, rmax, total, &lo, &elo, &hi, &ehi);
                 double x = lo + (target - elo) / (ehi - elo) * (hi - lo);
                 if (!(x > lo && x < hi)) x = 0.5 * (lo + hi);
                 double dx = hi - lo, dxold = dx;

@@ -180,20 +180,31 @@ struct Ctx {
 
 int set_error(Ctx* c, int code, const char* fmt, ...);
 
-// raise cudaFuncAttributeMaxDynamicSharedMemorySize of `func` to `bytes` once per context
+// Raise cudaFuncAttributeMaxDynamicSharedMemorySize of `func` to at least `bytes`, never lower it.  The attribute
+// belongs to the function on the device, shared by every context of the process, so lowering it would break a
+// context that cached a larger value.
+template <class F>
+inline cudaError_t raise_dynamic_smem(F* func, size_t bytes) {
+    cudaFuncAttributes a;
+    cudaError_t e = cudaFuncGetAttributes(&a, func);
+    if (e != cudaSuccess || (size_t)a.maxDynamicSharedSizeBytes >= bytes) return e;
+    return cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
+
+// raise_dynamic_smem once per context and size: the attribute only grows, so a cached size stays valid
 template <class F>
 inline int ensure_dynamic_smem(Ctx* c, F* func, size_t bytes) {
     const void* key = reinterpret_cast<const void*>(func);
     for (int i = 0; i < c->n_smem_funcs; ++i)
         if (c->smem_funcs[i] == key) {
             if (c->smem_bytes[i] >= bytes) return PSFR_OK;
-            cudaError_t e = cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+            cudaError_t e = raise_dynamic_smem(func, bytes);
             if (e != cudaSuccess) return set_error(c, PSFR_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
             c->smem_bytes[i] = bytes;
             return PSFR_OK;
         }
     if (bytes > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+        cudaError_t e = raise_dynamic_smem(func, bytes);
         if (e != cudaSuccess) return set_error(c, PSFR_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     }
     if (c->n_smem_funcs < 64) {

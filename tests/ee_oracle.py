@@ -17,10 +17,14 @@ def _quadrant(x, y, r):
     x, y = np.minimum(np.abs(x), r), np.minimum(np.abs(y), r)
     r2 = r * r
 
-    def prim(X):     # integral of sqrt(r^2 - X^2) from 0 to X
-        return (X * np.sqrt(np.maximum(r2 - X * X, 0)) + r2 * np.arcsin(np.clip(X / r, -1, 1))) / 2
+    def chord(X):    # sqrt(r^2 - X^2) as sqrt((r - X)(r + X)): no cancellation where X is within an ulp of r
+        return np.sqrt(np.maximum((r - X) * (r + X), 0))
 
-    xa = np.minimum(np.sqrt(np.maximum(r2 - y * y, 0)), x)      # the arc is above Y = y for X < xa
+    def prim(X):     # integral of sqrt(r^2 - X^2) from 0 to X; arcsin(X / r) as atan2, exact near X = r too
+        s = chord(X)
+        return (X * s + r2 * np.arctan2(X, s)) / 2
+
+    xa = np.minimum(chord(y), x)      # the arc is above Y = y for X < xa
     return sx * sy * (xa * y + prim(x) - prim(xa))
 
 
