@@ -130,6 +130,32 @@ enum {
  *                         1e-10 px below r
  * Radii must be finite and >= 0, fractions in (0, 1), centres finite; otherwise PSFR_E_ARG, nothing written. */
 
+/* AO summaries of every PSF (DESIGN.md section 5.5).  N = dim, L = 16 m (the PSD grid step is 1/L), OTF_tel the
+ * telescope OTF on the N x N grid and D_lambda = (2 pi / lambda_nm)^2 D_unit the structure function at lambda.
+ *
+ * Strehl ratio S(lambda) = sum_f OTF_tel(f) exp(-D_lambda(f) / 2) / sum_f OTF_tel(f) over the full N x N grid: the
+ * centre ratio psf[N/2][N/2] / psf_diff[N/2][N/2] of the reference's psd_to_psf, the first PSF from the PSD and
+ * the second from a PSD of zeros (both unit-sum).  In field-mean mode (ndir > 1 without field) it is the mean of
+ * the per-direction values, the origin value of the field-mean PSF.  It is the AO Strehl, before the tip-tilt and
+ * MUSE-intrinsic kernels: those act on the 0.2" grid, which does not resolve the diffraction core, and a
+ * "delivered" Strehl after them is not computed.
+ *
+ * Residual-phase variance record of every (draw, direction) plane, nm^2, independent of lambda (multiply by
+ * (2 pi / lambda_nm)^2 for rad^2 at lambda).  TOTAL = sum over the plane's merged N x N PSD / L^2 (psfrec.py:148-151,
+ * the bg[0,0] of psfrec.py:718).  Each cell counts to exactly one source: outside the 80 x 80 AO zone to FIT; inside
+ * it, where the merged value max(fit, ao) is the fit (fit >= ao), to FIT; otherwise its ao value splits into NOISE
+ * (err_noise) and PROJ = sum_l err_rec_l, each err_rec_l also in LAYER0 + l (unused layer slots 0).  PROJ is the
+ * reference's |P beta_l - corr_l|^2 Cphi_l: servo lag, anisoplanatism and aliasing do not add up separately in
+ * that formula, so it is not split further.  TOTAL = FIT + NOISE + PROJ up to rounding. */
+enum {
+    PSFR_VAR_TOTAL = 0,
+    PSFR_VAR_FIT = 1,
+    PSFR_VAR_NOISE = 2,
+    PSFR_VAR_PROJ = 3,
+    PSFR_VAR_LAYER0 = 4,     /* LAYER0 + l, l < PSFR_MAX_LAYERS */
+    PSFR_VAR_NPAR = 12
+};
+
 /* Context ------------------------------------------------------------------------- */
 
 /* dim: PSD grid size (1280; the reference hard-codes it in compute_psf, psfrec.py:955).
@@ -255,6 +281,19 @@ PSFR_API int psfr_compute_energy(psfr_ctx* ctx, int field, int ndraw, const doub
                        int ngroup, const int* group_end, int nrad, const double* radii_px, int nfrac,
                        const double* fracs, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
                        double* out_efit, double* out_mean_efit, double* out_ee, double* out_mean_ee, void* stream);
+
+/* psfr_compute_energy plus the AO summaries of every draw (PSFR_VAR_* above): out_strehl [ndraw][P][nlam] (P = ndir
+ * with field, 1 without), the Strehl ratio of each PSF the pipeline forms, and out_var [ndraw][ndir][PSFR_VAR_NPAR],
+ * the variance record of each (draw, direction) plane in either mode.  Both are computed in the chunk of their draws
+ * and depend on a draw's data only (the same bits at every chunk size and through either mode for the variance).
+ * Exposure means of them are not formed: they are a few doubles per draw.  Every output may be NULL, and a NULL
+ * output launches nothing; the other outputs are those of psfr_compute_energy, bit for bit. */
+PSFR_API int psfr_compute_ao(psfr_ctx* ctx, int field, int ndraw, const double* draws, int npos,
+                       const double* poslgs, int ndir, const double* dirs, int nlam, const double* lambda_nm,
+                       int ngroup, const int* group_end, int nrad, const double* radii_px, int nfrac,
+                       const double* fracs, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
+                       double* out_efit, double* out_mean_efit, double* out_ee, double* out_mean_ee,
+                       double* out_strehl, double* out_var, void* stream);
 
 /* Time-mean of ncube cubes + refit (psfrec.py:1104-1105). cubes [ncube][nlam][40][40]. */
 PSFR_API int psfr_mean_refit(psfr_ctx* ctx, int ncube, int nlam, const double* cubes,

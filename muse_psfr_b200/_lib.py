@@ -43,6 +43,10 @@ def ee_slots(nrad, nfrac):
     nrad, nfrac = int(nrad), int(nfrac)
     return slice(0, nrad), nrad, slice(nrad + 1, nrad + 1 + nfrac), nrad + 1 + nfrac
 
+# residual-phase variance record of a (draw, direction) plane (PSFR_VAR_*), nm^2
+VAR_TOTAL, VAR_FIT, VAR_NOISE, VAR_PROJ, VAR_LAYER0 = 0, 1, 2, 3, 4
+VAR_NPAR = 12
+
 AO_DIM = 80
 PSF_DIM = 40
 
@@ -89,6 +93,8 @@ _SIGNATURES = {
     'psfr_encircled_energy': (_I, [_P, _I, _I, _I, _P, _P, _I, _P, _I, _P, _P, _P]),
     'psfr_compute_energy': (_I, [_P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P,
                                  _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'psfr_compute_ao': (_I, [_P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P,
+                             _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     'psfr_mean_refit': (_I, [_P, _I, _I, _P, _P, _P, _P]),
     'psfr_polyfit': (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     'psfr_set_option': (_I, [_P, _I, _D]),
@@ -326,6 +332,17 @@ class Context:
                      out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit),
                      energy=(rad, fr, out_ee, out_mean_ee))
 
+    def compute_ao(self, field, draws, dirs, poslgs, lambda_nm, radii_px=(), fracs=(), group_end=None,
+                   out_cube=None, out_fit=None, out_mean=None, out_mean_fit=None, out_efit=None, out_mean_efit=None,
+                   out_ee=None, out_mean_ee=None, out_strehl=None, out_var=None, stream=None):
+        """psfr_compute_ao: ``compute_energy`` plus the Strehl ratio of every PSF it forms, ``out_strehl`` [ndraw, P,
+        nl] (P = npos with ``field``, 1 without), and the variance record of every (draw, direction) plane,
+        ``out_var`` [ndraw, ndir, VAR_NPAR] in nm^2 (``VAR_*``)."""
+        rad, fr = f64(radii_px).ravel(), f64(fracs).ravel()
+        self._groups(self._lib.psfr_compute_ao, bool(field), draws, dirs, poslgs, lambda_nm, group_end, out_cube,
+                     out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit),
+                     energy=(rad, fr, out_ee, out_mean_ee), ao=(out_strehl, out_var))
+
     def compute_batch(self, draws, dirs, poslgs, lambda_nm, out_cube=None, out_fit=None, stream=None):
         if not hasattr(draws, 'data_ptr'):      # numpy / sequence; torch tensors pass through as buffers
             draws = f64(draws)
@@ -363,7 +380,7 @@ class Context:
                          out_cube, out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit))
 
     def _groups(self, fn, field, draws, dirs, poslgs, lambda_nm, group_end, out_cube, out_fit, out_mean,
-                out_mean_fit, stream, shapes=None, energy=None):
+                out_mean_fit, stream, shapes=None, energy=None, ao=None):
         if not hasattr(draws, 'data_ptr'):
             draws = f64(draws)
         if len(draws.shape) != 2 or draws.shape[1] != DRAW_NPAR:
@@ -390,6 +407,9 @@ class Context:
             rec = ee_slots(energy[0].size, energy[1].size)[3]
             args += [self._buf(energy[2], nd * nimg * rec, 'out_ee', True),
                      self._buf(energy[3], ng * nimg * rec, 'out_mean_ee', True)]
+        if ao is not None:
+            args += [self._buf(ao[0], nd * nimg, 'out_strehl', True),
+                     self._buf(ao[1], nd * dirs.shape[1] * VAR_NPAR, 'out_var', True)]
         self._check(fn(*args, stream))
 
     def mean_refit(self, ncube, nlam, cubes, out_mean=None, out_fit=None, stream=None):

@@ -309,14 +309,15 @@ static int hot_begin(Ctx* c) {
 // max_planes / ndir draws: PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit, and
 // with ngroup > 0 the time mean of every exposure (draws [group_end[g-1], group_end[g])) and its fit in the
 // chunk where the exposure's last draw lies.  field: every (draw, direction) plane keeps its own PSF instead
-// of the draw's field mean, so a draw owns ndir x nlam images in every output.  Host outputs leave through
+// of the draw's field mean, so a draw owns ndir x nlam images in every output (out_var: ndir records in either
+// mode).  Host outputs leave through
 // a second stream: the results of chunk i are copied out while chunk i + 1 computes, from staging buffers
 // that alternate between two sets.
 static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs, int npos,
                      const double* poslgs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                      bool field, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
                      double* out_efit, double* out_mean_efit, int nrad, int nfrac, double* out_ee,
-                     double* out_mean_ee, cudaStream_t s) {
+                     double* out_mean_ee, double* out_strehl, double* out_var, cudaStream_t s) {
     PSFR_CUDA(c, cudaSetDevice(c->device));
     std::vector<double> lam;
     int rc = small_to_host(c, lam, lambda_nm, nlam > 0 ? nlam : 0, s);
@@ -337,6 +338,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     const size_t fits = imgs * PSFR_FIT_NPAR;   // fit records per draw
     const size_t efits = imgs * PSFR_EFIT_NPAR;  // elliptical records per draw
     const size_t ees = imgs * (size_t)(nrad + 1 + nfrac);   // encircled-energy values per draw
+    const size_t vars = (size_t)ndir * PSFR_VAR_NPAR;       // variance values per draw
     const bool cube_dev = out_cube && is_device_ptr(out_cube);
     const bool fit_dev = out_fit && is_device_ptr(out_fit);
     const bool mean_dev = out_mean && is_device_ptr(out_mean);
@@ -345,10 +347,13 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     const bool mefit_dev = out_mean_efit && is_device_ptr(out_mean_efit);
     const bool ee_dev = out_ee && is_device_ptr(out_ee);
     const bool mee_dev = out_mean_ee && is_device_ptr(out_mean_ee);
+    const bool strehl_dev = out_strehl && is_device_ptr(out_strehl);
+    const bool var_dev = out_var && is_device_ptr(out_var);
     const bool means = out_mean || out_mean_fit || out_mean_efit || out_mean_ee;
     const bool host_out = (out_cube && !cube_dev) || (out_fit && !fit_dev) || (out_mean && !mean_dev) ||
                           (out_mean_fit && !mfit_dev) || (out_efit && !efit_dev) || (out_mean_efit && !mefit_dev) ||
-                          (out_ee && !ee_dev) || (out_mean_ee && !mee_dev);
+                          (out_ee && !ee_dev) || (out_mean_ee && !mee_dev) || (out_strehl && !strehl_dev) ||
+                          (out_var && !var_dev);
     int* seg_dev = reinterpret_cast<int*>(c->d_misc + misc_groups(c->max_planes));
     std::vector<int> seg;
     int g0 = 0;   // first exposure not finished in an earlier chunk
@@ -368,6 +373,12 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
             rc = set_error(c, PSFR_E_CUDA, "stream wait failed: %s", cudaGetErrorString(cudaGetLastError()));
             break;
         }
+        // the AO records of the chunk: d_psdq / d_ao still hold its PSDs and d_samp its raw samples, and staging
+        // set b is free again
+        double* var = var_dev ? out_var + (size_t)d0 * vars : c->d_var[b];
+        if (out_var && (rc = run_var(c, nd, ndir, ngs, npos, var, s))) break;
+        double* strehl = strehl_dev ? out_strehl + (size_t)d0 * imgs : c->d_strehl[b];
+        if (out_strehl && (rc = run_strehl(c, nd * (int)imgs, strehl, s))) break;
         double* conv = cube_dev ? out_cube + (size_t)d0 * elems : (b ? c->d_cube3 : c->d_cube2);
         if ((rc = run_convolve(c, nd, ppd, nlam, c->d_cube, conv, s))) break;
         double* fit = fit_dev ? out_fit + (size_t)d0 * fits : (b ? c->d_fit2 : c->d_fit);
@@ -430,6 +441,12 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
             if (e == cudaSuccess && ndone && out_mean_ee && !mee_dev)
                 e = cudaMemcpyAsync(out_mean_ee + (size_t)g0 * ees, mee, (size_t)ndone * ees * sizeof(double),
                                     cudaMemcpyDefault, c->copy_stream);
+            if (e == cudaSuccess && out_var && !var_dev)
+                e = cudaMemcpyAsync(out_var + (size_t)d0 * vars, var, (size_t)nd * vars * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
+            if (e == cudaSuccess && out_strehl && !strehl_dev)
+                e = cudaMemcpyAsync(out_strehl + (size_t)d0 * imgs, strehl, (size_t)nd * imgs * sizeof(double),
+                                    cudaMemcpyDefault, c->copy_stream);
             if (e == cudaSuccess) e = cudaEventRecord(c->ev_copied[b], c->copy_stream);
             if (e != cudaSuccess) {
                 rc = set_error(c, PSFR_E_CUDA, "result copy failed: %s", cudaGetErrorString(e));
@@ -450,7 +467,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 104; }
+int psfr_version(void) { return 105; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -465,7 +482,7 @@ void psfr_destroy(psfr_ctx* c) {
     cudaFree(c->d_twc); cudaFree(c->d_wsamp); cudaFree(c->d_wcol); cudaFree(c->d_kcol); cudaFree(c->d_xmap); cudaFree(c->d_khat_tt); cudaFree(c->d_khat_mu);
     cudaFree(c->d_cube3); cudaFree(c->d_fit2); cudaFree(c->d_carry); cudaFree(c->d_efit); cudaFree(c->d_efit2);
     for (int i = 0; i < 2; ++i) { cudaFree(c->d_mean[i]); cudaFree(c->d_mfit[i]); cudaFree(c->d_mefit[i]); }
-    for (int i = 0; i < 2; ++i) { cudaFree(c->d_ee[i]); cudaFree(c->d_mee[i]); }
+    for (int i = 0; i < 2; ++i) { cudaFree(c->d_ee[i]); cudaFree(c->d_mee[i]); cudaFree(c->d_strehl[i]); cudaFree(c->d_var[i]); }
     cudaFree(c->d_eepar); cudaFree(c->d_eecen);
     cudaFree(c->d_dphi32); cudaFree(c->d_otf32); cudaFree(c->d_tw32); cudaFree(c->d_twg); cudaFree(c->d_twg32); cudaFree(c->d_p3); cudaFree(c->d_p2mask); cudaFree(c->d_csort); cudaFree(c->d_lorder); cudaFree(c->d_kaddr);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
@@ -591,6 +608,8 @@ int psfr_create(int device, int dim, int max_planes, int max_lambda, psfr_ctx** 
         CK(dev_alloc(c, &c->d_mefit[i], P * LM * PSFR_EFIT_NPAR));
         CK(dev_alloc(c, &c->d_ee[i], P * LM * kEeMaxRecord));
         CK(dev_alloc(c, &c->d_mee[i], P * LM * kEeMaxRecord));
+        CK(dev_alloc(c, &c->d_strehl[i], P * LM));
+        CK(dev_alloc(c, &c->d_var[i], P * PSFR_VAR_NPAR));
     }
     CK(dev_alloc(c, &c->d_eepar, (size_t)PSFR_EE_MAX_RADII + PSFR_EE_MAX_FRACTIONS));
     CK(dev_alloc(c, &c->d_eecen, P * LM * 2));
@@ -635,6 +654,7 @@ int psfr_create(int device, int dim, int max_planes, int max_lambda, psfr_ctx** 
         CKC(cudaMemcpy(c->d_twc, twc.data(), twc.size() * sizeof(double2), cudaMemcpyHostToDevice));
     }
     CK(run_build_otf(c, 0));
+    CK(run_otf_sum(c, 0));
     CKC(cudaDeviceSynchronize());
 #undef CK
 #undef CKC
@@ -876,7 +896,7 @@ int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, co
     if (ngs < 1) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
     return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, false, out_cube,
                      out_fit, nullptr, nullptr, nullptr, nullptr, 0, 0, nullptr, nullptr,
-                     static_cast<cudaStream_t>(stream));
+                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 // the arguments of psfr_compute_groups and psfr_compute_field that run_batch does not check itself
@@ -904,7 +924,7 @@ int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, c
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, false,
                      out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, 0, 0, nullptr, nullptr,
-                     static_cast<cudaStream_t>(stream));
+                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
@@ -914,7 +934,7 @@ int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, co
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
                      out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, 0, 0, nullptr, nullptr,
-                     static_cast<cudaStream_t>(stream));
+                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field_shapes(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
@@ -926,7 +946,7 @@ int psfr_compute_field_shapes(psfr_ctx* c, int ndraw, const double* draws, int n
         return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
                      out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, 0, 0, nullptr, nullptr,
-                     static_cast<cudaStream_t>(stream));
+                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_energy(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs,
@@ -942,7 +962,23 @@ int psfr_compute_energy(psfr_ctx* c, int field, int ndraw, const double* draws, 
     if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
                      out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
-                     out_mean_ee, s);
+                     out_mean_ee, nullptr, nullptr, s);
+}
+
+int psfr_compute_ao(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
+                    const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end, int nrad,
+                    const double* radii_px, int nfrac, const double* fracs, double* out_cube, double* out_fit,
+                    double* out_mean, double* out_mean_fit, double* out_efit, double* out_mean_efit, double* out_ee,
+                    double* out_mean_ee, double* out_strehl, double* out_var, void* stream) {
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
+                              out_mean || out_mean_fit || out_mean_efit || out_mean_ee))
+        return rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
+                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
+                     out_mean_ee, out_strehl, out_var, s);
 }
 
 int psfr_mean_refit(psfr_ctx* c, int ncube, int nlam, const double* cubes, double* out_mean, double* out_fit,

@@ -93,6 +93,7 @@ struct Ctx {
     int planes_loaded = 0;       // planes whose PSD sits in d_psd
     int planes_struct = 0;       // planes whose structure function sits in d_dphi
     double pup_sum = 0;
+    double otf_sum = 0;          // sum of the telescope OTF over the full N x N grid (run_otf_sum): Strehl denominator
 
     double2* d_tw = nullptr;     // twiddles: TW1 then TW2
     double2* d_twc = nullptr;    // [1280] combine twiddles exp(+2 pi i k / N) (NF = 2)
@@ -152,6 +153,8 @@ struct Ctx {
     double* d_eepar = nullptr;   // [PSFR_EE_MAX_RADII + PSFR_EE_MAX_FRACTIONS] radii then fractions of the call
     double* d_eecen = nullptr;   // [max_planes*max_lambda][2] staging for host centres (psfr_encircled_energy)
     std::vector<double> ee_par;  // host copy of d_eepar's contents (outlives the asynchronous upload)
+    double* d_strehl[2] = {nullptr, nullptr}; // [max_planes*max_lambda] Strehl ratios (double-buffered as d_ee)
+    double* d_var[2] = {nullptr, nullptr};    // [max_planes][PSFR_VAR_NPAR] variance records (double-buffered)
     cudaStream_t copy_stream = nullptr;      // device -> host copies of finished chunks
     cudaEvent_t ev_done[2] = {nullptr, nullptr};    // chunk results ready (compute stream)
     cudaEvent_t ev_copied[2] = {nullptr, nullptr};  // chunk results copied out (copy stream)
@@ -255,6 +258,16 @@ int run_group_rows(Ctx* c, int nplanes, int nlam, cudaStream_t s);
 // ngs: guide stars of every draw, or 0 for each draw's own count (slot PSFR_DRAW_NGS); the positions
 // are the first ngs columns of the [2][npos] table at d_misc + kMiscPos
 int run_psd(Ctx* c, int ndraw, int ndir, int ngs, int npos, cudaStream_t s, bool full = true);
+
+// residual-phase variance record [ndraw * ndir][PSFR_VAR_NPAR] of the planes whose quadrant-form PSD run_psd(...,
+// full = false) left in d_psdq / d_ao (same draws, directions and guide stars)
+int run_var(Ctx* c, int ndraw, int ndir, int ngs, int npos, double* out_dev, cudaStream_t s);
+
+// ---- psfr_ao.cu ----------------------------------------------------------------------
+// context init, after run_build_otf: c->otf_sum = sum of the telescope OTF over the full grid (one sync)
+int run_otf_sum(Ctx* c, cudaStream_t s);
+// Strehl ratio of the nimg PSFs run_pruned_psf left in d_samp (raw samples, before clip and normalisation)
+int run_strehl(Ctx* c, int nimg, double* out_dev, cudaStream_t s);
 
 // ---- psfr_plane.cu -------------------------------------------------------------------
 int run_build_kernels(Ctx* c, int ndraw, int nlam, const double* lambda_nm_host, bool tt, bool mu,

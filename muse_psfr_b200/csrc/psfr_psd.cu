@@ -8,6 +8,8 @@
 //  psd_fill_kernel: the dim x dim fitting PSD (psd_fit, :616-626), one pow() per four
 //                   mirror-symmetric cells, merged with the AO zone by max() (:148-149) and
 //                   scaled to nm^2 (:151), written with coalesced FP64 stores.
+//  var_kernel     : residual-phase variance record of every plane (fitting / noise / projection
+//                   error budget, DESIGN.md 5.5) from the same AO-zone terms and fitting quadrant.
 #include "psfr_internal.h"
 
 namespace psfr {
@@ -41,11 +43,13 @@ struct PsdParams {
     int npos;              // columns of pos: a draw uses the first ngs of them
 };
 
-__global__ void ao_zone_kernel(PsdParams p) {
-    const int cell = blockIdx.x * blockDim.x + threadIdx.x;
-    const int plane = blockIdx.y;
-    if (cell >= kAO * kAO) return;
-    const int u = cell / kAO, v = cell % kAO;
+// The residual-PSD terms of AO-zone cell `cell` (u * 80 + v, before the transpose and shift of the zone
+// mapping) of plane `plane`, unscaled: returns the propagated noise err_noise and calls layer(l, err_rec_l) for
+// l = 0 .. nlayers - 1 in layer order, err_rec_l = |P beta_l - corr_l|^2 Cphi_l the projection error of layer l
+// (servo lag, anisoplanatism and aliasing of that layer together: they do not add up separately).
+// ao_zone_kernel and var_kernel share it, so both see the same terms.
+template <class Layer>
+__device__ __forceinline__ double ao_cell_terms(const PsdParams& p, int cell, int plane, Layer&& layer) {
     const int draw = plane / p.ndir, dir = plane % p.ndir;
     const double* dr = p.draws + (size_t)draw * PSFR_DRAW_NPAR;
     const double f = p.geom[cell], fx = p.geom[kAO * kAO + cell], fy = p.geom[2 * kAO * kAO + cell];
@@ -91,7 +95,6 @@ __global__ void ao_zone_kernel(PsdParams p) {
     const int nl = (int)dr[PSFR_DRAW_NLAYERS];
     const double L0 = dr[PSFR_DRAW_L0];
     const double vk = pow_m11_6(f * f + (1 / L0) * (1 / L0));
-    double err_rec = 0.0;
     for (int l = 0; l < nl; ++l) {
         const double* ly = dr + PSFR_DRAW_LAYER0 + PSFR_LAYER_NPAR * l;
         const double h = ly[PSFR_LAYER_H];
@@ -111,8 +114,18 @@ __global__ void ao_zone_kernel(PsdParams p) {
         }
         const cd pb = cexp_i(2 * pi * (h * 60 / 206265 * bf - (wx * dT * fx + wy * dT * fy)));
         const double prx = pb.x - acc.x, pry = pb.y - acc.y;
-        err_rec += (prx * prx + pry * pry) * (ly[PSFR_LAYER_CPHI] * vk);
+        layer(l, (prx * prx + pry * pry) * (ly[PSFR_LAYER_CPHI] * vk));
     }
+    return err_noise;
+}
+
+__global__ void ao_zone_kernel(PsdParams p) {
+    const int cell = blockIdx.x * blockDim.x + threadIdx.x;
+    const int plane = blockIdx.y;
+    if (cell >= kAO * kAO) return;
+    const int u = cell / kAO, v = cell % kAO;
+    double err_rec = 0.0;
+    const double err_noise = ao_cell_terms(p, cell, plane, [&](int, double t) { err_rec += t; });
     double dsp = err_rec + err_noise;
     if (cell == 0) dsp = 0.0;
     // reference: transpose (moveaxis, :613) then fftshift (:149): zone[i][j] = dsp[(j+40)%80][(i+40)%80]
@@ -189,6 +202,83 @@ psd_quad_kernel(const double* __restrict__ draws, double* __restrict__ q, int kN
     __syncthreads();
 #pragma unroll
     for (int r = ty; r < 32; r += 8) base[(size_t)(tb * 32 + r) * kNH + ta * 32 + tx] = tile[tx][r];
+}
+
+// Residual-phase variance record of every (draw, direction) plane (DESIGN.md 5.5) from the quadrant form of the
+// chunk's PSDs (d_psdq, d_ao).  One CTA per plane:
+//  * the draw's fitting PSD over the whole grid, 4 x the sum of its quadrant;
+//  * the 80 x 80 zone cells, each with the fit at the same full-grid cell (the value LoadEvenRowsQuad merges):
+//    a cell whose AO value exceeds its fit moves that fit out of FIT and splits the AO value into NOISE and
+//    PROJ = sum_l LAYER0 + l with ao_cell_terms.
+// Each thread accumulates a fixed strided subset in order and the CTA adds the threads up in a fixed tree, so a
+// record depends on its plane's data only: the same bits at every chunk size and through every entry point.
+constexpr int kVarThreads = 256;
+enum { kAccQuad = 0, kAccWonFit, kAccWonAo, kAccNoise, kAccProj, kAccLayer0, kAccN = kAccLayer0 + PSFR_MAX_LAYERS };
+
+__global__ void __launch_bounds__(kVarThreads)
+var_kernel(PsdParams p, const double* __restrict__ q, int kN, double* __restrict__ out) {
+    __shared__ double acc[kAccN][kVarThreads];   // column t belongs to thread t alone until the tree sum
+    const int t = threadIdx.x, plane = blockIdx.x;
+    const int kNH = kN / 2, lo = kNH - kAO / 2;
+    const double* qd = q + (size_t)(plane / p.ndir) * kNH * kNH;
+    const double* z = p.ao + (size_t)plane * kAO * kAO;
+    for (int k = 0; k < kAccN; ++k) acc[k][t] = 0.0;
+
+    const double2* q2 = reinterpret_cast<const double2*>(qd);
+    const int n2 = kNH * kNH / 2;
+    double quad = 0.0;
+#pragma unroll 8
+    for (int i = t; i < n2; i += kVarThreads) {
+        const double2 v = __ldg(q2 + i);
+        quad += v.x;
+        quad += v.y;
+    }
+    acc[kAccQuad][t] = quad;
+
+    for (int zc = t; zc < kAO * kAO; zc += kVarThreads) {
+        const int i = zc / kAO, j = zc % kAO;            // zone[i][j] sits at full-grid cell (lo + i, lo + j)
+        const int a = lo + i, n = lo + j;
+        const int qa = a < kNH ? a : kN - 1 - a, qn = n < kNH ? n : kN - 1 - n;
+        const double fit = __ldg(qd + (size_t)qa * kNH + qn);
+        const double ao = __ldg(z + zc);
+        if (!(ao > fit)) continue;                       // fmax(fit, ao) is the fit: the cell counts to FIT
+        // zone[i][j] = dsp[(j + 40) % 80][(i + 40) % 80] (ao_zone_kernel)
+        const int cell = ((j + kAO / 2) % kAO) * kAO + (i + kAO / 2) % kAO;
+        double proj = 0.0;
+        const double noise = ao_cell_terms(p, cell, plane, [&](int l, double e) {
+            acc[kAccLayer0 + l][t] += e;
+            proj += e;
+        });
+        acc[kAccWonFit][t] += fit;
+        acc[kAccWonAo][t] += ao;
+        acc[kAccNoise][t] += noise;
+        acc[kAccProj][t] += proj;
+    }
+    for (int s = kVarThreads / 2; s > 0; s >>= 1) {
+        __syncthreads();
+        if (t < s)
+            for (int k = 0; k < kAccN; ++k) acc[k][t] += acc[k][t + s];
+    }
+    __syncthreads();
+    // unscaled PSD -> nm^2 (psfrec.py:151, run_psd) and the grid step 1/L, L = 16 m: sum PSD / L^2
+    const double k = 0.5 * 1000 / (2 * 3.141592653589793), L = 16.0;
+    const double unit = (k * k) / (L * L);
+    double* o = out + (size_t)plane * PSFR_VAR_NPAR;
+    if (t < PSFR_MAX_LAYERS) o[PSFR_VAR_LAYER0 + t] = acc[kAccLayer0 + t][0] * unit;
+    if (t == 0) {
+        const double fit = 4.0 * acc[kAccQuad][0] - acc[kAccWonFit][0];
+        o[PSFR_VAR_TOTAL] = (fit + acc[kAccWonAo][0]) * unit;
+        o[PSFR_VAR_FIT] = fit * unit;
+        o[PSFR_VAR_NOISE] = acc[kAccNoise][0] * unit;
+        o[PSFR_VAR_PROJ] = acc[kAccProj][0] * unit;
+    }
+}
+
+int run_var(Ctx* c, int ndraw, int ndir, int ngs, int npos, double* out_dev, cudaStream_t s) {
+    PsdParams p{c->d_draws, c->d_geom, c->d_misc + kMiscDirs, c->d_misc + kMiscPos, c->d_ao, ndraw, ndir, ngs, npos};
+    var_kernel<<<ndraw * ndir, kVarThreads, 0, s>>>(p, c->d_psdq, c->N, out_dev);
+    PSFR_LAUNCH_CHECK(c);
+    return PSFR_OK;
 }
 
 int run_psd(Ctx* c, int ndraw, int ndir, int ngs, int npos, cudaStream_t s, bool full) {

@@ -356,6 +356,23 @@ def _ee_table(lbda, ee, radii, fractions, pixscale=_PIXSCALE):
     }, meta={'radii': radii, 'fractions': fractions})
 
 
+def _ao_table(lbda, strehl, var):
+    """Columns of the AO summary table (DESIGN.md section 5.5): ``strehl`` [n] (the AO Strehl ratio at each
+    wavelength) and, from the variance records ``var`` [n, VAR_NPAR] or one record [VAR_NPAR] for every row, the
+    residual-phase variance ``var_total`` = ``var_fit`` + ``var_noise`` + ``var_proj`` in nm^2 (independent of the
+    wavelength; multiply by (2 pi / lbda_nm)^2 for rad^2)."""
+    lbda = np.asarray(lbda, dtype=float)
+    var = np.broadcast_to(np.asarray(var, dtype=float), (lbda.size, _lib.VAR_NPAR))
+    return FitTable({
+        'lbda': lbda,
+        'strehl': np.asarray(strehl, dtype=float).reshape(lbda.size).copy(),
+        'var_total': var[:, _lib.VAR_TOTAL].copy(),
+        'var_fit': var[:, _lib.VAR_FIT].copy(),
+        'var_noise': var[:, _lib.VAR_NOISE].copy(),
+        'var_proj': var[:, _lib.VAR_PROJ].copy(),
+    })
+
+
 # --------------------------------------------------------------------------- reference API
 def simul_psd_wfm(Cn2, h, seeing, L0, zenith=0., plot=False, npsflin=1, dim=1280,
                   three_lgs_mode=False, verbose=True, wind_dir=None):
@@ -597,7 +614,8 @@ def _planes_context(nd, ndir, nlam, max_planes, device, dim):
 
 def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs_mode=False,
                       out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None, stream=None,
-                      dim=_DIM, zenith=0., Cn2=None, wind_dir=None, ee_radii=None, ee_fractions=(0.5, 0.8)):
+                      dim=_DIM, zenith=0., Cn2=None, wind_dir=None, ee_radii=None, ee_fractions=(0.5, 0.8),
+                      ao_budget=False):
     """Batched ``compute_psf``: one fused device pipeline for many (seeing, GL, L0[, h]) draws.
 
     ``h`` is one (h0, h1) pair or an array [ndraw, 2].  ``three_lgs_mode`` is one flag for all draws or
@@ -609,7 +627,12 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     computed on the device right after its fit (``encircled_energy``): the result gains a third entry, the raw
     records [ndraw, nl, nrad + 1 + nfrac] in pixels (``_lib.ee_slots``; ``_ee_table`` turns them into the
     columns of ``encircled_energy``), for the fractions ``ee_fractions``.  With ``want_cube=False`` no cube leaves
-    the device.  fit and cube are those of a call without ``ee_radii``, bit for bit."""
+    the device.  fit and cube are those of a call without ``ee_radii``, bit for bit.
+
+    ``ao_budget=True`` appends (strehl [ndraw, nl], var [ndraw, npsflin**2, VAR_NPAR]) after the other results:
+    the AO Strehl ratio of every PSF and the residual-phase variance record (nm^2, ``_lib.VAR_*``) of every
+    (draw, direction) plane, computed on the device in the same pass (DESIGN.md section 5.5; ``_ao_table`` turns
+    them into columns).  Every other result is that of a call without it, bit for bit."""
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
     seeing, GL, L0 = (np.atleast_1d(np.asarray(v, dtype=float)) for v in (seeing, GL, L0))
     nd = seeing.size
@@ -622,16 +645,18 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     if energy:
         rad_px, frac = _ee_params(ee_radii, ee_fractions)
         ee = np.empty((nd, lam.size, _lib.ee_slots(rad_px.size, frac.size)[3]))
+    ndir = npsflin * npsflin
+    ao = (np.empty((nd, lam.size)), np.empty((nd, ndir, _lib.VAR_NPAR))) if ao_budget else ()
+    extra = ((ee,) if energy else ()) + ao
     if nd == 0 or lam.size == 0:
         # nothing to compute: empty results of the right shape, written through nothing
-        empty = (np.empty((nd, lam.size, _lib.FIT_NPAR)),
-                 np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None)
-        return empty + (ee,) if energy else empty
+        return (np.empty((nd, lam.size, _lib.FIT_NPAR)),
+                np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None) + extra
     if per_draw:
         recs = _mode_records(three, seeing, GL, L0, h, zenith, Cn2, wind_dir)
     else:
         recs = _batch_records(seeing, GL, L0, h, zenith, Cn2, wind_dir)
-        if energy:      # the groups path takes each draw's guide-star count from its record
+        if energy or ao_budget:      # the groups path takes each draw's guide-star count from its record
             recs[:, _lib.DRAW_NGS] = 3 if three_lgs_mode else 4
     dirs = direction_perf(npsflin)
     dim = _check_dim(dim)
@@ -641,7 +666,11 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        if energy:
+        if ao_budget:
+            ctx.compute_ao(False, recs, dirs, _lgs_positions(False), lam, rad_px if energy else (),
+                           frac if energy else (), out_cube=out_cube, out_fit=out_fit, out_ee=ee if energy else None,
+                           out_strehl=ao[0], out_var=ao[1], stream=stream)
+        elif energy:
             ctx.compute_energy(False, recs, dirs, _lgs_positions(False), lam, rad_px, frac, out_cube=out_cube,
                                out_fit=out_fit, out_ee=ee, stream=stream)
         elif per_draw:    # the three-laser asterism is the first three stars of the four-laser one
@@ -654,13 +683,13 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
         raise
-    return (out_fit, out_cube, ee) if energy else (out_fit, out_cube)
+    return (out_fit, out_cube) + extra
 
 
 def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_size=60, h=(100, 10000),
                       three_lgs_mode=False, out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None,
                       stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None, elliptical=False, ee_radii=None,
-                      ee_fractions=(0.5, 0.8)):
+                      ee_fractions=(0.5, 0.8), ao_budget=False):
     """Field-resolved ``compute_psf_batch``: the PSF of every draw at every field position instead of
     their average.
 
@@ -678,7 +707,11 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     cube are those of a call without it, bit for bit.
 
     ``ee_radii`` [arcsec] appends the encircled-energy records [ndraw, npos, nl, nrad + 1 + nfrac] of every PSF, in
-    pixels, as ``compute_psf_batch(ee_radii=...)`` does, after ``efit`` where present."""
+    pixels, as ``compute_psf_batch(ee_radii=...)`` does, after ``efit`` where present.
+
+    ``ao_budget=True`` appends (strehl [ndraw, npos, nl], var [ndraw, npos, VAR_NPAR]) last, as
+    ``compute_psf_batch(ao_budget=True)`` does: the Strehl ratio of each position's PSF and the variance record of
+    each (draw, position) plane."""
     pos = _field_positions(direction_perf(npsflin, field_size) if positions is None else positions)
     npos = pos.shape[1]
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
@@ -692,7 +725,8 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     if energy:
         rad_px, frac = _ee_params(ee_radii, ee_fractions)
         ee = np.empty((nd, npos, lam.size, _lib.ee_slots(rad_px.size, frac.size)[3]))
-    extra = ((efit,) if elliptical else ()) + ((ee,) if energy else ())
+    ao = (np.empty((nd, npos, lam.size)), np.empty((nd, npos, _lib.VAR_NPAR))) if ao_budget else ()
+    extra = ((efit,) if elliptical else ()) + ((ee,) if energy else ()) + ao
     if nd == 0 or lam.size == 0:
         return (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
                 np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None) + extra
@@ -706,7 +740,11 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        if energy:
+        if ao_budget:
+            ctx.compute_ao(True, recs, pos, _lgs_positions(False), lam, rad_px if energy else (),
+                           frac if energy else (), out_cube=out_cube, out_fit=out_fit, out_efit=efit,
+                           out_ee=ee if energy else None, out_strehl=ao[0], out_var=ao[1], stream=stream)
+        elif energy:
             ctx.compute_energy(True, recs, pos, _lgs_positions(False), lam, rad_px, frac, out_cube=out_cube,
                                out_fit=out_fit, out_efit=efit, out_ee=ee, stream=stream)
         else:
@@ -799,6 +837,15 @@ def _ee_columns(lam, ee, radii, fractions):
     return {k: tab[k] for k in tab.colnames}
 
 
+def _draw_mean(x):
+    """Mean of ``x`` over its first axis, summed in order (the mean of an exposure's draws, in draw order)."""
+    x = np.asarray(x, dtype=float)
+    acc = np.zeros(x.shape[1:])
+    for row in x:
+        acc = acc + row
+    return acc / len(x)
+
+
 def _ee_cards(meta, radii, fractions):
     """``meta`` plus one card per radius [arcsec] (EERADk) and per fraction (EEFRACk), k from 1."""
     cards = dict(meta)
@@ -810,7 +857,7 @@ def _ee_cards(meta, radii, fractions):
 def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                             lbda=None, h=(100, 10000), n_jobs=-1, plot=False, mean_of_lgs=True,
                             verbose=True, device=None, field_positions=None, elliptical=False, ee_radii=None,
-                            ee_fractions=(0.5, 0.8)):
+                            ee_fractions=(0.5, 0.8), ao_budget=False):
     """Reconstruct a PSF from SPARTA data (psfrec.py:981-1120).
 
     ``filename``: path of a FITS file, a binary file object, or an HDUList (this package's or
@@ -820,20 +867,20 @@ def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin
     FIT_MEAN, PSF_MEAN] - an ``astropy.io.fits.HDUList`` when astropy is installed, otherwise
     the equivalent object of ``muse_psfr_b200._fits`` - or None when no row is valid.  With
     ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow, with ``elliptical=True``
-    SHAPE_MEAN (and SHAPE_FIELD), and with ``ee_radii`` EE_MEAN (and EE_FIELD): see
-    ``compute_psf_from_sparta_batch``."""
+    SHAPE_MEAN (and SHAPE_FIELD), with ``ee_radii`` EE_MEAN (and EE_FIELD), and with ``ao_budget=True`` AO_MEAN
+    (and AO_FIELD): see ``compute_psf_from_sparta_batch``."""
     if plot:
         raise NotImplementedError('plotting is outside the B200 hot path')
     return compute_psf_from_sparta_batch([filename], extname=extname, npsflin=npsflin, lmin=lmin, lmax=lmax, nl=nl,
                                          lbda=lbda, h=h, n_jobs=n_jobs, mean_of_lgs=mean_of_lgs, verbose=verbose,
                                          device=device, field_positions=field_positions, elliptical=elliptical,
-                                         ee_radii=ee_radii, ee_fractions=ee_fractions)[0]
+                                         ee_radii=ee_radii, ee_fractions=ee_fractions, ao_budget=ao_budget)[0]
 
 
 def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                                   lbda=None, h=(100, 10000), n_jobs=-1, mean_of_lgs=True, verbose=True,
                                   device=None, max_planes=None, field_positions=None, elliptical=False,
-                                  ee_radii=None, ee_fractions=(0.5, 0.8)):
+                                  ee_radii=None, ee_fractions=(0.5, 0.8), ao_budget=False):
     """``compute_psf_from_sparta`` for many exposures in one device pass: returns one entry per source,
     the HDUList ``compute_psf_from_sparta(source, ...)`` returns, bit for bit, or None for a table
     without a valid row.
@@ -859,7 +906,14 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     ``ee_fractions``) with the cards of FIT_MEAN plus EERADk / EEFRACk, and with ``field_positions`` EE_FIELD, the
     same columns plus ``x`` and ``y`` for the PSFs of PSF_FIELD, position-major.  Both are computed on the device
     in the passes that form the means, and follow the SHAPE_* HDUs; every HDU before them is that of a call
-    without ``ee_radii``, bit for bit."""
+    without ``ee_radii``, bit for bit.
+
+    ``ao_budget=True`` appends AO_MEAN, one row per wavelength with the ``_ao_table`` columns and the cards of
+    FIT_MEAN: the Strehl ratio and the residual-phase variance budget (nm^2) of the exposure, each the mean over
+    its draws in draw order (for the variance, over the directions of each draw too), from the Strehl ratios and
+    variance records the mean pass computes on the device.  With ``field_positions`` AO_FIELD follows, the same
+    columns plus ``x`` and ``y`` per (position, wavelength), position-major, from the field pass.  Every HDU before
+    them is that of a call without ``ao_budget``, bit for bit."""
     if lbda is None:
         lbda = np.linspace(lmin, lmax, nl)
     lbda = np.atleast_1d(np.asarray(lbda, dtype=float))
@@ -906,6 +960,13 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     try:
         if energy:
             ee_mean = np.empty((ng, nlam, ee_rec))
+        if ao_budget:
+            strehl = np.empty((nd, nlam))
+            var = np.empty((nd, dirs.shape[1], _lib.VAR_NPAR))
+            ctx.compute_ao(False, draws, dirs, _lgs_positions(False), lbda, rad_px if energy else (),
+                           frac if energy else (), group_end, out_fit=fit, out_mean=psftot, out_mean_fit=fit_mean,
+                           out_mean_ee=ee_mean if energy else None, out_strehl=strehl, out_var=var)
+        elif energy:
             ctx.compute_energy(False, draws, dirs, _lgs_positions(False), lbda, rad_px, frac, group_end, out_fit=fit,
                                out_mean=psftot, out_mean_fit=fit_mean, out_mean_ee=ee_mean)
         else:
@@ -919,6 +980,14 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
             shape_field = np.empty((ng, npos, nlam, _lib.EFIT_NPAR)) if elliptical else None
             if energy:
                 ee_field = np.empty((ng, npos, nlam, ee_rec))
+            if ao_budget:
+                strehl_field = np.empty((nd, npos, nlam))
+                var_field = np.empty((nd, npos, _lib.VAR_NPAR))
+                ctx.compute_ao(True, draws, pos, _lgs_positions(False), lbda, rad_px if energy else (),
+                               frac if energy else (), group_end, out_mean=psf_field, out_mean_fit=fit_field,
+                               out_mean_efit=shape_field, out_mean_ee=ee_field if energy else None,
+                               out_strehl=strehl_field, out_var=var_field)
+            elif energy:
                 ctx.compute_energy(True, draws, pos, _lgs_positions(False), lbda, rad_px, frac, group_end,
                                    out_mean=psf_field, out_mean_fit=fit_field, out_mean_efit=shape_field,
                                    out_mean_ee=ee_field)
@@ -976,6 +1045,17 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
                 cols['x'] = np.repeat(pos[0], nlam)
                 cols['y'] = np.repeat(pos[1], nlam)
                 out.append(_fits.table_to_hdu(cols, meta=cards, name='EE_FIELD'))
+        if ao_budget:
+            tab = _ao_table(lbda, _draw_mean(strehl[d0:d0 + nj]),
+                            _draw_mean(var[d0:d0 + nj].reshape(-1, _lib.VAR_NPAR)))
+            out.append(_fits.table_to_hdu({k: tab[k] for k in tab.colnames}, meta=meta, name='AO_MEAN'))
+            if pos is not None:
+                s_f, v_f = _draw_mean(strehl_field[d0:d0 + nj]), _draw_mean(var_field[d0:d0 + nj])
+                tab = FitTable.vstack([_ao_table(lbda, s_f[k], v_f[k]) for k in range(npos)])
+                cols = {k: tab[k] for k in tab.colnames}
+                cols['x'] = np.repeat(pos[0], nlam)
+                cols['y'] = np.repeat(pos[1], nlam)
+                out.append(_fits.table_to_hdu(cols, meta=meta, name='AO_FIELD'))
         try:
             results.append(_fits.to_astropy(out))
         except ImportError:
