@@ -201,7 +201,15 @@ PSFR_API int psfr_psf_cube(psfr_ctx* ctx, int ndraw, int ndir, int nlam, const d
 
 /* convolve_final_psf (psfrec.py:874-930): tip-tilt Moffat (beta=2, alpha_tt[draw] in px)
  * then MUSE intrinsic Moffat (muse_intrinsic_psf, psfrec.py:1144-1171) per wavelength.
- * cube [ndraw][nlam][40][40] in -> out (may alias). */
+ * cube [ndraw][nlam][40][40] in -> out (may alias).
+ * Domain of the kernels (outside, the kernel would be 0/0; nothing is launched or written):
+ *   alpha_tt[d] > 0 with pi alpha_tt^2 a finite, normal double (alpha_tt in about [8.5e-155, 7.5e153]), else
+ *   PSFR_E_ARG (tiptilt_alpha is 0 at GL = 1 and NaN at GL > 1); the same holds for the PSFR_DRAW_ALPHA_TT slot
+ *   in every batch call that convolves;
+ *   lambda finite and > 0, else PSFR_E_ARG;
+ *   MUSE beta(lambda) > 0 and != 1 and pi gamma^2 finite and normal, else PSFR_E_UNSUPPORTED: beta crosses 0 at
+ *   lambda ~ 1188.99 nm, so the convolutions (and every batch call) stop there; beta = 1 at ~ 1132.77 nm and
+ *   fwhm = 0 at ~ 303.85 nm are isolated points. */
 PSFR_API int psfr_convolve(psfr_ctx* ctx, int ndraw, int nlam, const double* lambda_nm,
                   const double* alpha_tt, const double* cube, double* out_cube, void* stream);
 

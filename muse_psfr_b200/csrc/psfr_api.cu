@@ -219,11 +219,25 @@ static int small_to_host(Ctx* c, std::vector<double>& dst, const double* src, si
     return PSFR_OK;
 }
 
+// The tip-tilt Moffat width of every draw: alpha > 0 with pi alpha^2 a finite, normal double.  Outside, the
+// kernel is 0/0: alpha = 0 (GL = 1 in tiptilt_alpha) or alpha^2 underflowing to 0 leaves its centre 0/0, pi alpha^2
+// = inf its amplitude 0, and NaN (GL > 1) propagates.
+static int check_alpha_tt(Ctx* c, int ndraw, const double* alpha, size_t stride) {
+    for (int d = 0; d < ndraw; ++d) {
+        const double a = alpha[(size_t)d * stride];
+        if (!(a > 0 && moffat_width_ok(a)))
+            return set_error(c, PSFR_E_ARG, "draw %d has tip-tilt alpha %g px; the kernel needs alpha > 0 with "
+                             "pi alpha^2 finite and normal", d, a);
+    }
+    return PSFR_OK;
+}
+
 // geometry of a call: directions and guide-star positions [2][npos]; validates the whole draw list once
 // (the host keeps the reference's ValueError for > 2 layers without explicit wind directions).  ngs: guide
-// stars of every draw, or 0 when each draw gives its own count in slot PSFR_DRAW_NGS.  One host sync at most.
+// stars of every draw, or 0 when each draw gives its own count in slot PSFR_DRAW_NGS.  One host sync at most;
+// h receives the host copy of the draw records.
 static int upload_geometry(Ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs,
-                           int npos, const double* pos, cudaStream_t s) {
+                           int npos, const double* pos, std::vector<double>& h, cudaStream_t s) {
     if (ndraw < 1 || ndir < 1) return set_error(c, PSFR_E_ARG, "ndraw=%d ndir=%d", ndraw, ndir);
     if (ngs < 0 || ngs > kMaxGS) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
     if (npos < 1 || npos > kMaxGS) return set_error(c, PSFR_E_ARG, "npos=%d outside [1,%d]", npos, kMaxGS);
@@ -233,7 +247,6 @@ static int upload_geometry(Ctx* c, int ndraw, const double* draws, int ndir, con
     if (rc) return rc;
     rc = to_device(c, c->d_misc + kMiscPos, pos, (size_t)2 * npos * sizeof(double), s);
     if (rc) return rc;
-    std::vector<double> h;
     rc = small_to_host(c, h, draws, (size_t)ndraw * PSFR_DRAW_NPAR, s);
     if (rc) return rc;
     for (int d = 0; d < ndraw; ++d) {
@@ -326,7 +339,10 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     if (rc) return rc;
     rc = run_build_kernels(c, 0, nlam, lam.data(), false, true, s);
     if (rc) return rc;
-    rc = upload_geometry(c, ndraw, draws, ndir, dirs, ngs, npos, poslgs, s);
+    std::vector<double> h;
+    rc = upload_geometry(c, ndraw, draws, ndir, dirs, ngs, npos, poslgs, h, s);
+    if (rc) return rc;
+    rc = check_alpha_tt(c, ndraw, h.data() + PSFR_DRAW_ALPHA_TT, PSFR_DRAW_NPAR);
     if (rc) return rc;
     hot_begin(c);
     c->hot_timed = true;
@@ -679,7 +695,8 @@ int psfr_psd(psfr_ctx* c, int ndraw, const double* draws, int ndir, const double
     if (ngs < 1) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     PSFR_CUDA(c, cudaSetDevice(c->device));
-    int rc = upload_geometry(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, s);
+    std::vector<double> h;   // psfr_psd never reads the tip-tilt alpha: records with any value in it pass
+    int rc = upload_geometry(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, h, s);
     if (rc) return rc;
     if ((rc = upload_draws(c, ndraw, draws, ndir, s))) return rc;
     rc = run_psd(c, ndraw, ndir, ngs, ngs, s);
@@ -760,9 +777,14 @@ int psfr_convolve(psfr_ctx* c, int ndraw, int nlam, const double* lambda_nm, con
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d nlam=%d exceed the context capacity", ndraw, nlam);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     PSFR_CUDA(c, cudaSetDevice(c->device));
-    std::vector<double> lam;
+    std::vector<double> lam, att;
     int rc = small_to_host(c, lam, lambda_nm, nlam, s);
+    if (!rc) rc = small_to_host(c, att, alpha_tt, ndraw, s);
     if (rc) return rc;
+    for (int l = 0; l < nlam; ++l)
+        if (!(std::isfinite(lam[l]) && lam[l] > 0))
+            return set_error(c, PSFR_E_ARG, "wavelength %g nm is not finite and positive", lam[l]);
+    if ((rc = check_alpha_tt(c, ndraw, att.data(), 1))) return rc;
     rc = to_device(c, c->d_misc + misc_alpha_tt(c->max_planes), alpha_tt, ndraw * sizeof(double), s);
     if (rc) return rc;
     rc = run_build_kernels(c, ndraw, nlam, lam.data(), true, true, s);

@@ -1,5 +1,6 @@
 // Internal declarations shared by the translation units of libpsfr_b200.so.
 #pragma once
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cuda_runtime.h>
@@ -270,6 +271,9 @@ int run_otf_sum(Ctx* c, cudaStream_t s);
 int run_strehl(Ctx* c, int nimg, double* out_dev, cudaStream_t s);
 
 // ---- psfr_plane.cu -------------------------------------------------------------------
+// moffat_kernels_kernel divides by pi * gamma^2, evaluated as (pi * gamma) * gamma: the kernel is finite for
+// every gamma that leaves that product a finite, normal double (|gamma| in about [8.5e-155, 7.5e153])
+inline bool moffat_width_ok(double gamma) { return std::isnormal(3.141592653589793 * gamma * gamma); }
 int run_build_kernels(Ctx* c, int ndraw, int nlam, const double* lambda_nm_host, bool tt, bool mu,
                       cudaStream_t s);
 // samples -> 40x40 resampled + normalised cube (psf_muse tail)

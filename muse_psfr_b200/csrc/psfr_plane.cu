@@ -6,6 +6,7 @@
 //                     analytic Jacobian (fit_psf_cube -> mpdaf moffat_fit, :861-871)
 //   mean / polyfit  : time mean of cubes (:1104) and polynomial smoothing (:1174-1210)
 #include <algorithm>
+#include <cmath>
 #include "psfr_internal.h"
 #include "fast_exp.cuh"
 
@@ -744,6 +745,31 @@ __global__ void polyfit_kernel(const double* __restrict__ lb, int nlam, int deg,
 // ---------------------------------------------------------------- drivers
 int run_build_kernels(Ctx* c, int ndraw, int nlam, const double* lambda_nm_host, bool tt, bool mu,
                       cudaStream_t s) {
+    if (mu && (int)c->lam_kernels.size() == nlam &&
+        std::equal(lambda_nm_host, lambda_nm_host + nlam, c->lam_kernels.begin()))
+        mu = false;   // the MUSE kernels of these wavelengths and their spectra are already on the device
+    std::vector<double> gb(mu ? 2 * nlam : 0);   // gamma[nlam], beta[nlam]
+    for (int l = 0; mu && l < nlam; ++l) {
+        // muse_intrinsic_psf (psfrec.py:1160-1168, np.polyval = Horner) and alpha = fwhm/0.2/(2 sqrt(2^(1/beta)-1)) (:923-924)
+        static const double pol_beta[6] = {-0.83704697, 1.1337153, 0.0609222, -1.35581762, 1.15237178, 2.2106042};
+        static const double pol_fwhm[6] = {0.60467385, -1.58905792, 1.75293264, -1.0368302, 0.21487023, 0.34851139};
+        const double lb = (10 * lambda_nm_host[l] - 4750) / (9350 - 4750);
+        double fw = 0.0, be = 0.0;
+        for (int k = 0; k < 6; ++k) {
+            fw = fw * lb + pol_fwhm[k];
+            be = be * lb + pol_beta[k];
+        }
+        fw = fw / 0.2;
+        const double g = fw / (2 * sqrt(pow(2.0, 1. / be) - 1));
+        // the kernel's domain: beta <= 0 (lambda >~ 1189 nm) makes gamma NaN or 0, beta == 1 zeroes the amplitude,
+        // fwhm == 0 (~303.85 nm) zeroes gamma; each would give a 0/0 kernel
+        if (!(be > 0) || be == 1.0 || !moffat_width_ok(g))
+            return set_error(c, PSFR_E_UNSUPPORTED,
+                             "wavelength %g nm: the MUSE Moffat has beta = %g, gamma = %g px; the kernel needs beta > 0, "
+                             "beta != 1 and pi gamma^2 finite and normal", lambda_nm_host[l], be, g);
+        gb[l] = g;
+        gb[nlam + l] = be;
+    }
     if (tt) {
         // gamma = alpha_tt per draw (slot PSFR_DRAW_ALPHA_TT), Moffat power 2
         double* two = c->d_misc + kMiscTwo;   // holds the constant 2.0
@@ -754,26 +780,10 @@ int run_build_kernels(Ctx* c, int ndraw, int nlam, const double* lambda_nm_host,
         int rc = run_kernel_spectra(c, ndraw, c->d_kern_tt, c->d_khat_tt, s);
         if (rc) return rc;
     }
-    if (mu && (int)c->lam_kernels.size() == nlam &&
-        std::equal(lambda_nm_host, lambda_nm_host + nlam, c->lam_kernels.begin()))
-        mu = false;   // the MUSE kernels of these wavelengths and their spectra are already on the device
     if (mu) {
         c->lam_kernels.clear();
-        // muse_intrinsic_psf (psfrec.py:1160-1168, np.polyval = Horner) and alpha = fwhm/0.2/(2 sqrt(2^(1/beta)-1)) (:923-924)
-        static const double pol_beta[6] = {-0.83704697, 1.1337153, 0.0609222, -1.35581762, 1.15237178, 2.2106042};
-        static const double pol_fwhm[6] = {0.60467385, -1.58905792, 1.75293264, -1.0368302, 0.21487023, 0.34851139};
         double* h = static_cast<double*>(c->h_pinned);
-        for (int l = 0; l < nlam; ++l) {
-            const double lb = (10 * lambda_nm_host[l] - 4750) / (9350 - 4750);
-            double fw = 0.0, be = 0.0;
-            for (int k = 0; k < 6; ++k) {
-                fw = fw * lb + pol_fwhm[k];
-                be = be * lb + pol_beta[k];
-            }
-            fw = fw / 0.2;
-            h[l] = fw / (2 * sqrt(pow(2.0, 1. / be) - 1));
-            h[nlam + l] = be;
-        }
+        std::copy(gb.begin(), gb.end(), h);
         double* d = c->d_misc + kMiscMuse;    // gamma[nlam], beta[nlam]
         PSFR_CUDA(c, cudaMemcpyAsync(d, h, 2 * nlam * sizeof(double), cudaMemcpyHostToDevice, s));
         PSFR_CUDA(c, cudaStreamSynchronize(s));   // pinned bounce buffer is reused by the caller
