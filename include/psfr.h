@@ -156,6 +156,16 @@ enum {
     PSFR_VAR_NPAR = 12
 };
 
+/* Band images (DESIGN.md section 5.6): throughput-weighted sums of the wavelength planes of an image set, the PSF of a
+ * white-light, narrow-band or filter image.  A call carries 1 <= nband <= PSFR_MAX_BANDS bands with weights
+ * w [nband][nlam], finite and >= 0, and every band sum W_b = sum_k w[b][k] (added in ascending k) finite and > 0;
+ * otherwise PSFR_E_ARG before any launch, nothing written.  The band image of a set of planes C[k] is
+ *   B[b][pix] = acc / W_b,  acc = fma(w[b][k], C[k][pix], acc) in ascending k from acc = 0, in FP64,
+ * with no clip and no renormalisation: B keeps the flux scale of the planes.  One-hot weights give plane k bit for
+ * bit, and scaling a band's weights by a power of two leaves its bits unchanged.  The reference has no band PSF:
+ * parity with it is unpinned. */
+#define PSFR_MAX_BANDS 16
+
 /* Context ------------------------------------------------------------------------- */
 
 /* dim: PSD grid size (1280; the reference hard-codes it in compute_psf, psfrec.py:955).
@@ -302,6 +312,29 @@ PSFR_API int psfr_compute_ao(psfr_ctx* ctx, int field, int ndraw, const double* 
                        const double* fracs, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
                        double* out_efit, double* out_mean_efit, double* out_ee, double* out_mean_ee,
                        double* out_strehl, double* out_var, void* stream);
+
+/* Band images (PSFR_MAX_BANDS above) of ncube image sets cubes [ncube][nlam][ny][nx] -> out [ncube][nband][ny][nx],
+ * weights [nband][nlam].  Host or device pointers; host arrays go through the staging buffers in chunks.  nlam must
+ * not exceed max_lambda (PSFR_E_CAPACITY). */
+PSFR_API int psfr_band_psf(psfr_ctx* ctx, int ncube, int nlam, int ny, int nx, const double* cubes, int nband,
+                           const double* weights, double* out, void* stream);
+
+/* psfr_compute_ao plus the band images of every image set it forms (P = ndir with field, 1 without):
+ * out_band [ndraw][P][nband][40][40], the bands of the planes in out_cube; out_band_fit [ndraw][P][nband][PSFR_FIT_NPAR]
+ * and out_band_ee [ndraw][P][nband][nrad + 1 + nfrac], psfr_moffat_fit and psfr_encircled_energy (default centre) of
+ * those band images, bit for bit; out_mean_band, out_mean_band_fit and out_mean_band_ee [ngroup][P][nband]... the same
+ * for the exposure means, bit for bit psfr_band_psf of out_mean (not the mean of the per-draw bands).  The bands of a
+ * chunk run after its convolutions, those of the means after the exposure's mean is formed.  Every output may be NULL,
+ * and a NULL output launches nothing; with nband = 0 and every band output NULL the call is psfr_compute_ao (weights
+ * may then be NULL).  The other outputs are those of psfr_compute_ao, bit for bit. */
+PSFR_API int psfr_compute_bands(psfr_ctx* ctx, int field, int ndraw, const double* draws, int npos,
+                       const double* poslgs, int ndir, const double* dirs, int nlam, const double* lambda_nm,
+                       int ngroup, const int* group_end, int nrad, const double* radii_px, int nfrac,
+                       const double* fracs, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
+                       double* out_efit, double* out_mean_efit, double* out_ee, double* out_mean_ee,
+                       double* out_strehl, double* out_var, int nband, const double* weights, double* out_band,
+                       double* out_band_fit, double* out_band_ee, double* out_mean_band, double* out_mean_band_fit,
+                       double* out_mean_band_ee, void* stream);
 
 /* Time-mean of ncube cubes + refit (psfrec.py:1104-1105). cubes [ncube][nlam][40][40]. */
 PSFR_API int psfr_mean_refit(psfr_ctx* ctx, int ncube, int nlam, const double* cubes,

@@ -46,6 +46,8 @@ def ee_slots(nrad, nfrac):
 # residual-phase variance record of a (draw, direction) plane (PSFR_VAR_*), nm^2
 VAR_TOTAL, VAR_FIT, VAR_NOISE, VAR_PROJ, VAR_LAYER0 = 0, 1, 2, 3, 4
 VAR_NPAR = 12
+# band images (PSFR_MAX_BANDS): at most this many filter-weighted wavelength sums per call
+MAX_BANDS = 16
 
 AO_DIM = 80
 PSF_DIM = 40
@@ -95,6 +97,9 @@ _SIGNATURES = {
                                  _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     'psfr_compute_ao': (_I, [_P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P,
                              _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'psfr_band_psf': (_I, [_P, _I, _I, _I, _I, _P, _I, _P, _P, _P]),
+    'psfr_compute_bands': (_I, [_P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P,
+                                _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     'psfr_mean_refit': (_I, [_P, _I, _I, _P, _P, _P, _P]),
     'psfr_polyfit': (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     'psfr_set_option': (_I, [_P, _I, _D]),
@@ -163,6 +168,17 @@ def group_end_ptr(group_end):
     if not group_end.flags['C_CONTIGUOUS']:
         raise ValueError('group_end must be C-contiguous')
     return int(group_end.size), (group_end.ctypes.data if group_end.size else None)
+
+
+def band_weights_array(weights, nlam):
+    """Band weights as a C-contiguous float64 array [nband, nlam] (one band from a 1-D array, [0, nlam] from None);
+    the library checks their values."""
+    if weights is None:
+        return np.empty((0, int(nlam)))
+    w = np.array(weights, dtype=np.float64, ndmin=2, order='C')
+    if w.ndim != 2 or w.shape[1] != int(nlam):
+        raise ValueError('band weights must be [nband, %d] (got shape %s)' % (int(nlam), w.shape))
+    return w
 
 
 def checked_ptr(a, count, device, name, writable=False):
@@ -343,6 +359,32 @@ class Context:
                      out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit),
                      energy=(rad, fr, out_ee, out_mean_ee), ao=(out_strehl, out_var))
 
+    def compute_bands(self, field, draws, dirs, poslgs, lambda_nm, weights, radii_px=(), fracs=(), group_end=None,
+                      out_cube=None, out_fit=None, out_mean=None, out_mean_fit=None, out_efit=None, out_mean_efit=None,
+                      out_ee=None, out_mean_ee=None, out_strehl=None, out_var=None, out_band=None, out_band_fit=None,
+                      out_band_ee=None, out_mean_band=None, out_mean_band_fit=None, out_mean_band_ee=None,
+                      stream=None):
+        """psfr_compute_bands: ``compute_ao`` plus the band images of every image set it forms for the weights
+        [nband, nl] (or None: no bands), ``out_band`` [ndraw, P, nband, 40, 40], ``out_band_fit`` [ndraw, P, nband,
+        FIT_NPAR], ``out_band_ee`` [ndraw, P, nband, rec], and the same of the exposure means, ``out_mean_band*``
+        [ngroup, P, nband, ...] (P = npos with ``field``, 1 without)."""
+        rad, fr = f64(radii_px).ravel(), f64(fracs).ravel()
+        self._groups(self._lib.psfr_compute_bands, bool(field), draws, dirs, poslgs, lambda_nm, group_end, out_cube,
+                     out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit),
+                     energy=(rad, fr, out_ee, out_mean_ee), ao=(out_strehl, out_var),
+                     bands=(weights, out_band, out_band_fit, out_band_ee, out_mean_band, out_mean_band_fit,
+                            out_mean_band_ee))
+
+    def band_psf(self, ncube, nlam, ny, nx, cubes, weights, out, stream=None):
+        """psfr_band_psf: band images ``out`` [ncube, nband, ny, nx] of ``cubes`` [ncube, nlam, ny, nx] for the
+        weights [nband, nlam]."""
+        ncube, nlam, ny, nx = int(ncube), int(nlam), int(ny), int(nx)
+        w = band_weights_array(weights, nlam)
+        self._check(self._lib.psfr_band_psf(self._handle(), ncube, nlam, ny, nx,
+                                            self._buf(cubes, ncube * nlam * ny * nx, 'cubes'), w.shape[0],
+                                            ptr(w) if w.size else None,
+                                            self._buf(out, ncube * w.shape[0] * ny * nx, 'out', True), stream))
+
     def compute_batch(self, draws, dirs, poslgs, lambda_nm, out_cube=None, out_fit=None, stream=None):
         if not hasattr(draws, 'data_ptr'):      # numpy / sequence; torch tensors pass through as buffers
             draws = f64(draws)
@@ -380,7 +422,7 @@ class Context:
                          out_cube, out_fit, out_mean, out_mean_fit, stream, shapes=(out_efit, out_mean_efit))
 
     def _groups(self, fn, field, draws, dirs, poslgs, lambda_nm, group_end, out_cube, out_fit, out_mean,
-                out_mean_fit, stream, shapes=None, energy=None, ao=None):
+                out_mean_fit, stream, shapes=None, energy=None, ao=None, bands=None):
         if not hasattr(draws, 'data_ptr'):
             draws = f64(draws)
         if len(draws.shape) != 2 or draws.shape[1] != DRAW_NPAR:
@@ -410,6 +452,17 @@ class Context:
         if ao is not None:
             args += [self._buf(ao[0], nd * nimg, 'out_strehl', True),
                      self._buf(ao[1], nd * dirs.shape[1] * VAR_NPAR, 'out_var', True)]
+        if bands is not None:
+            w = band_weights_array(bands[0], lam.size)
+            sets = w.shape[0] * (dirs.shape[1] if field else 1)     # band images per draw and per exposure
+            rec = ee_slots(energy[0].size, energy[1].size)[3]
+            args += [w.shape[0], ptr(w) if w.size else None]
+            img1 = PSF_DIM * PSF_DIM
+            for name, a, n, per in (('out_band', bands[1], nd, img1), ('out_band_fit', bands[2], nd, FIT_NPAR),
+                                    ('out_band_ee', bands[3], nd, rec), ('out_mean_band', bands[4], ng, img1),
+                                    ('out_mean_band_fit', bands[5], ng, FIT_NPAR),
+                                    ('out_mean_band_ee', bands[6], ng, rec)):
+                args.append(self._buf(a, n * sets * per, name, True))
         self._check(fn(*args, stream))
 
     def mean_refit(self, ncube, nlam, cubes, out_mean=None, out_fit=None, stream=None):

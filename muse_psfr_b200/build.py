@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libpsfr_b200.so')
 SOURCES = ['psfr_api.cu', 'psfr_passes.cu', 'psfr_hot.cu', 'psfr_hot2.cu', 'psfr_psd.cu', 'psfr_plane.cu', 'psfr_conv.cu',
-           'psfr_energy.cu', 'psfr_ao.cu']
+           'psfr_energy.cu', 'psfr_ao.cu', 'psfr_band.cu']
 HEADERS = ['psfr_internal.h', 'warp_fft.cuh', 'pass_kernel.cuh', 'fft_tables.h', 'fast_exp.cuh', 'tma.cuh', 'ee_geometry.h', '../../include/psfr.h']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=hidden', '--expt-relaxed-constexpr']

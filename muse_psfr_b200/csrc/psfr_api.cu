@@ -298,6 +298,71 @@ static int upload_ee_params(Ctx* c, int nrad, const double* radii, int nfrac, co
     return PSFR_OK;
 }
 
+// Band weights of a call [nband][nlam] (either side): checked on the host, their ascending-k sums to `sums`, and the
+// k-major zero-padded copy band_kernel reads to c->band_w, then to d_bandw (allocated on first use), stream-ordered.
+static int upload_band_weights(Ctx* c, int nband, int nlam, const double* weights, BandSums& sums, cudaStream_t s) {
+    if (nband < 1 || nband > PSFR_MAX_BANDS)
+        return set_error(c, PSFR_E_ARG, "nband=%d outside [1, %d]", nband, PSFR_MAX_BANDS);
+    if (!weights) return set_error(c, PSFR_E_ARG, "NULL band weights");
+    if (nlam < 1) return set_error(c, PSFR_E_ARG, "nlam=%d", nlam);
+    std::vector<double> h;
+    if (int rc = small_to_host(c, h, weights, (size_t)nband * nlam, s)) return rc;
+    for (int b = 0; b < PSFR_MAX_BANDS; ++b) sums.w[b] = 1.0;
+    for (int b = 0; b < nband; ++b) {
+        double W = 0.0;
+        for (int k = 0; k < nlam; ++k) {
+            const double v = h[(size_t)b * nlam + k];
+            if (!(std::isfinite(v) && v >= 0.0))
+                return set_error(c, PSFR_E_ARG, "band %d: weight %d is %g; weights must be finite and >= 0", b, k, v);
+            W += v;
+        }
+        if (!(std::isfinite(W) && W > 0.0))
+            return set_error(c, PSFR_E_ARG, "band %d: the weights sum to %g; the sum must be finite and > 0", b, W);
+        sums.w[b] = W;
+    }
+    if (nlam > c->max_lambda) return set_error(c, PSFR_E_CAPACITY, "nlam=%d exceeds max_lambda=%d", nlam, c->max_lambda);
+    if (!c->d_bandw) {
+        int rc = dev_alloc(c, &c->d_bandw, (size_t)c->max_lambda * PSFR_MAX_BANDS);
+        if (rc) return rc;
+    }
+    c->band_w.assign((size_t)nlam * PSFR_MAX_BANDS, 0.0);
+    for (int b = 0; b < nband; ++b)
+        for (int k = 0; k < nlam; ++k) c->band_w[(size_t)k * PSFR_MAX_BANDS + b] = h[(size_t)b * nlam + k];
+    PSFR_CUDA(c, cudaMemcpyAsync(c->d_bandw, c->band_w.data(), c->band_w.size() * sizeof(double),
+                                 cudaMemcpyHostToDevice, s));
+    return PSFR_OK;
+}
+
+// the double-buffered band staging of the fused pipeline, allocated by the first call that computes bands: a context
+// that never does keeps its footprint
+static int alloc_band_staging(Ctx* c) {
+    if (c->d_mbee[1]) return PSFR_OK;   // the last buffer allocated below
+    const size_t sets = (size_t)c->max_planes * PSFR_MAX_BANDS;
+    for (int i = 0; i < 2; ++i) {   // after a failed attempt, start again
+        cudaFree(c->d_band[i]); cudaFree(c->d_bfit[i]); cudaFree(c->d_bee[i]);
+        cudaFree(c->d_mband[i]); cudaFree(c->d_mbfit[i]); cudaFree(c->d_mbee[i]);
+        c->d_band[i] = c->d_bfit[i] = c->d_bee[i] = c->d_mband[i] = c->d_mbfit[i] = c->d_mbee[i] = nullptr;
+    }
+    for (int i = 0; i < 2; ++i) {
+        int rc = dev_alloc(c, &c->d_band[i], sets * kPSF * kPSF);
+        if (!rc) rc = dev_alloc(c, &c->d_bfit[i], sets * PSFR_FIT_NPAR);
+        if (!rc) rc = dev_alloc(c, &c->d_bee[i], sets * kEeMaxRecord);
+        if (!rc) rc = dev_alloc(c, &c->d_mband[i], sets * kPSF * kPSF);
+        if (!rc) rc = dev_alloc(c, &c->d_mbfit[i], sets * PSFR_FIT_NPAR);
+        if (!rc) rc = dev_alloc(c, &c->d_mbee[i], sets * kEeMaxRecord);
+        if (rc) return rc;
+    }
+    return PSFR_OK;
+}
+
+// band outputs of a run_batch call: per-draw images, fits and EE records, then those of the exposure means
+struct BandOut {
+    int nband = 0;
+    BandSums sums;
+    double* out[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+};
+enum { kBand = 0, kBandFit = 1, kBandEe = 2, kMeanBand = 3, kMeanBandFit = 4, kMeanBandEe = 5 };
+
 constexpr int kMaxHotEvents = 512;
 struct HotTimer {
     cudaEvent_t ev[2 * kMaxHotEvents];
@@ -330,7 +395,8 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                      const double* poslgs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                      bool field, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
                      double* out_efit, double* out_mean_efit, int nrad, int nfrac, double* out_ee,
-                     double* out_mean_ee, double* out_strehl, double* out_var, cudaStream_t s) {
+                     double* out_mean_ee, double* out_strehl, double* out_var, cudaStream_t s,
+                     const BandOut* bo = nullptr) {
     PSFR_CUDA(c, cudaSetDevice(c->device));
     std::vector<double> lam;
     int rc = small_to_host(c, lam, lambda_nm, nlam > 0 ? nlam : 0, s);
@@ -365,11 +431,24 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     const bool mee_dev = out_mean_ee && is_device_ptr(out_mean_ee);
     const bool strehl_dev = out_strehl && is_device_ptr(out_strehl);
     const bool var_dev = out_var && is_device_ptr(out_var);
-    const bool means = out_mean || out_mean_fit || out_mean_efit || out_mean_ee;
+    // band outputs (DESIGN.md 5.6): bout[i] NULL or a pointer on either side, bdev[i] whether it is on the device
+    double* bout[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    bool bdev[6] = {false, false, false, false, false, false}, band_host = false;
+    const int nband = bo ? bo->nband : 0;
+    for (int i = 0; bo && i < 6; ++i) {
+        bout[i] = bo->out[i];
+        bdev[i] = bout[i] && is_device_ptr(bout[i]);
+        band_host |= bout[i] && !bdev[i];
+    }
+    const bool bands = bout[kBand] || bout[kBandFit] || bout[kBandEe];
+    const bool mbands = bout[kMeanBand] || bout[kMeanBandFit] || bout[kMeanBandEe];
+    const size_t bsets = (size_t)ppd * nband;                     // band images per draw and per exposure
+    const size_t belems = bsets * img, bfits = bsets * PSFR_FIT_NPAR, bees = bsets * (size_t)(nrad + 1 + nfrac);
+    const bool means = out_mean || out_mean_fit || out_mean_efit || out_mean_ee || mbands;
     const bool host_out = (out_cube && !cube_dev) || (out_fit && !fit_dev) || (out_mean && !mean_dev) ||
                           (out_mean_fit && !mfit_dev) || (out_efit && !efit_dev) || (out_mean_efit && !mefit_dev) ||
                           (out_ee && !ee_dev) || (out_mean_ee && !mee_dev) || (out_strehl && !strehl_dev) ||
-                          (out_var && !var_dev);
+                          (out_var && !var_dev) || band_host;
     int* seg_dev = reinterpret_cast<int*>(c->d_misc + misc_groups(c->max_planes));
     std::vector<int> seg;
     int g0 = 0;   // first exposure not finished in an earlier chunk
@@ -404,12 +483,22 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
         if (out_efit && (rc = run_efit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, efit, s))) break;
         double* ee = ee_dev ? out_ee + (size_t)d0 * ees : c->d_ee[b];
         if (out_ee && (rc = run_ee(c, nd * (int)imgs, kPSF, kPSF, conv, nullptr, nrad, nfrac, ee, s))) break;
+        // the band images of the chunk's image sets, read from the convolved planes, then their fits and EE
+        double* band = bdev[kBand] ? bout[kBand] + (size_t)d0 * belems : c->d_band[b];
+        if (bands && (rc = run_band(c, (long long)nd * ppd, nlam, (int)img, nband, bo->sums, conv, band, s))) break;
+        double* bfit = bdev[kBandFit] ? bout[kBandFit] + (size_t)d0 * bfits : c->d_bfit[b];
+        if (bout[kBandFit] && (rc = run_fit(c, nd * (int)bsets, kPSF, kPSF, band, bfit, s))) break;
+        double* bee = bdev[kBandEe] ? bout[kBandEe] + (size_t)d0 * bees : c->d_bee[b];
+        if (bout[kBandEe] && (rc = run_ee(c, nd * (int)bsets, kPSF, kPSF, band, nullptr, nrad, nfrac, bee, s))) break;
         // exposures g0, g0 + 1, ... that have draws in [d0, d0 + nd): all but possibly the last end here
         int ndone = 0;
         double* mean = mean_dev ? out_mean + (size_t)g0 * elems : c->d_mean[b];
         double* mfit = mfit_dev ? out_mean_fit + (size_t)g0 * fits : c->d_mfit[b];
         double* mefit = mefit_dev ? out_mean_efit + (size_t)g0 * efits : c->d_mefit[b];
         double* mee = mee_dev ? out_mean_ee + (size_t)g0 * ees : c->d_mee[b];
+        double* mband = bdev[kMeanBand] ? bout[kMeanBand] + (size_t)g0 * belems : c->d_mband[b];
+        double* mbfit = bdev[kMeanBandFit] ? bout[kMeanBandFit] + (size_t)g0 * bfits : c->d_mbfit[b];
+        double* mbee = bdev[kMeanBandEe] ? bout[kMeanBandEe] + (size_t)g0 * bees : c->d_mbee[b];
         if (means) {
             seg.clear();
             for (int g = g0; g < ngroup && (g == g0 || group_end[g - 1] < d0 + nd); ++g) {
@@ -428,6 +517,13 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                 break;
             if (out_mean_efit && ndone && (rc = run_efit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, mefit, s))) break;
             if (out_mean_ee && ndone && (rc = run_ee(c, ndone * (int)imgs, kPSF, kPSF, mean, nullptr, nrad, nfrac, mee, s)))
+                break;
+            if (mbands && ndone &&
+                (rc = run_band(c, (long long)ndone * ppd, nlam, (int)img, nband, bo->sums, mean, mband, s)))
+                break;
+            if (bout[kMeanBandFit] && ndone && (rc = run_fit(c, ndone * (int)bsets, kPSF, kPSF, mband, mbfit, s))) break;
+            if (bout[kMeanBandEe] && ndone &&
+                (rc = run_ee(c, ndone * (int)bsets, kPSF, kPSF, mband, nullptr, nrad, nfrac, mbee, s)))
                 break;
         }
         if (host_out) {
@@ -463,6 +559,15 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
             if (e == cudaSuccess && out_strehl && !strehl_dev)
                 e = cudaMemcpyAsync(out_strehl + (size_t)d0 * imgs, strehl, (size_t)nd * imgs * sizeof(double),
                                     cudaMemcpyDefault, c->copy_stream);
+            // band results: per-draw ones of the chunk's nd draws, those of the ndone exposures that end here
+            const double* bsrc[6] = {band, bfit, bee, mband, mbfit, mbee};
+            const size_t bper[6] = {belems, bfits, bees, belems, bfits, bees};
+            for (int i = 0; i < 6 && e == cudaSuccess; ++i) {
+                const size_t first = i < kMeanBand ? (size_t)d0 : (size_t)g0, count = i < kMeanBand ? nd : ndone;
+                if (bout[i] && !bdev[i] && count)
+                    e = cudaMemcpyAsync(bout[i] + first * bper[i], bsrc[i], count * bper[i] * sizeof(double),
+                                        cudaMemcpyDefault, c->copy_stream);
+            }
             if (e == cudaSuccess) e = cudaEventRecord(c->ev_copied[b], c->copy_stream);
             if (e != cudaSuccess) {
                 rc = set_error(c, PSFR_E_CUDA, "result copy failed: %s", cudaGetErrorString(e));
@@ -483,7 +588,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 105; }
+int psfr_version(void) { return 106; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -499,7 +604,11 @@ void psfr_destroy(psfr_ctx* c) {
     cudaFree(c->d_cube3); cudaFree(c->d_fit2); cudaFree(c->d_carry); cudaFree(c->d_efit); cudaFree(c->d_efit2);
     for (int i = 0; i < 2; ++i) { cudaFree(c->d_mean[i]); cudaFree(c->d_mfit[i]); cudaFree(c->d_mefit[i]); }
     for (int i = 0; i < 2; ++i) { cudaFree(c->d_ee[i]); cudaFree(c->d_mee[i]); cudaFree(c->d_strehl[i]); cudaFree(c->d_var[i]); }
-    cudaFree(c->d_eepar); cudaFree(c->d_eecen);
+    cudaFree(c->d_eepar); cudaFree(c->d_eecen); cudaFree(c->d_bandw);
+    for (int i = 0; i < 2; ++i) {
+        cudaFree(c->d_band[i]); cudaFree(c->d_bfit[i]); cudaFree(c->d_bee[i]);
+        cudaFree(c->d_mband[i]); cudaFree(c->d_mbfit[i]); cudaFree(c->d_mbee[i]);
+    }
     cudaFree(c->d_dphi32); cudaFree(c->d_otf32); cudaFree(c->d_tw32); cudaFree(c->d_twg); cudaFree(c->d_twg32); cudaFree(c->d_p3); cudaFree(c->d_p2mask); cudaFree(c->d_csort); cudaFree(c->d_lorder); cudaFree(c->d_kaddr);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     for (int i = 0; i < 2; ++i) {
@@ -1001,6 +1110,70 @@ int psfr_compute_ao(psfr_ctx* c, int field, int ndraw, const double* draws, int 
     return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
                      out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
                      out_mean_ee, out_strehl, out_var, s);
+}
+
+int psfr_compute_bands(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs,
+                       int ndir, const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
+                       int nrad, const double* radii_px, int nfrac, const double* fracs, double* out_cube,
+                       double* out_fit, double* out_mean, double* out_mean_fit, double* out_efit, double* out_mean_efit,
+                       double* out_ee, double* out_mean_ee, double* out_strehl, double* out_var, int nband,
+                       const double* weights, double* out_band, double* out_band_fit, double* out_band_ee,
+                       double* out_mean_band, double* out_mean_band_fit, double* out_mean_band_ee, void* stream) {
+    BandOut bo;
+    double* outs[6] = {out_band, out_band_fit, out_band_ee, out_mean_band, out_mean_band_fit, out_mean_band_ee};
+    bool any = false;
+    for (int i = 0; i < 6; ++i) {
+        bo.out[i] = outs[i];
+        any |= outs[i] != nullptr;
+    }
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
+                              out_mean || out_mean_fit || out_mean_efit || out_mean_ee || out_mean_band ||
+                              out_mean_band_fit || out_mean_band_ee))
+        return rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    if (any || nband != 0) {
+        if (int rc = upload_band_weights(c, nband, nlam, weights, bo.sums, s)) return rc;
+        bo.nband = nband;
+    }
+    if (any)
+        if (int rc = alloc_band_staging(c)) return rc;
+    if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
+                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
+                     out_mean_ee, out_strehl, out_var, s, any ? &bo : nullptr);
+}
+
+int psfr_band_psf(psfr_ctx* c, int ncube, int nlam, int ny, int nx, const double* cubes, int nband,
+                  const double* weights, double* out, void* stream) {
+    if (!c || !cubes || !out) return set_error(c, PSFR_E_ARG, "NULL argument");
+    if (ncube < 1 || nlam < 1 || ny < 1 || nx < 1)
+        return set_error(c, PSFR_E_ARG, "ncube=%d nlam=%d ny=%d nx=%d", ncube, nlam, ny, nx);
+    if ((long long)ny * nx > 0x7fffffff) return set_error(c, PSFR_E_ARG, "image %dx%d is too large", ny, nx);
+    if (nlam > c->max_lambda) return set_error(c, PSFR_E_CAPACITY, "nlam=%d exceeds max_lambda=%d", nlam, c->max_lambda);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    BandSums sums;
+    int rc = upload_band_weights(c, nband, nlam, weights, sums, s);
+    if (rc) return rc;
+    const size_t per = (size_t)ny * nx, in_set = (size_t)nlam * per, out_set = (size_t)nband * per;
+    const bool in_dev = is_device_ptr(cubes), out_dev = is_device_ptr(out);
+    // host arrays go through d_cube (inputs) and d_cube2 (outputs), each of cap doubles
+    const size_t cap = (size_t)c->max_planes * c->max_lambda * kPSF * kPSF;
+    const size_t chunk = (in_dev && out_dev) ? (size_t)ncube : cap / std::max(in_set, out_set);
+    if (chunk < 1) return set_error(c, PSFR_E_CAPACITY, "image set %dx%dx%d does not fit the staging buffer", nlam, ny, nx);
+    for (size_t i0 = 0; i0 < (size_t)ncube; i0 += chunk) {
+        const size_t n = std::min(chunk, (size_t)ncube - i0);
+        const double* src = cubes + i0 * in_set;
+        if (!in_dev) {
+            if ((rc = to_device(c, c->d_cube, src, n * in_set * sizeof(double), s))) return rc;
+            src = c->d_cube;
+        }
+        double* dst = out_dev ? out + i0 * out_set : c->d_cube2;
+        if ((rc = run_band(c, (long long)n, nlam, (int)per, nband, sums, src, dst, s))) return rc;
+        if (!out_dev && (rc = from_device(c, out + i0 * out_set, dst, n * out_set * sizeof(double), s))) return rc;
+    }
+    return PSFR_OK;
 }
 
 int psfr_mean_refit(psfr_ctx* c, int ncube, int nlam, const double* cubes, double* out_mean, double* out_fit,

@@ -156,6 +156,17 @@ struct Ctx {
     std::vector<double> ee_par;  // host copy of d_eepar's contents (outlives the asynchronous upload)
     double* d_strehl[2] = {nullptr, nullptr}; // [max_planes*max_lambda] Strehl ratios (double-buffered as d_ee)
     double* d_var[2] = {nullptr, nullptr};    // [max_planes][PSFR_VAR_NPAR] variance records (double-buffered)
+    // band images (DESIGN.md 5.6), allocated by the first call that needs them (alloc_band_staging): weights
+    // [max_lambda][PSFR_MAX_BANDS] k-major, and per staging set b images [max_planes * PSFR_MAX_BANDS][40][40], fit and
+    // EE records of the per-draw bands and of the exposure means' bands
+    double* d_bandw = nullptr;
+    std::vector<double> band_w;  // host copy of d_bandw's contents (outlives the asynchronous upload)
+    double* d_band[2] = {nullptr, nullptr};
+    double* d_bfit[2] = {nullptr, nullptr};
+    double* d_bee[2] = {nullptr, nullptr};
+    double* d_mband[2] = {nullptr, nullptr};
+    double* d_mbfit[2] = {nullptr, nullptr};
+    double* d_mbee[2] = {nullptr, nullptr};
     cudaStream_t copy_stream = nullptr;      // device -> host copies of finished chunks
     cudaEvent_t ev_done[2] = {nullptr, nullptr};    // chunk results ready (compute stream)
     cudaEvent_t ev_copied[2] = {nullptr, nullptr};  // chunk results copied out (copy stream)
@@ -269,6 +280,16 @@ int run_var(Ctx* c, int ndraw, int ndir, int ngs, int npos, double* out_dev, cud
 int run_otf_sum(Ctx* c, cudaStream_t s);
 // Strehl ratio of the nimg PSFs run_pruned_psf left in d_samp (raw samples, before clip and normalisation)
 int run_strehl(Ctx* c, int nimg, double* out_dev, cudaStream_t s);
+
+// ---- psfr_band.cu --------------------------------------------------------------------
+// W_b = sum_k w[b][k] in ascending k of every band; unused slots hold 1
+struct BandSums {
+    double w[PSFR_MAX_BANDS];
+};
+// band images out [nset][nband][npix] of the image sets in [nset][nlam][npix]: (sum_k fma(w[b][k], in[k], .)) / W_b in
+// ascending k, with the weights c->d_bandw [nlam][PSFR_MAX_BANDS] holds
+int run_band(Ctx* c, long long nset, int nlam, int npix, int nband, const BandSums& sums, const double* in_dev,
+             double* out_dev, cudaStream_t s);
 
 // ---- psfr_plane.cu -------------------------------------------------------------------
 // moffat_kernels_kernel divides by pi * gamma^2, evaluated as (pi * gamma) * gamma: the kernel is finite for

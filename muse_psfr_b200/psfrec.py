@@ -17,7 +17,7 @@ from ._lib import PsfrError
 
 __all__ = ['compute_psf_from_sparta', 'compute_psf_from_sparta_batch', 'compute_psf', 'compute_psf_batch',
            'reconstruct_psf', 'create_sparta_table', 'fit_psf_with_polynom', 'simul_psd_wfm', 'psd_to_psf', 'psf_muse',
-           'convolve_final_psf', 'fit_psf_cube', 'compute_psf_field', 'encircled_energy',
+           'convolve_final_psf', 'fit_psf_cube', 'compute_psf_field', 'encircled_energy', 'band_weights', 'band_psf',
            'muse_intrinsic_psf', 'direction_perf', 'seeing2r01', 'pupil_mask', 'select_sparta_rows', 'FitTable',
            'PsfrError', 'MIN_L0', 'MAX_L0']
 
@@ -373,6 +373,96 @@ def _ao_table(lbda, strehl, var):
     })
 
 
+def band_weights(lbda, band_lbda, throughput):
+    """Weights [nl] of one band on the wavelength grid ``lbda`` [nm] (DESIGN.md section 5.6): the trapezoid-rule
+    quadrature of the throughput curve ``T = np.interp(lbda, band_lbda, throughput, left=0, right=0)`` on that grid,
+    ``w_k = T(lbda_k) * delta_k`` with ``delta_k`` half the distance between the neighbours of k (of its one neighbour
+    at either end; 1 for a single wavelength).  ``sum(w)`` is the trapezoid integral of T over the grid.
+
+    A top-hat is ``band_lbda=[lo, hi], throughput=[1, 1]``; stack several calls for several bands.  The weights are
+    those of a photon-flat source: an SED and photon-counting factors (such as lambda) are the caller's, folded into
+    ``throughput``.  Raises ValueError for a grid (``lbda`` or ``band_lbda``) that is not strictly increasing, a
+    negative or non-finite throughput, and a band that puts no weight on the grid."""
+    lam = np.array(lbda, dtype=float, ndmin=1)
+    bl = np.array(band_lbda, dtype=float, ndmin=1)
+    tp = np.array(throughput, dtype=float, ndmin=1)
+    for name, x in (('lbda', lam), ('band_lbda', bl)):
+        if x.ndim != 1 or x.size == 0 or not np.all(np.isfinite(x)) or np.any(np.diff(x) <= 0):
+            raise ValueError('%s must be a finite, strictly increasing 1-D grid' % name)
+    if tp.shape != bl.shape:
+        raise ValueError('throughput must hold one value per band_lbda (got %d for %d)' % (tp.size, bl.size))
+    if not np.all(np.isfinite(tp)) or np.any(tp < 0):
+        raise ValueError('throughput must be finite and >= 0')
+    delta = np.ones(1)
+    if lam.size > 1:
+        delta = np.empty(lam.size)
+        delta[0], delta[-1] = (lam[1] - lam[0]) / 2, (lam[-1] - lam[-2]) / 2
+        delta[1:-1] = (lam[2:] - lam[:-2]) / 2
+    w = np.interp(lam, bl, tp, left=0, right=0) * delta
+    if not w.sum() > 0:
+        raise ValueError('the band [%g, %g] nm puts no weight on the grid [%g, %g] nm' % (bl[0], bl[-1], lam[0], lam[-1]))
+    return w
+
+
+def _band_params(bands, nl):
+    """Band weights of a request, [nband, nl] or [nl] for one band, checked as the library checks them (DESIGN.md
+    section 5.6): 1 to MAX_BANDS bands, weights finite and >= 0, each band's sum in ascending order finite and > 0.
+    Returns a C-contiguous float64 array [nband, nl]."""
+    w = np.array(bands, dtype=float, ndmin=2)
+    if w.ndim != 2 or w.shape[1] != nl:
+        raise ValueError('bands must be [nband, %d] or [%d] (got shape %s)' % (nl, nl, w.shape))
+    if not 1 <= w.shape[0] <= _lib.MAX_BANDS:
+        raise ValueError('bands must hold 1 to %d bands (got %d)' % (_lib.MAX_BANDS, w.shape[0]))
+    if not np.all(np.isfinite(w)) or np.any(w < 0):
+        raise ValueError('band weights must be finite and >= 0')
+    total = _band_sums(w)
+    if not np.all(np.isfinite(total) & (total > 0)):
+        raise ValueError('every band\'s weights must sum to a finite value > 0 (sums %s)' % total.tolist())
+    return np.ascontiguousarray(w)
+
+
+def _band_sums(w):
+    """W_b = sum_k w[b][k], added in ascending k (the order of the library's sums)."""
+    return np.cumsum(w, axis=1)[:, -1] if w.shape[1] else np.zeros(len(w))
+
+
+def _band_lbda_eff(lbda, w):
+    """Effective wavelength of every band [nband]: sum_k w[b][k] lbda[k] / W_b, summed in ascending k."""
+    return _band_sums(w * np.asarray(lbda, dtype=float)) / _band_sums(w)
+
+
+def _band_columns(lbda, w, fit, ee=None, radii=(), fractions=()):
+    """Columns of a band table for the band fit records [n, nband, FIT_NPAR] (flattened; n = 1 or the positions):
+    the ``_fit_columns`` with ``lbda`` the band's effective wavelength, ``band`` (index), ``weights`` [nl] per row,
+    and the ``_ee_columns`` of the band EE records [n, nband, rec] when given."""
+    lbda_eff = _band_lbda_eff(lbda, w)
+    cols = _fit_columns(lbda_eff, fit)
+    reps = len(cols['lbda']) // len(w)
+    cols['band'] = np.tile(np.arange(len(w), dtype=np.int64), reps)
+    cols['weights'] = np.tile(w, (reps, 1))
+    if ee is not None:
+        cols.update(_ee_columns(lbda_eff, ee, radii, fractions))
+    return cols
+
+
+def band_psf(psfcube, weights):
+    """Band images of a cube [nl, ny, nx] -> [nband, ny, nx], or of cubes [n, nl, ny, nx] -> [n, nband, ny, nx], on
+    the device (DESIGN.md section 5.6): ``B[b] = sum_k w[b][k] C[k] / W_b`` with the FP64 sum in ascending k, for
+    ``weights`` [nband, nl] or [nl] (``band_weights``).  The band image keeps the flux scale of the planes.  Invalid
+    weights raise ValueError before any device call."""
+    data = getattr(psfcube, 'data', psfcube)
+    data = np.ascontiguousarray(np.ma.getdata(data), dtype=np.float64)
+    if data.ndim not in (3, 4):
+        raise ValueError('psfcube must be [nl, ny, nx] or [n, nl, ny, nx]')
+    cubes = data if data.ndim == 4 else data[None]
+    n, nl, ny, nx = cubes.shape
+    w = _band_params(weights, nl)
+    out = np.empty((n, w.shape[0], ny, nx))
+    if out.size:
+        get_context(max_lambda=nl).band_psf(n, nl, ny, nx, cubes, w, out)
+    return out if data.ndim == 4 else out[0]
+
+
 # --------------------------------------------------------------------------- reference API
 def simul_psd_wfm(Cn2, h, seeing, L0, zenith=0., plot=False, npsflin=1, dim=1280,
                   three_lgs_mode=False, verbose=True, wind_dir=None):
@@ -612,10 +702,20 @@ def _planes_context(nd, ndir, nlam, max_planes, device, dim):
                        dim=dim)
 
 
+def _band_outputs(bands, nl, lead, ee_rec):
+    """(band_fit, band_cube[, band_ee]) buffers [*lead, nband, ...] of a ``bands=`` request (checked by
+    ``_band_params``; ValueError before any device call), or () without one."""
+    if bands is None:
+        return ()
+    nb = _band_params(bands, nl).shape[0]
+    out = (np.empty(lead + (nb, _lib.FIT_NPAR)), np.empty(lead + (nb, _lib.PSF_DIM, _lib.PSF_DIM)))
+    return out + ((np.empty(lead + (nb, ee_rec)),) if ee_rec is not None else ())
+
+
 def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs_mode=False,
                       out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None, stream=None,
                       dim=_DIM, zenith=0., Cn2=None, wind_dir=None, ee_radii=None, ee_fractions=(0.5, 0.8),
-                      ao_budget=False):
+                      ao_budget=False, bands=None):
     """Batched ``compute_psf``: one fused device pipeline for many (seeing, GL, L0[, h]) draws.
 
     ``h`` is one (h0, h1) pair or an array [ndraw, 2].  ``three_lgs_mode`` is one flag for all draws or
@@ -632,7 +732,14 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     ``ao_budget=True`` appends (strehl [ndraw, nl], var [ndraw, npsflin**2, VAR_NPAR]) after the other results:
     the AO Strehl ratio of every PSF and the residual-phase variance record (nm^2, ``_lib.VAR_*``) of every
     (draw, direction) plane, computed on the device in the same pass (DESIGN.md section 5.5; ``_ao_table`` turns
-    them into columns).  Every other result is that of a call without it, bit for bit."""
+    them into columns).  Every other result is that of a call without it, bit for bit.
+
+    ``bands`` (weights [nband, nl] or [nl], ``band_weights``) appends (band_fit [ndraw, nband, FIT_NPAR], band_cube
+    [ndraw, nband, 40, 40]) after every other result, and band_ee [ndraw, nband, nrad + 1 + nfrac] when ``ee_radii``
+    is given: the band image of every draw, ``sum_k w[b][k] cube[k] / W_b``, its Moffat fit and encircled energy,
+    formed on the device from the convolved planes (DESIGN.md section 5.6).  band_cube is returned with
+    ``want_cube=False`` too.  Every other result is that of a call without ``bands``, bit for bit; invalid weights
+    raise ValueError before any device call."""
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
     seeing, GL, L0 = (np.atleast_1d(np.asarray(v, dtype=float)) for v in (seeing, GL, L0))
     nd = seeing.size
@@ -647,7 +754,8 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         ee = np.empty((nd, lam.size, _lib.ee_slots(rad_px.size, frac.size)[3]))
     ndir = npsflin * npsflin
     ao = (np.empty((nd, lam.size)), np.empty((nd, ndir, _lib.VAR_NPAR))) if ao_budget else ()
-    extra = ((ee,) if energy else ()) + ao
+    band = _band_outputs(bands, lam.size, (nd,), ee.shape[-1] if energy else None)
+    extra = ((ee,) if energy else ()) + ao + band
     if nd == 0 or lam.size == 0:
         # nothing to compute: empty results of the right shape, written through nothing
         return (np.empty((nd, lam.size, _lib.FIT_NPAR)),
@@ -656,7 +764,7 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         recs = _mode_records(three, seeing, GL, L0, h, zenith, Cn2, wind_dir)
     else:
         recs = _batch_records(seeing, GL, L0, h, zenith, Cn2, wind_dir)
-        if energy or ao_budget:      # the groups path takes each draw's guide-star count from its record
+        if energy or ao_budget or band:      # the groups path takes each draw's guide-star count from its record
             recs[:, _lib.DRAW_NGS] = 3 if three_lgs_mode else 4
     dirs = direction_perf(npsflin)
     dim = _check_dim(dim)
@@ -666,7 +774,13 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        if ao_budget:
+        if band:
+            ctx.compute_bands(False, recs, dirs, _lgs_positions(False), lam, _band_params(bands, lam.size),
+                              rad_px if energy else (), frac if energy else (), out_cube=out_cube, out_fit=out_fit,
+                              out_ee=ee if energy else None, out_strehl=ao[0] if ao else None,
+                              out_var=ao[1] if ao else None, out_band=band[1], out_band_fit=band[0],
+                              out_band_ee=band[2] if energy else None, stream=stream)
+        elif ao_budget:
             ctx.compute_ao(False, recs, dirs, _lgs_positions(False), lam, rad_px if energy else (),
                            frac if energy else (), out_cube=out_cube, out_fit=out_fit, out_ee=ee if energy else None,
                            out_strehl=ao[0], out_var=ao[1], stream=stream)
@@ -689,7 +803,7 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
 def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_size=60, h=(100, 10000),
                       three_lgs_mode=False, out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None,
                       stream=None, dim=_DIM, zenith=0., Cn2=None, wind_dir=None, elliptical=False, ee_radii=None,
-                      ee_fractions=(0.5, 0.8), ao_budget=False):
+                      ee_fractions=(0.5, 0.8), ao_budget=False, bands=None):
     """Field-resolved ``compute_psf_batch``: the PSF of every draw at every field position instead of
     their average.
 
@@ -711,7 +825,11 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
 
     ``ao_budget=True`` appends (strehl [ndraw, npos, nl], var [ndraw, npos, VAR_NPAR]) last, as
     ``compute_psf_batch(ao_budget=True)`` does: the Strehl ratio of each position's PSF and the variance record of
-    each (draw, position) plane."""
+    each (draw, position) plane.
+
+    ``bands`` appends (band_fit [ndraw, npos, nband, FIT_NPAR], band_cube [ndraw, npos, nband, 40, 40]) and, with
+    ``ee_radii``, band_ee [ndraw, npos, nband, nrad + 1 + nfrac] after everything else, as ``compute_psf_batch(bands=...)``
+    does, for the PSF of each position."""
     pos = _field_positions(direction_perf(npsflin, field_size) if positions is None else positions)
     npos = pos.shape[1]
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
@@ -726,7 +844,8 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
         rad_px, frac = _ee_params(ee_radii, ee_fractions)
         ee = np.empty((nd, npos, lam.size, _lib.ee_slots(rad_px.size, frac.size)[3]))
     ao = (np.empty((nd, npos, lam.size)), np.empty((nd, npos, _lib.VAR_NPAR))) if ao_budget else ()
-    extra = ((efit,) if elliptical else ()) + ((ee,) if energy else ()) + ao
+    band = _band_outputs(bands, lam.size, (nd, npos), ee.shape[-1] if energy else None)
+    extra = ((efit,) if elliptical else ()) + ((ee,) if energy else ()) + ao + band
     if nd == 0 or lam.size == 0:
         return (np.empty((nd, npos, lam.size, _lib.FIT_NPAR)),
                 np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM)) if want_cube else None) + extra
@@ -740,7 +859,13 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
     try:
-        if ao_budget:
+        if band:
+            ctx.compute_bands(True, recs, pos, _lgs_positions(False), lam, _band_params(bands, lam.size),
+                              rad_px if energy else (), frac if energy else (), out_cube=out_cube, out_fit=out_fit,
+                              out_efit=efit, out_ee=ee if energy else None, out_strehl=ao[0] if ao else None,
+                              out_var=ao[1] if ao else None, out_band=band[1], out_band_fit=band[0],
+                              out_band_ee=band[2] if energy else None, stream=stream)
+        elif ao_budget:
             ctx.compute_ao(True, recs, pos, _lgs_positions(False), lam, rad_px if energy else (),
                            frac if energy else (), out_cube=out_cube, out_fit=out_fit, out_efit=efit,
                            out_ee=ee if energy else None, out_strehl=ao[0], out_var=ao[1], stream=stream)
@@ -857,7 +982,7 @@ def _ee_cards(meta, radii, fractions):
 def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                             lbda=None, h=(100, 10000), n_jobs=-1, plot=False, mean_of_lgs=True,
                             verbose=True, device=None, field_positions=None, elliptical=False, ee_radii=None,
-                            ee_fractions=(0.5, 0.8), ao_budget=False):
+                            ee_fractions=(0.5, 0.8), ao_budget=False, bands=None):
     """Reconstruct a PSF from SPARTA data (psfrec.py:981-1120).
 
     ``filename``: path of a FITS file, a binary file object, or an HDUList (this package's or
@@ -867,20 +992,22 @@ def compute_psf_from_sparta(filename, extname='SPARTA_ATM_DATA', npsflin=1, lmin
     FIT_MEAN, PSF_MEAN] - an ``astropy.io.fits.HDUList`` when astropy is installed, otherwise
     the equivalent object of ``muse_psfr_b200._fits`` - or None when no row is valid.  With
     ``field_positions`` [2, npos] (arcsec), FIT_FIELD and PSF_FIELD follow, with ``elliptical=True``
-    SHAPE_MEAN (and SHAPE_FIELD), with ``ee_radii`` EE_MEAN (and EE_FIELD), and with ``ao_budget=True`` AO_MEAN
-    (and AO_FIELD): see ``compute_psf_from_sparta_batch``."""
+    SHAPE_MEAN (and SHAPE_FIELD), with ``ee_radii`` EE_MEAN (and EE_FIELD), with ``ao_budget=True`` AO_MEAN
+    (and AO_FIELD), and with ``bands`` BAND_MEAN and PSF_BAND (and BAND_FIELD, PSF_BAND_FIELD): see
+    ``compute_psf_from_sparta_batch``."""
     if plot:
         raise NotImplementedError('plotting is outside the B200 hot path')
     return compute_psf_from_sparta_batch([filename], extname=extname, npsflin=npsflin, lmin=lmin, lmax=lmax, nl=nl,
                                          lbda=lbda, h=h, n_jobs=n_jobs, mean_of_lgs=mean_of_lgs, verbose=verbose,
                                          device=device, field_positions=field_positions, elliptical=elliptical,
-                                         ee_radii=ee_radii, ee_fractions=ee_fractions, ao_budget=ao_budget)[0]
+                                         ee_radii=ee_radii, ee_fractions=ee_fractions, ao_budget=ao_budget,
+                                         bands=bands)[0]
 
 
 def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1, lmin=490, lmax=930, nl=35,
                                   lbda=None, h=(100, 10000), n_jobs=-1, mean_of_lgs=True, verbose=True,
                                   device=None, max_planes=None, field_positions=None, elliptical=False,
-                                  ee_radii=None, ee_fractions=(0.5, 0.8), ao_budget=False):
+                                  ee_radii=None, ee_fractions=(0.5, 0.8), ao_budget=False, bands=None):
     """``compute_psf_from_sparta`` for many exposures in one device pass: returns one entry per source,
     the HDUList ``compute_psf_from_sparta(source, ...)`` returns, bit for bit, or None for a table
     without a valid row.
@@ -913,11 +1040,22 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     its draws in draw order (for the variance, over the directions of each draw too), from the Strehl ratios and
     variance records the mean pass computes on the device.  With ``field_positions`` AO_FIELD follows, the same
     columns plus ``x`` and ``y`` per (position, wavelength), position-major, from the field pass.  Every HDU before
-    them is that of a call without ``ao_budget``, bit for bit."""
+    them is that of a call without ``ao_budget``, bit for bit.
+
+    ``bands`` (weights [nband, nl] or [nl] on ``lbda``, ``band_weights``) appends BAND_MEAN and PSF_BAND after every
+    other HDU.  PSF_BAND is an image [nband, 40, 40], the band images of PSF_MEAN (DESIGN.md section 5.6), formed on
+    the device in the mean pass; it is the band of the exposure's mean cube, not the mean of its draws' bands.
+    BAND_MEAN holds one row per band: the columns of FIT_MEAN for the Moffat fit of the band image, with ``lbda`` the
+    band's effective wavelength sum_k w_k lbda_k / sum_k w_k, a ``band`` index, the band's ``weights`` [nl], and the
+    ``encircled_energy`` columns when ``ee_radii`` is given; the cards of FIT_MEAN (plus EERADk / EEFRACk with
+    ``ee_radii``).  With ``field_positions`` BAND_FIELD (the same columns plus ``x`` and ``y``, one row per (position,
+    band), position-major) and PSF_BAND_FIELD [npos, nband, 40, 40] follow, from the field pass.  Every HDU before
+    them is that of a call without ``bands``, bit for bit; invalid weights raise ValueError before any device call."""
     if lbda is None:
         lbda = np.linspace(lmin, lmax, nl)
     lbda = np.atleast_1d(np.asarray(lbda, dtype=float))
     pos = None if field_positions is None else _field_positions(field_positions)
+    w_band = None if bands is None else _band_params(bands, lbda.size)
     energy = ee_radii is not None
     if energy:
         rad_px, frac = _ee_params(ee_radii, ee_fractions)
@@ -963,6 +1101,14 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
         if ao_budget:
             strehl = np.empty((nd, nlam))
             var = np.empty((nd, dirs.shape[1], _lib.VAR_NPAR))
+        if w_band is not None:
+            band_mean = _band_outputs(w_band, nlam, (ng,), ee_rec if energy else None)
+            ctx.compute_bands(False, draws, dirs, _lgs_positions(False), lbda, w_band, rad_px if energy else (),
+                              frac if energy else (), group_end, out_fit=fit, out_mean=psftot, out_mean_fit=fit_mean,
+                              out_mean_ee=ee_mean if energy else None, out_strehl=strehl if ao_budget else None,
+                              out_var=var if ao_budget else None, out_mean_band=band_mean[1],
+                              out_mean_band_fit=band_mean[0], out_mean_band_ee=band_mean[2] if energy else None)
+        elif ao_budget:
             ctx.compute_ao(False, draws, dirs, _lgs_positions(False), lbda, rad_px if energy else (),
                            frac if energy else (), group_end, out_fit=fit, out_mean=psftot, out_mean_fit=fit_mean,
                            out_mean_ee=ee_mean if energy else None, out_strehl=strehl, out_var=var)
@@ -983,6 +1129,15 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
             if ao_budget:
                 strehl_field = np.empty((nd, npos, nlam))
                 var_field = np.empty((nd, npos, _lib.VAR_NPAR))
+            if w_band is not None:
+                band_field = _band_outputs(w_band, nlam, (ng, npos), ee_rec if energy else None)
+                ctx.compute_bands(True, draws, pos, _lgs_positions(False), lbda, w_band, rad_px if energy else (),
+                                  frac if energy else (), group_end, out_mean=psf_field, out_mean_fit=fit_field,
+                                  out_mean_efit=shape_field, out_mean_ee=ee_field if energy else None,
+                                  out_strehl=strehl_field if ao_budget else None,
+                                  out_var=var_field if ao_budget else None, out_mean_band=band_field[1],
+                                  out_mean_band_fit=band_field[0], out_mean_band_ee=band_field[2] if energy else None)
+            elif ao_budget:
                 ctx.compute_ao(True, draws, pos, _lgs_positions(False), lbda, rad_px if energy else (),
                                frac if energy else (), group_end, out_mean=psf_field, out_mean_fit=fit_field,
                                out_mean_efit=shape_field, out_mean_ee=ee_field if energy else None,
@@ -1056,6 +1211,19 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
                 cols['x'] = np.repeat(pos[0], nlam)
                 cols['y'] = np.repeat(pos[1], nlam)
                 out.append(_fits.table_to_hdu(cols, meta=meta, name='AO_FIELD'))
+        if w_band is not None:
+            cards = _ee_cards(meta, ee_rad, frac) if energy else meta
+            ee_args = (band_mean[2][g], ee_rad, frac) if energy else ()
+            out.append(_fits.table_to_hdu(_band_columns(lbda, w_band, band_mean[0][g], *ee_args), meta=cards,
+                                          name='BAND_MEAN'))
+            out.append(_fits.ImageHDU(data=band_mean[1][g], name='PSF_BAND'))
+            if pos is not None:
+                ee_args = (band_field[2][g], ee_rad, frac) if energy else ()
+                cols = _band_columns(lbda, w_band, band_field[0][g], *ee_args)
+                cols['x'] = np.repeat(pos[0], len(w_band))
+                cols['y'] = np.repeat(pos[1], len(w_band))
+                out.append(_fits.table_to_hdu(cols, meta=cards, name='BAND_FIELD'))
+                out.append(_fits.ImageHDU(data=band_field[1][g], name='PSF_BAND_FIELD'))
         try:
             results.append(_fits.to_astropy(out))
         except ImportError:
