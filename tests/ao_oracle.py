@@ -33,7 +33,9 @@ def ao_terms(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=False, win
     if wind_dir is None:
         wind_dir = orc.WIND_DIR[:h.size]
     wind_dir = np.asarray(wind_dir, dtype=float)
-    layer_psd = (0.0229 * (Cn2[:, None, None] ** (-3 / 5) * r0ref) ** (-5 / 3) * (f ** 2 + (1 / L0) ** 2) ** (-11 / 6))
+    with np.errstate(divide='ignore'):         # a zero-weight layer: 0^(-3/5) = inf, its PSD exactly 0
+        layer_psd = (0.0229 * (Cn2[:, None, None] ** (-3 / 5) * r0ref) ** (-5 / 3) *
+                     (f ** 2 + (1 / L0) ** 2) ** (-11 / 6))
     ngs = pos.shape[1]
     pitch = orc.D_PUP / orc.N_ACT
     sig2 = np.repeat(orc.NOISE_LGS2, ngs)
@@ -69,14 +71,20 @@ def ao_terms(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=False, win
     return rec, noise, r0ref
 
 
-def variance_record(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=False, wind_dir=None, dim=1280,
-                    dirs=None):
-    """PSFR_VAR_* records [ndir, VAR_NPAR] in nm^2 by the attribution rule of DESIGN.md 5.5."""
+def _zone(Cn2, h, seeing, L0, zenith, npsflin, three_lgs_mode, wind_dir, dim, dirs):
+    """The terms of ``ao_terms``, the fitting PSD on the 80 x 80 zone and the sum of the fitting PSD over the
+    whole dim x dim grid."""
     rec, noise, r0ref = ao_terms(Cn2, h, seeing, L0, zenith, npsflin, three_lgs_mode, wind_dir, dirs)
     fit = orc.psd_fit(dim, L, r0ref, L0, 1 / (2 * (orc.D_PUP / orc.N_ACT)))
     sl = slice(dim // 2 - orc.DIM_PUP, dim // 2 + orc.DIM_PUP)
-    fz = fit[sl, sl]
-    fit_total = fit.sum()
+    return rec, noise, fit[sl, sl], fit.sum()
+
+
+def variance_record(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=False, wind_dir=None, dim=1280,
+                    dirs=None):
+    """PSFR_VAR_* records [ndir, VAR_NPAR] in nm^2 by the attribution rule of DESIGN.md 5.5.  ``dirs`` [2, ndir]
+    (arcsec) replaces the directions of ``direction_perf(npsflin)``."""
+    rec, noise, fz, fit_total = _zone(Cn2, h, seeing, L0, zenith, npsflin, three_lgs_mode, wind_dir, dim, dirs)
     out = np.zeros((rec.shape[0], VAR_NPAR))
     unit = NM2 / L ** 2
     for b in range(rec.shape[0]):
@@ -88,6 +96,21 @@ def variance_record(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=Fal
         out[b, 3] = out[b, 4:4 + rec.shape[1]].sum()
         out[b, 0] = out[b, 1] + ao[won].sum()
     return out * unit
+
+
+def zone_margin(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=False, wind_dir=None, dim=1280,
+                dirs=None):
+    """Smallest |ao - fit| / fit over the zone cells of every direction where the fit is positive.
+
+    A cell whose AO value and fit agree to within rounding can fall on different sides of ``ao > fit`` here and
+    on the device, which moves its fit, noise and projection terms between the slots of the record: a comparison
+    with the record is only meaningful when this margin is well above the rounding of either side.  Where the fit
+    is 0 (inside the correction radius) any positive AO value wins on both sides, and the centre cell is 0 on
+    both."""
+    rec, noise, fz, _ = _zone(Cn2, h, seeing, L0, zenith, npsflin, three_lgs_mode, wind_dir, dim, dirs)
+    ao = rec.sum(axis=1) + noise
+    live = fz > 0
+    return float((np.abs(ao[:, live] - fz[live]) / fz[live]).min())
 
 
 def psd_total(Cn2, h, seeing, L0, zenith=0., npsflin=1, three_lgs_mode=False, wind_dir=None, dim=1280):

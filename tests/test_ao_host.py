@@ -90,3 +90,49 @@ def test_restatement_identities(case):
         assert abs(r[4:].sum() - r[3]) <= 1e-13 * r[3]
         assert np.all(r[4 + len(case['Cn2']):] == 0)
     assert np.allclose(rec[:, 0], ao.psd_total(**case), rtol=1e-12, atol=0)
+
+
+def assert_identities(rec, nl):
+    for r in rec:
+        assert abs(r[1] + r[2] + r[3] - r[0]) <= 1e-13 * r[0]
+        assert abs(r[4:].sum() - r[3]) <= 1e-13 * r[3]
+        assert np.all(r[4 + nl:] == 0)
+
+
+def test_restatement_dim2560():
+    """At dim 2560 the zone sits at the same frequencies as at 1280: NOISE, PROJ and the layers are the same,
+    FIT and TOTAL gain the fitting PSD of the wider grid (0.3 % of FIT for config 1)."""
+    case = dict(Cn2=[0.7, 0.3], h=(100, 10000), seeing=1.0, L0=25.0, npsflin=2)
+    big, small = ao.variance_record(dim=2560, **case), ao.variance_record(**case)
+    assert_identities(big, 2)
+    assert np.allclose(big[:, 0], ao.psd_total(dim=2560, **case), rtol=1e-12, atol=0)
+    assert np.allclose(big[:, 2:], small[:, 2:], rtol=1e-13, atol=0)
+    assert np.all(big[:, 1] / small[:, 1] - 1 > 2e-3)
+    assert ao.zone_margin(dim=2560, **case) > 1e-12
+
+
+def test_restatement_with_dirs():
+    """dirs = direction_perf(n) is npsflin = n bit for bit, and every direction's record is that of a call with
+    that direction alone, far outside the laser asterism too."""
+    case = dict(Cn2=[0.6, 0.4], h=(300.0, 9000.0), seeing=1.3, L0=18.0, zenith=15.0, three_lgs_mode=True)
+    assert np.array_equal(ao.variance_record(dirs=psfrec.direction_perf(3), **case),
+                          ao.variance_record(npsflin=3, **case))
+    pos = np.array([[0., -30., 12.5, 120., -120., 300.], [0., 30., -7.3, 60., 60., 0.]])
+    rec = ao.variance_record(dirs=pos, **case)
+    assert_identities(rec, 2)
+    for k in range(pos.shape[1]):
+        assert np.array_equal(rec[k], ao.variance_record(dirs=pos[:, k:k + 1], **case)[0])
+    assert ao.zone_margin(dirs=pos, **case) > 1e-12
+
+
+def test_restatement_zero_weight_layer():
+    """A layer of weight 0 has the slot 0 exactly, and the record is that of the profile without the layer."""
+    kw = dict(seeing=0.8, L0=30.0, zenith=45.0)
+    rec = ao.variance_record([0.5, 0.0, 0.3, 0.2], (50.0, 2000.0, 6000.0, 14000.0), wind_dir=[0.3, 1.1, -2.0, 2.6],
+                             dirs=[[0.0, 40.0], [0.0, -20.0]], **kw)
+    assert_identities(rec, 4)
+    assert np.all(rec[:, 5] == 0) and np.all(rec[:, [4, 6, 7]] > 0)
+    ref = ao.variance_record([0.5, 0.3, 0.2], (50.0, 6000.0, 14000.0), wind_dir=[0.3, -2.0, 2.6],
+                             dirs=[[0.0, 40.0], [0.0, -20.0]], **kw)
+    assert np.array_equal(rec[:, :4], ref[:, :4])
+    assert np.array_equal(rec[:, [4, 6, 7]], ref[:, 4:7])
