@@ -400,6 +400,7 @@ __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx
     }
 }
 
+template <bool kCoarse>
 __global__ void __launch_bounds__(kFitWarps * 32, PSFR_FIT_MINBLOCKS)
 fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __restrict__ out,
            int* __restrict__ next_image) {
@@ -466,10 +467,17 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     }
     // Stage 1: Levenberg-Marquardt on every eighth pixel down to a relative step of 1e-3 - it
     // only moves the start point (the converged minimum does not depend on it); stage 2: all
-    // pixels down to MINPACK's own tolerance, 1.49e-8.
-    int iter = 0, status = -1;
-    lm_solve<CircularMoffat, PSFR_FIT_COARSE_STEP>(img, npx, nx, x, sums, PSFR_FIT_COARSE_TOL2, 12, iter, status);
-    const int coarse_iter = iter;
+    // pixels down to MINPACK's own tolerance, 1.49e-8.  Stage 1 visits pixels lane + 256 k of each
+    // lane's pair loop: on an image of at most 512 pixels that is one or two 32-pixel strips (the
+    // first rows of a 16 x 16, rows 0, 1, 15 and 16 of a 17 x 17), wings that can drive the start
+    // away from the core, so run_fit launches the kCoarse = false instance on such images: stage 2 from the
+    // moments start directly.
+    int iter = 0, status = -1, coarse_iter = 0;
+    if constexpr (kCoarse) {
+        lm_solve<CircularMoffat, PSFR_FIT_COARSE_STEP>(img, npx, nx, x, sums, PSFR_FIT_COARSE_TOL2, 12, iter,
+                                                       status);
+        coarse_iter = iter;
+    }
     lm_solve<CircularMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, 200, iter, status);
     iter += coarse_iter;
     if (status > 0) status += coarse_iter;
@@ -624,6 +632,49 @@ __device__ void write_efit_record(const double* x, const double* sums, int npx, 
     o[PSFR_EFIT_ERR_FLUX] = err(g_flux);
 }
 
+// Start point of the elliptical fit from the image alone (warp-collective): peak pixel value, the centroid and
+// second moments of the pixels at or above half of it (each pixel a unit square, hence + 1/12 per axis), and the
+// quadratic form whose n = 2.5 Moffat has its half maximum on the ellipse of those moments (a uniform ellipse of
+// semi-axes h has variance h^2 / 4 along each).
+__device__ __forceinline__ void moments_start(const double* __restrict__ img, int npx, int nx, double* x) {
+    const int lane = threadIdx.x & 31;
+    double vmax = -INFINITY;
+    for (int i = lane; i < npx; i += 32) vmax = fmax(vmax, img[i]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) vmax = fmax(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
+    double m[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    for (int i = lane; i < npx; i += 32) {
+        if (!(img[i] >= 0.5 * vmax)) continue;
+        const double p = (double)(i / nx), q = (double)(i % nx);
+        m[0] += 1.0;
+        m[1] += p;
+        m[2] += q;
+        m[3] += p * p;
+        m[4] += q * q;
+        m[5] += p * q;
+    }
+    warp_sum_vec<6>(m);
+    const double mp = m[1] / m[0], mq = m[2] / m[0];
+    const double spp = m[3] / m[0] - mp * mp + 1.0 / 12.0, sqq = m[4] / m[0] - mq * mq + 1.0 / 12.0;
+    const double spq = m[5] / m[0] - mp * mq;
+    const double k = 0.25 * (pow(2.0, 0.4) - 1.0) / (spp * sqq - spq * spq);
+    x[0] = vmax;
+    x[1] = mp;
+    x[2] = mq;
+    x[3] = k * sqq;
+    x[4] = k * spp;
+    x[5] = -2.0 * k * spq;
+    x[6] = 2.5;
+}
+
+// A solution whose minor semi-axis is under 0.05 px (largest eigenvalue of the form above 400) leaves the model
+// under 401^-n of its peak on every pixel but the nearest: one pixel sets the width and any narrower one fits as
+// well (a lone hot pixel), so it is no answer and is reported as not converged.
+__device__ __forceinline__ bool resolved(const double* x) {
+    const double hd = 0.5 * (x[3] - x[4]), hc = 0.5 * x[5];
+    return 0.5 * (x[3] + x[4]) + sqrt(hd * hd + hc * hc) <= 400.0;
+}
+
 // Elliptical Moffat fit of every image, one warp per image as fit_kernel, from the image's converged
 // circular record circ [nimg][PSFR_FIT_NPAR]: (I, y0, x0, 1/a^2, 1/a^2, 0, n), all pixels, down to the
 // final stage's tolerance.  out [nimg][PSFR_EFIT_NPAR].
@@ -650,6 +701,27 @@ efit_kernel(const double* __restrict__ imgs, const double* __restrict__ circ, in
         double sums[kNSUM];
         int iter = 0, status = -1;
         lm_solve<EllipticalMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
+        // A circular fit that did not converge (typically collapsed onto a one-pixel spike, alpha -> 0, on a PSF
+        // narrower than a pixel along one axis) is no start for the ellipse, and neither start is sure to
+        // converge: then fit again from the half-maximum moments and keep the converged result of lower chi^2.
+        // Both conditions are warp-uniform; images whose two fits converge keep the bits of the first.
+        if (status <= 0 || !(c[PSFR_FIT_ITER] > 0.0)) {
+            double x1[kNP];
+#pragma unroll
+            for (int i = 0; i < kNP; ++i) x1[i] = x[i];
+            const double cost1 = sums[kNSUM - 1];
+            const int iter1 = iter, status1 = status;
+            moments_start(img, npx, nx, x);
+            lm_solve<EllipticalMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
+            if (!(status > 0 && resolved(x) && (status1 <= 0 || sums[kNSUM - 1] < cost1))) {
+#pragma unroll
+                for (int i = 0; i < kNP; ++i) x[i] = x1[i];
+                iter = iter1;
+                status = status1;
+                accumulate<EllipticalMoffat, 1>(img, npx, nx, x, sums);   // the bits lm_solve left at x1
+            }
+        }
+        if (!resolved(x)) status = -1;       // reported as not converged after iter iterations
         if (lane == 0) write_efit_record(x, sums, npx, iter, status, out + (size_t)image * PSFR_EFIT_NPAR);
         __syncwarp();
     }
@@ -811,10 +883,12 @@ int run_convolve(Ctx* c, int ndraw, int ndir, int nlam, const double* in_dev, do
 int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit_dev, cudaStream_t s) {
     const size_t smem = (size_t)kFitWarps * (ny * nx + nx) * sizeof(double);
     if (smem > 200 * 1024) return set_error(c, PSFR_E_UNSUPPORTED, "image %dx%d too large for the fitter", ny, nx);
-    if (int rc = ensure_dynamic_smem(c, fit_kernel, smem)) return rc;
+    // the coarse stage needs more than its two 32-pixel strips of the image (fit_kernel)
+    const auto kernel = ny * nx > 2 * 32 * PSFR_FIT_COARSE_STEP ? fit_kernel<true> : fit_kernel<false>;
+    if (int rc = ensure_dynamic_smem(c, kernel, smem)) return rc;
     int grid = (nimg + kFitWarps - 1) / kFitWarps;
     int per_sm = 2;                                  // persistent grid: as many CTAs as are resident at once
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fit_kernel, kFitWarps * 32, smem) != cudaSuccess ||
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kFitWarps * 32, smem) != cudaSuccess ||
         per_sm < 1) {
         cudaGetLastError();
         per_sm = 2;
@@ -822,7 +896,7 @@ int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit
     const int resident = c->sm_count * per_sm;
     if (grid > resident) grid = resident;
     PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 1, 0, sizeof(int), s));
-    fit_kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, nimg, ny, nx, fit_dev, c->d_counter + 1);
+    kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, nimg, ny, nx, fit_dev, c->d_counter + 1);
     PSFR_LAUNCH_CHECK(c);
     return PSFR_OK;
 }

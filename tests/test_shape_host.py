@@ -97,3 +97,82 @@ def test_oracle_delta_method_matches_finite_differences():
             d[i] = h * max(1.0, abs(theta[i]))
             g[i] = (eo.record(theta + d, jtj, 1.0, 1)[slot] - eo.record(theta - d, jtj, 1.0, 1)[slot]) / (2 * d[i])
         assert_allclose(base[err], np.sqrt(g @ sigma @ g), rtol=1e-6, err_msg=str(slot))
+
+
+def test_oracle_delta_method_matches_finite_differences_long_double():
+    """The same gradients through record_ld: the long-double record's errors against central differences of its
+    own derived columns, with J^T J, chi^2 and dof over a noisy render."""
+    truth = (1.3, 19.1, 20.4, 3.1, 2.2, 37.0, 2.7)
+    img = eo.render_noisy((40, 40), truth, 1e-2, 3)
+    theta = eo.theta_of(*truth)
+    base = eo.record_ld(theta, img)
+    p, q = (a.ravel().astype(float) for a in np.indices(img.shape))
+    J = eo.jacobian(theta, p, q)
+    r = eo.model(theta, p, q) - img.ravel()
+    sigma = np.linalg.inv(J.T @ J) * (r @ r) / (img.size - 7)
+    h = 1e-6
+    for slot, err in ((eo.PEAK, eo.ERR_PEAK), (eo.Y0, eo.ERR_Y0), (eo.X0, eo.ERR_X0), (eo.N, eo.ERR_N),
+                      (eo.A_MAJOR, eo.ERR_A_MAJOR), (eo.A_MINOR, eo.ERR_A_MINOR), (eo.PA, eo.ERR_PA),
+                      (eo.FWHM_MAJOR, eo.ERR_FWHM_MAJOR), (eo.FWHM_MINOR, eo.ERR_FWHM_MINOR),
+                      (eo.AXIS_RATIO, eo.ERR_AXIS_RATIO), (eo.FLUX, eo.ERR_FLUX)):
+        g = np.empty(7)
+        for i in range(7):
+            d = np.zeros(7)
+            d[i] = h * max(1.0, abs(theta[i]))
+            up, dn = eo.record(theta + d, np.eye(7), 1.0, 1), eo.record(theta - d, np.eye(7), 1.0, 1)
+            g[i] = (up[slot] - dn[slot]) / (2 * d[i])
+        assert_allclose(base[err], np.sqrt(g @ sigma @ g), rtol=1e-6, err_msg=str(slot))
+
+
+@pytest.mark.parametrize('seed', range(8))
+def test_record_ld_matches_record_in_fp64(seed):
+    """record_ld on random theta and a noisy image against record() fed the same J^T J, chi^2 and dof in FP64."""
+    rng = np.random.default_rng(seed)
+    shape = (int(rng.integers(8, 41)), int(rng.integers(8, 41)))
+    amaj = rng.uniform(1.0, min(shape) / 4)
+    truth = (rng.uniform(0.5, 3), (shape[0] - 1) / 2 + rng.uniform(-1, 1), (shape[1] - 1) / 2 + rng.uniform(-1, 1),
+             amaj, amaj * rng.uniform(0.2, 0.99), rng.uniform(0, 180), rng.uniform(1.3, 6))
+    img = eo.render_noisy(shape, truth, 10 ** rng.uniform(-4, -1), seed)
+    theta = eo.theta_of(*truth) * (1 + 1e-4 * rng.normal(size=7))
+    p, q = (a.ravel().astype(float) for a in np.indices(shape))
+    J = eo.jacobian(theta, p, q)
+    r = eo.model(theta, p, q) - img.ravel()
+    ref = eo.record(theta, J.T @ J, r @ r, img.size - 7)
+    got = eo.record_ld(theta, img)
+    assert_allclose(got, ref, rtol=1e-12, atol=0)
+
+
+@pytest.mark.parametrize('pa', [0.0, 1e-7, 30.0, 90.0 - 1e-6, 90.0, 135.0, 180.0 - 1e-7])
+def test_theta_of_record_round_trips(pa):
+    theta = eo.theta_of(1.7, 12.3, 15.8, 4.0, 2.5, pa, 2.2)
+    rec = eo.record(theta, np.eye(7), 1.0, 1)
+    back = eo.theta_of_record(rec)
+    assert_allclose(back, theta, rtol=0, atol=1e-13 * np.abs(theta).max())
+    assert_allclose(eo.record(back, np.eye(7), 1.0, 1), rec, rtol=1e-12)
+
+
+@pytest.mark.parametrize('truth,shape', [
+    ((1.0, 8.0, 8.0, 300.0, 270.0, 20.0, 1.05), (17, 17)),    # flat to 1e-3 over the image: I, a and n trade off
+    ((1.0, 8.3, 7.7, 0.7, 0.14, 20.0, 10.0), (17, 17)),       # the whole PSF inside one pixel
+])
+def test_well_posed_refuses_ill_posed_images(truth, shape):
+    with pytest.raises(AssertionError):
+        eo.well_posed(eo.render(shape, *truth), truth)
+
+
+@pytest.mark.parametrize('shape', [(40, 40), (17, 17)])
+def test_grid_removals_are_exactly_the_ill_posed_cases(shape):
+    """Every case the GPU grid keeps passes the guard; every case it removes fails it; every axis value is kept at
+    least once."""
+    kept, removed = eo.grid(shape)
+    for i, t in kept:
+        eo.well_posed(eo.render(shape, *t), t)
+    for i, t in removed:
+        with pytest.raises(AssertionError):
+            eo.well_posed(eo.render(shape, *t), t)
+    truths = [t for _, t in kept]
+    assert {t[3] for t in truths} == set(eo.GRID_A_MAJOR)
+    assert {round(t[4] / t[3], 6) for t in truths} == set(eo.GRID_Q)
+    assert {t[6] for t in truths} == set(eo.GRID_N)
+    assert {t[5] for t in truths} == set(eo.GRID_PA)
+
