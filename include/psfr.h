@@ -115,6 +115,32 @@ enum {
     PSFR_EFIT_NPAR = 24
 };
 
+/* Moffat fits of observed star images (DESIGN.md section 5.7, psfr_moffat_fit_weighted).  The fit minimises
+ * sum_i w_i (f(p_i, q_i; theta) + c - d_i)^2 over the used pixels, f the circular or elliptical Moffat of the records
+ * above and c a constant background when it is requested (otherwise c = 0, not fitted).
+ *  - A pixel is used when w_i > 0.  A pixel with w_i = 0 takes part in no sum, the start point included, whatever its
+ *    data value (NaN and +-inf included).
+ *  - An image fails when it has a weight that is negative or not finite, a used pixel whose data is not finite, or
+ *    npix_used <= NP (NP = 5 circular, 7 elliptical, plus 1 with a background).  A failed image gets ITER = 0 and NaN
+ *    in every other slot of its record and in CONT / ERR_CONT; the other images of the call are unaffected.
+ *  - Errors as the records above with chi^2 = sum w r^2 and dof = npix_used - NP: sqrt(diag((J^T W J)^-1) chi^2/dof),
+ *    the delta method over the same Sigma for the elliptical record.  With w = 1 / variance, chi^2/dof ~ 1.
+ *  - Start point: with every weight 1 and no background, the start of psfr_moffat_fit bit for bit.  Otherwise the
+ *    peak and column moments are taken over the used pixels only; with a background, c0 = the mean of the used
+ *    pixels on the outermost ring of the stamp (rows 0 and ny - 1, columns 0 and nx - 1; 0 when none is used), and
+ *    the moments are taken of d - c0.  The elliptical fit starts from the image's own circular star-fit record
+ *    with its c, as psfr_moffat_fit_elliptical.
+ *  - FIT / EFIT records as above: PEAK and FLUX are above the background.  Side record [nimg][PSFR_BACK_NPAR]: */
+enum {
+    PSFR_BACK_CONT = 0,      /* c (0 without a background) */
+    PSFR_BACK_ERR_CONT = 1,  /* its error (0 without a background) */
+    PSFR_BACK_NPIX = 2,      /* used pixels */
+    PSFR_BACK_NPAR = 3
+};
+/* Shared memory of the star fits: the image and its weights, 4 images per CTA.  The circular fit needs
+ * 4 (2 ny nx + nx) doubles, the elliptical one also 4 * 2 ny nx doubles, each at most 200 KiB; otherwise
+ * PSFR_E_UNSUPPORTED.  The largest accepted square stamp is 56 x 56 (57 x 57 is refused). */
+
 /* Encircled energy (DESIGN.md section 5.4).  Pixel (p, q) is the unit square [p - 1/2, p + 1/2] x [q - 1/2, q + 1/2]
  * with its value spread uniformly over it; EE(r) = sum img[p][q] * area(pixel AND disc(centre, r)), the exact
  * overlap area in FP64, over the pixels of the image only (a circle that leaves the image is clipped by its edge),
@@ -234,6 +260,19 @@ PSFR_API int psfr_moffat_fit(psfr_ctx* ctx, int nimg, int ny, int nx, const doub
  * handling and refusals as psfr_moffat_fit, and ny*nx must exceed 7.  params [nimg][PSFR_EFIT_NPAR]. */
 PSFR_API int psfr_moffat_fit_elliptical(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs,
                                         double* params, void* stream);
+
+/* Moffat fit of star images with per-pixel weights and an optional constant background (DESIGN.md section 5.7; the
+ * definitions are above PSFR_BACK_CONT).  imgs and weights [nimg][ny][nx]; weights NULL means every weight is 1.
+ * fit_back != 0 fits the background; elliptical != 0 writes PSFR_EFIT_* records to params [nimg][PSFR_EFIT_NPAR],
+ * otherwise PSFR_FIT_* records to params [nimg][PSFR_FIT_NPAR].  back [nimg][PSFR_BACK_NPAR] may be NULL.  Host or
+ * device arrays in any mix; host arrays are chunked through the staging buffers as psfr_moffat_fit (images and
+ * weights each take one, at the same chunk size), and an image that does not fit them is PSFR_E_CAPACITY.  NULL imgs
+ * or params, nimg < 1 or a side under 3 are PSFR_E_ARG, a stamp over the shared-memory limit above
+ * PSFR_E_UNSUPPORTED: all before any launch, nothing written.  With weights NULL and fit_back = 0 the records are
+ * those of psfr_moffat_fit / psfr_moffat_fit_elliptical bit for bit, and back holds (0, 0, ny nx). */
+PSFR_API int psfr_moffat_fit_weighted(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs,
+                                      const double* weights, int fit_back, int elliptical, double* params,
+                                      double* back, void* stream);
 
 /* compute_psf (psfrec.py:933-978) for a batch of draws, fused on the device:
  * PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit.

@@ -33,6 +33,9 @@ FIT_NPAR = 16
 (EFIT_ERR_PEAK, EFIT_ERR_Y0, EFIT_ERR_X0, EFIT_ERR_A_MAJOR, EFIT_ERR_A_MINOR, EFIT_ERR_PA, EFIT_ERR_N,
  EFIT_ERR_FWHM_MAJOR, EFIT_ERR_FWHM_MINOR, EFIT_ERR_AXIS_RATIO, EFIT_FLUX, EFIT_ERR_FLUX) = range(12, 24)
 EFIT_NPAR = 24
+# side record of the star fits (PSFR_BACK_*): background, its error, used pixels
+BACK_CONT, BACK_ERR_CONT, BACK_NPIX = range(3)
+BACK_NPAR = 3
 # encircled-energy record (include/psfr.h): EE at nrad radii, TOTAL, then the radius at each of nfrac fractions
 EE_MAX_RADII = 64
 EE_MAX_FRACTIONS = 16
@@ -88,6 +91,7 @@ _SIGNATURES = {
     'psfr_convolve': (_I, [_P, _I, _I, _P, _P, _P, _P, _P]),
     'psfr_moffat_fit': (_I, [_P, _I, _I, _I, _P, _P, _P]),
     'psfr_moffat_fit_elliptical': (_I, [_P, _I, _I, _I, _P, _P, _P]),
+    'psfr_moffat_fit_weighted': (_I, [_P, _I, _I, _I, _P, _P, _I, _I, _P, _P, _P]),
     'psfr_compute_batch': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P]),
     'psfr_compute_groups': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     'psfr_compute_field': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
@@ -324,6 +328,17 @@ class Context:
         self._check(self._lib.psfr_moffat_fit_elliptical(
             self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
             self._buf(params, nimg * EFIT_NPAR, 'params', True), stream))
+
+    def moffat_fit_weighted(self, nimg, ny, nx, imgs, weights, params, back=None, fit_back=False, elliptical=False,
+                            stream=None):
+        """psfr_moffat_fit_weighted: ``weights`` [nimg, ny, nx] or None (every weight 1); ``params`` [nimg, FIT_NPAR]
+        or, with ``elliptical``, [nimg, EFIT_NPAR]; ``back`` [nimg, BACK_NPAR] or None."""
+        nimg, ny, nx = int(nimg), int(ny), int(nx)
+        npar = EFIT_NPAR if elliptical else FIT_NPAR
+        self._check(self._lib.psfr_moffat_fit_weighted(
+            self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
+            self._buf(weights, nimg * ny * nx, 'weights'), int(bool(fit_back)), int(bool(elliptical)),
+            self._buf(params, nimg * npar, 'params', True), self._buf(back, nimg * BACK_NPAR, 'back', True), stream))
 
     def encircled_energy(self, nimg, ny, nx, imgs, radii_px, fracs, out, centres=None, stream=None):
         """psfr_encircled_energy: ``out`` [nimg, len(radii_px) + 1 + len(fracs)]; ``centres`` [nimg, 2] (y0, x0)

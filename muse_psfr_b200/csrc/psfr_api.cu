@@ -588,7 +588,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 106; }
+int psfr_version(void) { return 107; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -973,6 +973,54 @@ int psfr_moffat_fit_elliptical(psfr_ctx* c, int nimg, int ny, int nx, const doub
             rc = from_device(c, params + i0 * PSFR_EFIT_NPAR, dst, (size_t)n * PSFR_EFIT_NPAR * sizeof(double), s);
             if (rc) return rc;
         }
+    }
+    return PSFR_OK;
+}
+
+int psfr_moffat_fit_weighted(psfr_ctx* c, int nimg, int ny, int nx, const double* imgs, const double* weights,
+                             int fit_back, int elliptical, double* params, double* back, void* stream) {
+    if (!c || !imgs || !params) return set_error(c, PSFR_E_ARG, "NULL argument");
+    if (nimg < 1 || ny < 3 || nx < 3) return set_error(c, PSFR_E_ARG, "nimg=%d ny=%d nx=%d", nimg, ny, nx);
+    if (int rc = check_star_fit_size(c, ny, nx, elliptical != 0)) return rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    const size_t cap = (size_t)c->max_planes * c->max_lambda;
+    const size_t per = (size_t)ny * nx;
+    const int npar = elliptical ? PSFR_EFIT_NPAR : PSFR_FIT_NPAR;
+    const bool in_dev = is_device_ptr(imgs), w_dev = !weights || is_device_ptr(weights);
+    const bool out_dev = is_device_ptr(params), back_dev = back && is_device_ptr(back);
+    // host images and weights go through d_cube and d_cube2, host records through d_fit (circular) or d_efit
+    // (elliptical; d_fit then holds the circular start records), and the side records through d_fit2 unless the
+    // caller's are on the device: each holds cap images' worth
+    const size_t chunk_imgs = std::min(cap, (cap * kPSF * kPSF) / per);
+    if (chunk_imgs < 1) return set_error(c, PSFR_E_CAPACITY, "image %dx%d does not fit the staging buffer", ny, nx);
+    for (size_t i0 = 0; i0 < (size_t)nimg; i0 += chunk_imgs) {
+        const int n = (int)std::min(chunk_imgs, (size_t)nimg - i0);
+        const size_t bytes = (size_t)n * per * sizeof(double);
+        const double* src = imgs + i0 * per;
+        const double* w = weights ? weights + i0 * per : nullptr;
+        int rc;
+        if (!in_dev) {
+            if ((rc = to_device(c, c->d_cube, src, bytes, s))) return rc;
+            src = c->d_cube;
+        }
+        if (!w_dev) {
+            if ((rc = to_device(c, c->d_cube2, w, bytes, s))) return rc;
+            w = c->d_cube2;
+        }
+        double* dst = out_dev ? params + i0 * npar : (elliptical ? c->d_efit : c->d_fit);
+        double* bdst = back_dev ? back + i0 * PSFR_BACK_NPAR : c->d_fit2;
+        if (elliptical) {
+            if ((rc = run_star_fit(c, n, ny, nx, src, w, fit_back != 0, c->d_fit, bdst, s))) return rc;
+            rc = run_star_efit(c, n, ny, nx, src, w, fit_back != 0, c->d_fit, bdst, dst, bdst, s);
+        } else {
+            rc = run_star_fit(c, n, ny, nx, src, w, fit_back != 0, dst, bdst, s);
+        }
+        if (rc) return rc;
+        if (!out_dev && (rc = from_device(c, params + i0 * npar, dst, (size_t)n * npar * sizeof(double), s))) return rc;
+        if (back && !back_dev &&
+            (rc = from_device(c, back + i0 * PSFR_BACK_NPAR, bdst, (size_t)n * PSFR_BACK_NPAR * sizeof(double), s)))
+            return rc;
     }
     return PSFR_OK;
 }

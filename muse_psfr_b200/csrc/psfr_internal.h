@@ -309,6 +309,14 @@ int run_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, double* fit
 // elliptical fit of every image from its circular record circ_dev [nimg][PSFR_FIT_NPAR]
 int run_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* circ_dev, double* efit_dev,
              cudaStream_t s);
+// star fits (DESIGN.md 5.7): weights w_dev may be NULL (all 1); back_dev [nimg][PSFR_BACK_NPAR]; the elliptical one
+// starts from run_star_fit's records circ_dev / circ_back_dev (back_dev may be circ_back_dev)
+int check_star_fit_size(Ctx* c, int ny, int nx, bool elliptical);
+int run_star_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, bool fit_back,
+                 double* fit_dev, double* back_dev, cudaStream_t s);
+int run_star_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, bool fit_back,
+                  const double* circ_dev, const double* circ_back_dev, double* efit_dev, double* back_dev,
+                  cudaStream_t s);
 // psfr_energy.cu: encircled-energy record [nimg][nrad + 1 + nfrac] of every image, radii and fractions from
 // d_eepar, centres_dev [nimg][2] (row, column) or nullptr for (ny / 2, nx / 2)
 int run_ee(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* centres_dev, int nrad, int nfrac,

@@ -7,6 +7,7 @@
 //   mean / polyfit  : time mean of cubes (:1104) and polynomial smoothing (:1174-1210)
 #include <algorithm>
 #include <cmath>
+#include <type_traits>
 #include "psfr_internal.h"
 #include "fast_exp.cuh"
 
@@ -188,6 +189,22 @@ __device__ __forceinline__ void add_normal(const double* J, double r, double* su
     sums[NJJ + NP] = fma(r, r, sums[NJJ + NP]);
 }
 
+// the same with a pixel weight w: J^T W J, J^T W r and r^T W r.  w = 1 gives add_normal's bits (w J_i and w r are
+// exact), so a unit-weight star fit reproduces the plain fit.
+template <int NP>
+__device__ __forceinline__ void add_normal_w(const double* J, double r, double w, double* sums) {
+    constexpr int NJJ = Normal<NP>::NJJ;
+#pragma unroll
+    for (int i = 0; i < NP; ++i) {
+        const double wj = w * J[i];
+#pragma unroll
+        for (int j = i; j < NP; ++j) sums[pk<NP>(i, j)] = fma(wj, J[j], sums[pk<NP>(i, j)]);
+        sums[NJJ + i] = fma(wj, r, sums[NJJ + i]);
+    }
+    const double wr = w * r;
+    sums[NJJ + NP] = fma(wr, r, sums[NJJ + NP]);
+}
+
 // The models the Levenberg-Marquardt driver below fits.  Each is built from the parameter vector x once
 // per pass over the image (per-pass constants), gives one pixel's contribution to the normal equations at
 // offset (dp, dq) = (row - y0, column - x0), and says which trial points it refuses.
@@ -198,19 +215,25 @@ struct CircularMoffat {
     double I, n, ia2, ia;
     __device__ __forceinline__ explicit CircularMoffat(const double* x)
         : I(x[0]), n(x[4]), ia2(1.0 / (x[3] * x[3])), ia(1.0 / x[3]) {}
-    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double* sums) const {
+    static constexpr bool kWeighted = false;
+    // model value at offset (dp, dq); J receives its NP derivatives
+    __device__ __forceinline__ double eval(double dp, double dq, double* J) const {
         const double rho2 = (dp * dp + dq * dq) * ia2;
         const double uu = 1.0 + rho2;
         const double lu = log_ge1(uu);
         const double m = fast_exp(-n * lu);        // u^-n
         const double f = I * m;
         const double g = 2.0 * n * f * rcp_pos(uu);  // 2 I n u^(-n-1)
-        double J[NP];
         J[0] = m;
         J[1] = g * dp * ia2;
         J[2] = g * dq * ia2;
         J[3] = g * rho2 * ia;
         J[4] = -f * lu;
+        return f;
+    }
+    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double* sums) const {
+        double J[NP];
+        const double f = eval(dp, dq, J);
         add_normal<NP>(J, f - pix, sums);
     }
     static __device__ __forceinline__ bool refuses(const double* xt) {
@@ -226,14 +249,14 @@ struct EllipticalMoffat {
     double I, A, B, C, n;
     __device__ __forceinline__ explicit EllipticalMoffat(const double* x)
         : I(x[0]), A(x[3]), B(x[4]), C(x[5]), n(x[6]) {}
-    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double* sums) const {
+    static constexpr bool kWeighted = false;
+    __device__ __forceinline__ double eval(double dp, double dq, double* J) const {
         const double pp = dp * dp, qq = dq * dq, pq = dp * dq;
         const double uu = 1.0 + fma(A, pp, fma(B, qq, C * pq));
         const double lu = log_ge1(uu);
         const double m = fast_exp(-n * lu);        // u^-n
         const double f = I * m;
         const double g = n * f * rcp_pos(uu);        // I n u^(-n-1)
-        double J[NP];
         J[0] = m;
         J[1] = g * fma(2.0 * A, dp, C * dq);
         J[2] = g * fma(2.0 * B, dq, C * dp);
@@ -241,12 +264,38 @@ struct EllipticalMoffat {
         J[4] = -g * qq;
         J[5] = -g * pq;
         J[6] = -f * lu;
+        return f;
+    }
+    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double* sums) const {
+        double J[NP];
+        const double f = eval(dp, dq, J);
         add_normal<NP>(J, f - pix, sums);
     }
     // the form must stay positive definite (u >= 1 everywhere)
     static __device__ __forceinline__ bool refuses(const double* xt) {
         return !(xt[3] > 0.0) || !(xt[4] > 0.0) || !(4.0 * xt[3] * xt[4] - xt[5] * xt[5] > 0.0) || !(xt[6] > 0.0) ||
                !isfinite(xt[0]);
+    }
+};
+
+// A star fit of model M (DESIGN.md 5.7): every pixel carries a weight w, stored in shared memory right after the image
+// (npx further doubles; 0 on unused pixels, whose data were zeroed on load), and with kBack the model gains a constant
+// background c, the last parameter, with the Jacobian column dc = 1.
+template <class M, bool kBack>
+struct StarModel {
+    static constexpr int NP = M::NP + (kBack ? 1 : 0);
+    static constexpr bool kWeighted = true;
+    M m;
+    double c;
+    __device__ __forceinline__ explicit StarModel(const double* x) : m(x), c(kBack ? x[M::NP] : 0.0) {}
+    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double w, double* sums) const {
+        double J[NP];
+        const double f = m.eval(dp, dq, J);
+        if constexpr (kBack) J[M::NP] = 1.0;
+        add_normal_w<NP>(J, kBack ? (f + c) - pix : f - pix, w, sums);
+    }
+    static __device__ __forceinline__ bool refuses(const double* xt) {
+        return M::refuses(xt) || (kBack && !isfinite(xt[NP - 1]));
     }
 };
 
@@ -278,10 +327,20 @@ __device__ __forceinline__ void accumulate(const double* __restrict__ img, int n
         step();
         const double dp1 = (double)pr - y0, dq1 = (double)qc - x0;
         step();
-        model.pixel(dp0, dq0, img[idx], sums);
-        model.pixel(dp1, dq1, img[idx + 32 * STEP], sums);
+        if constexpr (M::kWeighted) {   // the weights follow the image
+            model.pixel(dp0, dq0, img[idx], img[npx + idx], sums);
+            model.pixel(dp1, dq1, img[idx + 32 * STEP], img[npx + idx + 32 * STEP], sums);
+        } else {
+            model.pixel(dp0, dq0, img[idx], sums);
+            model.pixel(dp1, dq1, img[idx + 32 * STEP], sums);
+        }
     }
-    if (idx < npx) model.pixel((double)pr - y0, (double)qc - x0, img[idx], sums);
+    if (idx < npx) {
+        if constexpr (M::kWeighted)
+            model.pixel((double)pr - y0, (double)qc - x0, img[idx], img[npx + idx], sums);
+        else
+            model.pixel((double)pr - y0, (double)qc - x0, img[idx], sums);
+    }
     warp_sum_vec<Normal<M::NP>::NSUM>(sums);
 }
 
@@ -400,14 +459,81 @@ __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx
     }
 }
 
-template <bool kCoarse>
-__global__ void __launch_bounds__(kFitWarps * 32, PSFR_FIT_MINBLOCKS)
-fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __restrict__ out,
-           int* __restrict__ next_image) {
-    constexpr int kNP = CircularMoffat::NP, kNSUM = Normal<kNP>::NSUM, COST = Normal<kNP>::COST;
+// ---------------------------------------------------------------- star fits (DESIGN.md 5.7)
+// Load image `image` and its weights (wts NULL: every weight 1) into the warp's shared memory, img[npx] then w[npx].
+// A pixel is used when w > 0; the data and weight of every other pixel are zeroed here - selected, never multiplied -
+// so that whatever it holds (NaN, inf) reaches no sum.  Returns the number of used pixels; `bad` is set when the
+// image has a negative or non-finite weight, or non-finite data on a used pixel.  Warp-collective and warp-uniform.
+__device__ __forceinline__ int load_star_image(const double* __restrict__ imgs, const double* __restrict__ wts,
+                                               int image, int npx, double* img, bool& bad) {
+    const int lane = threadIdx.x & 31;
+    const double* src = imgs + (size_t)image * npx;
+    const double* wsrc = wts ? wts + (size_t)image * npx : nullptr;
+    int used = 0;
+    bool b = false;
+    for (int i = lane; i < npx; i += 32) {
+        const double w = wsrc ? wsrc[i] : 1.0, d = src[i];
+        const bool u = w > 0.0;
+        b = b || !(w >= 0.0 && isfinite(w)) || (u && !isfinite(d));
+        used += u ? 1 : 0;
+        img[i] = u ? d : 0.0;
+        img[npx + i] = u ? w : 0.0;
+    }
+    used = __reduce_add_sync(0xffffffffu, used);
+    bad = __any_sync(0xffffffffu, b);
+    __syncwarp();
+    return used;
+}
+
+// Start value c0 of the background: the mean of the used pixels on the outermost ring of the stamp (rows 0 and
+// ny - 1, columns 0 and nx - 1), 0 when none of them is used.  Warp-collective; the same bits in every lane.
+__device__ __forceinline__ double ring_background(const double* img, int ny, int nx) {
+    const int lane = threadIdx.x & 31, npx = ny * nx, nring = 2 * nx + 2 * (ny - 2);
+    double v[2] = {0.0, 0.0};
+    for (int k = lane; k < nring; k += 32) {
+        const int r = k - 2 * nx;
+        const int i = k < nx ? k : k < 2 * nx ? (ny - 1) * nx + (k - nx) : (r / 2 + 1) * nx + (r % 2) * (nx - 1);
+        if (img[npx + i] > 0.0) {
+            v[0] += img[i];
+            v[1] += 1.0;
+        }
+    }
+    warp_sum_vec<2>(v);
+    return v[1] > 0.0 ? v[0] / v[1] : 0.0;
+}
+
+// record of an image that fails the star fit's check: ITER = 0 and every other slot NaN
+__device__ __forceinline__ void fail_record(double* o, int npar, int iter_slot) {
+    for (int i = 0; i < npar; ++i) o[i] = (i == iter_slot) ? 0.0 : nan("");
+}
+
+__device__ __forceinline__ void back_record(double* b, double cont, double err_cont, int npix) {
+    b[PSFR_BACK_CONT] = cont;
+    b[PSFR_BACK_ERR_CONT] = err_cont;
+    b[PSFR_BACK_NPIX] = (double)npix;
+}
+
+// pixel i in the start-point statistics: its data, above c0 with a background (unused pixels hold 0)
+template <bool kBack>
+__device__ __forceinline__ double start_value(const double* img, int npx, int i, double c0) {
+    if constexpr (kBack) return img[npx + i] > 0.0 ? img[i] - c0 : 0.0;
+    else return img[i];
+}
+
+// ---------------------------------------------------------------- circular Moffat fit
+// One driver for every circular fit.  kW = false, kBack = false is the reconstruction's fitter (fit_kernel); kW is a
+// star fit (weights after the image in shared memory, the per-image check, dof over used pixels and the side record
+// `back`), kBack adds the background parameter c.
+template <bool kCoarse, bool kW, bool kBack>
+__device__ __forceinline__ void fit_images(const double* __restrict__ imgs, const double* __restrict__ wts, int nimg,
+                                           int ny, int nx, double* __restrict__ out, double* __restrict__ back,
+                                           int* __restrict__ next_image) {
+    using Model = std::conditional_t<kW, StarModel<CircularMoffat, kBack>, CircularMoffat>;
+    constexpr int kNP = Model::NP, kNSUM = Normal<kNP>::NSUM, COST = Normal<kNP>::COST;
     extern __shared__ double sm[];
     const int npx = ny * nx, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double* img = sm + (size_t)warp * (npx + nx);    // npx pixels + nx column weights
+    const int img_len = kW ? 2 * npx : npx;          // npx pixels (and npx weights)
+    double* img = sm + (size_t)warp * (img_len + nx);    // ... + nx column weights
     // images are handed to the warps by a global counter: the LM iteration count varies 3x
     // between images, so a static one-image-per-warp grid ends in a long tail
 #pragma unroll 1
@@ -417,14 +543,31 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     image = __shfl_sync(0xffffffffu, image, 0);
     if (image >= nimg) return;                       // whole warp leaves; no block barrier is used below
     __syncwarp();
-    double* colw = img + npx;
-    const double* src = imgs + (size_t)image * npx;
-    for (int i = lane; i < npx; i += 32) img[i] = src[i];
-    __syncwarp();
-    // ---- start point as mpdaf: peak pixel, width from Image.moments(), n = 2
+    double* colw = img + img_len;
+    int npu = npx;                                   // pixels in the fit
+    double c0 = 0.0;                                 // start of the background
+    if constexpr (kW) {
+        bool bad;
+        npu = load_star_image(imgs, wts, image, npx, img, bad);
+        if (bad || npu <= kNP) {
+            if (lane == 0) {
+                fail_record(out + (size_t)image * PSFR_FIT_NPAR, PSFR_FIT_NPAR, PSFR_FIT_ITER);
+                back_record(back + (size_t)image * PSFR_BACK_NPAR, nan(""), nan(""), npu);
+            }
+            __syncwarp();
+            continue;
+        }
+        if constexpr (kBack) c0 = ring_background(img, ny, nx);
+    } else {
+        const double* src = imgs + (size_t)image * npx;
+        for (int i = lane; i < npx; i += 32) img[i] = src[i];
+        __syncwarp();
+    }
+    // ---- start point as mpdaf: peak pixel, width from Image.moments(), n = 2; a star fit takes them over the used
+    // pixels (the others hold 0) and of the data above c0
     for (int q = lane; q < nx; q += 32) {
         double t = 0.0;
-        for (int p = 0; p < ny; ++p) t += p * fabs(img[p * nx + q]);
+        for (int p = 0; p < ny; ++p) t += p * fabs(start_value<kBack>(img, npx, p * nx + q, c0));
         colw[q] = t;
     }
     __syncwarp();
@@ -434,7 +577,10 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     for (int q = lane; q < nx; q += 32)
         if (colw[q] > bestw) { bestw = colw[q]; qb = q; }
     for (int i = lane; i < npx; i += 32)
-        if (img[i] > bestv) { bestv = img[i]; ib = i; }
+        if ((!kW || img[npx + i] > 0.0) && start_value<kBack>(img, npx, i, c0) > bestv) {
+            bestv = start_value<kBack>(img, npx, i, c0);
+            ib = i;
+        }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         const double ow = __shfl_xor_sync(0xffffffffu, bestw, o);
@@ -446,7 +592,7 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     }
     double num = 0.0, den = 0.0;
     for (int p = lane; p < ny; p += 32) {
-        const double v = img[p * nx + qb];
+        const double v = start_value<kBack>(img, npx, p * nx + qb, c0);
         num += fabs((p - qb) * v);
         den += fabs(v);
     }
@@ -464,6 +610,7 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
         x[2] = ib % nx;
         x[3] = fwhm0 / (2.0 * sqrt(sqrt(2.0) - 1.0));
         x[4] = 2.0;
+        if constexpr (kBack) x[kNP - 1] = c0;
     }
     // Stage 1: Levenberg-Marquardt on every eighth pixel down to a relative step of 1e-3 - it
     // only moves the start point (the converged minimum does not depend on it); stage 2: all
@@ -474,11 +621,10 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
     // moments start directly.
     int iter = 0, status = -1, coarse_iter = 0;
     if constexpr (kCoarse) {
-        lm_solve<CircularMoffat, PSFR_FIT_COARSE_STEP>(img, npx, nx, x, sums, PSFR_FIT_COARSE_TOL2, 12, iter,
-                                                       status);
+        lm_solve<Model, PSFR_FIT_COARSE_STEP>(img, npx, nx, x, sums, PSFR_FIT_COARSE_TOL2, 12, iter, status);
         coarse_iter = iter;
     }
-    lm_solve<CircularMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, 200, iter, status);
+    lm_solve<Model, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, 200, iter, status);
     iter += coarse_iter;
     if (status > 0) status += coarse_iter;
     const int max_iter = 212;
@@ -494,7 +640,7 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
         o[PSFR_FIT_FWHM] = a * kf;
         o[PSFR_FIT_CHISQ] = sums[COST];
         o[PSFR_FIT_ITER] = (status > 0) ? (double)status : -(double)(iter > max_iter ? max_iter : iter);
-        const double dof = (double)(npx - kNP);
+        const double dof = (double)(npu - kNP);
         double L[kNP][kNP];
         if (cholesky(sums, 0.0, L)) {
             double e[kNP];
@@ -515,14 +661,35 @@ fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __
             // with err_e = 0 for a circular fit (restated from mpdaf 3.x; the package is not in the reference tree)
             o[PSFR_FIT_ERR_FWHM] = e[3] * n;
             o[PSFR_FIT_ERR_FLUX] = e[0] * e[4] * e[3] * e[3] * 0.0;
+            if constexpr (kW)
+                back_record(back + (size_t)image * PSFR_BACK_NPAR, kBack ? x[kNP - 1] : 0.0, kBack ? e[kNP - 1] : 0.0,
+                            npu);
         } else {
             for (int i = PSFR_FIT_ERR_PEAK; i <= PSFR_FIT_ERR_FWHM; ++i) o[i] = nan("");
             o[PSFR_FIT_ERR_FLUX] = nan("");
+            if constexpr (kW)
+                back_record(back + (size_t)image * PSFR_BACK_NPAR, kBack ? x[kNP - 1] : 0.0, kBack ? nan("") : 0.0,
+                            npu);
         }
         o[PSFR_FIT_FLUX] = x[0] / (n - 1.0) * (3.141592653589793 * a * a);
     }
     __syncwarp();
     }   // next image
+}
+
+template <bool kCoarse>
+__global__ void __launch_bounds__(kFitWarps * 32, PSFR_FIT_MINBLOCKS)
+fit_kernel(const double* __restrict__ imgs, int nimg, int ny, int nx, double* __restrict__ out,
+           int* __restrict__ next_image) {
+    fit_images<kCoarse, false, false>(imgs, nullptr, nimg, ny, nx, out, nullptr, next_image);
+}
+
+// circular star fit: weights [nimg][ny][nx] (NULL: all 1), back [nimg][PSFR_BACK_NPAR]
+template <bool kCoarse, bool kBack>
+__global__ void __launch_bounds__(kFitWarps * 32, PSFR_FIT_MINBLOCKS)
+star_fit_kernel(const double* __restrict__ imgs, const double* __restrict__ wts, int nimg, int ny, int nx,
+                double* __restrict__ out, double* __restrict__ back, int* __restrict__ next_image) {
+    fit_images<kCoarse, true, kBack>(imgs, wts, nimg, ny, nx, out, back, next_image);
 }
 
 // ---------------------------------------------------------------- elliptical Moffat fit
@@ -548,8 +715,11 @@ __device__ __forceinline__ double inv_quad(const double (&L)[NP][NP], const doub
 
 // The elliptical record of x = [I, y0, x0, A, B, C, n] (include/psfr.h, PSFR_EFIT_*).  Each derived quantity
 // q gets the error sqrt(grad q^T Sigma grad q), Sigma = (J^T J)^-1 chi^2/dof, with the gradient written out.
+// NT = 8: x and the sums also hold the background c (star fits, DESIGN.md 5.7); npx is the number of pixels in
+// the fit.
+template <int NT>
 __device__ void write_efit_record(const double* x, const double* sums, int npx, int iter, int status, double* o) {
-    constexpr int NP = EllipticalMoffat::NP, COST = Normal<NP>::COST;
+    constexpr int NP = NT, COST = Normal<NP>::COST;
     constexpr double kPi = 3.141592653589793, kDeg = 180.0 / kPi;
     const double I = x[0], A = x[3], B = x[4], C = x[5], n = x[6];
     // eigenvalues of [[A, C/2], [C/2, B]]: the major axis belongs to the smaller one
@@ -600,7 +770,7 @@ __device__ void write_efit_record(const double* x, const double* sums, int npx, 
     const double g_amin[NP] = {0, 0, 0, gmin * (0.5 + ca), gmin * (0.5 - ca), gmin * cc, 0};
     double g[NP];
 #pragma unroll
-    for (int c = 0; c < NP; ++c) {
+    for (int c = 0; c < EllipticalMoffat::NP; ++c) {
         if (c == 3 || c == 4 || c == 5) continue;
 #pragma unroll
         for (int i = 0; i < NP; ++i) g[i] = (i == c) ? 1.0 : 0.0;
@@ -632,19 +802,33 @@ __device__ void write_efit_record(const double* x, const double* sums, int npx, 
     o[PSFR_EFIT_ERR_FLUX] = err(g_flux);
 }
 
+// error of the background of an elliptical star fit: sqrt((J^T W J)^-1_cc chi^2/dof), NaN where J^T W J is singular
+__device__ __forceinline__ double efit_err_back(const double* sums, int npu) {
+    constexpr int NP = EllipticalMoffat::NP + 1, COST = Normal<NP>::COST;
+    double L[NP][NP];
+    if (!cholesky<NP>(sums, 0.0, L)) return nan("");
+    double g[NP];
+#pragma unroll
+    for (int i = 0; i < NP; ++i) g[i] = (i == NP - 1) ? 1.0 : 0.0;
+    return sqrt(fabs(inv_quad<NP>(L, g)) * fabs(sums[COST] / (double)(npu - NP)));
+}
+
 // Start point of the elliptical fit from the image alone (warp-collective): peak pixel value, the centroid and
 // second moments of the pixels at or above half of it (each pixel a unit square, hence + 1/12 per axis), and the
 // quadratic form whose n = 2.5 Moffat has its half maximum on the ellipse of those moments (a uniform ellipse of
-// semi-axes h has variance h^2 / 4 along each).
-__device__ __forceinline__ void moments_start(const double* __restrict__ img, int npx, int nx, double* x) {
+// semi-axes h has variance h^2 / 4 along each).  A star fit (kW) takes the used pixels only and, with a background,
+// their data above c0, the background's start; x[7] = c0.
+template <bool kW, bool kBack>
+__device__ __forceinline__ void moments_start(const double* __restrict__ img, int npx, int nx, double c0, double* x) {
     const int lane = threadIdx.x & 31;
     double vmax = -INFINITY;
-    for (int i = lane; i < npx; i += 32) vmax = fmax(vmax, img[i]);
+    for (int i = lane; i < npx; i += 32)
+        if (!kW || img[npx + i] > 0.0) vmax = fmax(vmax, start_value<kBack>(img, npx, i, c0));
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) vmax = fmax(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
     double m[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     for (int i = lane; i < npx; i += 32) {
-        if (!(img[i] >= 0.5 * vmax)) continue;
+        if (!(start_value<kBack>(img, npx, i, c0) >= 0.5 * vmax) || (kW && !(img[npx + i] > 0.0))) continue;
         const double p = (double)(i / nx), q = (double)(i % nx);
         m[0] += 1.0;
         m[1] += p;
@@ -665,6 +849,7 @@ __device__ __forceinline__ void moments_start(const double* __restrict__ img, in
     x[4] = k * spp;
     x[5] = -2.0 * k * spq;
     x[6] = 2.5;
+    if constexpr (kBack) x[7] = c0;
 }
 
 // A solution whose minor semi-axis is under 0.05 px (largest eigenvalue of the form above 400) leaves the model
@@ -677,14 +862,18 @@ __device__ __forceinline__ bool resolved(const double* x) {
 
 // Elliptical Moffat fit of every image, one warp per image as fit_kernel, from the image's converged
 // circular record circ [nimg][PSFR_FIT_NPAR]: (I, y0, x0, 1/a^2, 1/a^2, 0, n), all pixels, down to the
-// final stage's tolerance.  out [nimg][PSFR_EFIT_NPAR].
-__global__ void __launch_bounds__(kFitWarps * 32, PSFR_EFIT_MINBLOCKS)
-efit_kernel(const double* __restrict__ imgs, const double* __restrict__ circ, int nimg, int ny, int nx,
-            double* __restrict__ out, int* __restrict__ next_image) {
-    constexpr int kNP = EllipticalMoffat::NP, kNSUM = Normal<kNP>::NSUM;
+// final stage's tolerance.  out [nimg][PSFR_EFIT_NPAR].  kW, kBack as fit_images: a star fit also starts c from
+// the circular star fit's side record circ_back and writes its own to back (the two may be the same array).
+template <bool kW, bool kBack>
+__device__ __forceinline__ void efit_images(const double* __restrict__ imgs, const double* __restrict__ wts,
+                                            const double* __restrict__ circ, const double* circ_back, int nimg,
+                                            int ny, int nx, double* __restrict__ out, double* back,
+                                            int* __restrict__ next_image) {
+    using Model = std::conditional_t<kW, StarModel<EllipticalMoffat, kBack>, EllipticalMoffat>;
+    constexpr int kNP = Model::NP, kNSUM = Normal<kNP>::NSUM;
     extern __shared__ double sm[];
     const int npx = ny * nx, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double* img = sm + (size_t)warp * npx;
+    double* img = sm + (size_t)warp * (kW ? 2 * npx : npx);
 #pragma unroll 1
     for (;;) {
         int image = 0;
@@ -692,15 +881,32 @@ efit_kernel(const double* __restrict__ imgs, const double* __restrict__ circ, in
         image = __shfl_sync(0xffffffffu, image, 0);
         if (image >= nimg) return;
         __syncwarp();
-        const double* src = imgs + (size_t)image * npx;
-        for (int i = lane; i < npx; i += 32) img[i] = src[i];
-        __syncwarp();
+        int npu = npx;
+        double c0 = 0.0;
+        if constexpr (kW) {
+            bool bad;
+            npu = load_star_image(imgs, wts, image, npx, img, bad);
+            if (bad || npu <= kNP) {
+                if (lane == 0) {
+                    fail_record(out + (size_t)image * PSFR_EFIT_NPAR, PSFR_EFIT_NPAR, PSFR_EFIT_ITER);
+                    back_record(back + (size_t)image * PSFR_BACK_NPAR, nan(""), nan(""), npu);
+                }
+                __syncwarp();
+                continue;
+            }
+            if constexpr (kBack) c0 = ring_background(img, ny, nx);
+        } else {
+            const double* src = imgs + (size_t)image * npx;
+            for (int i = lane; i < npx; i += 32) img[i] = src[i];
+            __syncwarp();
+        }
         const double* c = circ + (size_t)image * PSFR_FIT_NPAR;
         const double ia2 = 1.0 / (c[PSFR_FIT_ALPHA] * c[PSFR_FIT_ALPHA]);
         double x[kNP] = {c[PSFR_FIT_PEAK], c[PSFR_FIT_Y0], c[PSFR_FIT_X0], ia2, ia2, 0.0, c[PSFR_FIT_N]};
+        if constexpr (kBack) x[kNP - 1] = circ_back[(size_t)image * PSFR_BACK_NPAR + PSFR_BACK_CONT];
         double sums[kNSUM];
         int iter = 0, status = -1;
-        lm_solve<EllipticalMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
+        lm_solve<Model, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
         // A circular fit that did not converge (typically collapsed onto a one-pixel spike, alpha -> 0, on a PSF
         // narrower than a pixel along one axis) is no start for the ellipse, and neither start is sure to
         // converge: then fit again from the half-maximum moments and keep the converged result of lower chi^2.
@@ -711,20 +917,40 @@ efit_kernel(const double* __restrict__ imgs, const double* __restrict__ circ, in
             for (int i = 0; i < kNP; ++i) x1[i] = x[i];
             const double cost1 = sums[kNSUM - 1];
             const int iter1 = iter, status1 = status;
-            moments_start(img, npx, nx, x);
-            lm_solve<EllipticalMoffat, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
+            moments_start<kW, kBack>(img, npx, nx, c0, x);
+            lm_solve<Model, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kEfitMaxIter, iter, status);
             if (!(status > 0 && resolved(x) && (status1 <= 0 || sums[kNSUM - 1] < cost1))) {
 #pragma unroll
                 for (int i = 0; i < kNP; ++i) x[i] = x1[i];
                 iter = iter1;
                 status = status1;
-                accumulate<EllipticalMoffat, 1>(img, npx, nx, x, sums);   // the bits lm_solve left at x1
+                accumulate<Model, 1>(img, npx, nx, x, sums);   // the bits lm_solve left at x1
             }
         }
         if (!resolved(x)) status = -1;       // reported as not converged after iter iterations
-        if (lane == 0) write_efit_record(x, sums, npx, iter, status, out + (size_t)image * PSFR_EFIT_NPAR);
+        if (lane == 0) {
+            write_efit_record<kNP>(x, sums, npu, iter, status, out + (size_t)image * PSFR_EFIT_NPAR);
+            if constexpr (kW)
+                back_record(back + (size_t)image * PSFR_BACK_NPAR, kBack ? x[kNP - 1] : 0.0,
+                            kBack ? efit_err_back(sums, npu) : 0.0, npu);
+        }
         __syncwarp();
     }
+}
+
+__global__ void __launch_bounds__(kFitWarps * 32, PSFR_EFIT_MINBLOCKS)
+efit_kernel(const double* __restrict__ imgs, const double* __restrict__ circ, int nimg, int ny, int nx,
+            double* __restrict__ out, int* __restrict__ next_image) {
+    efit_images<false, false>(imgs, nullptr, circ, nullptr, nimg, ny, nx, out, nullptr, next_image);
+}
+
+// elliptical star fit from the circular star fit's records circ and circ_back (which back may overwrite in place)
+template <bool kBack>
+__global__ void __launch_bounds__(kFitWarps * 32, PSFR_EFIT_MINBLOCKS)
+star_efit_kernel(const double* __restrict__ imgs, const double* __restrict__ wts, const double* __restrict__ circ,
+                 const double* circ_back, int nimg, int ny, int nx, double* __restrict__ out, double* back,
+                 int* __restrict__ next_image) {
+    efit_images<true, kBack>(imgs, wts, circ, circ_back, nimg, ny, nx, out, back, next_image);
 }
 
 // ---------------------------------------------------------------- mean of cubes
@@ -917,6 +1143,67 @@ int run_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const doub
     if (grid > resident) grid = resident;
     PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 2, 0, sizeof(int), s));
     efit_kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, circ_dev, nimg, ny, nx, efit_dev, c->d_counter + 2);
+    PSFR_LAUNCH_CHECK(c);
+    return PSFR_OK;
+}
+
+// Shared memory of the star fits (the image and its weights per warp), or 0 when a stamp is over the fitter's
+// 200 KiB: the circular fit always runs, the elliptical one after it.
+static size_t star_fit_smem(int ny, int nx, bool elliptical) {
+    const size_t npx = (size_t)ny * nx, circ = kFitWarps * (2 * npx + nx) * sizeof(double);
+    const size_t ell = kFitWarps * 2 * npx * sizeof(double);
+    const size_t lim = 200 * 1024;
+    return circ > lim || (elliptical && ell > lim) ? 0 : circ;
+}
+
+int check_star_fit_size(Ctx* c, int ny, int nx, bool elliptical) {
+    if (!star_fit_smem(ny, nx, elliptical))
+        return set_error(c, PSFR_E_UNSUPPORTED,
+                         "image %dx%d too large for the star fit: its image and weights need %zu bytes of shared memory "
+                         "per CTA, over 200 KiB", ny, nx,
+                         (size_t)kFitWarps * (2 * (size_t)ny * nx + (elliptical ? 0 : nx)) * sizeof(double));
+    return PSFR_OK;
+}
+
+// persistent grid of a fit kernel: as many CTAs as are resident at once, at most one warp per image
+template <class K>
+static int fit_grid(Ctx* c, K* kernel, size_t smem, int nimg, int per_sm_default) {
+    int grid = (nimg + kFitWarps - 1) / kFitWarps;
+    int per_sm = per_sm_default;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kFitWarps * 32, smem) != cudaSuccess ||
+        per_sm < 1) {
+        cudaGetLastError();
+        per_sm = per_sm_default;
+    }
+    return std::min(grid, c->sm_count * per_sm);
+}
+
+int run_star_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, bool fit_back,
+                 double* fit_dev, double* back_dev, cudaStream_t s) {
+    if (int rc = check_star_fit_size(c, ny, nx, false)) return rc;
+    const size_t smem = star_fit_smem(ny, nx, false);
+    const bool coarse = ny * nx > 2 * 32 * PSFR_FIT_COARSE_STEP;   // as run_fit
+    const auto kernel = coarse ? (fit_back ? star_fit_kernel<true, true> : star_fit_kernel<true, false>)
+                               : (fit_back ? star_fit_kernel<false, true> : star_fit_kernel<false, false>);
+    if (int rc = ensure_dynamic_smem(c, kernel, smem)) return rc;
+    const int grid = fit_grid(c, kernel, smem, nimg, 2);
+    PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 1, 0, sizeof(int), s));
+    kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, w_dev, nimg, ny, nx, fit_dev, back_dev, c->d_counter + 1);
+    PSFR_LAUNCH_CHECK(c);
+    return PSFR_OK;
+}
+
+int run_star_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, bool fit_back,
+                  const double* circ_dev, const double* circ_back_dev, double* efit_dev, double* back_dev,
+                  cudaStream_t s) {
+    if (int rc = check_star_fit_size(c, ny, nx, true)) return rc;
+    const size_t smem = (size_t)kFitWarps * 2 * ny * nx * sizeof(double);
+    const auto kernel = fit_back ? star_efit_kernel<true> : star_efit_kernel<false>;
+    if (int rc = ensure_dynamic_smem(c, kernel, smem)) return rc;
+    const int grid = fit_grid(c, kernel, smem, nimg, 1);
+    PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 2, 0, sizeof(int), s));
+    kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, w_dev, circ_dev, circ_back_dev, nimg, ny, nx, efit_dev,
+                                              back_dev, c->d_counter + 2);
     PSFR_LAUNCH_CHECK(c);
     return PSFR_OK;
 }

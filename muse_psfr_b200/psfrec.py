@@ -558,26 +558,87 @@ def convolve_final_psf(lbda, seeing, GL, L0, psf):
     return out
 
 
-def fit_psf_cube(lbda, psfcube, circular=True):
+def fit_psf_cube(lbda, psfcube, circular=True, var=None, mask=None, fit_back=False):
     """Fit a Moffat PSF on each wavelength plane (psfrec.py:861-871).  ``psfcube`` is an
     array [nl, ny, nx] (or anything with a ``.data`` array, like an mpdaf Cube).
 
     ``circular=False`` (mpdaf's keyword; the reference passes True) fits an elliptical Moffat instead and
     returns the columns of ``_shape_table_from_fit``: ``fwhm`` = (major, minor), ``axis_ratio``, ``pa`` [deg]
-    and their errors."""
-    data = getattr(psfcube, 'data', psfcube)
-    data = np.ascontiguousarray(np.ma.getdata(data), dtype=np.float64)
+    and their errors.
+
+    Star images (DESIGN.md section 5.7): ``var`` (the cube's variance), ``mask`` (True = bad pixel) and
+    ``fit_back`` (fit a constant background) turn the fit into a weighted one.  ``var`` and ``mask`` have the
+    cube's shape or [ny, nx] for every plane.  The weights are 1 / ``var`` (1 without ``var``) and 0 where ``mask``
+    is true, where a masked input is masked, or where the data or the variance is not finite (NaN marks bad
+    pixels in MUSE cubes).  The table then also holds ``cont`` (the background, 0 without ``fit_back``),
+    ``err_cont`` and ``npix`` (the pixels used); ``peak`` and ``flux`` are above the background.  ``var <= 0`` on a
+    pixel that would be used, and shapes that do not match, raise ValueError before any device call.  With all
+    three keywords at their defaults the fit is the reference's unweighted one, unchanged."""
+    if var is None and mask is None and not fit_back:
+        data = getattr(psfcube, 'data', psfcube)
+        data = np.ascontiguousarray(np.ma.getdata(data), dtype=np.float64)
+        lam = np.atleast_1d(np.asarray(lbda, dtype=float))
+        nimg, ny, nx = data.shape
+        if not circular:
+            efit = np.empty((nimg, _lib.EFIT_NPAR))
+            if nimg:
+                get_context().moffat_fit_elliptical(nimg, ny, nx, data, efit)
+            return _shape_table_from_fit(lam, efit)
+        ctx = get_context()
+        fit = np.empty((nimg, _lib.FIT_NPAR))
+        ctx.moffat_fit(nimg, ny, nx, data, fit)
+        return _table_from_fit(lam, fit)
     lam = np.atleast_1d(np.asarray(lbda, dtype=float))
+    data, weights = _star_weights(psfcube, var, mask)
     nimg, ny, nx = data.shape
-    if not circular:
-        efit = np.empty((nimg, _lib.EFIT_NPAR))
-        if nimg:
-            get_context().moffat_fit_elliptical(nimg, ny, nx, data, efit)
-        return _shape_table_from_fit(lam, efit)
-    ctx = get_context()
-    fit = np.empty((nimg, _lib.FIT_NPAR))
-    ctx.moffat_fit(nimg, ny, nx, data, fit)
-    return _table_from_fit(lam, fit)
+    npar = _lib.FIT_NPAR if circular else _lib.EFIT_NPAR
+    rec = np.empty((nimg, npar))
+    back = np.empty((nimg, _lib.BACK_NPAR))
+    if nimg:
+        get_context().moffat_fit_weighted(nimg, ny, nx, data, weights, rec, back, fit_back=fit_back,
+                                          elliptical=not circular)
+    tab = _table_from_fit(lam, rec) if circular else _shape_table_from_fit(lam, rec)
+    tab['cont'] = back[:, _lib.BACK_CONT].copy()
+    tab['err_cont'] = back[:, _lib.BACK_ERR_CONT].copy()
+    tab['npix'] = back[:, _lib.BACK_NPIX].astype(np.int64)
+    return tab
+
+
+def _star_weights(psfcube, var, mask):
+    """(data, weights) of a star fit, both C-contiguous float64 [nl, ny, nx]; see ``fit_psf_cube``.  Unused pixels
+    (weight 0) keep whatever data they hold: the library never reads them into a sum."""
+    raw = psfcube if np.ma.isMaskedArray(psfcube) else getattr(psfcube, 'data', psfcube)   # an mpdaf Cube's .data
+    data = np.array(np.ma.getdata(raw), dtype=np.float64, order='C')
+    if data.ndim != 3:
+        raise ValueError('psfcube must be [nl, ny, nx] (got shape %s)' % (data.shape,))
+    shape = data.shape
+
+    def planes(a, name):
+        a = np.asarray(a)
+        if a.shape == shape[1:]:
+            a = np.broadcast_to(a, shape)
+        if a.shape != shape:
+            raise ValueError('%s must have the cube\'s shape %s or %s (got %s)' % (name, shape, shape[1:], a.shape))
+        return a
+
+    bad = ~np.isfinite(data)
+    inmask = np.ma.getmask(raw)
+    if inmask is not np.ma.nomask:
+        bad |= planes(inmask, 'the mask of psfcube').astype(bool)
+    if mask is not None:
+        bad |= planes(np.ma.filled(mask, True) if np.ma.isMaskedArray(mask) else mask, 'mask').astype(bool)
+    if var is None:
+        weights = np.where(bad, 0.0, 1.0)
+    else:
+        v = planes(np.ma.filled(var, np.nan) if np.ma.isMaskedArray(var) else var, 'var').astype(np.float64)
+        bad |= ~np.isfinite(v)
+        if np.any(v[~bad] <= 0):
+            i = np.argwhere((v <= 0) & ~bad)[0]
+            raise ValueError('var must be > 0 on every used pixel (var[%d, %d, %d] = %g)'
+                             % (i[0], i[1], i[2], v[tuple(i)]))
+        weights = np.zeros(shape)
+        np.divide(1.0, v, out=weights, where=~bad)
+    return data, np.ascontiguousarray(weights)
 
 
 def encircled_energy(lbda, psfcube, radii, fractions=(0.5, 0.8), center=None, pixscale=_PIXSCALE):
