@@ -355,13 +355,20 @@ static int alloc_band_staging(Ctx* c) {
     return PSFR_OK;
 }
 
-// band outputs of a run_batch call: per-draw images, fits and EE records, then those of the exposure means
-struct BandOut {
-    int nband = 0;
+// Outputs of a fused call (run_batch), each NULL or an array on either side: the per-draw ones first, then those
+// of the exposure means.  nrad / nfrac size the EE records, nband and sums the band images.
+enum { kCube, kFit, kEfit, kEe, kStrehl, kVar, kBand, kBandFit, kBandEe,
+       kMean, kMeanFit, kMeanEfit, kMeanEe, kMeanBand, kMeanBandFit, kMeanBandEe, kNumOut };
+struct BatchOut {
+    double* out[kNumOut] = {};
+    int nrad = 0, nfrac = 0, nband = 0;
     BandSums sums;
-    double* out[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    bool any(int first, int last) const {   // whether one of the outputs first..last is requested
+        for (int i = first; i <= last; ++i)
+            if (out[i]) return true;
+        return false;
+    }
 };
-enum { kBand = 0, kBandFit = 1, kBandEe = 2, kMeanBand = 3, kMeanBandFit = 4, kMeanBandEe = 5 };
 
 constexpr int kMaxHotEvents = 512;
 struct HotTimer {
@@ -387,16 +394,12 @@ static int hot_begin(Ctx* c) {
 // max_planes / ndir draws: PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit, and
 // with ngroup > 0 the time mean of every exposure (draws [group_end[g-1], group_end[g])) and its fit in the
 // chunk where the exposure's last draw lies.  field: every (draw, direction) plane keeps its own PSF instead
-// of the draw's field mean, so a draw owns ndir x nlam images in every output (out_var: ndir records in either
-// mode).  Host outputs leave through
-// a second stream: the results of chunk i are copied out while chunk i + 1 computes, from staging buffers
-// that alternate between two sets.
+// of the draw's field mean, so a draw owns ndir x nlam images in every output (kVar: ndir records in either
+// mode).  Host outputs leave through a second stream: the results of chunk i are copied out while chunk i + 1
+// computes, from staging buffers that alternate between two sets.
 static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const double* dirs, int ngs, int npos,
                      const double* poslgs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
-                     bool field, double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
-                     double* out_efit, double* out_mean_efit, int nrad, int nfrac, double* out_ee,
-                     double* out_mean_ee, double* out_strehl, double* out_var, cudaStream_t s,
-                     const BandOut* bo = nullptr) {
+                     bool field, const BatchOut& o, cudaStream_t s) {
     PSFR_CUDA(c, cudaSetDevice(c->device));
     std::vector<double> lam;
     int rc = small_to_host(c, lam, lambda_nm, nlam > 0 ? nlam : 0, s);
@@ -411,7 +414,6 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     rc = check_alpha_tt(c, ndraw, h.data() + PSFR_DRAW_ALPHA_TT, PSFR_DRAW_NPAR);
     if (rc) return rc;
     hot_begin(c);
-    c->hot_timed = true;
     const int per_chunk = c->max_planes / ndir;
     // output planes per draw; a chunk's nd * ppd * nlam images fit every [max_planes * max_lambda]-image
     // buffer (d_samp, d_cube*, d_fit*, d_mean[b], d_mfit[b], d_carry) because nd * ndir <= max_planes
@@ -419,36 +421,25 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     const size_t img = (size_t)kPSF * kPSF, imgs = (size_t)ppd * nlam, elems = imgs * img;
     const size_t fits = imgs * PSFR_FIT_NPAR;   // fit records per draw
     const size_t efits = imgs * PSFR_EFIT_NPAR;  // elliptical records per draw
-    const size_t ees = imgs * (size_t)(nrad + 1 + nfrac);   // encircled-energy values per draw
-    const size_t vars = (size_t)ndir * PSFR_VAR_NPAR;       // variance values per draw
-    const bool cube_dev = out_cube && is_device_ptr(out_cube);
-    const bool fit_dev = out_fit && is_device_ptr(out_fit);
-    const bool mean_dev = out_mean && is_device_ptr(out_mean);
-    const bool mfit_dev = out_mean_fit && is_device_ptr(out_mean_fit);
-    const bool efit_dev = out_efit && is_device_ptr(out_efit);
-    const bool mefit_dev = out_mean_efit && is_device_ptr(out_mean_efit);
-    const bool ee_dev = out_ee && is_device_ptr(out_ee);
-    const bool mee_dev = out_mean_ee && is_device_ptr(out_mean_ee);
-    const bool strehl_dev = out_strehl && is_device_ptr(out_strehl);
-    const bool var_dev = out_var && is_device_ptr(out_var);
-    // band outputs (DESIGN.md 5.6): bout[i] NULL or a pointer on either side, bdev[i] whether it is on the device
-    double* bout[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    bool bdev[6] = {false, false, false, false, false, false}, band_host = false;
-    const int nband = bo ? bo->nband : 0;
-    for (int i = 0; bo && i < 6; ++i) {
-        bout[i] = bo->out[i];
-        bdev[i] = bout[i] && is_device_ptr(bout[i]);
-        band_host |= bout[i] && !bdev[i];
+    const size_t ees = imgs * (size_t)(o.nrad + 1 + o.nfrac);   // encircled-energy values per draw
+    const size_t vars = (size_t)ndir * PSFR_VAR_NPAR;           // variance values per draw
+    const size_t bsets = (size_t)ppd * o.nband;                 // band images per draw and per exposure
+    const size_t belems = bsets * img, bfits = bsets * PSFR_FIT_NPAR, bees = bsets * (size_t)(o.nrad + 1 + o.nfrac);
+    // values per draw or exposure of each output, and the staging sets that hold it when it is not on the device
+    const size_t per[kNumOut] = {elems, fits, efits, ees, imgs, vars, belems, bfits, bees,
+                                 elems, fits, efits, ees, belems, bfits, bees};
+    double* const stage[kNumOut][2] = {
+        {c->d_cube2, c->d_cube3}, {c->d_fit, c->d_fit2}, {c->d_efit, c->d_efit2}, {c->d_ee[0], c->d_ee[1]},
+        {c->d_strehl[0], c->d_strehl[1]}, {c->d_var[0], c->d_var[1]}, {c->d_band[0], c->d_band[1]},
+        {c->d_bfit[0], c->d_bfit[1]}, {c->d_bee[0], c->d_bee[1]}, {c->d_mean[0], c->d_mean[1]},
+        {c->d_mfit[0], c->d_mfit[1]}, {c->d_mefit[0], c->d_mefit[1]}, {c->d_mee[0], c->d_mee[1]},
+        {c->d_mband[0], c->d_mband[1]}, {c->d_mbfit[0], c->d_mbfit[1]}, {c->d_mbee[0], c->d_mbee[1]}};
+    bool dev[kNumOut], host_out = false;
+    for (int i = 0; i < kNumOut; ++i) {
+        dev[i] = o.out[i] && is_device_ptr(o.out[i]);
+        host_out |= o.out[i] && !dev[i];
     }
-    const bool bands = bout[kBand] || bout[kBandFit] || bout[kBandEe];
-    const bool mbands = bout[kMeanBand] || bout[kMeanBandFit] || bout[kMeanBandEe];
-    const size_t bsets = (size_t)ppd * nband;                     // band images per draw and per exposure
-    const size_t belems = bsets * img, bfits = bsets * PSFR_FIT_NPAR, bees = bsets * (size_t)(nrad + 1 + nfrac);
-    const bool means = out_mean || out_mean_fit || out_mean_efit || out_mean_ee || mbands;
-    const bool host_out = (out_cube && !cube_dev) || (out_fit && !fit_dev) || (out_mean && !mean_dev) ||
-                          (out_mean_fit && !mfit_dev) || (out_efit && !efit_dev) || (out_mean_efit && !mefit_dev) ||
-                          (out_ee && !ee_dev) || (out_mean_ee && !mee_dev) || (out_strehl && !strehl_dev) ||
-                          (out_var && !var_dev) || band_host;
+    const bool bands = o.any(kBand, kBandEe), mbands = o.any(kMeanBand, kMeanBandEe), means = o.any(kMean, kMeanBandEe);
     int* seg_dev = reinterpret_cast<int*>(c->d_misc + misc_groups(c->max_planes));
     std::vector<int> seg;
     int g0 = 0;   // first exposure not finished in an earlier chunk
@@ -456,6 +447,11 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
     for (int d0 = 0; d0 < ndraw; d0 += per_chunk, ++chunk) {
         const int nd = std::min(per_chunk, ndraw - d0);
         const int b = chunk & 1;
+        // where each output of the chunk is written: the caller's array at its first draw (exposure g0 for the
+        // means) when that array is on the device, staging set b otherwise
+        double* dst[kNumOut];
+        for (int i = 0; i < kNumOut; ++i)
+            dst[i] = dev[i] ? o.out[i] + (size_t)(i < kMean ? d0 : g0) * per[i] : stage[i][b];
         rc = upload_draws(c, nd, draws + (size_t)d0 * PSFR_DRAW_NPAR, ndir, s);
         if (rc) break;
         if ((rc = run_psd(c, nd, ndir, ngs, npos, s, false))) break;
@@ -470,35 +466,26 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
         }
         // the AO records of the chunk: d_psdq / d_ao still hold its PSDs and d_samp its raw samples, and staging
         // set b is free again
-        double* var = var_dev ? out_var + (size_t)d0 * vars : c->d_var[b];
-        if (out_var && (rc = run_var(c, nd, ndir, ngs, npos, var, s))) break;
-        double* strehl = strehl_dev ? out_strehl + (size_t)d0 * imgs : c->d_strehl[b];
-        if (out_strehl && (rc = run_strehl(c, nd * (int)imgs, strehl, s))) break;
-        double* conv = cube_dev ? out_cube + (size_t)d0 * elems : (b ? c->d_cube3 : c->d_cube2);
-        if ((rc = run_convolve(c, nd, ppd, nlam, c->d_cube, conv, s))) break;
-        double* fit = fit_dev ? out_fit + (size_t)d0 * fits : (b ? c->d_fit2 : c->d_fit);
+        if (o.out[kVar] && (rc = run_var(c, nd, ndir, ngs, npos, dst[kVar], s))) break;
+        if (o.out[kStrehl] && (rc = run_strehl(c, nd * (int)imgs, dst[kStrehl], s))) break;
+        if ((rc = run_convolve(c, nd, ppd, nlam, c->d_cube, dst[kCube], s))) break;
         // the elliptical fit starts from the circular records of the same images
-        if ((out_fit || out_efit) && (rc = run_fit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, s))) break;
-        double* efit = efit_dev ? out_efit + (size_t)d0 * efits : (b ? c->d_efit2 : c->d_efit);
-        if (out_efit && (rc = run_efit(c, nd * (int)imgs, kPSF, kPSF, conv, fit, efit, s))) break;
-        double* ee = ee_dev ? out_ee + (size_t)d0 * ees : c->d_ee[b];
-        if (out_ee && (rc = run_ee(c, nd * (int)imgs, kPSF, kPSF, conv, nullptr, nrad, nfrac, ee, s))) break;
+        if ((o.out[kFit] || o.out[kEfit]) && (rc = run_fit(c, nd * (int)imgs, kPSF, kPSF, dst[kCube], dst[kFit], s)))
+            break;
+        if (o.out[kEfit] && (rc = run_efit(c, nd * (int)imgs, kPSF, kPSF, dst[kCube], dst[kFit], dst[kEfit], s))) break;
+        if (o.out[kEe] &&
+            (rc = run_ee(c, nd * (int)imgs, kPSF, kPSF, dst[kCube], nullptr, o.nrad, o.nfrac, dst[kEe], s)))
+            break;
         // the band images of the chunk's image sets, read from the convolved planes, then their fits and EE
-        double* band = bdev[kBand] ? bout[kBand] + (size_t)d0 * belems : c->d_band[b];
-        if (bands && (rc = run_band(c, (long long)nd * ppd, nlam, (int)img, nband, bo->sums, conv, band, s))) break;
-        double* bfit = bdev[kBandFit] ? bout[kBandFit] + (size_t)d0 * bfits : c->d_bfit[b];
-        if (bout[kBandFit] && (rc = run_fit(c, nd * (int)bsets, kPSF, kPSF, band, bfit, s))) break;
-        double* bee = bdev[kBandEe] ? bout[kBandEe] + (size_t)d0 * bees : c->d_bee[b];
-        if (bout[kBandEe] && (rc = run_ee(c, nd * (int)bsets, kPSF, kPSF, band, nullptr, nrad, nfrac, bee, s))) break;
+        if (bands &&
+            (rc = run_band(c, (long long)nd * ppd, nlam, (int)img, o.nband, o.sums, dst[kCube], dst[kBand], s)))
+            break;
+        if (o.out[kBandFit] && (rc = run_fit(c, nd * (int)bsets, kPSF, kPSF, dst[kBand], dst[kBandFit], s))) break;
+        if (o.out[kBandEe] &&
+            (rc = run_ee(c, nd * (int)bsets, kPSF, kPSF, dst[kBand], nullptr, o.nrad, o.nfrac, dst[kBandEe], s)))
+            break;
         // exposures g0, g0 + 1, ... that have draws in [d0, d0 + nd): all but possibly the last end here
         int ndone = 0;
-        double* mean = mean_dev ? out_mean + (size_t)g0 * elems : c->d_mean[b];
-        double* mfit = mfit_dev ? out_mean_fit + (size_t)g0 * fits : c->d_mfit[b];
-        double* mefit = mefit_dev ? out_mean_efit + (size_t)g0 * efits : c->d_mefit[b];
-        double* mee = mee_dev ? out_mean_ee + (size_t)g0 * ees : c->d_mee[b];
-        double* mband = bdev[kMeanBand] ? bout[kMeanBand] + (size_t)g0 * belems : c->d_mband[b];
-        double* mbfit = bdev[kMeanBandFit] ? bout[kMeanBandFit] + (size_t)g0 * bfits : c->d_mbfit[b];
-        double* mbee = bdev[kMeanBandEe] ? bout[kMeanBandEe] + (size_t)g0 * bees : c->d_mbee[b];
         if (means) {
             seg.clear();
             for (int g = g0; g < ngroup && (g == g0 || group_end[g - 1] < d0 + nd); ++g) {
@@ -512,60 +499,36 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
                 rc = set_error(c, PSFR_E_CUDA, "segment upload failed: %s", cudaGetErrorString(cudaGetLastError()));
                 break;
             }
-            if ((rc = run_group_mean(c, (int)elems, conv, seg_dev, (int)seg.size() / 2, carry_in, mean, s))) break;
-            if ((out_mean_fit || out_mean_efit) && ndone && (rc = run_fit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, s)))
+            if ((rc = run_group_mean(c, (int)elems, dst[kCube], seg_dev, (int)seg.size() / 2, carry_in, dst[kMean], s)))
                 break;
-            if (out_mean_efit && ndone && (rc = run_efit(c, ndone * (int)imgs, kPSF, kPSF, mean, mfit, mefit, s))) break;
-            if (out_mean_ee && ndone && (rc = run_ee(c, ndone * (int)imgs, kPSF, kPSF, mean, nullptr, nrad, nfrac, mee, s)))
+            if ((o.out[kMeanFit] || o.out[kMeanEfit]) && ndone &&
+                (rc = run_fit(c, ndone * (int)imgs, kPSF, kPSF, dst[kMean], dst[kMeanFit], s)))
+                break;
+            if (o.out[kMeanEfit] && ndone &&
+                (rc = run_efit(c, ndone * (int)imgs, kPSF, kPSF, dst[kMean], dst[kMeanFit], dst[kMeanEfit], s)))
+                break;
+            if (o.out[kMeanEe] && ndone &&
+                (rc = run_ee(c, ndone * (int)imgs, kPSF, kPSF, dst[kMean], nullptr, o.nrad, o.nfrac, dst[kMeanEe], s)))
                 break;
             if (mbands && ndone &&
-                (rc = run_band(c, (long long)ndone * ppd, nlam, (int)img, nband, bo->sums, mean, mband, s)))
+                (rc = run_band(c, (long long)ndone * ppd, nlam, (int)img, o.nband, o.sums, dst[kMean], dst[kMeanBand], s)))
                 break;
-            if (bout[kMeanBandFit] && ndone && (rc = run_fit(c, ndone * (int)bsets, kPSF, kPSF, mband, mbfit, s))) break;
-            if (bout[kMeanBandEe] && ndone &&
-                (rc = run_ee(c, ndone * (int)bsets, kPSF, kPSF, mband, nullptr, nrad, nfrac, mbee, s)))
+            if (o.out[kMeanBandFit] && ndone &&
+                (rc = run_fit(c, ndone * (int)bsets, kPSF, kPSF, dst[kMeanBand], dst[kMeanBandFit], s)))
+                break;
+            if (o.out[kMeanBandEe] && ndone &&
+                (rc = run_ee(c, ndone * (int)bsets, kPSF, kPSF, dst[kMeanBand], nullptr, o.nrad, o.nfrac,
+                             dst[kMeanBandEe], s)))
                 break;
         }
         if (host_out) {
+            // the host outputs of the chunk's nd draws and of the ndone exposures that end in it
             cudaError_t e = cudaEventRecord(c->ev_done[b], s);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(c->copy_stream, c->ev_done[b], 0);
-            if (e == cudaSuccess && out_cube && !cube_dev)
-                e = cudaMemcpyAsync(out_cube + (size_t)d0 * elems, conv, (size_t)nd * elems * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && out_fit && !fit_dev)
-                e = cudaMemcpyAsync(out_fit + (size_t)d0 * fits, fit, (size_t)nd * fits * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && ndone && out_mean && !mean_dev)
-                e = cudaMemcpyAsync(out_mean + (size_t)g0 * elems, mean, (size_t)ndone * elems * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && ndone && out_mean_fit && !mfit_dev)
-                e = cudaMemcpyAsync(out_mean_fit + (size_t)g0 * fits, mfit, (size_t)ndone * fits * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && out_efit && !efit_dev)
-                e = cudaMemcpyAsync(out_efit + (size_t)d0 * efits, efit, (size_t)nd * efits * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && ndone && out_mean_efit && !mefit_dev)
-                e = cudaMemcpyAsync(out_mean_efit + (size_t)g0 * efits, mefit, (size_t)ndone * efits * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && out_ee && !ee_dev)
-                e = cudaMemcpyAsync(out_ee + (size_t)d0 * ees, ee, (size_t)nd * ees * sizeof(double), cudaMemcpyDefault,
-                                    c->copy_stream);
-            if (e == cudaSuccess && ndone && out_mean_ee && !mee_dev)
-                e = cudaMemcpyAsync(out_mean_ee + (size_t)g0 * ees, mee, (size_t)ndone * ees * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && out_var && !var_dev)
-                e = cudaMemcpyAsync(out_var + (size_t)d0 * vars, var, (size_t)nd * vars * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            if (e == cudaSuccess && out_strehl && !strehl_dev)
-                e = cudaMemcpyAsync(out_strehl + (size_t)d0 * imgs, strehl, (size_t)nd * imgs * sizeof(double),
-                                    cudaMemcpyDefault, c->copy_stream);
-            // band results: per-draw ones of the chunk's nd draws, those of the ndone exposures that end here
-            const double* bsrc[6] = {band, bfit, bee, mband, mbfit, mbee};
-            const size_t bper[6] = {belems, bfits, bees, belems, bfits, bees};
-            for (int i = 0; i < 6 && e == cudaSuccess; ++i) {
-                const size_t first = i < kMeanBand ? (size_t)d0 : (size_t)g0, count = i < kMeanBand ? nd : ndone;
-                if (bout[i] && !bdev[i] && count)
-                    e = cudaMemcpyAsync(bout[i] + first * bper[i], bsrc[i], count * bper[i] * sizeof(double),
+            for (int i = 0; i < kNumOut && e == cudaSuccess; ++i) {
+                const size_t first = i < kMean ? d0 : g0, count = i < kMean ? nd : ndone;
+                if (o.out[i] && !dev[i] && count)
+                    e = cudaMemcpyAsync(o.out[i] + first * per[i], dst[i], count * per[i] * sizeof(double),
                                         cudaMemcpyDefault, c->copy_stream);
             }
             if (e == cudaSuccess) e = cudaEventRecord(c->ev_copied[b], c->copy_stream);
@@ -576,7 +539,6 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
         }
         g0 += ndone;
     }
-    c->hot_timed = false;
     if (host_out) {
         // host outputs are complete on return; later work on `s` must not overtake the copies
         cudaError_t e = cudaStreamSynchronize(c->copy_stream);
@@ -1073,20 +1035,22 @@ int psfr_compute_batch(psfr_ctx* c, int ndraw, const double* draws, int ndir, co
     if (ndraw < 1 || ndir < 1 || ndir > c->max_planes)
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d ndir=%d max_planes=%d", ndraw, ndir, c->max_planes);
     if (ngs < 1) return set_error(c, PSFR_E_ARG, "ngs=%d outside [1,%d]", ngs, kMaxGS);
-    return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, false, out_cube,
-                     out_fit, nullptr, nullptr, nullptr, nullptr, 0, 0, nullptr, nullptr,
-                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    return run_batch(c, ndraw, draws, ndir, dirs, ngs, ngs, poslgs, nlam, lambda_nm, 0, nullptr, false, o,
+                     static_cast<cudaStream_t>(stream));
 }
 
 // the arguments of psfr_compute_groups and psfr_compute_field that run_batch does not check itself
 static int check_groups(Ctx* c, int ndraw, const double* draws, const double* poslgs, int ndir, const double* dirs,
-                        const double* lambda_nm, int ngroup, const int* group_end, bool means) {
+                        const double* lambda_nm, int ngroup, const int* group_end, const BatchOut& o) {
     if (!c || !draws || !dirs || !poslgs || !lambda_nm || (ngroup > 0 && !group_end))
         return set_error(c, PSFR_E_ARG, "NULL argument");
     if (ndraw < 1 || ndir < 1 || ndir > c->max_planes)
         return set_error(c, PSFR_E_CAPACITY, "ndraw=%d ndir=%d max_planes=%d", ndraw, ndir, c->max_planes);
     if (ngroup < 0) return set_error(c, PSFR_E_ARG, "ngroup=%d", ngroup);
-    if (ngroup == 0 && means)
+    if (ngroup == 0 && o.any(kMean, kMeanBandEe))
         return set_error(c, PSFR_E_ARG, "exposure means need at least one exposure (ngroup=0)");
     for (int g = 0; g < ngroup; ++g)
         if (group_end[g] <= (g ? group_end[g - 1] : 0))
@@ -1099,33 +1063,43 @@ static int check_groups(Ctx* c, int ndraw, const double* draws, const double* po
 int psfr_compute_groups(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
                         const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                         double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean || out_mean_fit))
-        return rc;
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, false,
-                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, 0, 0, nullptr, nullptr,
-                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    o.out[kMean] = out_mean;
+    o.out[kMeanFit] = out_mean_fit;
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, o)) return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, false, o,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
                        const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                        double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, out_mean || out_mean_fit))
-        return rc;
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
-                     out_cube, out_fit, out_mean, out_mean_fit, nullptr, nullptr, 0, 0, nullptr, nullptr,
-                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    o.out[kMean] = out_mean;
+    o.out[kMeanFit] = out_mean_fit;
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, o)) return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true, o,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_field_shapes(psfr_ctx* c, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
                               const double* dirs, int nlam, const double* lambda_nm, int ngroup, const int* group_end,
                               double* out_cube, double* out_fit, double* out_mean, double* out_mean_fit,
                               double* out_efit, double* out_mean_efit, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
-                              out_mean || out_mean_fit || out_mean_efit))
-        return rc;
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true,
-                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, 0, 0, nullptr, nullptr,
-                     nullptr, nullptr, static_cast<cudaStream_t>(stream));
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    o.out[kEfit] = out_efit;
+    o.out[kMean] = out_mean;
+    o.out[kMeanFit] = out_mean_fit;
+    o.out[kMeanEfit] = out_mean_efit;
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, o)) return rc;
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, true, o,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int psfr_compute_energy(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs,
@@ -1133,15 +1107,22 @@ int psfr_compute_energy(psfr_ctx* c, int field, int ndraw, const double* draws, 
                         int nrad, const double* radii_px, int nfrac, const double* fracs, double* out_cube,
                         double* out_fit, double* out_mean, double* out_mean_fit, double* out_efit,
                         double* out_mean_efit, double* out_ee, double* out_mean_ee, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
-                              out_mean || out_mean_fit || out_mean_efit || out_mean_ee))
-        return rc;
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    o.out[kEfit] = out_efit;
+    o.out[kEe] = out_ee;
+    o.out[kMean] = out_mean;
+    o.out[kMeanFit] = out_mean_fit;
+    o.out[kMeanEfit] = out_mean_efit;
+    o.out[kMeanEe] = out_mean_ee;
+    o.nrad = nrad;
+    o.nfrac = nfrac;
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, o)) return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     PSFR_CUDA(c, cudaSetDevice(c->device));
     if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
-                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
-                     out_mean_ee, nullptr, nullptr, s);
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0, o, s);
 }
 
 int psfr_compute_ao(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs, int ndir,
@@ -1149,15 +1130,24 @@ int psfr_compute_ao(psfr_ctx* c, int field, int ndraw, const double* draws, int 
                     const double* radii_px, int nfrac, const double* fracs, double* out_cube, double* out_fit,
                     double* out_mean, double* out_mean_fit, double* out_efit, double* out_mean_efit, double* out_ee,
                     double* out_mean_ee, double* out_strehl, double* out_var, void* stream) {
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
-                              out_mean || out_mean_fit || out_mean_efit || out_mean_ee))
-        return rc;
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    o.out[kEfit] = out_efit;
+    o.out[kEe] = out_ee;
+    o.out[kStrehl] = out_strehl;
+    o.out[kVar] = out_var;
+    o.out[kMean] = out_mean;
+    o.out[kMeanFit] = out_mean_fit;
+    o.out[kMeanEfit] = out_mean_efit;
+    o.out[kMeanEe] = out_mean_ee;
+    o.nrad = nrad;
+    o.nfrac = nfrac;
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, o)) return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     PSFR_CUDA(c, cudaSetDevice(c->device));
     if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
-                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
-                     out_mean_ee, out_strehl, out_var, s);
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0, o, s);
 }
 
 int psfr_compute_bands(psfr_ctx* c, int field, int ndraw, const double* draws, int npos, const double* poslgs,
@@ -1167,29 +1157,37 @@ int psfr_compute_bands(psfr_ctx* c, int field, int ndraw, const double* draws, i
                        double* out_ee, double* out_mean_ee, double* out_strehl, double* out_var, int nband,
                        const double* weights, double* out_band, double* out_band_fit, double* out_band_ee,
                        double* out_mean_band, double* out_mean_band_fit, double* out_mean_band_ee, void* stream) {
-    BandOut bo;
-    double* outs[6] = {out_band, out_band_fit, out_band_ee, out_mean_band, out_mean_band_fit, out_mean_band_ee};
-    bool any = false;
-    for (int i = 0; i < 6; ++i) {
-        bo.out[i] = outs[i];
-        any |= outs[i] != nullptr;
-    }
-    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end,
-                              out_mean || out_mean_fit || out_mean_efit || out_mean_ee || out_mean_band ||
-                              out_mean_band_fit || out_mean_band_ee))
-        return rc;
+    BatchOut o;
+    o.out[kCube] = out_cube;
+    o.out[kFit] = out_fit;
+    o.out[kEfit] = out_efit;
+    o.out[kEe] = out_ee;
+    o.out[kStrehl] = out_strehl;
+    o.out[kVar] = out_var;
+    o.out[kBand] = out_band;
+    o.out[kBandFit] = out_band_fit;
+    o.out[kBandEe] = out_band_ee;
+    o.out[kMean] = out_mean;
+    o.out[kMeanFit] = out_mean_fit;
+    o.out[kMeanEfit] = out_mean_efit;
+    o.out[kMeanEe] = out_mean_ee;
+    o.out[kMeanBand] = out_mean_band;
+    o.out[kMeanBandFit] = out_mean_band_fit;
+    o.out[kMeanBandEe] = out_mean_band_ee;
+    o.nrad = nrad;
+    o.nfrac = nfrac;
+    if (int rc = check_groups(c, ndraw, draws, poslgs, ndir, dirs, lambda_nm, ngroup, group_end, o)) return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     PSFR_CUDA(c, cudaSetDevice(c->device));
-    if (any || nband != 0) {
-        if (int rc = upload_band_weights(c, nband, nlam, weights, bo.sums, s)) return rc;
-        bo.nband = nband;
+    const bool band_out = o.any(kBand, kBandEe) || o.any(kMeanBand, kMeanBandEe);
+    if (band_out || nband != 0) {
+        if (int rc = upload_band_weights(c, nband, nlam, weights, o.sums, s)) return rc;
+        o.nband = nband;
     }
-    if (any)
+    if (band_out)
         if (int rc = alloc_band_staging(c)) return rc;
     if (int rc = upload_ee_params(c, nrad, radii_px, nfrac, fracs, s)) return rc;
-    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0,
-                     out_cube, out_fit, out_mean, out_mean_fit, out_efit, out_mean_efit, nrad, nfrac, out_ee,
-                     out_mean_ee, out_strehl, out_var, s, any ? &bo : nullptr);
+    return run_batch(c, ndraw, draws, ndir, dirs, 0, npos, poslgs, nlam, lambda_nm, ngroup, group_end, field != 0, o, s);
 }
 
 int psfr_band_psf(psfr_ctx* c, int ncube, int nlam, int ny, int nx, const double* cubes, int nband,

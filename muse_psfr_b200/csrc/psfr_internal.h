@@ -170,15 +170,13 @@ struct Ctx {
     cudaStream_t copy_stream = nullptr;      // device -> host copies of finished chunks
     cudaEvent_t ev_done[2] = {nullptr, nullptr};    // chunk results ready (compute stream)
     cudaEvent_t ev_copied[2] = {nullptr, nullptr};  // chunk results copied out (copy stream)
-    double* d_stage = nullptr;   // generic staging for host inputs (max_planes*N*N doubles)
     double* d_poly = nullptr;    // polynomial fit scratch
     void* h_pinned = nullptr;    // pinned bounce buffer
     size_t h_pinned_bytes = 0;
 
-    cudaEvent_t ev_hot0 = nullptr, ev_hot1 = nullptr;
+    cudaEvent_t ev_hot0 = nullptr;
     int hot_launches = 0;
     long long hot_psfs = 0;
-    bool hot_timed = false;
 
     // kernels whose dynamic shared-memory limit has been raised on THIS device (the attribute is
     // per device, so a process-wide flag would break a second context on another GPU)

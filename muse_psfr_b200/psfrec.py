@@ -773,6 +773,20 @@ def _band_outputs(bands, nl, lead, ee_rec):
     return out + ((np.empty(lead + (nb, ee_rec)),) if ee_rec is not None else ())
 
 
+def _fused(ctx, field, recs, dirs, lam, group_end=None, ee=None, bands=None, stream=None, **outs):
+    """One pass of the fused pipeline (``Context.compute_bands``) over draws that each carry their guide-star count:
+    ``ee`` (radii [px], fractions) or None, ``bands`` weights [nband, nl] or None, and the outputs ``outs`` (keywords
+    of ``compute_bands``).  PSFR_E_UNSUPPORTED (a wavelength or draw outside the library's range) raises ValueError."""
+    rad, frac = ((), ()) if ee is None else ee
+    try:
+        ctx.compute_bands(field, recs, dirs, _lgs_positions(False), lam, bands, rad, frac, group_end, stream=stream,
+                          **outs)
+    except PsfrError as exc:
+        if exc.code == _lib.E_UNSUPPORTED:
+            raise ValueError(str(exc))
+        raise
+
+
 def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs_mode=False,
                       out_cube=None, out_fit=None, want_cube=True, device=None, max_planes=None, stream=None,
                       dim=_DIM, zenith=0., Cn2=None, wind_dir=None, ee_radii=None, ee_fractions=(0.5, 0.8),
@@ -834,31 +848,22 @@ def compute_psf_batch(lbda, seeing, GL, L0, npsflin=1, h=(100, 10000), three_lgs
         out_fit = np.empty((nd, lam.size, _lib.FIT_NPAR))
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
+    if per_draw or energy or ao_budget or band:
+        # each draw's own guide-star count: the three-laser asterism is the first three stars of the four-laser one
+        _fused(ctx, False, recs, dirs, lam, ee=(rad_px, frac) if energy else None,
+               bands=_band_params(bands, lam.size) if band else None, stream=stream, out_cube=out_cube,
+               out_fit=out_fit, out_ee=ee if energy else None, out_strehl=ao[0] if ao else None,
+               out_var=ao[1] if ao else None, out_band=band[1] if band else None,
+               out_band_fit=band[0] if band else None, out_band_ee=band[2] if band and energy else None)
+        return (out_fit, out_cube) + extra
     try:
-        if band:
-            ctx.compute_bands(False, recs, dirs, _lgs_positions(False), lam, _band_params(bands, lam.size),
-                              rad_px if energy else (), frac if energy else (), out_cube=out_cube, out_fit=out_fit,
-                              out_ee=ee if energy else None, out_strehl=ao[0] if ao else None,
-                              out_var=ao[1] if ao else None, out_band=band[1], out_band_fit=band[0],
-                              out_band_ee=band[2] if energy else None, stream=stream)
-        elif ao_budget:
-            ctx.compute_ao(False, recs, dirs, _lgs_positions(False), lam, rad_px if energy else (),
-                           frac if energy else (), out_cube=out_cube, out_fit=out_fit, out_ee=ee if energy else None,
-                           out_strehl=ao[0], out_var=ao[1], stream=stream)
-        elif energy:
-            ctx.compute_energy(False, recs, dirs, _lgs_positions(False), lam, rad_px, frac, out_cube=out_cube,
-                               out_fit=out_fit, out_ee=ee, stream=stream)
-        elif per_draw:    # the three-laser asterism is the first three stars of the four-laser one
-            ctx.compute_groups(recs, dirs, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit,
-                               stream=stream)
-        else:
-            ctx.compute_batch(recs, dirs, _lgs_positions(three_lgs_mode), lam, out_cube=out_cube,
-                              out_fit=out_fit, stream=stream)
+        ctx.compute_batch(recs, dirs, _lgs_positions(three_lgs_mode), lam, out_cube=out_cube, out_fit=out_fit,
+                          stream=stream)
     except PsfrError as exc:
         if exc.code == _lib.E_UNSUPPORTED:
             raise ValueError(str(exc))
         raise
-    return (out_fit, out_cube) + extra
+    return out_fit, out_cube
 
 
 def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_size=60, h=(100, 10000),
@@ -919,27 +924,11 @@ def compute_psf_field(lbda, seeing, GL, L0, positions=None, npsflin=3, field_siz
         out_fit = np.empty((nd, npos, lam.size, _lib.FIT_NPAR))
     if out_cube is None and want_cube:
         out_cube = np.empty((nd, npos, lam.size, _lib.PSF_DIM, _lib.PSF_DIM))
-    try:
-        if band:
-            ctx.compute_bands(True, recs, pos, _lgs_positions(False), lam, _band_params(bands, lam.size),
-                              rad_px if energy else (), frac if energy else (), out_cube=out_cube, out_fit=out_fit,
-                              out_efit=efit, out_ee=ee if energy else None, out_strehl=ao[0] if ao else None,
-                              out_var=ao[1] if ao else None, out_band=band[1], out_band_fit=band[0],
-                              out_band_ee=band[2] if energy else None, stream=stream)
-        elif ao_budget:
-            ctx.compute_ao(True, recs, pos, _lgs_positions(False), lam, rad_px if energy else (),
-                           frac if energy else (), out_cube=out_cube, out_fit=out_fit, out_efit=efit,
-                           out_ee=ee if energy else None, out_strehl=ao[0], out_var=ao[1], stream=stream)
-        elif energy:
-            ctx.compute_energy(True, recs, pos, _lgs_positions(False), lam, rad_px, frac, out_cube=out_cube,
-                               out_fit=out_fit, out_efit=efit, out_ee=ee, stream=stream)
-        else:
-            ctx.compute_field(recs, pos, _lgs_positions(False), lam, out_cube=out_cube, out_fit=out_fit,
-                              stream=stream, out_efit=efit)
-    except PsfrError as exc:
-        if exc.code == _lib.E_UNSUPPORTED:
-            raise ValueError(str(exc))
-        raise
+    _fused(ctx, True, recs, pos, lam, ee=(rad_px, frac) if energy else None,
+           bands=_band_params(bands, lam.size) if band else None, stream=stream, out_cube=out_cube, out_fit=out_fit,
+           out_efit=efit, out_ee=ee if energy else None, out_strehl=ao[0] if ao else None,
+           out_var=ao[1] if ao else None, out_band=band[1] if band else None, out_band_fit=band[0] if band else None,
+           out_band_ee=band[2] if band and energy else None)
     return (out_fit, out_cube) + extra
 
 
@@ -1156,67 +1145,37 @@ def compute_psf_from_sparta_batch(sources, extname='SPARTA_ATM_DATA', npsflin=1,
     fit_mean = np.empty((ng, nlam, _lib.FIT_NPAR))
     dirs = direction_perf(npsflin)
     ctx = _planes_context(nd, dirs.shape[1], nlam, max_planes, device, _DIM)
-    try:
-        if energy:
-            ee_mean = np.empty((ng, nlam, ee_rec))
+    ee_par = (rad_px, frac) if energy else None
+    ee_mean = np.empty((ng, nlam, ee_rec)) if energy else None
+    if ao_budget:
+        strehl = np.empty((nd, nlam))
+        var = np.empty((nd, dirs.shape[1], _lib.VAR_NPAR))
+    band_mean = _band_outputs(w_band, nlam, (ng,), ee_rec if energy else None)
+    _fused(ctx, False, draws, dirs, lbda, group_end, ee=ee_par, bands=w_band, out_fit=fit, out_mean=psftot,
+           out_mean_fit=fit_mean, out_mean_ee=ee_mean, out_strehl=strehl if ao_budget else None,
+           out_var=var if ao_budget else None, out_mean_band=band_mean[1] if band_mean else None,
+           out_mean_band_fit=band_mean[0] if band_mean else None,
+           out_mean_band_ee=band_mean[2] if band_mean and energy else None)
+    if pos is not None:
+        npos = pos.shape[1]
+        psf_field = np.empty((ng, npos, nlam, _lib.PSF_DIM, _lib.PSF_DIM))
+        fit_field = np.empty((ng, npos, nlam, _lib.FIT_NPAR))
+        ctx = _planes_context(nd, npos, nlam, max_planes, device, _DIM)
+        shape_field = np.empty((ng, npos, nlam, _lib.EFIT_NPAR)) if elliptical else None
+        ee_field = np.empty((ng, npos, nlam, ee_rec)) if energy else None
         if ao_budget:
-            strehl = np.empty((nd, nlam))
-            var = np.empty((nd, dirs.shape[1], _lib.VAR_NPAR))
-        if w_band is not None:
-            band_mean = _band_outputs(w_band, nlam, (ng,), ee_rec if energy else None)
-            ctx.compute_bands(False, draws, dirs, _lgs_positions(False), lbda, w_band, rad_px if energy else (),
-                              frac if energy else (), group_end, out_fit=fit, out_mean=psftot, out_mean_fit=fit_mean,
-                              out_mean_ee=ee_mean if energy else None, out_strehl=strehl if ao_budget else None,
-                              out_var=var if ao_budget else None, out_mean_band=band_mean[1],
-                              out_mean_band_fit=band_mean[0], out_mean_band_ee=band_mean[2] if energy else None)
-        elif ao_budget:
-            ctx.compute_ao(False, draws, dirs, _lgs_positions(False), lbda, rad_px if energy else (),
-                           frac if energy else (), group_end, out_fit=fit, out_mean=psftot, out_mean_fit=fit_mean,
-                           out_mean_ee=ee_mean if energy else None, out_strehl=strehl, out_var=var)
-        elif energy:
-            ctx.compute_energy(False, draws, dirs, _lgs_positions(False), lbda, rad_px, frac, group_end, out_fit=fit,
-                               out_mean=psftot, out_mean_fit=fit_mean, out_mean_ee=ee_mean)
-        else:
-            ctx.compute_groups(draws, dirs, _lgs_positions(False), lbda, group_end, out_fit=fit, out_mean=psftot,
-                               out_mean_fit=fit_mean)
-        if pos is not None:
-            npos = pos.shape[1]
-            psf_field = np.empty((ng, npos, nlam, _lib.PSF_DIM, _lib.PSF_DIM))
-            fit_field = np.empty((ng, npos, nlam, _lib.FIT_NPAR))
-            ctx = _planes_context(nd, npos, nlam, max_planes, device, _DIM)
-            shape_field = np.empty((ng, npos, nlam, _lib.EFIT_NPAR)) if elliptical else None
-            if energy:
-                ee_field = np.empty((ng, npos, nlam, ee_rec))
-            if ao_budget:
-                strehl_field = np.empty((nd, npos, nlam))
-                var_field = np.empty((nd, npos, _lib.VAR_NPAR))
-            if w_band is not None:
-                band_field = _band_outputs(w_band, nlam, (ng, npos), ee_rec if energy else None)
-                ctx.compute_bands(True, draws, pos, _lgs_positions(False), lbda, w_band, rad_px if energy else (),
-                                  frac if energy else (), group_end, out_mean=psf_field, out_mean_fit=fit_field,
-                                  out_mean_efit=shape_field, out_mean_ee=ee_field if energy else None,
-                                  out_strehl=strehl_field if ao_budget else None,
-                                  out_var=var_field if ao_budget else None, out_mean_band=band_field[1],
-                                  out_mean_band_fit=band_field[0], out_mean_band_ee=band_field[2] if energy else None)
-            elif ao_budget:
-                ctx.compute_ao(True, draws, pos, _lgs_positions(False), lbda, rad_px if energy else (),
-                               frac if energy else (), group_end, out_mean=psf_field, out_mean_fit=fit_field,
-                               out_mean_efit=shape_field, out_mean_ee=ee_field if energy else None,
-                               out_strehl=strehl_field, out_var=var_field)
-            elif energy:
-                ctx.compute_energy(True, draws, pos, _lgs_positions(False), lbda, rad_px, frac, group_end,
-                                   out_mean=psf_field, out_mean_fit=fit_field, out_mean_efit=shape_field,
-                                   out_mean_ee=ee_field)
-            else:
-                ctx.compute_field(draws, pos, _lgs_positions(False), lbda, group_end, out_mean=psf_field,
-                                  out_mean_fit=fit_field, out_mean_efit=shape_field)
-        if elliptical:      # the time means are on the host already: one standalone fit of all of them
-            shape_mean = np.empty((ng, nlam, _lib.EFIT_NPAR))
-            ctx.moffat_fit_elliptical(ng * nlam, _lib.PSF_DIM, _lib.PSF_DIM, psftot, shape_mean)
-    except PsfrError as exc:
-        if exc.code == _lib.E_UNSUPPORTED:
-            raise ValueError(str(exc))
-        raise
+            strehl_field = np.empty((nd, npos, nlam))
+            var_field = np.empty((nd, npos, _lib.VAR_NPAR))
+        band_field = _band_outputs(w_band, nlam, (ng, npos), ee_rec if energy else None)
+        _fused(ctx, True, draws, pos, lbda, group_end, ee=ee_par, bands=w_band, out_mean=psf_field,
+               out_mean_fit=fit_field, out_mean_efit=shape_field, out_mean_ee=ee_field,
+               out_strehl=strehl_field if ao_budget else None, out_var=var_field if ao_budget else None,
+               out_mean_band=band_field[1] if band_field else None,
+               out_mean_band_fit=band_field[0] if band_field else None,
+               out_mean_band_ee=band_field[2] if band_field and energy else None)
+    if elliptical:      # the time means are on the host already: one standalone fit of all of them
+        shape_mean = np.empty((ng, nlam, _lib.EFIT_NPAR))
+        ctx.moffat_fit_elliptical(ng * nlam, _lib.PSF_DIM, _lib.PSF_DIM, psftot, shape_mean)
 
     results, g = [], 0
     for entry in files:
