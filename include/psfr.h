@@ -141,6 +141,45 @@ enum {
  * 4 (2 ny nx + nx) doubles, the elliptical one also 4 * 2 ny nx doubles, each at most 200 KiB; otherwise
  * PSFR_E_UNSUPPORTED.  The largest accepted square stamp is 56 x 56 (57 x 57 is refused). */
 
+/* Template fits of star images (DESIGN.md section 5.8, psfr_template_fit): each stamp d [ny][nx] with weights w is
+ * fitted as F * T(shifted) + c, T the reconstructed PSF tpl [ty][tx] of the same wavelength.
+ *  - s(u, v) is the interpolating cubic B-spline of tpl with mirror boundary conditions, exactly
+ *    scipy.ndimage.map_coordinates(tpl, [[u], [v]], order=3, mode='mirror'); outside [0, ty - 1] x [0, tx - 1] s and
+ *    its derivatives are 0.
+ *  - Pixel (p, q) has the model m = F * s(p - y0 + ty/2, q - x0 + tx/2) / S + c (integer halves), S the sum of tpl's
+ *    pixels in FP64 in row-major order: F is the flux of the template's whole footprint.  c is fitted only with a
+ *    background, otherwise 0.  Parameters x = [F, y0, x0(, c)], NP = 3 or 4.
+ *  - Used pixels, objective and errors as the star fits above: minimise sum w r^2 over the pixels with w > 0, errors
+ *    sqrt(diag((J^T W J)^-1) chi^2/dof), dof = npix_used - NP.
+ *  - Start point: c0 = the ring background of the star fits (0 without a background); (y0, x0) = the used pixel with
+ *    the largest d - c0 (lowest row-major index on a tie); F0 = sum w s~ (d - c0) / sum w s~^2 at that centre,
+ *    s~ = s / S.  Levenberg-Marquardt over every pixel to the relative step 1.49e-8, at most 200 iterations
+ *    (ITER < 0: not converged); a trial point with a non-finite parameter or a centre outside
+ *    [-0.5, ny - 0.5] x [-0.5, nx - 0.5] is refused.
+ *  - An image fails for the star fits' causes (NP as above), for a template with a non-finite pixel or S <= 0, and when
+ *    no used pixel overlaps the template (sum w s~^2 = 0 at the start): ITER = 0 and NaN in every other slot of its
+ *    record and of its model image; the other images of the call are unaffected.
+ *  Record [nimg][PSFR_TFIT_NPAR]: */
+enum {
+    PSFR_TFIT_FLUX = 0,      /* F */
+    PSFR_TFIT_Y0 = 1,        /* centre row [px] */
+    PSFR_TFIT_X0 = 2,        /* centre column [px] */
+    PSFR_TFIT_CONT = 3,      /* c (0 without a background) */
+    PSFR_TFIT_CHISQ = 4,     /* sum w r^2 */
+    PSFR_TFIT_QFIT = 5,      /* sum_used |r| / |F|: the template's misfit, independent of the weights */
+    PSFR_TFIT_ITER = 6,      /* LM iterations (< 0: not converged, 0: failed) */
+    PSFR_TFIT_NPIX = 7,      /* used pixels */
+    PSFR_TFIT_ERR_FLUX = 8,
+    PSFR_TFIT_ERR_Y0 = 9,
+    PSFR_TFIT_ERR_X0 = 10,
+    PSFR_TFIT_ERR_CONT = 11, /* 0 without a background */
+    PSFR_TFIT_NPAR = 12
+};
+/* Shared memory of the template fit: the image, its weights and the template's B-spline coefficients, 4 images per
+ * CTA: 4 (2 ny nx + ty tx') doubles with tx' = tx rounded up to odd (a row stride free of bank conflicts), at most
+ * 200 KiB; otherwise PSFR_E_UNSUPPORTED.  With a 40 x 40 template the largest accepted square stamp is 48 x 48
+ * (49 x 49 is refused). */
+
 /* Encircled energy (DESIGN.md section 5.4).  Pixel (p, q) is the unit square [p - 1/2, p + 1/2] x [q - 1/2, q + 1/2]
  * with its value spread uniformly over it; EE(r) = sum img[p][q] * area(pixel AND disc(centre, r)), the exact
  * overlap area in FP64, over the pixels of the image only (a circle that leaves the image is clipped by its edge),
@@ -273,6 +312,20 @@ PSFR_API int psfr_moffat_fit_elliptical(psfr_ctx* ctx, int nimg, int ny, int nx,
 PSFR_API int psfr_moffat_fit_weighted(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs,
                                       const double* weights, int fit_back, int elliptical, double* params,
                                       double* back, void* stream);
+
+/* Template fit of star images (DESIGN.md section 5.8; the definitions are above PSFR_TFIT_FLUX).  imgs and weights
+ * [nimg][ny][nx]; weights NULL means every weight is 1.  tpls [ntpl][ty][tx]: image i is fitted with template
+ * i % ntpl, so stamps stacked star-major share one template cube.  fit_back != 0 fits the background.  params
+ * [nimg][PSFR_TFIT_NPAR]; model [nimg][ny][nx] (may be NULL) receives the model m at the final parameters on every
+ * pixel, used or not.  Host or device arrays in any mix; host stamps, weights, records and models are chunked through
+ * the staging buffers as psfr_moffat_fit_weighted, and host templates are uploaded once per call (PSFR_E_CAPACITY when
+ * they exceed the staging buffer, max_planes * max_lambda * 1600 doubles).  When imgs, weights, params and model are
+ * all device arrays (or NULL), one launch fits every image, whatever the context's capacity.  NULL imgs, tpls or params, nimg < 1, ny or nx < 3, ntpl < 1, nimg % ntpl != 0 and
+ * ty or tx < 4 are PSFR_E_ARG, a stamp and template over the shared-memory limit above PSFR_E_UNSUPPORTED: all before
+ * any launch, nothing written. */
+PSFR_API int psfr_template_fit(psfr_ctx* ctx, int nimg, int ny, int nx, const double* imgs, const double* weights,
+                               int ntpl, int ty, int tx, const double* tpls, int fit_back, double* params,
+                               double* model, void* stream);
 
 /* compute_psf (psfrec.py:933-978) for a batch of draws, fused on the device:
  * PSD -> structure function -> pruned PSFs -> resample -> convolutions -> fit.

@@ -36,6 +36,10 @@ EFIT_NPAR = 24
 # side record of the star fits (PSFR_BACK_*): background, its error, used pixels
 BACK_CONT, BACK_ERR_CONT, BACK_NPIX = range(3)
 BACK_NPAR = 3
+# template-fit record (PSFR_TFIT_*): flux, centre [px], background, chi^2, QFIT, iterations, used pixels, errors
+(TFIT_FLUX, TFIT_Y0, TFIT_X0, TFIT_CONT, TFIT_CHISQ, TFIT_QFIT, TFIT_ITER, TFIT_NPIX, TFIT_ERR_FLUX, TFIT_ERR_Y0,
+ TFIT_ERR_X0, TFIT_ERR_CONT) = range(12)
+TFIT_NPAR = 12
 # encircled-energy record (include/psfr.h): EE at nrad radii, TOTAL, then the radius at each of nfrac fractions
 EE_MAX_RADII = 64
 EE_MAX_FRACTIONS = 16
@@ -92,6 +96,7 @@ _SIGNATURES = {
     'psfr_moffat_fit': (_I, [_P, _I, _I, _I, _P, _P, _P]),
     'psfr_moffat_fit_elliptical': (_I, [_P, _I, _I, _I, _P, _P, _P]),
     'psfr_moffat_fit_weighted': (_I, [_P, _I, _I, _I, _P, _P, _I, _I, _P, _P, _P]),
+    'psfr_template_fit': (_I, [_P, _I, _I, _I, _P, _P, _I, _I, _I, _P, _I, _P, _P, _P]),
     'psfr_compute_batch': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P]),
     'psfr_compute_groups': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     'psfr_compute_field': (_I, [_P, _I, _P, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
@@ -339,6 +344,18 @@ class Context:
             self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
             self._buf(weights, nimg * ny * nx, 'weights'), int(bool(fit_back)), int(bool(elliptical)),
             self._buf(params, nimg * npar, 'params', True), self._buf(back, nimg * BACK_NPAR, 'back', True), stream))
+
+    def template_fit(self, nimg, ny, nx, imgs, weights, tpls, params, model=None, fit_back=False, stream=None):
+        """psfr_template_fit: ``weights`` [nimg, ny, nx] or None (every weight 1); ``tpls`` [ntpl, ty, tx] with nimg a
+        multiple of ntpl (image i uses template i % ntpl); ``params`` [nimg, TFIT_NPAR]; ``model`` [nimg, ny, nx] or
+        None."""
+        nimg, ny, nx = int(nimg), int(ny), int(nx)
+        ntpl, ty, tx = (int(v) for v in tpls.shape)
+        self._check(self._lib.psfr_template_fit(
+            self._handle(), nimg, ny, nx, self._buf(imgs, nimg * ny * nx, 'imgs'),
+            self._buf(weights, nimg * ny * nx, 'weights'), ntpl, ty, tx, self._buf(tpls, ntpl * ty * tx, 'tpls'),
+            int(bool(fit_back)), self._buf(params, nimg * TFIT_NPAR, 'params', True),
+            self._buf(model, nimg * ny * nx, 'model', True), stream))
 
     def encircled_energy(self, nimg, ny, nx, imgs, radii_px, fracs, out, centres=None, stream=None):
         """psfr_encircled_energy: ``out`` [nimg, len(radii_px) + 1 + len(fracs)]; ``centres`` [nimg, 2] (y0, x0)

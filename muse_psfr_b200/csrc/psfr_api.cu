@@ -550,7 +550,7 @@ static int run_batch(Ctx* c, int ndraw, const double* draws, int ndir, const dou
 
 extern "C" {
 
-int psfr_version(void) { return 107; }
+int psfr_version(void) { return 108; }
 
 const char* psfr_last_error(const psfr_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
 
@@ -983,6 +983,60 @@ int psfr_moffat_fit_weighted(psfr_ctx* c, int nimg, int ny, int nx, const double
         if (back && !back_dev &&
             (rc = from_device(c, back + i0 * PSFR_BACK_NPAR, bdst, (size_t)n * PSFR_BACK_NPAR * sizeof(double), s)))
             return rc;
+    }
+    return PSFR_OK;
+}
+
+int psfr_template_fit(psfr_ctx* c, int nimg, int ny, int nx, const double* imgs, const double* weights, int ntpl,
+                      int ty, int tx, const double* tpls, int fit_back, double* params, double* model, void* stream) {
+    if (!c || !imgs || !tpls || !params) return set_error(c, PSFR_E_ARG, "NULL argument");
+    if (nimg < 1 || ny < 3 || nx < 3 || ntpl < 1 || nimg % ntpl != 0 || ty < 4 || tx < 4)
+        return set_error(c, PSFR_E_ARG, "nimg=%d ny=%d nx=%d ntpl=%d ty=%d tx=%d (nimg must be a multiple of ntpl)",
+                         nimg, ny, nx, ntpl, ty, tx);
+    if (int rc = check_template_fit_size(c, ny, nx, ty, tx)) return rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PSFR_CUDA(c, cudaSetDevice(c->device));
+    const size_t cap = (size_t)c->max_planes * c->max_lambda * kPSF * kPSF;   // doubles per staging buffer
+    const size_t per = (size_t)ny * nx, tpl_len = (size_t)ntpl * ty * tx;
+    const bool in_dev = is_device_ptr(imgs), w_dev = !weights || is_device_ptr(weights);
+    const bool t_dev = is_device_ptr(tpls), out_dev = is_device_ptr(params), m_dev = model && is_device_ptr(model);
+    // host stamps, weights and models go through d_cube, d_cube2 and d_cube3, host records through d_fit, and host
+    // templates, which every chunk reads whole, through d_mean[0]; when no stamp-sized array is on the host, one
+    // launch fits every image
+    const bool all_dev = in_dev && w_dev && out_dev && (!model || m_dev);
+    const size_t chunk_imgs = all_dev ? (size_t)nimg : std::min((size_t)c->max_planes * c->max_lambda, cap / per);
+    if (chunk_imgs < 1) return set_error(c, PSFR_E_CAPACITY, "image %dx%d does not fit the staging buffer", ny, nx);
+    if (!t_dev && tpl_len > cap)
+        return set_error(c, PSFR_E_CAPACITY, "%d host templates of %dx%d do not fit the staging buffer (%zu doubles)",
+                         ntpl, ty, tx, cap);
+    int rc;
+    const double* tpl = tpls;
+    if (!t_dev) {
+        if ((rc = to_device(c, c->d_mean[0], tpls, tpl_len * sizeof(double), s))) return rc;
+        tpl = c->d_mean[0];
+    }
+    for (size_t i0 = 0; i0 < (size_t)nimg; i0 += chunk_imgs) {
+        const int n = (int)std::min(chunk_imgs, (size_t)nimg - i0);
+        const size_t bytes = (size_t)n * per * sizeof(double);
+        const double* src = imgs + i0 * per;
+        const double* w = weights ? weights + i0 * per : nullptr;
+        if (!in_dev) {
+            if ((rc = to_device(c, c->d_cube, src, bytes, s))) return rc;
+            src = c->d_cube;
+        }
+        if (!w_dev) {
+            if ((rc = to_device(c, c->d_cube2, w, bytes, s))) return rc;
+            w = c->d_cube2;
+        }
+        double* dst = out_dev ? params + i0 * PSFR_TFIT_NPAR : c->d_fit;
+        double* mdst = !model ? nullptr : m_dev ? model + i0 * per : c->d_cube3;
+        if ((rc = run_template_fit(c, n, ny, nx, src, w, ntpl, ty, tx, tpl, (long long)i0, fit_back != 0, dst, mdst,
+                                   s)))
+            return rc;
+        if (!out_dev &&
+            (rc = from_device(c, params + i0 * PSFR_TFIT_NPAR, dst, (size_t)n * PSFR_TFIT_NPAR * sizeof(double), s)))
+            return rc;
+        if (model && !m_dev && (rc = from_device(c, model + i0 * per, mdst, bytes, s))) return rc;
     }
     return PSFR_OK;
 }

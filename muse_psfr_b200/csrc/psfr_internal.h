@@ -315,6 +315,12 @@ int run_star_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const 
 int run_star_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, bool fit_back,
                   const double* circ_dev, const double* circ_back_dev, double* efit_dev, double* back_dev,
                   cudaStream_t s);
+// template fit (DESIGN.md 5.8): tpl_dev [ntpl][ty][tx]; image i of the call uses template (first + i) % ntpl;
+// model_dev [nimg][ny][nx] or NULL
+int check_template_fit_size(Ctx* c, int ny, int nx, int ty, int tx);
+int run_template_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, int ntpl, int ty,
+                     int tx, const double* tpl_dev, long long first, bool fit_back, double* fit_dev, double* model_dev,
+                     cudaStream_t s);
 // psfr_energy.cu: encircled-energy record [nimg][nrad + 1 + nfrac] of every image, radii and fractions from
 // d_eepar, centres_dev [nimg][2] (row, column) or nullptr for (ny / 2, nx / 2)
 int run_ee(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* centres_dev, int nrad, int nfrac,

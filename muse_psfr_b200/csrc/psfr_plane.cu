@@ -302,14 +302,15 @@ struct StarModel {
 // accumulate normal equations at x over this lane's pixels (two independent pixel chains per
 // trip so that the log / exp latencies overlap), then reduce over the warp.  STEP = 1 visits every
 // pixel; STEP = 4 every fourth pixel of each lane (a quasi-uniform quarter of the image), used
-// by the coarse first stage of the fit.
-template <class M, int STEP>
+// by the coarse first stage of the fit.  `env` is whatever the model needs besides x (the template fit's
+// coefficient array); the Moffat models take none.
+template <class M, int STEP, class... Env>
 __device__ __forceinline__ void accumulate(const double* __restrict__ img, int npx, int nx, const double* x,
-                                           double* sums) {
+                                           double* sums, const Env&... env) {
 #pragma unroll
     for (int k = 0; k < Normal<M::NP>::NSUM; ++k) sums[k] = 0.0;
     const double y0 = x[1], x0 = x[2];
-    const M model(x);
+    const M model(x, env...);
     const int lane = threadIdx.x & 31;
     int pr = lane / nx, qc = lane % nx;          // once per call; then stepped incrementally
     const int dpr = (32 * STEP) / nx, dqc = (32 * STEP) % nx;
@@ -389,13 +390,13 @@ __device__ __forceinline__ void chol_solve(const double (&L)[NP][NP], double* z)
 
 // Levenberg-Marquardt of model M on the pixel subset STEP from the start point x (updated in place);
 // sums holds the normal equations at the final x.  tol2 = square of the relative step at which
-// to stop (MINPACK, the reference's solver, stops at 1.49e-8; so does the final stage).
-template <class M, int STEP>
+// to stop (MINPACK, the reference's solver, stops at 1.49e-8; so does the final stage).  env as accumulate.
+template <class M, int STEP, class... Env>
 __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx, int nx, double* x, double* sums,
-                                         double tol2, int max_iter, int& iter, int& status) {
+                                         double tol2, int max_iter, int& iter, int& status, const Env&... env) {
     constexpr int kNP = M::NP, NJJ = Normal<kNP>::NJJ, kNSUM = Normal<kNP>::NSUM, COST = Normal<kNP>::COST;
     double trial[kNSUM], xt[kNP], d[kNP];
-    accumulate<M, STEP>(img, npx, nx, x, sums);
+    accumulate<M, STEP>(img, npx, nx, x, sums, env...);
     double mu = 1e-3, nu = 2.0;
     status = -1;
     constexpr DiagIndex<kNP> dia;
@@ -421,13 +422,13 @@ __device__ __forceinline__ void lm_solve(const double* __restrict__ img, int npx
             // predicted decrease of r.r : d.(mu D d - g)
             pred += d[i] * (mu * sc2 * d[i] - sums[NJJ + i]);
         }
-        if (M::refuses(xt)) {
+        if (M::refuses(xt, env...)) {
             mu *= nu;
             nu *= 2.0;
             if (mu > 1e15) break;
             continue;
         }
-        accumulate<M, STEP>(img, npx, nx, xt, trial);
+        accumulate<M, STEP>(img, npx, nx, xt, trial, env...);
         const double actual = sums[COST] - trial[COST];
         // near the minimum the cost is flat to rounding: tolerate a noise-level increase so that
         // Gauss-Newton steps keep contracting, and stop on the (column-scaled) step size
@@ -953,6 +954,256 @@ star_efit_kernel(const double* __restrict__ imgs, const double* __restrict__ wts
     efit_images<true, kBack>(imgs, wts, circ, circ_back, nimg, ny, nx, out, back, next_image);
 }
 
+// ---------------------------------------------------------------- template fit (DESIGN.md 5.8)
+// resident CTAs per SM the template fitter is compiled for; shared memory (image, weights and template per warp)
+// allows two at 25 x 25 stamps and 40 x 40 templates
+#ifndef PSFR_TFIT_MINBLOCKS
+#define PSFR_TFIT_MINBLOCKS 2
+#endif
+constexpr int kTfitMaxIter = 200;   // the circular fit's final-stage cap
+
+// Row stride of the coefficient array in shared memory: tx rounded up to an odd number of doubles, so that the
+// prefilter's row pass (one lane per row, all lanes at the same column) hits 32 different 8-byte bank pairs.
+__host__ __device__ constexpr int tpl_stride(int tx) { return tx | 1; }
+
+// The warp's template: interpolating cubic B-spline coefficients [ty][tpl_stride(tx)] in shared memory, 1 / S, and
+// the stamp's size (the bounds of the centre).
+struct TemplateView {
+    const double* coef;
+    int ty, tx, ny, nx;
+    double inv_s;
+};
+
+// cubic B-spline weights of the four taps floor(u) - 1 .. floor(u) + 2 at fraction t, and their derivatives in t
+__device__ __forceinline__ void bspline3(double t, double* w, double* dw) {
+    const double s = 1.0 - t, t2 = t * t, s2 = s * s;
+    w[0] = s2 * s * (1.0 / 6.0);
+    w[1] = 2.0 / 3.0 - 0.5 * t2 * (2.0 - t);
+    w[2] = 2.0 / 3.0 - 0.5 * s2 * (2.0 - s);
+    w[3] = t2 * t * (1.0 / 6.0);
+    dw[0] = -0.5 * s2;
+    dw[1] = t * (1.5 * t - 2.0);
+    dw[2] = -s * (1.5 * s - 2.0);
+    dw[3] = 0.5 * t2;
+}
+
+// tap index k of a line of n samples under mirror boundary conditions (d c b | a b c d | c b a); k in [-1, n + 1]
+// (the taps of a point at n - 1 reach n + 1), which n >= 4 keeps inside the line
+__device__ __forceinline__ int mirror_tap(int k, int n) { return k < 0 ? -k : k > n - 1 ? 2 * (n - 1) - k : k; }
+
+// Template model m = F s(u, v) / S + c, x = [F, y0, x0(, c)], (u, v) = (row - y0 + ty/2, column - x0 + tx/2): 16 taps of
+// the coefficients, no transcendental.  The weights follow the image in shared memory, as StarModel.
+template <bool kBack>
+struct TemplateModel {
+    static constexpr int NP = kBack ? 4 : 3;
+    static constexpr bool kWeighted = true;
+    TemplateView v;
+    double hy, hx, fs, c;   // template centre, F / S, background
+    __device__ __forceinline__ TemplateModel(const double* x, const TemplateView& tv)
+        : v(tv), hy((double)(tv.ty / 2)), hx((double)(tv.tx / 2)), fs(x[0] * tv.inv_s), c(kBack ? x[3] : 0.0) {}
+    // s and its derivatives in u and v; all 0 outside [0, ty - 1] x [0, tx - 1]
+    __device__ __forceinline__ double sample(double u, double vv, double& su, double& sv) const {
+        su = sv = 0.0;
+        if (!(u >= 0.0 && u <= (double)(v.ty - 1) && vv >= 0.0 && vv <= (double)(v.tx - 1))) return 0.0;
+        const double fu = floor(u), fv = floor(vv);
+        const int iu = (int)fu, iv = (int)fv;
+        double wu[4], dwu[4], wv[4], dwv[4];
+        bspline3(u - fu, wu, dwu);
+        bspline3(vv - fv, wv, dwv);
+        int col[4];
+#pragma unroll
+        for (int l = 0; l < 4; ++l) col[l] = mirror_tap(iv - 1 + l, v.tx);
+        double val = 0.0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const double* row = v.coef + mirror_tap(iu - 1 + k, v.ty) * tpl_stride(v.tx);
+            double rv = 0.0, rd = 0.0;
+#pragma unroll
+            for (int l = 0; l < 4; ++l) {
+                const double cf = row[col[l]];
+                rv = fma(wv[l], cf, rv);
+                rd = fma(dwv[l], cf, rd);
+            }
+            val = fma(wu[k], rv, val);
+            su = fma(dwu[k], rv, su);
+            sv = fma(wu[k], rd, sv);
+        }
+        return val;
+    }
+    // model value at offset (dp, dq) = (row - y0, column - x0)
+    __device__ __forceinline__ double value(double dp, double dq) const {
+        double su, sv;
+        return fma(fs, sample(dp + hy, dq + hx, su, sv), c);
+    }
+    __device__ __forceinline__ void pixel(double dp, double dq, double pix, double w, double* sums) const {
+        double su, sv, J[NP];
+        const double s = sample(dp + hy, dq + hx, su, sv);
+        J[0] = s * v.inv_s;
+        J[1] = -fs * su;
+        J[2] = -fs * sv;
+        if constexpr (kBack) J[3] = 1.0;
+        add_normal_w<NP>(J, fma(fs, s, c) - pix, w, sums);
+    }
+    static __device__ __forceinline__ bool refuses(const double* xt, const TemplateView& tv) {
+        bool bad = !(xt[1] >= -0.5 && xt[1] <= tv.ny - 0.5 && xt[2] >= -0.5 && xt[2] <= tv.nx - 0.5);
+#pragma unroll
+        for (int i = 0; i < NP; ++i) bad = bad || !isfinite(xt[i]);
+        return bad;
+    }
+};
+
+// scipy's spline_filter1d(order=3, mode='mirror') of one line of n samples at stride st, in place: the gain, then the
+// causal recursion from its exact mirror initialisation and the anticausal one, pole z = sqrt(3) - 2
+__device__ __forceinline__ void prefilter_line(double* c, int n, int st) {
+    const double z = -0.26794919243112270;   // sqrt(3) - 2
+    const double gain = (1.0 - z) * (1.0 - 1.0 / z);
+    for (int i = 0; i < n; ++i) c[i * st] *= gain;
+    const double zn1 = pow(z, (double)(n - 1));
+    double c0 = c[0] + zn1 * c[(n - 1) * st], zi = z;
+    for (int i = 1; i < n - 1; ++i) {
+        c0 += zi * (c[i * st] + zn1 * c[(n - 1 - i) * st]);
+        zi *= z;
+    }
+    c[0] = c0 / (1.0 - zn1 * zn1);
+    for (int i = 1; i < n; ++i) c[i * st] += z * c[(i - 1) * st];
+    c[(n - 1) * st] = (z * c[(n - 2) * st] + c[(n - 1) * st]) * z / (z * z - 1.0);
+    for (int i = n - 2; i >= 0; --i) c[i * st] = z * (c[(i + 1) * st] - c[i * st]);
+}
+
+// Template fit of every image, one warp per image, images handed out by a global counter as fit_images.  Shared
+// memory per warp: image [npx], weights [npx], template coefficients [ty][tpl_stride(tx)].  Image i (counted from
+// `first`, the chunk's offset in the call) uses template (first + i) % ntpl of tpls.  out [nimg][PSFR_TFIT_NPAR];
+// model [nimg][ny][nx] or NULL.
+template <bool kBack>
+__global__ void __launch_bounds__(kFitWarps * 32, PSFR_TFIT_MINBLOCKS)
+template_fit_kernel(const double* __restrict__ imgs, const double* __restrict__ wts, int nimg, int ny, int nx,
+                    const double* __restrict__ tpls, int ntpl, int ty, int tx, long long first,
+                    double* __restrict__ out, double* __restrict__ model, int* __restrict__ next_image) {
+    using Model = TemplateModel<kBack>;
+    constexpr int kNP = Model::NP, kNSUM = Normal<kNP>::NSUM, COST = Normal<kNP>::COST;
+    extern __shared__ double sm[];
+    const int npx = ny * nx, ntp = ty * tx, ts = tpl_stride(tx), lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double* img = sm + (size_t)warp * (2 * npx + ty * ts);
+    double* coef = img + 2 * npx;
+#pragma unroll 1
+    for (;;) {
+        int image = 0;
+        if (lane == 0) image = atomicAdd(next_image, 1);
+        image = __shfl_sync(0xffffffffu, image, 0);
+        if (image >= nimg) return;
+        __syncwarp();
+        bool bad;
+        const int npu = load_star_image(imgs, wts, image, npx, img, bad);
+        const double* tsrc = tpls + (size_t)((first + image) % ntpl) * ntp;
+        bool tb = false;
+        for (int i = lane; i < ntp; i += 32) {
+            const double t = tsrc[i];
+            tb = tb || !isfinite(t);
+            coef[(i / tx) * ts + i % tx] = t;
+        }
+        bad = bad || __any_sync(0xffffffffu, tb) || npu <= kNP;
+        __syncwarp();
+        double S = 0.0;                 // every lane, row-major: the same bits in each
+        for (int r = 0; r < ty; ++r)
+            for (int q = 0; q < tx; ++q) S += coef[r * ts + q];
+        bad = bad || !(S > 0.0);
+        double* mo = model ? model + (size_t)image * npx : nullptr;
+        double x[kNP], sums[kNSUM];
+        if (!bad) {
+            __syncwarp();
+            for (int r = lane; r < ty; r += 32) prefilter_line(coef + r * ts, tx, 1);
+            __syncwarp();
+            for (int q = lane; q < tx; q += 32) prefilter_line(coef + q, ty, ts);
+            __syncwarp();
+            const double c0 = kBack ? ring_background(img, ny, nx) : 0.0;
+            // start: the used pixel of largest d - c0 (first in row-major order on a tie)
+            double bestv = -INFINITY;
+            int ib = npx;
+            for (int i = lane; i < npx; i += 32)
+                if (img[npx + i] > 0.0 && img[i] - c0 > bestv) {
+                    bestv = img[i] - c0;
+                    ib = i;
+                }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const double ov = __shfl_xor_sync(0xffffffffu, bestv, o);
+                const int oi = __shfl_xor_sync(0xffffffffu, ib, o);
+                if (ov > bestv || (ov == bestv && oi < ib)) { bestv = ov; ib = oi; }
+            }
+            x[0] = 1.0;
+            x[1] = ib / nx;
+            x[2] = ib % nx;
+            if constexpr (kBack) x[3] = 0.0;
+            // F0: closed-form linear least-squares flux at that centre
+            const TemplateView tv{coef, ty, tx, ny, nx, 1.0 / S};
+            {
+                const Model m0(x, tv);
+                double v2[2] = {0.0, 0.0};
+                for (int i = lane; i < npx; i += 32) {
+                    const double w = img[npx + i];
+                    const double st = m0.value((double)(i / nx) - x[1], (double)(i % nx) - x[2]);   // s / S
+                    v2[0] += w * st * (img[i] - c0);
+                    v2[1] += w * st * st;
+                }
+                warp_sum_vec<2>(v2);
+                bad = !(v2[1] > 0.0);
+                x[0] = v2[0] / v2[1];
+                if constexpr (kBack) x[3] = c0;
+            }
+            if (!bad) {
+                int iter = 0, status = -1;
+                lm_solve<Model, 1>(img, npx, nx, x, sums, PSFR_FIT_TOL2, kTfitMaxIter, iter, status, tv);
+                // QFIT and the model image at the final parameters
+                const Model mf(x, tv);
+                double ares = 0.0;
+                for (int i = lane; i < npx; i += 32) {
+                    const double m = mf.value((double)(i / nx) - x[1], (double)(i % nx) - x[2]);
+                    if (img[npx + i] > 0.0) ares += fabs(img[i] - m);
+                    if (mo) mo[i] = m;
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) ares += __shfl_xor_sync(0xffffffffu, ares, o);
+                if (lane == 0) {
+                    double* o = out + (size_t)image * PSFR_TFIT_NPAR;
+                    o[PSFR_TFIT_FLUX] = x[0];
+                    o[PSFR_TFIT_Y0] = x[1];
+                    o[PSFR_TFIT_X0] = x[2];
+                    o[PSFR_TFIT_CONT] = kBack ? x[kNP - 1] : 0.0;
+                    o[PSFR_TFIT_CHISQ] = sums[COST];
+                    o[PSFR_TFIT_QFIT] = ares / fabs(x[0]);
+                    o[PSFR_TFIT_ITER] =
+                        (status > 0) ? (double)status : -(double)(iter > kTfitMaxIter ? kTfitMaxIter : iter);
+                    o[PSFR_TFIT_NPIX] = (double)npu;
+                    const double dof = (double)(npu - kNP);
+                    double L[kNP][kNP], e[4] = {0.0, 0.0, 0.0, 0.0};
+                    if (cholesky(sums, 0.0, L)) {
+#pragma unroll
+                        for (int k = 0; k < kNP; ++k) {
+                            double z[kNP];
+#pragma unroll
+                            for (int i = 0; i < kNP; ++i) z[i] = (i == k) ? 1.0 : 0.0;
+                            chol_solve(L, z);
+                            e[k] = sqrt(fabs(z[k]) * fabs(sums[COST] / dof));
+                        }
+                    } else {
+                        for (int k = 0; k < kNP; ++k) e[k] = nan("");
+                    }
+                    o[PSFR_TFIT_ERR_FLUX] = e[0];
+                    o[PSFR_TFIT_ERR_Y0] = e[1];
+                    o[PSFR_TFIT_ERR_X0] = e[2];
+                    o[PSFR_TFIT_ERR_CONT] = e[3];
+                }
+            }
+        }
+        if (bad) {
+            if (lane == 0) fail_record(out + (size_t)image * PSFR_TFIT_NPAR, PSFR_TFIT_NPAR, PSFR_TFIT_ITER);
+            if (mo)
+                for (int i = lane; i < npx; i += 32) mo[i] = nan("");
+        }
+        __syncwarp();
+    }
+}
+
 // ---------------------------------------------------------------- mean of cubes
 __global__ void mean_kernel(const double* __restrict__ cubes, int ncube, size_t elems,
                             double* __restrict__ out, int first, int last, int ntotal) {
@@ -1204,6 +1455,36 @@ int run_star_efit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const
     PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 2, 0, sizeof(int), s));
     kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, w_dev, circ_dev, circ_back_dev, nimg, ny, nx, efit_dev,
                                               back_dev, c->d_counter + 2);
+    PSFR_LAUNCH_CHECK(c);
+    return PSFR_OK;
+}
+
+// shared memory of the template fit (image, weights and template per warp), or 0 when it is over 200 KiB
+static size_t template_fit_smem(int ny, int nx, int ty, int tx) {
+    const size_t b = (size_t)kFitWarps * (2 * (size_t)ny * nx + (size_t)ty * tpl_stride(tx)) * sizeof(double);
+    return b > 200 * 1024 ? 0 : b;
+}
+
+int check_template_fit_size(Ctx* c, int ny, int nx, int ty, int tx) {
+    if (!template_fit_smem(ny, nx, ty, tx))
+        return set_error(c, PSFR_E_UNSUPPORTED,
+                         "image %dx%d with a %dx%d template too large for the template fit: image, weights and "
+                         "template need %zu bytes of shared memory per CTA, over 200 KiB", ny, nx, ty, tx,
+                         (size_t)kFitWarps * (2 * (size_t)ny * nx + (size_t)ty * tpl_stride(tx)) * sizeof(double));
+    return PSFR_OK;
+}
+
+int run_template_fit(Ctx* c, int nimg, int ny, int nx, const double* img_dev, const double* w_dev, int ntpl, int ty,
+                     int tx, const double* tpl_dev, long long first, bool fit_back, double* fit_dev, double* model_dev,
+                     cudaStream_t s) {
+    if (int rc = check_template_fit_size(c, ny, nx, ty, tx)) return rc;
+    const size_t smem = template_fit_smem(ny, nx, ty, tx);
+    const auto kernel = fit_back ? template_fit_kernel<true> : template_fit_kernel<false>;
+    if (int rc = ensure_dynamic_smem(c, kernel, smem)) return rc;
+    const int grid = fit_grid(c, kernel, smem, nimg, 1);
+    PSFR_CUDA(c, cudaMemsetAsync(c->d_counter + 4, 0, sizeof(int), s));
+    kernel<<<grid, kFitWarps * 32, smem, s>>>(img_dev, w_dev, nimg, ny, nx, tpl_dev, ntpl, ty, tx, first, fit_dev,
+                                              model_dev, c->d_counter + 4);
     PSFR_LAUNCH_CHECK(c);
     return PSFR_OK;
 }

@@ -17,7 +17,8 @@ from ._lib import PsfrError
 
 __all__ = ['compute_psf_from_sparta', 'compute_psf_from_sparta_batch', 'compute_psf', 'compute_psf_batch',
            'reconstruct_psf', 'create_sparta_table', 'fit_psf_with_polynom', 'simul_psd_wfm', 'psd_to_psf', 'psf_muse',
-           'convolve_final_psf', 'fit_psf_cube', 'compute_psf_field', 'encircled_energy', 'band_weights', 'band_psf',
+           'convolve_final_psf', 'fit_psf_cube', 'fit_psf_template', 'compute_psf_field', 'encircled_energy',
+           'band_weights', 'band_psf',
            'muse_intrinsic_psf', 'direction_perf', 'seeing2r01', 'pupil_mask', 'select_sparta_rows', 'FitTable',
            'PsfrError', 'MIN_L0', 'MAX_L0']
 
@@ -639,6 +640,67 @@ def _star_weights(psfcube, var, mask):
         weights = np.zeros(shape)
         np.divide(1.0, v, out=weights, where=~bad)
     return data, np.ascontiguousarray(weights)
+
+
+def fit_psf_template(lbda, psfcube, template, var=None, mask=None, fit_back=False, return_model=False):
+    """Fit each star stamp with a reconstructed PSF as the model (DESIGN.md section 5.8): plane i of ``psfcube``
+    [n, ny, nx] (an array, a masked array or anything with a ``.data`` array) is fitted as F * T(shifted) + c, T =
+    ``template[i % ntpl]`` interpolated by a cubic B-spline (``scipy.ndimage.map_coordinates(order=3,
+    mode='mirror')``) and shifted so that its pixel (ty // 2, tx // 2) lands on the fitted centre.  ``template`` is
+    [ntpl, ty, tx] with ``n % ntpl == 0`` (ten stars stacked star-major share one template cube) or [ty, tx].
+
+    ``var``, ``mask`` and ``fit_back`` build the weights and the background as ``fit_psf_cube``.  The table has one
+    row per stamp: ``lbda``, ``center`` (y, x) [px] and ``err_center``, ``flux`` (the flux of the template's whole
+    footprint, template normalised to unit sum) and ``err_flux``, ``cont`` and ``err_cont`` (0 without
+    ``fit_back``), ``chisq`` (sum w r^2; ``chisq / (npix - NP)`` ~ 1 when the template describes the star, NP = 3, or
+    4 with ``fit_back``), ``qfit`` (sum |r| / |flux| over the used pixels), ``npix`` and ``converged``.  With
+    ``return_model`` the call returns ``(table, model)``, model [n, ny, nx] the fitted image on every pixel (NaN for
+    a failed stamp); the residual image is ``psfcube - model``.  Shape mismatches, ``var <= 0`` on a used pixel and a
+    template that is not finite or does not sum to > 0 raise ValueError before any device call."""
+    lam = np.atleast_1d(np.asarray(lbda, dtype=float))
+    data, weights = _star_weights(psfcube, var, mask)
+    nimg, ny, nx = data.shape
+    tpl = np.array(template, dtype=np.float64, order='C')
+    if tpl.ndim == 2:
+        tpl = tpl[None]
+    if tpl.ndim != 3 or tpl.shape[0] < 1 or nimg % tpl.shape[0]:
+        raise ValueError('template must be [ty, tx] or [ntpl, ty, tx] with ntpl dividing the %d stamps (got shape %s)'
+                         % (nimg, np.shape(template)))
+    if lam.size != nimg:
+        raise ValueError('lbda holds %d wavelengths for %d stamps' % (lam.size, nimg))
+    if not np.all(np.isfinite(tpl)):
+        raise ValueError('template has non-finite pixels (first at %s)' % (tuple(np.argwhere(~np.isfinite(tpl))[0]),))
+    sums = tpl.reshape(tpl.shape[0], -1).sum(axis=1)
+    if np.any(sums <= 0):
+        raise ValueError('template %d sums to %g; every template must sum to > 0' % (np.argmax(sums <= 0),
+                                                                                      sums[sums <= 0][0]))
+    rec = np.empty((nimg, _lib.TFIT_NPAR))
+    model = np.empty((nimg, ny, nx)) if return_model else None
+    if nimg:
+        # the host templates are staged whole on the device: grow the context until they fit its staging buffer
+        # (max_planes * max_lambda 40 x 40 planes)
+        ctx = get_context()
+        ctx = get_context(max_lambda=-(-tpl.size // (ctx.max_planes * _lib.PSF_DIM * _lib.PSF_DIM)))
+        ctx.template_fit(nimg, ny, nx, data, weights, tpl, rec, model, fit_back=fit_back)
+    converged = rec[:, _lib.TFIT_ITER] > 0
+    if not converged.all():
+        bad = np.flatnonzero(~converged)
+        logger.warning('template fit did not converge for %d of %d images (first at index %d)',
+                       bad.size, nimg, bad[0])
+    tab = FitTable({
+        'lbda': lam,
+        'center': rec[:, [_lib.TFIT_Y0, _lib.TFIT_X0]].copy(),
+        'err_center': rec[:, [_lib.TFIT_ERR_Y0, _lib.TFIT_ERR_X0]].copy(),
+        'flux': rec[:, _lib.TFIT_FLUX].copy(),
+        'err_flux': rec[:, _lib.TFIT_ERR_FLUX].copy(),
+        'cont': rec[:, _lib.TFIT_CONT].copy(),
+        'err_cont': rec[:, _lib.TFIT_ERR_CONT].copy(),
+        'chisq': rec[:, _lib.TFIT_CHISQ].copy(),
+        'qfit': rec[:, _lib.TFIT_QFIT].copy(),
+        'npix': np.nan_to_num(rec[:, _lib.TFIT_NPIX]).astype(np.int64),
+        'converged': converged.astype(np.int64),
+    })
+    return (tab, model) if return_model else tab
 
 
 def encircled_energy(lbda, psfcube, radii, fractions=(0.5, 0.8), center=None, pixscale=_PIXSCALE):
